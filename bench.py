@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the VNect per-frame hot path (BASELINE.json: frames/s @368x368, 2 scales, on 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of 64 synthetic 368x368 BGR frames per GPU (config C2 of
 SURVEY.md section 8d: scales [1.0, 0.7] => 128 CNN forwards), OneEuroFilter state live across steps (each frame slot is
@@ -17,6 +17,12 @@ roofline = the implicit-GEMM convolution kernel family (the dominant kernel): al
            (BASELINE.md section 3) / summed device time of its launches, against the measured bf16 tensor peak.
 cpu_baseline = the CPU restatement of the reference (oracle/: torch-CPU fp32 CNN + cv2/numpy pre/post) on a bounded
            sample, timed on this box's host cores.  `--impl reference` times only that.
+
+--dump-outputs DIR writes what the last of the K timed `value` steps returned to its caller: DIR/joints_2d.npy
+(float64 [frames, 21, 2]) and DIR/joints_3d.npy (float32 [frames, 21, 3]) of rank 0, plus DIR/results_all.npy (the
+gathered float64 [streams, 21, 5] rows) when N > 1.  Frames, weights and clock readings are seeded and the filter state
+at that point depends only on --warmup and --steps, so two builds run with the same arguments can be compared file by
+file.
 """
 import argparse
 import json
@@ -264,7 +270,10 @@ def main():
     ap.add_argument("--frames", type=int, default=FRAMES_PER_GPU, help="frames per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the C4 strong-scaling leg (256 streams x 32 steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args, out)
 
@@ -352,6 +361,14 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = n_streams * args.steps / (ms_max * 1e-3)
+    # results of the last timed step, taken before the legs below move the filters on by a timing-dependent step count
+    if args.dump_outputs and rank == 0:
+        dump = {"joints_2d": d_j2.cpu().numpy(), "joints_3d": d_j3.cpu().numpy()}
+        if world > 1:
+            dump["results_all"] = g_all.cpu().numpy()[parallel.unshard_index(n_streams, world)]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     # the GEMM family's own time for the roofline, taken here: same thermal / power state as the `value` leg just timed
     # (after the 2 s sustained leg further down the chip sits at its power cap and the forward measures 10-15 % longer)

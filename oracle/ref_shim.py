@@ -1,8 +1,8 @@
-"""Run the reference's OWN estimator / utils / OneEuroFilter, unchanged, from /root/reference.
+"""Run the reference's OWN estimator / utils / OneEuroFilter, unchanged, from a checkout of the reference project.
 
-TEST INFRASTRUCTURE (see oracle/__init__.py).  Only usable in the dev container (the GPU box has no /root/reference);
-it is what ``tests/golden/make_golden.py`` uses to mint the committed fixtures, and what the optional
-``tests/test_reference_live.py`` uses when the reference tree is present.
+TEST INFRASTRUCTURE (see oracle/__init__.py).  Only usable where the environment variable VNECT_REFERENCE_ROOT names a
+checkout of XinArkh/VNect; it is what ``tests/golden/make_golden.py`` uses to mint the committed fixtures, and what the
+live comparisons of the test suite use when the reference tree is present.
 
 ``src/estimator.py`` imports ``tensorflow`` (not installable here) and ``src/utils.py`` imports matplotlib (not
 installed).  Both are replaced by stubs *in sys.modules only*: the stub ``tf.Session.run`` hands the fed batch to a
@@ -14,12 +14,12 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("VNECT_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("VNECT_REFERENCE_ROOT", "")
 TENSOR_NAMES = ("split_2:0", "split_2:1", "split_2:2", "split_2:3")
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "estimator.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "estimator.py"))
 
 
 class _Forward:
@@ -62,7 +62,7 @@ def _install_stubs():
 def load_reference_modules():
     """Import (utils, OneEuroFilter, estimator) from the reference tree, unchanged."""
     if not reference_available():
-        raise RuntimeError("reference tree not present at " + REFERENCE_ROOT)
+        raise RuntimeError("reference tree not found: set VNECT_REFERENCE_ROOT to a checkout of XinArkh/VNect")
     _install_stubs()
     src = os.path.join(REFERENCE_ROOT, "src")
     if src not in sys.path:

@@ -1,9 +1,9 @@
 #!/usr/bin/env python3
-"""Mint the golden fixtures of tests/golden/ by running the reference's OWN code (dev container only).
+"""Mint the golden fixtures of tests/golden/ by running the reference's OWN code.
 
-    python tests/golden/make_golden.py
+    VNECT_REFERENCE_ROOT=<checkout of XinArkh/VNect> python tests/golden/make_golden.py
 
-Needs /root/reference (read-only).  The reference's ``src/utils.py``, ``src/OneEuroFilter.py`` and ``src/estimator.py``
+The reference tree is only read.  The reference's ``src/utils.py``, ``src/OneEuroFilter.py`` and ``src/estimator.py``
 are imported unchanged through ``oracle.ref_shim``; TensorFlow is replaced by a stub whose ``Session.run`` returns
 either seeded synthetic maps (post-processing fixtures, machine independent) or ``oracle.forward.OracleNet`` output
 (end-to-end fixtures).  Library versions are recorded in every file.
@@ -62,6 +62,16 @@ POST_CASES = [  # (name, seed, scales, n_frames, dt pattern)
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def savez_bzip2(path, **arrays):
+    """np.savez_compressed with bzip2 instead of deflate entries (np.load reads either).  The decoded video frames
+    shrink to about 60 % of their deflate size, which keeps video.npz well under 1 MB."""
+    import zipfile
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_BZIP2) as z:
+        for name, a in arrays.items():
+            with z.open(name + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(a), allow_pickle=False)
 
 
 def timestamps(pattern, n, seed):
@@ -157,8 +167,8 @@ def make_video():
         x, y, w, h = ns["x"], ns["y"], ns["w"], ns["h"]
         j2s.append(joints_2d.copy())
         j3s.append(joints_3d.copy())
-    np.savez_compressed(os.path.join(OUT, "video.npz"), frames=frames, t=t, j2=np.array(j2s), j3=np.array(j3s),
-                        boxes=np.array(boxes, np.int32), versions=str(VERSIONS))
+    savez_bzip2(os.path.join(OUT, "video.npz"), frames=frames, t=t, j2=np.array(j2s), j3=np.array(j3s),
+                boxes=np.array(boxes, np.int32), versions=str(VERSIONS))
 
 
 REF_SCRIPTS = ("run_pic.py", "run_estimator.py")
@@ -210,7 +220,7 @@ def make_angles():
 
 
 def main():
-    assert ref_shim.reference_available(), "run in the dev container (needs /root/reference)"
+    assert ref_shim.reference_available(), "set VNECT_REFERENCE_ROOT to a checkout of XinArkh/VNect"
     utils, oef, est_mod = ref_shim.load_reference_modules()
     only = set(sys.argv[1:])
     if only:

@@ -1,10 +1,10 @@
 """SURVEY.md T5: the reference's own run scripts, executed UNCHANGED, against the drop-in.
 
-The scripts' text comes from tests/golden/ref_scripts.npz (minted from /root/reference by make_golden.py; the GPU box has
-no reference tree).  A working directory is laid out like the reference checkout:
+The scripts' text comes from tests/golden/ref_scripts.npz (minted from the reference checkout by make_golden.py), so no
+reference tree is needed.  A working directory is laid out like the reference checkout:
 
     src/__init__.py
-    src/estimator.py   <- the binding under test: on the GPU box the 4-line block of INTEGRATION.md section 1,
+    src/estimator.py   <- the binding under test: on a GPU machine the 4-line block of INTEGRATION.md section 1,
                           parsed out of that file; on a CPU box an oracle-backed stand-in (harness self-check)
     src/hog_box.py     <- re-exports the headless HOGBox replacement (vnect_b200/hog_box.py)
     src/utils.py       <- the only two helpers the scripts call outside drawing: img_scale (utils.py:13-21) + drawing no-ops
@@ -170,13 +170,22 @@ def walk_run_estimator(res, net, module_suffix, exact):
 
 
 # ------------------------------------------------------------------------------------------------ fixture provenance
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree only exists in the dev container")
+# sha256 of the reference's run_pic.py and run_estimator.py, taken when ref_scripts.npz was minted from them
+REF_SCRIPT_SHA256 = {
+    "run_pic.py": "da6ec6c628b3fbd819185ebe29accc606791575fddb07f4ec04247d18efd7970",
+    "run_estimator.py": "db3835a346ba0d9cdf4cf16b583c5b72a5d174997da6defeb2d38b8c1aaad4b1",
+}
+
+
 def test_script_fixture_is_the_unmodified_reference_text():
+    """The stored script text hashes to what the reference files hashed to (and equals them when the tree is present)."""
     import hashlib
     g = np.load(os.path.join(GOLDEN, "ref_scripts.npz"))
-    for name in ("run_pic.py", "run_estimator.py"):
-        data = open(os.path.join(ref_shim.REFERENCE_ROOT, name), "rb").read()
-        assert bytes(g[name]) == data and str(g[name + "/sha256"]) == hashlib.sha256(data).hexdigest()
+    for name, digest in REF_SCRIPT_SHA256.items():
+        data = bytes(g[name])
+        assert hashlib.sha256(data).hexdigest() == digest == str(g[name + "/sha256"])
+        if ref_shim.reference_available():
+            assert open(os.path.join(ref_shim.REFERENCE_ROOT, name), "rb").read() == data
 
 
 def test_hogbox_cal_rect_matches_reference_arithmetic():
