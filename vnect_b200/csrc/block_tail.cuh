@@ -12,7 +12,7 @@
 //
 // One CTA pair (tcgen05 cta_group::2) owns 256 GEMM rows and walks ALL output-channel tiles of those rows (256 columns
 // each), so the second accumulator sees the whole K = Cout.  TMEM: columns [0, 256) main accumulator (single
-// buffered), [256, 512) second accumulator (two of them when N2 <= 128).  K order of the second GEMM is channel order,
+// buffered), [256, 512) two second accumulators.  K order of the second GEMM is channel order,
 // the same as the stand-alone reduce conv, so both plans give bit-identical results.
 //
 // Scheduling (the first version serialised everything and ran 2x slower than the two kernels it replaces):
@@ -42,19 +42,18 @@ struct TailCfg {
   static constexpr int A_BYTES = kBlockM * 128;
   static constexpr int B_BYTES = (kTailBlockN / 2) * 128;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int W2_STAGES = N2 == 256 ? 2 : 4;
+  static constexpr int W2_STAGES = 4;
   static constexpr int W2_BYTES = (N2 / 2) * 128;
   static constexpr int OUT_BUFS = 2;                                   // staging tiles per epilogue group
   static constexpr int OUT_BYTES = kEpiGroups * OUT_BUFS * kEpiChunkBytes;
-  static constexpr int RES_STAGES = RES ? (N2 == 256 ? 2 : 4) : 0;
+  static constexpr int RES_STAGES = RES ? 4 : 0;
   static constexpr int RES_BYTES = RES_STAGES * kEpiChunkBytes;
-  static constexpr int ACC2_BUFS = N2 <= 128 ? 2 : 1;
   static constexpr int STAGES_RAW = (kSmemBudget - 1024 - 512 - OUT_BYTES - RES_BYTES - W2_STAGES * W2_BYTES) / STAGE_BYTES;
   static constexpr int STAGES = STAGES_RAW > 6 ? 6 : STAGES_RAW;
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + W2_STAGES * W2_BYTES + OUT_BYTES + RES_BYTES + 1024 + 512;
   static_assert(STAGES >= 2, "pipeline needs at least two stages");
-  static_assert(N2 == 64 || N2 == 128 || N2 == 256, "second GEMM width");
-  static_assert(kTailBlockN + ACC2_BUFS * N2 <= 512, "accumulators must fit TMEM");
+  static_assert(N2 == 64 || N2 == 128, "second GEMM width");
+  static_assert(kTailBlockN + 2 * N2 <= 512, "accumulators must fit TMEM");
 };
 
 template <int N2, bool RES>
@@ -71,7 +70,7 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
   constexpr int CH2 = N2 / 64;       // chunks of the second accumulator
   constexpr int W2S = Cfg::W2_STAGES;
   constexpr int RS = Cfg::RES_STAGES > 0 ? Cfg::RES_STAGES : 1;
-  constexpr int A2 = Cfg::ACC2_BUFS;
+  constexpr int A2 = 2;              // second accumulators (double buffered)
   constexpr uint32_t IDESC = make_idesc_f16(2 * kBlockM, BLOCK_N, false);
   constexpr uint32_t IDESC2 = make_idesc_f16(2 * kBlockM, N2, false);
   const ConvGemmParams& p = bp.g;

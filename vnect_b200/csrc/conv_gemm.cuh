@@ -1,4 +1,4 @@
-// Implicit-GEMM convolution for sm_100a: TMA (tiled, 5-D, zero OOB fill = SAME padding) -> 128B/64B-swizzled smem
+// Implicit-GEMM convolution for sm_100a: TMA (tiled, 5-D, zero OOB fill = SAME padding) -> 128B-swizzled smem
 // -> tcgen05.mma (fp16 operands, fp32 accumulators in TMEM) -> fused epilogue (bias / folded BN / residual / ReLU).
 //
 // GEMM view: D[M = pixels, N = Cout] = A[M, K] * B[N, K]^T with K = taps * Cin. Activations are NHWC fp16, so A is
@@ -8,9 +8,8 @@
 //
 // Every conv of src/vnect_model.py:27-214 (reference) maps onto this one kernel:
 //   1x1 convs           flat rows (M = n*H*W), 1 tap
-//   3x3 convs           spatial tiles tw x th (<=128 px) of one image, 9 taps
+//   3x3 convs           9 taps: halo patches or spatial tiles tw x th (<=128 px) of one image, or flat rows (im2col)
 //   4x4/2 transposed    4 output phases, each a 2x2-tap conv (SURVEY.md App. A.2), epilogue scatters to (2y+py, 2x+px)
-//   conv1 7x7/2, Cin=3  7 row taps; a K block is an 8-pixel x 4-channel window of the padded, parity-split input
 //
 // Warp roles (256 threads, persistent over tiles): warp 0 = TMA producer, warp 1 = MMA issuer (one thread),
 // warp 2 = TMEM allocator, warps 4-7 = epilogue (TMEM lane quarter = warp % 4). TMEM accumulators are double
@@ -26,7 +25,6 @@ constexpr int kGemmThreadsTma = 384;   // TMA epilogues: two epilogue warpgroups
 constexpr int kSmemBudget = 227 * 1024;
 
 enum EpiKind : int {
-  EPI_NHWC_F16 = 0,    // fp16 NHWC, bias (+residual) (+ReLU)
   EPI_PLANAR_F32 = 1,  // fp32 channel-planar [n][c][OH][OW] (heat-map / location-map output, read by the post-process)
   EPI_DECONV_HEAD = 2, // fused res5c head: BN(folded)+ReLU on cols 0-127, deltas on 128-190, bone lengths -> 191-211
   EPI_TMA = 3,         // fp16 NHWC through swizzled smem staging + TMA tensor store (coalesced, clipped), bias (+ReLU)
@@ -34,17 +32,9 @@ enum EpiKind : int {
 };
 
 constexpr int kEpiChunkBytes = kBlockM * 128;  // one 64-column fp16 chunk of a tile: 128 rows x 128 B
-// Experiment switches (selftest builds only, `make experiments`): each removes one stage of the TMA epilogue so that the
-// per-chunk cost can be attributed; results are wrong by construction, only the timing is read.
-#ifndef VNECT_EXP_OUT_STAGES
-#define VNECT_EXP_OUT_STAGES 1
-#endif
-constexpr int kOutStages = VNECT_EXP_OUT_STAGES;   // per epilogue warpgroup (two groups alternate, so each ring needs one slot)
+constexpr int kOutStages = 1;   // per epilogue warpgroup (two groups alternate, so each ring needs one slot)
 constexpr int kEpiGroups = 2;
-#ifndef VNECT_EXP_RES_STAGES
-#define VNECT_EXP_RES_STAGES 4
-#endif
-constexpr int kResStages = VNECT_EXP_RES_STAGES;
+constexpr int kResStages = 4;
 
 struct ConvGemmParams {
   // ---- tiling of the GEMM rows
@@ -58,7 +48,7 @@ struct ConvGemmParams {
   int cblocks2;          // ... followed by cblocks2 blocks read from a SECOND activation tensor (1x1, same rows):
                          // a projection shortcut folded into the block's last conv as extra K (W = [W_2c | W_1])
   int b_rows_per_phase;  // padded Cout
-  signed char tap_dx[16], tap_dy[16], tap_dp[16];  // [phase * taps + tap]
+  signed char tap_dx[16], tap_dy[16];  // [phase * taps + tap]
   uint32_t stage_tx_bytes;
   uint32_t res_tx_bytes;  // bytes of one residual chunk box (EPI_TMA_RES)
   int reverse;            // 1: walk the tiles from last to first.  Consecutive layers alternate, so a layer starts on
@@ -69,13 +59,10 @@ struct ConvGemmParams {
   int n_valid;    // valid output columns
   int relu_cols;  // ReLU on columns < relu_cols (multiple of 32)
   const float* bias;
-  const __half* residual;
-  int ldr;
   void* out;
   int ldc;
   int OH, OW;    // output grid
   int oys, oxs;  // output pixel = (y*oys + py, x*oxs + px)
-  int decimate;  // 1: only rows with even (y, x) are stored, at (y/2, x/2) -- feeds the stride-2 1x1 convs
   int im2col;    // 1: flat-row 3x3 conv whose A operand comes through an im2col tensor map (tap_dx / tap_dy = filter offsets 0..2)
 };
 
@@ -99,11 +86,11 @@ constexpr int kHaloTW = 8, kHaloTH = 16;                  // output tile: 8 x 16
 constexpr int kHaloPW = kHaloTW + 2, kHaloPH = kHaloTH + 2;
 constexpr int kHaloPatchTx = kHaloPW * kHaloPH * 128;      // bytes one patch load delivers (OOB pixels are zero-filled)
 constexpr int kHaloABytes = ((kHaloPatchTx + 1023) / 1024) * 1024;
-template <int BLOCK_N, int SWZ, int EPI, int CG = 1, bool BRES = false, bool HALO = false>
+template <int BLOCK_N, int EPI, int CG = 1, bool BRES = false, bool HALO = false>
 struct GemmCfg {
-  static constexpr int BLOCK_K = SWZ / 2;  // fp16 elements per smem row
-  static constexpr int A_BYTES = kBlockM * SWZ;
-  static constexpr int B_BYTES = (BLOCK_N / CG) * SWZ;
+  static constexpr int BLOCK_K = 64;  // fp16 elements per 128-byte swizzled smem row
+  static constexpr int A_BYTES = kBlockM * 128;
+  static constexpr int B_BYTES = (BLOCK_N / CG) * 128;
   // ring stage: A + B tiles; activations only with resident weights; weight tiles only in HALO mode (the patches have
   // their own ring); HALO + BRES streams nothing through it (one dummy stage keeps the barrier arrays non-empty)
   static constexpr int STAGE_BYTES = HALO ? (BRES ? 1024 : B_BYTES) : (BRES ? A_BYTES : A_BYTES + B_BYTES);
@@ -125,8 +112,8 @@ struct GemmCfg {
                                         : (2 * BLOCK_N <= 256) ? 256
                                                                : 512;
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + BRES_BYTES + HALO_BYTES + EPI_BYTES + 1024 /*align slack*/ + 512 /*barriers*/;
-  static_assert(STAGES >= 2 || (HALO && BRES) || (VNECT_EXP_RES_STAGES > 4 && STAGES >= 1), "pipeline needs at least two stages");
-  static_assert(!HALO || (EPI == EPI_TMA && SWZ == 128), "the halo-patch path is the plain 3x3 conv: EPI_TMA, 128B swizzle");
+  static_assert(STAGES >= 2 || (HALO && BRES), "pipeline needs at least two stages");
+  static_assert(!HALO || EPI == EPI_TMA, "the halo-patch path is the plain 3x3 conv: EPI_TMA");
   static_assert(2 * STAGES + 5 + 2 * kResStages + 2 <= 64, "barriers must fit their 512-byte region");
   static_assert(2 * BLOCK_N <= 512, "two accumulator stages must fit TMEM");
   static_assert(BLOCK_N % 32 == 0 && BLOCK_N >= 32 && BLOCK_N <= 256, "epilogue walks 32-column chunks");
@@ -147,12 +134,12 @@ __device__ __forceinline__ uint32_t pack_half2_relu(float a, float b) {
   return d;
 }
 
-template <int BLOCK_N, int SWZ, int EPI, int CG = 1, bool BRES = false, bool HALO = false>
+template <int BLOCK_N, int EPI, int CG = 1, bool BRES = false, bool HALO = false>
 __global__ void __launch_bounds__((EPI == EPI_TMA || EPI == EPI_TMA_RES || EPI == EPI_DECONV_HEAD) ? kGemmThreadsTma : kGemmThreads, 1)
 conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                  const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_res,
                  const __grid_constant__ CUtensorMap tmap_a2, const __grid_constant__ ConvGemmParams p) {
-  using Cfg = GemmCfg<BLOCK_N, SWZ, EPI, CG, BRES, HALO>;
+  using Cfg = GemmCfg<BLOCK_N, EPI, CG, BRES, HALO>;
   static_assert(!BRES || CG == 1, "resident weights are a single-CTA variant");
   constexpr bool kTmaEpi = (EPI == EPI_TMA || EPI == EPI_TMA_RES);
   constexpr int BLOCK_K = Cfg::BLOCK_K;
@@ -293,7 +280,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         }
         for (int t = 0; t < p.taps; ++t) {
           const int ti = ph * p.taps + t;
-          const int ax = cx * p.in_stride + p.tap_dx[ti], ay = cy * p.in_stride + p.tap_dy[ti], ap = p.tap_dp[ti];
+          const int ax = cx * p.in_stride + p.tap_dx[ti], ay = cy * p.in_stride + p.tap_dy[ti];
           for (int cb = 0; cb < p.cblocks; ++cb) {
             mbar_wait(&empty_bar[stage], phase ^ 1);
             if (issuer) {
@@ -301,12 +288,12 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
               if constexpr (CG == 2) {  // both CTAs' bytes are counted on the leader's barrier
                 if (cta_rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * p.stage_tx_bytes);
                 if (p.im2col) tma_load_im2col_4d_pair(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, iw, ih, in_, p.tap_dx[ti], p.tap_dy[ti]);
-                else tma_load_5d_pair(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, ax, ay, ap, cn);
+                else tma_load_5d_pair(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, ax, ay, 0, cn);
                 tma_load_2d_pair(sa + Cfg::A_BYTES, &tmap_b, &full_bar[stage], (t * p.cblocks + cb) * BLOCK_K, b_row);
               } else {
                 mbar_arrive_expect_tx(&full_bar[stage], p.stage_tx_bytes);
                 if (p.im2col) tma_load_im2col_4d(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, iw, ih, in_, p.tap_dx[ti], p.tap_dy[ti]);
-                else tma_load_5d(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, ax, ay, ap, cn);
+                else tma_load_5d(sa, &tmap_a, &full_bar[stage], cb * BLOCK_K, ax, ay, 0, cn);
                 if constexpr (!BRES)
                   tma_load_2d(sa + Cfg::A_BYTES, &tmap_b, &full_bar[stage], (t * p.cblocks + cb) * BLOCK_K, b_row);
               }
@@ -383,11 +370,11 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
               const uint64_t a_desc = make_kmajor_desc_sbo(patch + static_cast<uint32_t>((ky * kHaloPW + kx) * 128), kHaloPW * 128);
               uint64_t b_desc;
               if constexpr (BRES) {
-                b_desc = make_kmajor_desc<SWZ>(smem_u32(b_res + (t * p.cblocks + cb) * Cfg::B_BYTES));
+                b_desc = make_kmajor_desc<128>(smem_u32(b_res + (t * p.cblocks + cb) * Cfg::B_BYTES));
               } else {
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
-                b_desc = make_kmajor_desc<SWZ>(smem_u32(smem + stage * Cfg::STAGE_BYTES));
+                b_desc = make_kmajor_desc<128>(smem_u32(smem + stage * Cfg::STAGE_BYTES));
               }
               if (issuer) {
 #pragma unroll
@@ -423,9 +410,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
           const uint32_t a_addr = smem_u32(smem + stage * Cfg::STAGE_BYTES);
-          const uint64_t a_desc = make_kmajor_desc<SWZ>(a_addr);
-          const uint64_t b_desc = BRES ? make_kmajor_desc<SWZ>(smem_u32(b_res + kb * Cfg::B_BYTES))
-                                       : make_kmajor_desc<SWZ>(a_addr + Cfg::A_BYTES);
+          const uint64_t a_desc = make_kmajor_desc<128>(a_addr);
+          const uint64_t b_desc = BRES ? make_kmajor_desc<128>(smem_u32(b_res + kb * Cfg::B_BYTES))
+                                       : make_kmajor_desc<128>(a_addr + Cfg::A_BYTES);
           if (issuer) {
 #pragma unroll
             for (int k = 0; k < BLOCK_K / 16; ++k) {  // +32 B per K step = +2 in the descriptor's (addr >> 4) field
@@ -572,14 +559,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           bias_hi = __ldg(p.bias + col_base + c0 + 32 + lane);
         }
         uint32_t v[64];
-#ifdef VNECT_EXP_NO_TMEM_LD
-#pragma unroll
-        for (int e = 0; e < 64; ++e) v[e] = static_cast<uint32_t>(e + lane);
-#else
         tmem_ld_32x32(t_row + c0, *reinterpret_cast<uint32_t(*)[32]>(&v[0]));
         tmem_ld_32x32(t_row + c0 + 32, *reinterpret_cast<uint32_t(*)[32]>(&v[32]));
         tmem_ld_wait();
-#endif
         if (c + 2 >= CH) {  // this group's last chunk of the tile: its share of the accumulator has been read
           tc_fence_before();
           __syncwarp();
@@ -597,13 +579,8 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         named_bar_sync(1 + grp, 128);
         const int col0 = col_base + c0;
         const bool relu = col0 < p.relu_cols;
-#ifdef VNECT_EXP_NO_PACK
-#pragma unroll
-        for (int j = 0; j < 0; ++j) {
-#else
 #pragma unroll
         for (int j = 0; j < 8; ++j) {  // 8 x 16 B = this row's 64 output channels
-#endif
           float f[8];
 #pragma unroll
           for (int e = 0; e < 8; ++e) f[e] = __uint_as_float(v[8 * j + e]);
@@ -611,11 +588,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           for (int e = 0; e < 8; ++e)  // column 8j+e of the chunk: lane (8j+e) & 31 of the low / high half holds its bias
             f[e] += __shfl_sync(0xffffffffu, j < 4 ? bias_lo : bias_hi, (8 * j + e) & 31);
           const uint32_t off = row_off + ((static_cast<uint32_t>(j) ^ sw) << 4);  // 128B swizzle, as the TMA unit does
-#ifndef VNECT_EXP_NO_RES
           if constexpr (EPI == EPI_TMA_RES) {
-#else
-          if constexpr (false) {
-#endif
             const uint4 rv = *reinterpret_cast<const uint4*>(rstage + off);
             const __half2* h = reinterpret_cast<const __half2*>(&rv);
 #pragma unroll
@@ -642,9 +615,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         fence_proxy_async_smem();  // generic-proxy smem writes -> visible to the TMA (async proxy)
         named_bar_sync(1 + grp, 128);
         if (leader) {
-#ifndef VNECT_EXP_NO_STORE
           tma_store_5d(&tmap_out, ostage, col0, cx, cy, 0, cn);
-#endif
           bulk_commit_group();
           if constexpr (EPI == EPI_TMA_RES) mbar_arrive(&res_empty[rb]);
         }
@@ -684,17 +655,8 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         x = (t2 % p.tiles_x) * p.tw + lx;
         valid = (ly < p.th) && (y < p.H) && (x < p.W) && (n < p.NB);
       }
-      int oy, ox;
-      if (p.decimate) {
-        valid = valid && !((y | x) & 1);
-        oy = y >> 1;
-        ox = x >> 1;
-      } else {
-        oy = y * p.oys + (ph >> 1);
-        ox = x * p.oxs + (ph & 1);
-      }
+      const int oy = y * p.oys + (ph >> 1), ox = x * p.oxs + (ph & 1);
       const size_t pix = (static_cast<size_t>(n) * p.OH + oy) * p.OW + ox;
-      const size_t rpix = (static_cast<size_t>(n) * p.H + y) * p.W + x;  // residual lives on the GEMM-row grid
       const int col_base = n_tile * BLOCK_N;
 
       mbar_wait(&tmem_full[acc], acc_phase);
@@ -741,20 +703,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           for (int j = 0; j < 32; ++j) st[(c0 + j) * kBlockM + r] = f[j];
         } else {
           if (valid) {
-            if (p.residual != nullptr) {
-              const uint4* rp = reinterpret_cast<const uint4*>(p.residual + rpix * p.ldr + col0);
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const uint4 rv = __ldg(rp + j);
-                const __half2* h = reinterpret_cast<const __half2*>(&rv);
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                  const float2 t = __half22float2(h[e]);
-                  f[8 * j + 2 * e] += t.x;
-                  f[8 * j + 2 * e + 1] += t.y;
-                }
-              }
-            }
             if (col0 < p.relu_cols) {
 #pragma unroll
               for (int j = 0; j < 32; ++j) f[j] = fmaxf(f[j], 0.f);
@@ -782,7 +730,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         }
       }
       if constexpr (EPI == EPI_PLANAR_F32) {
-        // flat rows only (1x1 conv, no decimation): row m = n * hw + rem, planes are [n][column][hw]; hw % 4 == 0
+        // flat rows only (1x1 conv): row m = n * hw + rem, planes are [n][column][hw]; hw % 4 == 0
         named_bar_sync(1, 128);
         const float* st = reinterpret_cast<const float*>(out_stage);
         float* o = reinterpret_cast<float*>(p.out);

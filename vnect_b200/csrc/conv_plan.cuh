@@ -68,6 +68,7 @@ inline bool encode_tmap_im2col_3x3(CUtensorMap* m, const void* ptr, int NB, int 
   return true;
 }
 
+// swz_bytes: 128 (every GEMM operand and output tile) or 0 (the stem's raw strips)
 inline bool encode_tmap(CUtensorMap* m, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                         const uint32_t* box, int swz_bytes, std::string* err, const uint32_t* elem_strides = nullptr) {
   PFN_encodeTiled enc = get_encode_tiled();
@@ -78,10 +79,7 @@ inline bool encode_tmap(CUtensorMap* m, const void* ptr, int rank, const uint64_
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   if (elem_strides)
     for (int i = 0; i < rank; ++i) estr[i] = elem_strides[i];
-  CUtensorMapSwizzle sw = swz_bytes == 128  ? CU_TENSOR_MAP_SWIZZLE_128B
-                          : swz_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
-                          : swz_bytes == 0  ? CU_TENSOR_MAP_SWIZZLE_NONE
-                                            : CU_TENSOR_MAP_SWIZZLE_32B;
+  const CUtensorMapSwizzle sw = swz_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE;
   CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, rank, const_cast<void*>(ptr), dims, strides_bytes, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -101,16 +99,13 @@ inline bool encode_tmap(CUtensorMap* m, const void* ptr, int rank, const uint64_
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-enum ConvKind : int { CONV_1x1 = 0, CONV_3x3 = 1, CONV_DECONV4 = 2, CONV_STEM7 = 3 };
+enum ConvKind : int { CONV_1x1 = 0, CONV_3x3 = 1, CONV_DECONV4 = 2 };
 
 struct ConvSpec {
   int kind = CONV_1x1;
-  // GEMM-row grid (= conv output grid before the phase scatter); for CONV_STEM7 this is the 184x184 output grid
-  int NB = 1, H = 1, W = 1;
-  const __half* in = nullptr;  // NHWC fp16 activation [NB,H,W,cin_pad]; CONV_STEM7: parity-split padded input
-  int cin_pad = 64;            // channels per pixel of `in` (multiple of 64); CONV_STEM7: ignored
-  // CONV_STEM7 input geometry: [NB][2 parities][rows_per_parity][row_pitch_elems]
-  int stem_rows_per_parity = 0, stem_row_pitch = 0;
+  int NB = 1, H = 1, W = 1;    // GEMM-row grid (= conv output grid before the phase scatter)
+  const __half* in = nullptr;  // NHWC fp16 activation [NB,H,W,cin_pad]
+  int cin_pad = 64;            // channels per pixel of `in` (multiple of 64)
   const __half* w = nullptr;  // packed [phases * n_pad][taps * cin_pad] fp16, K-major
   int n_pad = 64;             // padded Cout (multiple of block_n)
   int n_valid = 64;
@@ -121,30 +116,20 @@ struct ConvSpec {
   int ldr = 0;
   void* out = nullptr;
   int ldc = 0;
-  int epi = EPI_NHWC_F16;
-  int decimate = 0;
+  int epi = EPI_TMA;
   // stride-2 sampling (the stride-2 1x1 convs of res3a/res4a only read even pixels of res2c/res3d, so those two
   // blocks are computed at even pixels only): the conv reads `in` [NB, in_stride*H, in_stride*W, cin_pad] at every
   // in_stride-th pixel; the residual is [NB, res_stride*H, res_stride*W, ldr] read likewise. 1x1 convs with a
   // strided operand use spatial tiles.
   int in_stride = 1;
   int res_stride = 1;
-  int spatial_1x1 = 0;
   // folded projection shortcut (1x1 convs only): a second activation tensor [NB,H,W,cin2_pad] whose channels extend
   // the K dimension; `w` is then [n_pad][cin_pad + cin2_pad]
   const __half* in2 = nullptr;
   int cin2_pad = 0;
-  // 2: run on CTA pairs (tcgen05 cta_group::2, 256-row tiles); 1: one CTA per tile
-  int cg = 1;
-  // 1: keep the layer's whole weight matrix resident in smem (single N tile, <= kMaxResidentKBlocks K blocks, no pairs)
-  int b_resident = 0;
-  // 1: 3x3 stride-1 conv through one halo patch per channel block (8 x 16 pixel tiles, conv_gemm.cuh HALO)
-  int halo = 0;
-  // 1: 3x3 stride-1 conv on flat pixel rows through an im2col tensor map (no tile row wasted on small images)
-  int im2col = 0;
   // fused block tail (block_tail.cuh): this 1x1 conv (+ residual / folded shortcut) also feeds a second 1x1 conv
   // Y = relu(out * W2^T + bias2) of n2 output channels; w2 is [n2][n_pad] fp16 K-major, out2 NHWC [.., n2] on the
-  // same pixel grid as `out`.  Needs block_n = 256 on CTA pairs and a TMA epilogue.
+  // same pixel grid as `out`.  Needs block_n = 256 (CTA pairs) and n2 = 64 with EPI_TMA or n2 = 128 with EPI_TMA_RES.
   const __half* w2 = nullptr;
   const float* bias2 = nullptr;
   void* out2 = nullptr;
@@ -156,7 +141,7 @@ struct ConvLaunch {
   ConvGemmParams p;
   const float* bias2 = nullptr;
   int n2 = 0;  // > 0: fused block tail (block_tail_kernel)
-  int block_n = 0, swz = 128, epi = 0, grid = 0, cg = 1, b_resident = 0, halo = 0;
+  int block_n = 0, epi = 0, grid = 0, cg = 1, b_resident = 0, halo = 0;
   size_t smem = 0;
   double flops = 0;  // algorithmic: 2 * valid rows * n_valid * taps * real Cin is tracked by the caller; this is GEMM work
 };
@@ -202,28 +187,107 @@ inline bool halo_tiling_ok(int H, int W) {
   return halo_tiles * 10 <= free_tiles * 11;
 }
 
+// How a conv runs, from its shape, output tile width and epilogue.  build_conv applies these rules to every conv, so
+// the library and the self-test build exactly the configurations that have a kernel.
+struct ConvPath {
+  // CTA pairs (tcgen05 cta_group::2) pay off where the MMA's smem operand reads are the limit: N >= 128 tiles
+  // (measured 5-8 % on the tensor-bound layers, nothing at N = 64)
+  int cg;
+  // 64-channel convs whose whole weight matrix fits kMaxResidentKBlocks K blocks keep it resident in smem: the 3x3s of
+  // res2 are bound by L2->SM traffic (158 -> 135 us), the 1x1 256->64 convs gain a few percent.  Those 3x3s run on
+  // spatial tiles, one shifted box per tap, where the halo tiling does not apply (stride 2, small grids).
+  int b_resident;
+  // stride-1 3x3 convs on the larger grids read one halo patch per channel block instead of nine shifted boxes
+  // (conv_gemm.cuh HALO)
+  int halo;
+  // the other 3x3 convs (23 x 23 at box size 368: five 23 x 5 tiles fill 529 of 640 GEMM rows; stride-2 ones included,
+  // res3d's 3x3 at 46 -> 23: 31 -> 27 us) and the transposed conv (114 -> 103 us per 128 forwards) run on flat pixel
+  // rows through an im2col tensor map: every row of a 128-row tile is a real pixel.  Same K order, so the same results.
+  int im2col;
+};
+
+inline ConvPath conv_path(const ConvSpec& s) {
+  ConvPath r;
+  r.cg = s.block_n >= 128 ? 2 : 1;
+  const int taps = s.kind == CONV_3x3 ? 9 : 1;
+  r.b_resident = s.kind != CONV_DECONV4 && s.block_n == 64 && s.n_pad == 64 && s.epi == EPI_TMA && !s.in2 &&
+                 taps * s.cin_pad / 64 <= kMaxResidentKBlocks;
+  r.halo = s.kind == CONV_3x3 && s.in_stride == 1 && s.epi == EPI_TMA && s.block_n <= 128 && halo_tiling_ok(s.H, s.W);
+  r.im2col = s.kind == CONV_DECONV4 || (s.kind == CONV_3x3 && !r.halo && !r.b_resident);
+  return r;
+}
+
+// cudaFuncSetAttribute is per device (context): remember, per kernel instantiation, which devices of this process
+// already carry the opt-in.  One bit per device ordinal; a process holds at most one handle per GPU of an 8-GPU box.
+template <typename Kern>
+inline cudaError_t ensure_dyn_smem(Kern kern, int bytes, unsigned long long* done_mask) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  const unsigned long long bit = 1ull << (dev & 63);
+  if (__atomic_load_n(done_mask, __ATOMIC_ACQUIRE) & bit) return cudaSuccess;
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess) return e;
+  __atomic_fetch_or(done_mask, bit, __ATOMIC_RELEASE);
+  return cudaSuccess;
+}
+
+// One conv_gemm_kernel instantiation with its launch shape
+typedef void (*ConvKernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvGemmParams);
+struct ConvKernel {
+  ConvKernelFn fn = nullptr;
+  int threads = 0, smem = 0, cg = 1;
+  unsigned long long* smem_done = nullptr;  // ensure_dyn_smem's device mask of this instantiation
+};
+
+template <int BLOCK_N, int EPI, int CG, bool BRES = false, bool HALO = false>
+inline ConvKernel conv_kernel() {
+  using Cfg = GemmCfg<BLOCK_N, EPI, CG, BRES, HALO>;
+  static unsigned long long done = 0;
+  return {conv_gemm_kernel<BLOCK_N, EPI, CG, BRES, HALO>, Cfg::THREADS, Cfg::SMEM_BYTES, CG, &done};
+}
+
+// The instantiations the plans launch (see conv_path); any other combination has no kernel (fn == nullptr)
+inline ConvKernel find_conv_kernel(const ConvLaunch& L) {
+  const int bn = L.block_n, epi = L.epi, cg = L.cg;
+  if (epi == EPI_TMA && cg == 1 && bn == 64) {
+    if (L.halo) return L.b_resident ? conv_kernel<64, EPI_TMA, 1, true, true>() : conv_kernel<64, EPI_TMA, 1, false, true>();
+    return L.b_resident ? conv_kernel<64, EPI_TMA, 1, true>() : conv_kernel<64, EPI_TMA, 1>();
+  }
+  if (L.b_resident) return {};
+  if (epi == EPI_TMA && cg == 2 && bn == 128) return L.halo ? conv_kernel<128, EPI_TMA, 2, false, true>() : conv_kernel<128, EPI_TMA, 2>();
+  if (L.halo) return {};
+  if (epi == EPI_TMA && cg == 2 && bn == 256) return conv_kernel<256, EPI_TMA, 2>();
+  if (epi == EPI_TMA_RES && cg == 1 && bn == 64) return conv_kernel<64, EPI_TMA_RES, 1>();
+  if (epi == EPI_TMA_RES && cg == 2 && bn == 256) return conv_kernel<256, EPI_TMA_RES, 2>();
+  if (epi == EPI_PLANAR_F32 && cg == 1 && bn == 96) return conv_kernel<96, EPI_PLANAR_F32, 1>();
+  if (epi == EPI_DECONV_HEAD && cg == 2 && bn == 192) return conv_kernel<192, EPI_DECONV_HEAD, 2>();
+  return {};
+}
+
+// fused block tails: a 64-wide second conv after a folded projection, a 128-wide one after a residual add
+inline bool tail_supported(int n2, int epi) { return (n2 == 64 && epi == EPI_TMA) || (n2 == 128 && epi == EPI_TMA_RES); }
+
 inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::string* err) {
   memset(L, 0, sizeof(*L));
   ConvGemmParams& p = L->p;
-  const int swz = (s.kind == CONV_STEM7) ? 64 : 128;
-  const int block_k = swz / 2;
-  L->swz = swz;
+  constexpr int block_k = 64;
+  const ConvPath path = conv_path(s);
   L->block_n = s.block_n;
   L->epi = s.epi;
-  L->cg = s.cg;
-  L->b_resident = s.b_resident;
-  L->halo = s.halo;
-  if (s.halo && (s.kind != CONV_3x3 || s.in_stride != 1 || s.epi != EPI_TMA || (s.block_n != 64 && s.block_n != 128) ||
-                 (s.cg == 2 && s.block_n != 128) || (s.b_resident && s.block_n != 64))) {
-    if (err) *err = "the halo-patch path needs a stride-1 3x3 conv with an EPI_TMA output and a 64- or 128-column tile";
-    return false;
-  }
-  if (s.cg != 1 && (s.cg != 2 || s.kind == CONV_STEM7 || (s.block_n / 2) % 8 != 0)) {
-    if (err) *err = "unsupported CTA-pair configuration";
+  L->cg = path.cg;
+  L->b_resident = path.b_resident;
+  L->halo = path.halo;
+  if (s.cin_pad % 64 != 0 || s.cin2_pad % 64 != 0) {
+    if (err) *err = "input channels must be padded to multiples of 64";
     return false;
   }
   if (s.n_pad % s.block_n != 0) {
     if (err) *err = "n_pad must be a multiple of block_n";
+    return false;
+  }
+  if (s.kind == CONV_DECONV4 && s.in_stride != 1) {
+    if (err) *err = "the transposed conv reads every input pixel";
     return false;
   }
   p.NB = s.NB;
@@ -236,52 +300,48 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
   p.n_valid = s.n_valid;
   p.relu_cols = s.relu_cols;
   p.bias = s.bias;
-  p.residual = s.residual;
-  p.ldr = s.ldr;
   p.out = s.out;
   p.ldc = s.ldc;
-  p.decimate = s.decimate;
-  p.OH = s.decimate ? s.H / 2 : s.H;
-  p.OW = s.decimate ? s.W / 2 : s.W;
+  p.OH = s.H;
+  p.OW = s.W;
   p.oys = p.oxs = 1;
   p.in_stride = s.in_stride;
   p.res_stride = s.res_stride;
-  const bool spatial1 = s.kind == CONV_1x1 && (s.spatial_1x1 || s.in_stride != 1 || s.res_stride != 1);
+  const bool spatial1 = s.kind == CONV_1x1 && (s.in_stride != 1 || s.res_stride != 1);
   uint32_t estr[5] = {1, (uint32_t)s.in_stride, (uint32_t)s.in_stride, 1, 1};
 
   uint64_t dims[5], strides[4];
   uint32_t box[5];
   int k_total;
-  if (s.kind == CONV_1x1 && !spatial1) {
+  if ((s.kind == CONV_1x1 && !spatial1) || path.im2col) {  // flat pixel rows
     p.mode = 0;
-    p.taps = 1;
     p.cblocks = s.cin_pad / block_k;
     p.num_m_tiles = (p.M + kBlockM - 1) / kBlockM;
     p.tw = kBlockM;
     p.th = 1;
     p.tiles_x = p.tiles_y = 1;
+    // for im2col, dims / box describe the A tile for the byte count below; the map is built by encode_tmap_im2col_3x3
     dims[0] = s.cin_pad; dims[1] = p.M; dims[2] = 1; dims[3] = 1; dims[4] = 1;
     strides[0] = (uint64_t)s.cin_pad * 2;
     strides[1] = strides[2] = strides[3] = (uint64_t)s.cin_pad * 2 * p.M;
     box[0] = block_k; box[1] = kBlockM; box[2] = 1; box[3] = 1; box[4] = 1;
-    k_total = s.cin_pad + s.cin2_pad;
-    p.cblocks2 = s.cin2_pad / block_k;
-  } else if ((s.kind == CONV_3x3 || s.kind == CONV_DECONV4) && s.im2col) {
-    if (s.halo || (s.in_stride != 1 && s.kind != CONV_3x3) || s.cin_pad % 64 != 0 || swz != 128) {
-      if (err) *err = "the im2col path is the plain stride-1 3x3 conv (or the 4x4/2 transposed conv) with 128B-swizzled 64-channel K blocks";
-      return false;
-    }
-    p.mode = 0;
-    p.im2col = 1;
-    if (s.kind == CONV_3x3) {
+    if (s.kind == CONV_1x1) {
+      p.taps = 1;
+      p.cblocks2 = s.cin2_pad / block_k;
+    } else if (s.kind == CONV_3x3) {
+      p.im2col = 1;
       p.taps = 9;
       for (int ky = 0; ky < 3; ++ky)
         for (int kx = 0; kx < 3; ++kx) {  // filter offsets from the base pixel, not displacements from the output pixel
           p.tap_dy[ky * 3 + kx] = (signed char)ky;
           p.tap_dx[ky * 3 + kx] = (signed char)kx;
-          p.tap_dp[ky * 3 + kx] = 0;
         }
-    } else {  // the four output phases of the transposed conv, each a 2x2-tap conv inside the same 3x3 neighbourhood
+    } else {
+      // 4x4 stride-2 'SAME' transposed conv: output (2j+py, 2i+px); per axis, phase 0 uses kernel taps {1,3} at
+      // input offsets {0,-1}, phase 1 uses taps {0,2} at offsets {+1,0} (SURVEY.md App. A.2): each phase is a 2x2-tap
+      // conv inside the same 3x3 neighbourhood. Tap order here must match pack_deconv_weights(): tap = a*2 + b with a
+      // the row choice, b the column choice.
+      p.im2col = 1;
       p.taps = 4;
       p.phases = 4;
       p.oys = p.oxs = 2;
@@ -295,24 +355,13 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
             const int dx = px == 0 ? (b == 0 ? 0 : -1) : (b == 0 ? 1 : 0);
             p.tap_dy[ph * 4 + a * 2 + b] = (signed char)(dy + 1);
             p.tap_dx[ph * 4 + a * 2 + b] = (signed char)(dx + 1);
-            p.tap_dp[ph * 4 + a * 2 + b] = 0;
           }
       }
     }
-    p.cblocks = s.cin_pad / block_k;
-    p.num_m_tiles = (p.M + kBlockM - 1) / kBlockM;
-    p.tw = kBlockM;
-    p.th = 1;
-    p.tiles_x = p.tiles_y = 1;
-    // dims / box describe the A tile for the byte count below; the map itself is built by encode_tmap_im2col_3x3
-    dims[0] = s.cin_pad; dims[1] = p.M; dims[2] = 1; dims[3] = 1; dims[4] = 1;
-    strides[0] = (uint64_t)s.cin_pad * 2;
-    strides[1] = strides[2] = strides[3] = (uint64_t)s.cin_pad * 2 * p.M;
-    box[0] = block_k; box[1] = kBlockM; box[2] = 1; box[3] = 1; box[4] = 1;
-    k_total = p.taps * s.cin_pad;
-  } else if (s.kind == CONV_3x3 || s.kind == CONV_DECONV4 || spatial1) {
+    k_total = p.taps * s.cin_pad + s.cin2_pad;
+  } else {  // spatial tiles: halo-patch or resident-weight 3x3 convs, 1x1 convs with a strided operand
     p.mode = 1;
-    if (s.halo) {
+    if (path.halo) {
       p.tw = kHaloTW;
       p.th = kHaloTH;
     } else {
@@ -324,35 +373,14 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
     p.cblocks = s.cin_pad / block_k;
     if (spatial1) {
       p.taps = 1;
-      p.tap_dx[0] = p.tap_dy[0] = p.tap_dp[0] = 0;
-    } else if (s.kind == CONV_3x3) {
+      p.tap_dx[0] = p.tap_dy[0] = 0;
+    } else {
       p.taps = 9;
       for (int ky = 0; ky < 3; ++ky)
         for (int kx = 0; kx < 3; ++kx) {
           p.tap_dy[ky * 3 + kx] = (signed char)(ky - 1);
           p.tap_dx[ky * 3 + kx] = (signed char)(kx - 1);
-          p.tap_dp[ky * 3 + kx] = 0;
         }
-    } else {
-      // 4x4 stride-2 'SAME' transposed conv: output (2j+py, 2i+px); per axis, phase 0 uses kernel taps {1,3} at
-      // input offsets {0,-1}, phase 1 uses taps {0,2} at offsets {+1,0} (SURVEY.md App. A.2). Tap order here must
-      // match pack_deconv_weights(): tap = a*2 + b with a the row choice, b the column choice.
-      p.taps = 4;
-      p.phases = 4;
-      p.oys = p.oxs = 2;
-      p.OH = 2 * s.H;
-      p.OW = 2 * s.W;
-      for (int ph = 0; ph < 4; ++ph) {
-        const int py = ph >> 1, px = ph & 1;
-        for (int a = 0; a < 2; ++a)
-          for (int b = 0; b < 2; ++b) {
-            const int dy = py == 0 ? (a == 0 ? 0 : -1) : (a == 0 ? 1 : 0);
-            const int dx = px == 0 ? (b == 0 ? 0 : -1) : (b == 0 ? 1 : 0);
-            p.tap_dy[ph * 4 + a * 2 + b] = (signed char)dy;
-            p.tap_dx[ph * 4 + a * 2 + b] = (signed char)dx;
-            p.tap_dp[ph * 4 + a * 2 + b] = 0;
-          }
-      }
     }
     dims[0] = s.cin_pad; dims[1] = (uint64_t)s.W * s.in_stride; dims[2] = (uint64_t)s.H * s.in_stride; dims[3] = 1; dims[4] = s.NB;
     strides[0] = (uint64_t)s.cin_pad * 2;
@@ -360,50 +388,24 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
     strides[2] = strides[1] * dims[2];
     strides[3] = strides[2];
     box[0] = block_k; box[1] = p.tw * s.in_stride; box[2] = p.th * s.in_stride; box[3] = 1; box[4] = 1;
-    if (s.halo) {  // the A box is the whole patch: tile + one pixel of halo on every side
+    if (path.halo) {  // the A box is the whole patch: tile + one pixel of halo on every side
       box[1] = kHaloPW;
       box[2] = kHaloPH;
     }
     k_total = p.taps * s.cin_pad;
-  } else {  // CONV_STEM7
-    p.mode = 1;
-    choose_tile(s.H, s.W, &p.tw, &p.th);
-    p.tiles_x = (s.W + p.tw - 1) / p.tw;
-    p.tiles_y = (s.H + p.th - 1) / p.th;
-    p.num_m_tiles = s.NB * p.tiles_x * p.tiles_y;
-    p.cblocks = 1;
-    p.taps = 7;
-    for (int ky = 0; ky < 7; ++ky) {
-      p.tap_dy[ky] = (signed char)(ky >> 1);
-      p.tap_dx[ky] = 0;
-      p.tap_dp[ky] = (signed char)(ky & 1);
-    }
-    // window of 8 px x 4 ch (32 elements) per output column, consecutive output columns 2 px = 16 B apart
-    dims[0] = 32; dims[1] = s.W; dims[2] = s.stem_rows_per_parity; dims[3] = 2; dims[4] = s.NB;
-    strides[0] = 16;
-    strides[1] = (uint64_t)s.stem_row_pitch * 2;
-    strides[2] = strides[1] * s.stem_rows_per_parity;
-    strides[3] = strides[2] * 2;
-    box[0] = 32; box[1] = p.tw; box[2] = p.th; box[3] = 1; box[4] = 1;
-    k_total = 7 * 32;
   }
-  const int a_stride = (s.kind == CONV_STEM7 || p.im2col) ? 1 : s.in_stride;  // an im2col load is 128 pixels whatever the stride
+  const int a_stride = p.im2col ? 1 : s.in_stride;  // an im2col load is 128 pixels whatever the stride
   // per CTA: its A rows plus its share of the B tile (half of it in a CTA pair; nothing when the weights are resident)
   p.stage_tx_bytes = (uint32_t)(box[0] * (box[1] / a_stride) * (box[2] / a_stride) * 2 +
-                                (s.b_resident ? 0u : (uint32_t)(s.block_n / s.cg) * block_k * 2));
-  if (s.halo) p.stage_tx_bytes = 0;  // patch / weight-tile byte counts are compile-time constants of the HALO kernel
-  if (s.b_resident && (s.cg != 1 || p.num_n_tiles != 1 || p.phases != 1 || s.in2 || k_total / block_k > kMaxResidentKBlocks ||
-                       s.block_n != 64 || s.epi != EPI_TMA || swz != 128)) {
-    if (err) *err = "resident weights need a single-tile 64-column EPI_TMA layer of at most 9 K blocks";
-    return false;
-  }
+                                (path.b_resident ? 0u : (uint32_t)(s.block_n / path.cg) * block_k * 2));
+  if (path.halo) p.stage_tx_bytes = 0;  // patch / weight-tile byte counts are compile-time constants of the HALO kernel
   if (p.im2col) {
     if (!encode_tmap_im2col_3x3(&L->tmap_a, s.in, s.NB, s.H * s.in_stride, s.W * s.in_stride, s.cin_pad, err, s.in_stride)) return false;
-  } else if (!encode_tmap(&L->tmap_a, s.in, 5, dims, strides, box, swz, err, a_stride != 1 ? estr : nullptr)) return false;
+  } else if (!encode_tmap(&L->tmap_a, s.in, 5, dims, strides, box, 128, err, a_stride != 1 ? estr : nullptr)) return false;
   uint64_t bd[2] = {(uint64_t)k_total, (uint64_t)p.phases * s.n_pad};
   uint64_t bs[1] = {(uint64_t)k_total * 2};
-  uint32_t bb[2] = {(uint32_t)block_k, (uint32_t)(s.block_n / s.cg)};
-  if (!encode_tmap(&L->tmap_b, s.w, 2, bd, bs, bb, swz, err)) return false;
+  uint32_t bb[2] = {(uint32_t)block_k, (uint32_t)(s.block_n / path.cg)};
+  if (!encode_tmap(&L->tmap_b, s.w, 2, bd, bs, bb, 128, err)) return false;
   L->tmap_out = L->tmap_a;  // placeholders for the epilogues that do not use them
   L->tmap_res = L->tmap_a;
   L->tmap_a2 = L->tmap_a;
@@ -415,15 +417,15 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
     uint64_t d2[5] = {(uint64_t)s.cin2_pad, (uint64_t)p.M, 1, 1, 1};
     uint64_t s2[4] = {(uint64_t)s.cin2_pad * 2, (uint64_t)s.cin2_pad * 2 * p.M, (uint64_t)s.cin2_pad * 2 * p.M,
                       (uint64_t)s.cin2_pad * 2 * p.M};
-    if (!encode_tmap(&L->tmap_a2, s.in2, 5, d2, s2, box, swz, err)) return false;
+    if (!encode_tmap(&L->tmap_a2, s.in2, 5, d2, s2, box, 128, err)) return false;
   }
-  if (s.epi == EPI_PLANAR_F32 && (p.mode != 0 || s.decimate || (s.H * s.W) % 4 != 0)) {
+  if (s.epi == EPI_PLANAR_F32 && (p.mode != 0 || (s.H * s.W) % 4 != 0)) {
     if (err) *err = "the planar epilogue needs a flat 1x1 conv whose plane size is a multiple of 4";
     return false;
   }
   if (s.epi == EPI_TMA || s.epi == EPI_TMA_RES) {
     // output (and residual) tiles leave / enter through swizzled smem in 64-channel chunks: same row tiling as A
-    if (s.decimate || s.kind == CONV_DECONV4 || s.ldc % 8 != 0) {
+    if (s.kind == CONV_DECONV4 || s.ldc % 8 != 0) {
       if (err) *err = "TMA epilogue needs a plain NHWC output";
       return false;
     }
@@ -446,9 +448,8 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
     L->tmap_out2 = L->tmap_out;
     L->tmap_w2 = L->tmap_b;
     if (s.out2 != nullptr) {
-      if (s.block_n != kTailBlockN || s.cg != 2 || s.kind != CONV_1x1 || (s.n2 != 64 && s.n2 != 128 && s.n2 != 256) ||
-          !s.w2 || !s.bias2 || s.n_pad % kTailBlockN != 0 || s.b_resident || s.halo) {
-        if (err) *err = "a fused block tail needs a 1x1 conv on CTA pairs with 256-column tiles and a 64/128/256-wide second conv";
+      if (s.block_n != kTailBlockN || s.kind != CONV_1x1 || p.mode != 0 || !tail_supported(s.n2, s.epi) || !s.w2 || !s.bias2) {
+        if (err) *err = "a fused block tail needs a flat 1x1 conv with 256-column tiles and a 64-wide (EPI_TMA) or 128-wide (EPI_TMA_RES) second conv";
         return false;
       }
       if (!act_map(s.out2, s.n2, &L->tmap_out2, 1)) return false;
@@ -467,12 +468,24 @@ inline bool build_conv(const ConvSpec& s, int num_sms, ConvLaunch* L, std::strin
       if (!act_map(s.residual, s.ldr, &L->tmap_res, s.res_stride)) return false;
       p.res_tx_bytes = (ob[1] / s.res_stride) * (ob[2] / s.res_stride) * 128;
     }
+  } else if (s.residual) {
+    if (err) *err = "only the EPI_TMA_RES epilogue adds a residual";
+    return false;
   }
   if (s.out2 != nullptr && L->n2 == 0) {
     if (err) *err = "a fused block tail needs a TMA epilogue";
     return false;
   }
-  L->grid = L->n2 ? tail_grid(p, num_sms) : conv_grid(p, s.cg, num_sms);
+  if (L->n2 == 0 && find_conv_kernel(*L).fn == nullptr) {
+    if (err) {
+      char buf[160];
+      snprintf(buf, sizeof buf, "no conv kernel for a %d-column tile with epilogue %d (cg %d, resident %d, halo %d)", s.block_n,
+               s.epi, path.cg, path.b_resident, path.halo);
+      *err = buf;
+    }
+    return false;
+  }
+  L->grid = L->n2 ? tail_grid(p, num_sms) : conv_grid(p, path.cg, num_sms);
   L->flops = 2.0 * p.phases * (double)p.M * s.n_pad * k_total + 2.0 * (double)p.M * s.n_pad * L->n2;
   return true;
 }
@@ -506,51 +519,6 @@ inline cudaError_t launch_pdl(Kern kern, dim3 grid, dim3 block, size_t smem, cud
   return launch_pdl_cluster(kern, grid, block, smem, st, 1, args...);
 }
 
-// cudaFuncSetAttribute is per device (context): remember, per kernel instantiation, which devices of this process
-// already carry the opt-in.  One bit per device ordinal; a process holds at most one handle per GPU of an 8-GPU box.
-template <typename Kern>
-inline cudaError_t ensure_dyn_smem(Kern kern, int bytes, unsigned long long* done_mask) {
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  const unsigned long long bit = 1ull << (dev & 63);
-  if (__atomic_load_n(done_mask, __ATOMIC_ACQUIRE) & bit) return cudaSuccess;
-  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e != cudaSuccess) return e;
-  __atomic_fetch_or(done_mask, bit, __ATOMIC_RELEASE);
-  return cudaSuccess;
-}
-
-template <int BLOCK_N, int SWZ, int EPI, int CG = 1>
-inline cudaError_t launch_one(const ConvLaunch& L, cudaStream_t st) {
-  using Cfg = GemmCfg<BLOCK_N, SWZ, EPI, CG>;
-  static unsigned long long done = 0;
-  auto kern = conv_gemm_kernel<BLOCK_N, SWZ, EPI, CG>;
-  if (cudaError_t e = ensure_dyn_smem(kern, Cfg::SMEM_BYTES, &done); e != cudaSuccess) return e;
-  return launch_pdl_cluster(kern, dim3(L.grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, CG, L.tmap_a, L.tmap_b,
-                            L.tmap_out, L.tmap_res, L.tmap_a2, L.p);
-}
-
-template <int BLOCK_N, int SWZ, int EPI>
-inline cudaError_t launch_one_bres(const ConvLaunch& L, cudaStream_t st) {
-  using Cfg = GemmCfg<BLOCK_N, SWZ, EPI, 1, true>;
-  static unsigned long long done = 0;
-  auto kern = conv_gemm_kernel<BLOCK_N, SWZ, EPI, 1, true>;
-  if (cudaError_t e = ensure_dyn_smem(kern, Cfg::SMEM_BYTES, &done); e != cudaSuccess) return e;
-  return launch_pdl(kern, dim3(L.grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, L.tmap_a, L.tmap_b, L.tmap_out,
-                    L.tmap_res, L.tmap_a2, L.p);
-}
-
-template <int BLOCK_N, int CG, bool BRES>
-inline cudaError_t launch_one_halo(const ConvLaunch& L, cudaStream_t st) {
-  using Cfg = GemmCfg<BLOCK_N, 128, EPI_TMA, CG, BRES, true>;
-  static unsigned long long done = 0;
-  auto kern = conv_gemm_kernel<BLOCK_N, 128, EPI_TMA, CG, BRES, true>;
-  if (cudaError_t e = ensure_dyn_smem(kern, Cfg::SMEM_BYTES, &done); e != cudaSuccess) return e;
-  return launch_pdl_cluster(kern, dim3(L.grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, st, CG, L.tmap_a, L.tmap_b,
-                            L.tmap_out, L.tmap_res, L.tmap_a2, L.p);
-}
-
 template <int N2, bool RES>
 inline cudaError_t launch_one_tail(const ConvLaunch& L, cudaStream_t st) {
   using Cfg = TailCfg<N2, RES>;
@@ -567,57 +535,15 @@ inline cudaError_t launch_one_tail(const ConvLaunch& L, cudaStream_t st) {
 
 inline cudaError_t launch_conv(const ConvLaunch& L, cudaStream_t st) {
   if (L.n2) {
-    const bool res = L.epi == EPI_TMA_RES;
-    if (L.n2 == 64) return res ? launch_one_tail<64, true>(L, st) : launch_one_tail<64, false>(L, st);
-    if (L.n2 == 128) return res ? launch_one_tail<128, true>(L, st) : launch_one_tail<128, false>(L, st);
-    if (L.n2 == 256) return res ? launch_one_tail<256, true>(L, st) : launch_one_tail<256, false>(L, st);
+    if (L.n2 == 64 && L.epi == EPI_TMA) return launch_one_tail<64, false>(L, st);
+    if (L.n2 == 128 && L.epi == EPI_TMA_RES) return launch_one_tail<128, true>(L, st);
     return cudaErrorInvalidConfiguration;
   }
-  if (L.halo) {
-    if (L.b_resident) return launch_one_halo<64, 1, true>(L, st);
-    if (L.block_n == 128 && L.cg == 2) return launch_one_halo<128, 2, false>(L, st);
-    if (L.block_n == 128 && L.cg == 1) return launch_one_halo<128, 1, false>(L, st);
-    if (L.block_n == 64 && L.cg == 1) return launch_one_halo<64, 1, false>(L, st);
-    return cudaErrorInvalidConfiguration;
-  }
-  if (L.b_resident) return launch_one_bres<64, 128, EPI_TMA>(L, st);
-  if (L.cg == 2) {  // CTA pairs: the production epilogues only
-    if (L.swz != 128) return cudaErrorInvalidConfiguration;
-    if (L.epi == EPI_TMA) {
-      if (L.block_n == 64) return launch_one<64, 128, EPI_TMA, 2>(L, st);
-      if (L.block_n == 128) return launch_one<128, 128, EPI_TMA, 2>(L, st);
-      if (L.block_n == 256) return launch_one<256, 128, EPI_TMA, 2>(L, st);
-    }
-    if (L.epi == EPI_TMA_RES) {
-      if (L.block_n == 64) return launch_one<64, 128, EPI_TMA_RES, 2>(L, st);
-      if (L.block_n == 128) return launch_one<128, 128, EPI_TMA_RES, 2>(L, st);
-      if (L.block_n == 256) return launch_one<256, 128, EPI_TMA_RES, 2>(L, st);
-    }
-    if (L.epi == EPI_PLANAR_F32 && L.block_n == 96) return launch_one<96, 128, EPI_PLANAR_F32, 2>(L, st);
-    if (L.epi == EPI_DECONV_HEAD && L.block_n == 192) return launch_one<192, 128, EPI_DECONV_HEAD, 2>(L, st);
-    return cudaErrorInvalidConfiguration;
-  }
-  if (L.swz == 64 && L.block_n == 64 && L.epi == EPI_NHWC_F16) return launch_one<64, 64, EPI_NHWC_F16>(L, st);
-  if (L.swz == 128 && L.epi == EPI_NHWC_F16) {
-    if (L.block_n == 64) return launch_one<64, 128, EPI_NHWC_F16>(L, st);
-    if (L.block_n == 128) return launch_one<128, 128, EPI_NHWC_F16>(L, st);
-    if (L.block_n == 256) return launch_one<256, 128, EPI_NHWC_F16>(L, st);
-  }
-  if (L.swz == 64 && L.block_n == 64 && L.epi == EPI_TMA) return launch_one<64, 64, EPI_TMA>(L, st);
-  if (L.swz == 128 && L.epi == EPI_TMA) {
-    if (L.block_n == 64) return launch_one<64, 128, EPI_TMA>(L, st);
-    if (L.block_n == 128) return launch_one<128, 128, EPI_TMA>(L, st);
-    if (L.block_n == 256) return launch_one<256, 128, EPI_TMA>(L, st);
-  }
-  if (L.swz == 128 && L.epi == EPI_TMA_RES) {
-    if (L.block_n == 64) return launch_one<64, 128, EPI_TMA_RES>(L, st);
-    if (L.block_n == 128) return launch_one<128, 128, EPI_TMA_RES>(L, st);
-    if (L.block_n == 256) return launch_one<256, 128, EPI_TMA_RES>(L, st);
-  }
-  if (L.swz == 128 && L.epi == EPI_PLANAR_F32 && L.block_n == 96) return launch_one<96, 128, EPI_PLANAR_F32>(L, st);
-  if (L.swz == 128 && L.epi == EPI_DECONV_HEAD && L.block_n == 192)
-    return launch_one<192, 128, EPI_DECONV_HEAD>(L, st);
-  return cudaErrorInvalidConfiguration;
+  const ConvKernel k = find_conv_kernel(L);
+  if (k.fn == nullptr) return cudaErrorInvalidConfiguration;
+  if (cudaError_t e = ensure_dyn_smem(k.fn, k.smem, k.smem_done); e != cudaSuccess) return e;
+  return launch_pdl_cluster(k.fn, dim3(L.grid), dim3(k.threads), k.smem, st, k.cg, L.tmap_a, L.tmap_b, L.tmap_out,
+                            L.tmap_res, L.tmap_a2, L.p);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -695,10 +621,11 @@ inline void stem_roll_set_batch(StemRollParams& r, int nb, int num_sms, int* gri
   if (*grid == 0) *grid = 1;
 }
 
-// w_pair: pack_stem_pair's tables (or nullptr: single CTAs only); x1_halves: allocated size of the stem input
+// w_pair: pack_stem_pair's tables, used when the box splits into two x tiles (CTA pairs); x1_halves: allocated size of
+// the stem input
 inline bool build_stem_pool(const __half* x1, int S, int rows_per_parity, int row_pitch, const __half* w_stacked,
                             const float* bias, __half* pooled_out, int nb, int num_sms, StemPoolLaunch* L,
-                            std::string* err, const __half* w_pair = nullptr, size_t x1_halves = 0) {
+                            std::string* err, const __half* w_pair, size_t x1_halves) {
   memset(L, 0, sizeof(*L));
   L->cg = 1;
   StemRollParams& r = L->r;
@@ -729,8 +656,7 @@ inline bool build_stem_pool(const __half* x1, int S, int rows_per_parity, int ro
     ++r.n_xt;
     pb = pe;
   }
-  static const bool pairs_on = [] { const char* e = getenv("VNECT_B200_STEM_PAIRS"); return !(e && atoi(e) == 0); }();
-  if (pairs_on && w_pair != nullptr && r.n_xt == 2 && x1_halves >= 8 && num_sms >= 2) {
+  if (r.n_xt == 2 && x1_halves >= 8 && num_sms >= 2) {
     const uint64_t dims[2] = {8, (uint64_t)(x1_halves / 8)};
     const uint64_t strides[1] = {16};
     const uint32_t box[2] = {8, (uint32_t)(kRollStripLoad / 16)};
@@ -745,14 +671,15 @@ inline bool build_stem_pool(const __half* x1, int S, int rows_per_parity, int ro
 
 inline void stem_pool_set_batch(StemPoolLaunch& L, int nb, int num_sms) { stem_roll_set_batch(L.r, nb, num_sms, &L.grid); }
 
+// DBG = true: the cycle-counter variant (stem_roll.cuh), launched by the self-test only
+template <bool DBG = false>
 inline cudaError_t launch_stem_pool(const StemPoolLaunch& L, cudaStream_t st) {
-  static unsigned long long done[4] = {0, 0, 0, 0};
+  static unsigned long long done[2] = {0, 0};
   auto go = [&](auto kern, unsigned long long* mask) -> cudaError_t {
     if (cudaError_t e = ensure_dyn_smem(kern, StemRollSmem::BYTES, mask); e != cudaSuccess) return e;
     return launch_pdl_cluster(kern, dim3(L.grid), dim3(kRollThreads), StemRollSmem::BYTES, st, L.cg, L.r, L.tmap_x);
   };
-  if (L.cg == 2) return L.r.dbg != nullptr ? go(stem_roll_kernel<true, 2>, &done[3]) : go(stem_roll_kernel<false, 2>, &done[2]);
-  return L.r.dbg != nullptr ? go(stem_roll_kernel<true, 1>, &done[1]) : go(stem_roll_kernel<false, 1>, &done[0]);
+  return L.cg == 2 ? go(stem_roll_kernel<DBG, 2>, &done[1]) : go(stem_roll_kernel<DBG, 1>, &done[0]);
 }
 
 }  // namespace vnect

@@ -20,7 +20,8 @@ using namespace vnect;
   } while (0)
 
 struct NaiveGeom {
-  int kind, NB, H, W, cin_pad, n_pad, taps, phases, k_total;
+  int NB, H, W, cin_pad, n_pad, taps, phases, k_total;
+  int stem;  // 1: the 7x7/2 stem conv on the parity-split padded input [NB][2][stem_rpp][stem_pitch], row taps dy / dp
   int stem_rpp, stem_pitch;
   int in_stride;
   signed char dx[16], dy[16], dp[16];
@@ -44,7 +45,7 @@ __global__ void naive_acc_kernel(const __half* __restrict__ in, const __half* __
     float s = 0.f;
     for (int t = 0; t < g.taps; ++t) {
       const int ti = ph * g.taps + t;
-      if (g.kind == CONV_STEM7) {
+      if (g.stem) {
         const int row = y + g.dy[ti];
         if (row < 0 || row >= g.stem_rpp) continue;
         const __half* a = in + (((size_t)n * 2 + g.dp[ti]) * g.stem_rpp + row) * g.stem_pitch + (size_t)x * 8;
@@ -71,18 +72,16 @@ static float frand() {
   return ((rng_state >> 8) & 0xFFFF) / 32768.0f - 1.0f;
 }
 
+// build_conv picks the kernel path (CTA pairs, resident weights, halo patches, im2col) from the shape, block_n and
+// epilogue, as it does for the library's plans; every result line names the path taken
 struct Case {
   const char* name;
   int kind, NB, H, W, cin_pad, n_pad, n_valid, block_n, epi;
   bool bias, residual;
-  int relu_cols, decimate;
+  int relu_cols;
   int in_stride = 1, res_stride = 1;
   int cin2 = 0;  // folded shortcut: second input tensor with cin2 channels (1x1 only)
-  int cg = 1;    // 2: CTA pairs (tcgen05 cta_group::2)
-  int bres = 0;  // 1: weights resident in smem
-  int halo = 0;  // 1: 3x3 conv through halo patches (8 x 16 pixel tiles, nine taps read one smem patch)
   int n2 = 0;    // > 0: fused block tail, second 1x1 conv of n2 channels on this conv's output (block_tail.cuh)
-  int im2col = 0;  // 1: 3x3 conv on flat pixel rows through an im2col tensor map
 };
 
 // reference of the chained conv, from the fp16 X the kernel under test wrote: y[m][col] = relu(sum_c X[m][c] * W2[col][c] + b2[col])
@@ -112,27 +111,12 @@ static int run_case(const Case& c, int num_sms, bool timing) {
   s.block_n = c.block_n;
   s.epi = c.epi;
   s.relu_cols = c.relu_cols;
-  s.decimate = c.decimate;
   s.in_stride = c.in_stride;
   s.res_stride = c.res_stride;
-  s.cg = c.cg;
-  s.b_resident = c.bres;
-  s.halo = c.halo;
-  s.im2col = c.im2col;
   const int phases = c.kind == CONV_DECONV4 ? 4 : 1;
-  const int taps = c.kind == CONV_1x1 ? 1 : c.kind == CONV_3x3 ? 9 : c.kind == CONV_DECONV4 ? 4 : 7;
-  const int k_total = c.kind == CONV_STEM7 ? 7 * 32 : taps * c.cin_pad + c.cin2;
-  size_t in_elems;
-  int rpp = 0, pitch = 0;
-  if (c.kind == CONV_STEM7) {
-    rpp = c.H + 3;
-    pitch = (2 * c.W + 6) * 4;
-    in_elems = (size_t)c.NB * 2 * rpp * pitch;
-    s.stem_rows_per_parity = rpp;
-    s.stem_row_pitch = pitch;
-  } else {
-    in_elems = (size_t)c.NB * c.H * c.W * c.cin_pad * c.in_stride * c.in_stride;
-  }
+  const int taps = c.kind == CONV_1x1 ? 1 : c.kind == CONV_3x3 ? 9 : 4;
+  const int k_total = taps * c.cin_pad + c.cin2;
+  const size_t in_elems = (size_t)c.NB * c.H * c.W * c.cin_pad * c.in_stride * c.in_stride;
   std::vector<__half> h_in(in_elems), h_w((size_t)phases * c.n_pad * k_total);
   for (auto& v : h_in) v = __float2half(frand());
   const float wscale = 1.0f / sqrtf((float)k_total);
@@ -142,7 +126,6 @@ static int run_case(const Case& c, int num_sms, bool timing) {
 
   int OH = c.H, OW = c.W;
   if (c.kind == CONV_DECONV4) { OH = 2 * c.H; OW = 2 * c.W; }
-  if (c.decimate) { OH = c.H / 2; OW = c.W / 2; }
   const int ldc = c.epi == EPI_DECONV_HEAD ? 256 : c.n_pad;
   const size_t out_elems = c.epi == EPI_PLANAR_F32 ? (size_t)c.NB * c.n_valid * OH * OW : (size_t)c.NB * OH * OW * ldc;
   const size_t out_bytes = out_elems * (c.epi == EPI_PLANAR_F32 ? 4 : 2);
@@ -218,10 +201,11 @@ static int run_case(const Case& c, int num_sms, bool timing) {
   }
 
   NaiveGeom g;
-  g.kind = c.kind; g.NB = c.NB; g.H = c.H; g.W = c.W; g.cin_pad = c.cin_pad; g.n_pad = c.n_pad;
+  memset(&g, 0, sizeof g);
+  g.NB = c.NB; g.H = c.H; g.W = c.W; g.cin_pad = c.cin_pad; g.n_pad = c.n_pad;
   g.in_stride = c.in_stride;
-  g.taps = taps; g.phases = phases; g.k_total = k_total; g.stem_rpp = rpp; g.stem_pitch = pitch;
-  memcpy(g.dx, L.p.tap_dx, 16); memcpy(g.dy, L.p.tap_dy, 16); memcpy(g.dp, L.p.tap_dp, 16);
+  g.taps = taps; g.phases = phases; g.k_total = k_total;
+  memcpy(g.dx, L.p.tap_dx, 16); memcpy(g.dy, L.p.tap_dy, 16);
   if (L.p.im2col)  // the launch holds filter offsets from the base pixel (0..2); the reference wants displacements (-1..1)
     for (int t = 0; t < 16; ++t) { g.dx[t] = (signed char)(g.dx[t] - 1); g.dy[t] = (signed char)(g.dy[t] - 1); }
   naive_acc_kernel<<<1184, 256>>>(d_in, d_w, d_acc, g, d_in2, c.cin2);
@@ -252,10 +236,7 @@ static int run_case(const Case& c, int num_sms, bool timing) {
           const size_t m = ((size_t)n * c.H + y) * c.W + x;
           const float* a = &h_acc[((size_t)ph * c.NB * c.H * c.W + m) * c.n_pad];
           int oy, ox;
-          if (c.decimate) {
-            if ((y | x) & 1) continue;
-            oy = y / 2; ox = x / 2;
-          } else if (c.kind == CONV_DECONV4) {
+          if (c.kind == CONV_DECONV4) {
             oy = 2 * y + (ph >> 1); ox = 2 * x + (ph & 1);
           } else {
             oy = y; ox = x;
@@ -296,12 +277,12 @@ static int run_case(const Case& c, int num_sms, bool timing) {
     for (size_t i = 0; i < h_y.size(); ++i) check(__half2float(h_o2[i]), h_y[i]);
     cudaFree(d_y);
   }
-  printf("[%s] tiles=%d grid=%d tile=%dx%d checked=%lld bad=%lld max_abs_err=%.3e  %s\n", c.name,
-         L.p.phases * L.p.num_m_tiles * L.p.num_n_tiles, L.grid, L.p.tw, L.p.th, checked, bad, max_err,
+  printf("[%s] path=%s%s%s%sn%d/cg%d tiles=%d grid=%d tile=%dx%d checked=%lld bad=%lld max_abs_err=%.3e  %s\n", c.name,
+         L.n2 ? "tail " : "", L.b_resident ? "resident " : "", L.halo ? "halo " : "", L.p.im2col ? "im2col " : "",
+         L.block_n, L.cg, L.p.phases * L.p.num_m_tiles * L.p.num_n_tiles, L.grid, L.p.tw, L.p.th, checked, bad, max_err,
          bad == 0 ? "PASS" : "FAIL");
 
-  static const bool time_anyway = getenv("VNECT_SELFTEST_TIME_ANYWAY") != nullptr;  // experiment builds are wrong by design
-  if (timing && (bad == 0 || time_anyway)) {
+  if (timing && bad == 0) {
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
@@ -361,7 +342,7 @@ static int run_stem_pool(int NB, int S, int num_sms) {
   CK(cudaMalloc(&d_dbg, 8 * sizeof(unsigned long long)));
   CK(cudaMemset(d_dbg, 0, 8 * sizeof(unsigned long long)));
   L.r.dbg = d_dbg;
-  CK(launch_stem_pool(L, 0));
+  CK(launch_stem_pool<true>(L, 0));
   cudaError_t se = cudaDeviceSynchronize();
   if (se != cudaSuccess) {
     printf("[stem_pool] kernel FAILED: %s\n", cudaGetErrorString(se));
@@ -369,7 +350,7 @@ static int run_stem_pool(int NB, int S, int num_sms) {
   }
   NaiveGeom g;
   memset(&g, 0, sizeof g);
-  g.kind = CONV_STEM7; g.NB = NB; g.H = OH; g.W = OH; g.n_pad = 64; g.taps = 7; g.phases = 1;
+  g.stem = 1; g.NB = NB; g.H = OH; g.W = OH; g.n_pad = 64; g.taps = 7; g.phases = 1;
   g.k_total = 224; g.stem_rpp = rpp; g.stem_pitch = pitch; g.in_stride = 1;
   for (int ky = 0; ky < 7; ++ky) { g.dy[ky] = (signed char)(ky >> 1); g.dx[ky] = 0; g.dp[ky] = (signed char)(ky & 1); }
   const size_t acc_elems = (size_t)NB * OH * OH * 64;
@@ -554,7 +535,7 @@ int main(int argc, char** argv) {
     run_desc_probe();
     return 0;
   }
-  if (argc > 1 && strcmp(argv[1], "stem") == 0) {  // the fused conv1 + pool1 kernel only (VNECT_B200_STEM_PAIRS=0: single CTAs)
+  if (argc > 1 && strcmp(argv[1], "stem") == 0) {  // the fused conv1 + pool1 kernel only
     int f = 0;
     f += run_stem_pool(2, 368, sms);
     f += run_stem_pool(3, 448, sms);
@@ -565,149 +546,69 @@ int main(int argc, char** argv) {
     printf(f ? "SELFTEST FAILED (%d failing cases)\n" : "SELFTEST PASSED (%d failing cases)\n", f);
     return f ? 1 : 0;
   }
-  if (argc > 1 && strcmp(argv[1], "im2col") == 0) {  // 3x3 convs at 23 x 23 on flat pixel rows (im2col tensor map) against spatial tiles
-    Case a = {"IM2COL 3x3 256->256 relu 23x23 n64", CONV_3x3, 3, 23, 23, 256, 256, 256, 64, EPI_TMA, true, false, 256, 0};
-    Case b = {"IM2COL PAIR 3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256, 0};
-    Case c = {"IM2COL PAIR 3x3 512->512 relu 23x23 (odd tile count)", CONV_3x3, 5, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512, 0};
-    Case d = {"IM2COL 3x3 64->64 relu 13x9 n64", CONV_3x3, 2, 13, 9, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    Case e0 = {"BIG PAIR 3x3 256->256 23x23 nb128 (spatial tiles)", CONV_3x3, 128, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256, 0};
-    Case e1 = {"BIG IM2COL PAIR 3x3 256->256 23x23 nb128", CONV_3x3, 128, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256, 0};
-    Case f0 = {"BIG PAIR 3x3 512->512 23x23 nb128 (spatial tiles)", CONV_3x3, 128, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512, 0};
-    Case f1 = {"BIG IM2COL PAIR 3x3 512->512 23x23 nb128", CONV_3x3, 128, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512, 0};
-    Case i0 = {"S2 3x3 64->64 relu 92->46 (spatial tiles)", CONV_3x3, 2, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case i1 = {"IM2COL S2 3x3 64->64 relu 92->46", CONV_3x3, 2, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case i2 = {"IM2COL S2 3x3 128->128 relu 46->23", CONV_3x3, 3, 23, 23, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0, 2, 1};
-    Case j0 = {"BIG S2 3x3 64->64 92->46 nb128 (spatial tiles)", CONV_3x3, 128, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case j1 = {"BIG IM2COL S2 3x3 64->64 92->46 nb128", CONV_3x3, 128, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case j2 = {"BIG S2 PAIR 3x3 128->128 46->23 nb128 (spatial tiles)", CONV_3x3, 128, 23, 23, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0, 2, 1};
-    Case j3 = {"BIG IM2COL S2 PAIR 3x3 128->128 46->23 nb128", CONV_3x3, 128, 23, 23, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0, 2, 1};
-    Case j4 = {"BIG BRES S2 3x3 64->64 92->46 nb128 (spatial tiles, resident weights)", CONV_3x3, 128, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case j5 = {"BIG IM2COL BRES S2 3x3 64->64 92->46 nb128", CONV_3x3, 128, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case k0 = {"BIG HALO PAIR 3x3 256->128 46x46 nb128 (head)", CONV_3x3, 128, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case k1 = {"BIG IM2COL PAIR 3x3 256->128 46x46 nb128 (head)", CONV_3x3, 128, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case k2 = {"BIG HALO PAIR 3x3 128->128 46x46 nb128", CONV_3x3, 128, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case k3 = {"BIG IM2COL PAIR 3x3 128->128 46x46 nb128", CONV_3x3, 128, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    k0.halo = k2.halo = 1; k1.im2col = k3.im2col = 1;
-    k0.cg = k1.cg = k2.cg = k3.cg = 2;
-    i1.im2col = i2.im2col = j1.im2col = j3.im2col = j5.im2col = 1;
-    j2.cg = j3.cg = 2;
-    j4.bres = j5.bres = 1;
-    Case g0 = {"deconv4x4s2 256->192 head 23x23 (spatial tiles)", CONV_DECONV4, 3, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    Case g1 = {"IM2COL deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 3, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    Case h0 = {"BIG PAIR deconv4x4s2 256->192 head 23x23 nb128 (spatial tiles)", CONV_DECONV4, 128, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    Case h1 = {"BIG IM2COL PAIR deconv4x4s2 256->192 head 23x23 nb128", CONV_DECONV4, 128, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    a.im2col = b.im2col = c.im2col = d.im2col = e1.im2col = f1.im2col = g1.im2col = h1.im2col = 1;
-    b.cg = c.cg = e0.cg = e1.cg = f0.cg = f1.cg = h0.cg = h1.cg = 2;
-    int f = 0;
-    for (Case* k : {&a, &b, &c, &d, &e0, &e1, &f0, &f1, &g0, &g1, &h0, &h1, &i0, &i1, &i2, &j0, &j1, &j2, &j3, &j4, &j5, &k0, &k1, &k2, &k3}) f += run_case(*k, sms, true);
-    printf(f ? "SELFTEST FAILED (%d failing cases)\n" : "SELFTEST PASSED (%d failing cases)\n", f);
-    return f ? 1 : 0;
-  }
-  if (argc > 1 && strcmp(argv[1], "epi") == 0) {  // the epilogue-bound 1x1 layers only (experiment builds)
-    Case a = {"EPI TMARES 1x1 256->1024 +res 23x23 nb128", CONV_1x1, 128, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0};
-    Case b = {"EPI TMARES 1x1 128->512 +res 46x46 nb128", CONV_1x1, 128, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0};
-    Case c = {"EPI TMARES 1x1 64->256 +res 92x92 nb128", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0};
-    Case d = {"EPI TMA 1x1 1024->256 23x23 nb128", CONV_1x1, 128, 23, 23, 1024, 256, 256, 256, EPI_TMA, true, false, 256, 0};
-    a.cg = b.cg = c.cg = d.cg = 2;
-    for (Case* k : {&a, &b, &c, &d}) run_case(*k, prop.multiProcessorCount, true);
-    return 0;
-  }
+  // single-CTA tiles are 64 columns wide, as on the latency plans; the PAIR loop below reruns every TMA-epilogue case
+  // with the throughput plans' tile (256 columns from Cout 256, else 128) on CTA pairs
   std::vector<Case> cases = {
-      {"1x1 64->64 relu 92x92", CONV_1x1, 2, 92, 92, 64, 64, 64, 64, EPI_NHWC_F16, true, false, 64, 0},
-      {"1x1 256->512 +res relu 46x46", CONV_1x1, 4, 46, 46, 256, 512, 512, 256, EPI_NHWC_F16, true, true, 512, 0},
-      {"1x1 1024->256 relu 23x23 bn128", CONV_1x1, 8, 23, 23, 1024, 256, 256, 128, EPI_NHWC_F16, true, false, 256, 0},
-      {"1x1 64->256 +res relu decimate", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_NHWC_F16, true, true, 256, 1},
-      {"3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_NHWC_F16, true, false, 64, 0},
-      {"3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 128, EPI_NHWC_F16, true, false, 256, 0},
-      {"3x3 128->128 relu 46x46", CONV_3x3, 1, 46, 46, 128, 128, 128, 128, EPI_NHWC_F16, true, false, 128, 0},
-      {"TMA 1x1 64->64 relu 92x92", CONV_1x1, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-      {"TMA 1x1 64->256 lin 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 0, 0},
-      {"TMARES 1x1 64->256 +res relu 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0},
-      {"TMARES 1x1 256->1024 +res relu 23x23", CONV_1x1, 7, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0},
-      {"TMARES 1x1 128->512 +res relu 46x46 bn128", CONV_1x1, 3, 46, 46, 128, 512, 512, 128, EPI_TMA_RES, true, true, 512, 0},
-      {"TMA 3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-      {"TMA 3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 128, EPI_TMA, true, false, 256, 0},
-      {"TMA 3x3 128->128 relu 46x46", CONV_3x3, 1, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0},
-      {"TMA stem 7x7s2 3->64 relu 184x184", CONV_STEM7, 2, 184, 184, 0, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-      {"S2 3x3 64->64 relu 92->46", CONV_3x3, 2, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1},
-      {"S2 3x3 128->128 relu 46->23", CONV_3x3, 3, 23, 23, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0, 2, 1},
-      {"S2RES 1x1 64->256 +res(92) relu 46x46", CONV_1x1, 2, 46, 46, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0, 1, 2},
-      {"S2RES 1x1 128->512 +res(46) relu 23x23", CONV_1x1, 3, 23, 23, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0, 1, 2},
-      {"FOLD 1x1 64(+64)->256 relu 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 256, 0, 1, 1, 64},
-      {"FOLD 1x1 128(+256)->512 relu 46x46", CONV_1x1, 3, 46, 46, 128, 512, 512, 256, EPI_TMA, true, false, 512, 0, 1, 1, 256},
-      {"FOLD 1x1 512(+1024)->1024 relu 23x23", CONV_1x1, 5, 23, 23, 512, 1024, 1024, 256, EPI_TMA, true, false, 1024, 0, 1, 1, 1024},
-      {"deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 2, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false,
-       128, 0},
-      {"1x1 128->84 planar f32 46x46", CONV_1x1, 2, 46, 46, 128, 96, 84, 96, EPI_PLANAR_F32, false, false, 0, 0},
-      {"stem 7x7s2 3->64 relu 184x184", CONV_STEM7, 2, 184, 184, 0, 64, 64, 64, EPI_NHWC_F16, true, false, 64, 0},
+      {"1x1 64->64 relu 92x92", CONV_1x1, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64},
+      {"1x1 64->256 lin 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 64, EPI_TMA, true, false, 0},
+      {"TMARES 1x1 64->256 +res relu 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 64, EPI_TMA_RES, true, true, 256},
+      {"TMARES 1x1 256->1024 +res relu 23x23", CONV_1x1, 7, 23, 23, 256, 1024, 1024, 64, EPI_TMA_RES, true, true, 1024},
+      {"TMARES 1x1 128->512 +res relu 46x46", CONV_1x1, 3, 46, 46, 128, 512, 512, 64, EPI_TMA_RES, true, true, 512},
+      {"3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64},
+      {"3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 64, EPI_TMA, true, false, 256},
+      {"3x3 128->128 relu 46x46", CONV_3x3, 1, 46, 46, 128, 128, 128, 64, EPI_TMA, true, false, 128},
+      {"3x3 256->128 relu 23x23", CONV_3x3, 3, 23, 23, 256, 128, 128, 64, EPI_TMA, true, false, 128},
+      {"S2 3x3 64->64 relu 92->46", CONV_3x3, 2, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 2, 1},
+      {"S2 3x3 128->128 relu 46->23", CONV_3x3, 3, 23, 23, 128, 128, 128, 64, EPI_TMA, true, false, 128, 2, 1},
+      {"S2RES 1x1 64->256 +res(92) relu 46x46", CONV_1x1, 2, 46, 46, 64, 256, 256, 64, EPI_TMA_RES, true, true, 256, 1, 2},
+      {"S2RES 1x1 128->512 +res(46) relu 23x23", CONV_1x1, 3, 23, 23, 128, 512, 512, 64, EPI_TMA_RES, true, true, 512, 1, 2},
+      {"FOLD 1x1 64(+64)->256 relu 92x92", CONV_1x1, 2, 92, 92, 64, 256, 256, 64, EPI_TMA, true, false, 256, 1, 1, 64},
+      {"FOLD 1x1 128(+256)->512 relu 46x46", CONV_1x1, 3, 46, 46, 128, 512, 512, 64, EPI_TMA, true, false, 512, 1, 1, 256},
+      {"FOLD 1x1 512(+1024)->1024 relu 23x23", CONV_1x1, 5, 23, 23, 512, 1024, 1024, 64, EPI_TMA, true, false, 1024, 1, 1, 1024},
+      {"deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 2, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128},
+      {"1x1 128->84 planar f32 46x46", CONV_1x1, 2, 46, 46, 128, 96, 84, 96, EPI_PLANAR_F32, false, false, 0},
   };
   int fails = 0;
   for (const auto& c : cases) fails += run_case(c, sms, true);
-  // every production epilogue again on CTA pairs (odd tile counts included: 2x92x92 1x1 = 133 tiles)
+  // the same layers on CTA pairs (odd tile counts included: 2x92x92 1x1 = 133 tiles)
   std::vector<std::string> pair_names;
   pair_names.reserve(cases.size());
   for (const auto& c : cases) {
-    if (c.kind == CONV_STEM7 || c.epi == EPI_NHWC_F16) continue;
+    if ((c.epi != EPI_TMA && c.epi != EPI_TMA_RES) || c.n_pad < 128) continue;
     Case c2 = c;
     pair_names.push_back(std::string("PAIR ") + c.name);
     c2.name = pair_names.back().c_str();
-    c2.cg = 2;
+    c2.block_n = c.n_pad >= 256 ? 256 : 128;
     fails += run_case(c2, sms, true);
   }
-  {  // resident weights: the 64-channel 3x3 convs (stride 1 and stride 2) and a 1x1
-    Case r1 = {"BRES TMA 3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    Case r2 = {"BRES S2 3x3 64->64 relu 92->46", CONV_3x3, 2, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0, 2, 1};
-    Case r3 = {"BRES TMA 1x1 256->64 relu 92x92", CONV_1x1, 2, 92, 92, 256, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    r1.bres = r2.bres = r3.bres = 1;
-    fails += run_case(r1, sms, true);
-    fails += run_case(r2, sms, true);
-    fails += run_case(r3, sms, true);
+  {  // resident weights on spatial tiles: the 64-channel 3x3 convs on small grids (no halo tiling), and a 1x1
+    Case r1 = {"BRES 3x3 64->64 relu 23x23", CONV_3x3, 2, 23, 23, 64, 64, 64, 64, EPI_TMA, true, false, 64};
+    Case r2 = {"BRES 3x3 64->64 relu 17x9", CONV_3x3, 3, 17, 9, 64, 64, 64, 64, EPI_TMA, true, false, 64};
+    Case r3 = {"BRES 1x1 256->64 relu 92x92", CONV_1x1, 2, 92, 92, 256, 64, 64, 64, EPI_TMA, true, false, 64};
+    for (Case* c : {&r1, &r2, &r3}) fails += run_case(*c, sms, true);
   }
   {  // halo-patch 3x3 convs: every instantiation, image sizes that are / are not multiples of the 8 x 16 tile
-    Case h1 = {"HALO BRES 3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    Case h2 = {"HALO 3x3 64->64 relu 92x92 (streamed B)", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    Case h3 = {"HALO PAIR 3x3 128->128 relu 46x46", CONV_3x3, 3, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case h4 = {"HALO 3x3 128->128 relu 46x46 bn128 single", CONV_3x3, 3, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case h5 = {"HALO 3x3 128->128 relu 46x46 bn64", CONV_3x3, 1, 46, 46, 128, 128, 128, 64, EPI_TMA, true, false, 128, 0};
-    Case h6 = {"HALO PAIR 3x3 256->128 relu 46x46 (head)", CONV_3x3, 2, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-    Case h7 = {"HALO PAIR 3x3 128->128 lin 56x56", CONV_3x3, 1, 56, 56, 128, 128, 128, 128, EPI_TMA, true, false, 0, 0};
-    Case h8 = {"HALO BRES 3x3 64->64 relu 17x9", CONV_3x3, 3, 17, 9, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    h1.bres = h8.bres = 1;
-    h3.cg = h6.cg = h7.cg = 2;
-    for (Case* c : {&h1, &h2, &h3, &h4, &h5, &h6, &h7, &h8}) {
-      c->halo = 1;
-      fails += run_case(*c, sms, true);
-    }
+    Case h1 = {"HALO BRES 3x3 64->64 relu 92x92", CONV_3x3, 2, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64};
+    Case h2 = {"HALO BRES 3x3 64->64 relu 46x46", CONV_3x3, 3, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64};
+    Case h3 = {"HALO PAIR 3x3 128->128 relu 46x46", CONV_3x3, 3, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128};
+    Case h5 = {"HALO 3x3 128->128 relu 46x46 bn64", CONV_3x3, 1, 46, 46, 128, 128, 128, 64, EPI_TMA, true, false, 128};
+    Case h6 = {"HALO PAIR 3x3 256->128 relu 46x46 (head)", CONV_3x3, 2, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128};
+    Case h7 = {"HALO PAIR 3x3 128->128 lin 56x56", CONV_3x3, 1, 56, 56, 128, 128, 128, 128, EPI_TMA, true, false, 0};
+    Case h8 = {"HALO BRES 3x3 64->64 relu 13x15", CONV_3x3, 3, 13, 15, 64, 64, 64, 64, EPI_TMA, true, false, 64};
+    for (Case* c : {&h1, &h2, &h3, &h5, &h6, &h7, &h8}) fails += run_case(*c, sms, true);
   }
-  {  // fused block tails: every (N2, residual) instantiation, flat and spatial rows, folded shortcut, odd unit counts
-    Case t1 = {"TAIL 1x1 64->256 +res relu 92x92 > 64", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0};
-    Case t2 = {"TAIL FOLD 1x1 64(+64)->256 relu 92x92 > 64", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 256, 0, 1, 1, 64};
-    Case t3 = {"TAIL 1x1 128->512 +res relu 46x46 > 128", CONV_1x1, 3, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0};
-    Case t4 = {"TAIL FOLD 1x1 128(+256)->512 relu 46x46 > 128", CONV_1x1, 3, 46, 46, 128, 512, 512, 256, EPI_TMA, true, false, 512, 0, 1, 1, 256};
-    Case t5 = {"TAIL 1x1 256->1024 +res relu 23x23 > 256", CONV_1x1, 7, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0};
-    Case t6 = {"TAIL FOLD 1x1 512(+1024)->1024 relu 23x23 > 256", CONV_1x1, 5, 23, 23, 512, 1024, 1024, 256, EPI_TMA, true, false, 1024, 0, 1, 1, 1024};
-    Case t7 = {"TAIL S2RES 1x1 64->256 +res(92) relu 46x46 > 128", CONV_1x1, 2, 46, 46, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0, 1, 2};
-    Case t8 = {"TAIL S2RES 1x1 128->512 +res(46) relu 23x23 > 256", CONV_1x1, 3, 23, 23, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0, 1, 2};
-    t1.n2 = t2.n2 = 64;
-    t3.n2 = t4.n2 = t7.n2 = 128;
-    t5.n2 = t6.n2 = t8.n2 = 256;
-    for (Case* c : {&t1, &t2, &t3, &t4, &t5, &t6, &t7, &t8}) {
-      c->cg = 2;
-      fails += run_case(*c, sms, true);
-    }
+  {  // fused block tails: both (N2, residual) instantiations, odd unit counts
+    Case t2 = {"TAIL FOLD 1x1 64(+64)->256 relu 92x92 > 64", CONV_1x1, 2, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 256, 1, 1, 64, 64};
+    Case t3 = {"TAIL 1x1 128->512 +res relu 46x46 > 128", CONV_1x1, 3, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 1, 1, 0, 128};
+    for (Case* c : {&t2, &t3}) fails += run_case(*c, sms, true);
   }
   {  // 3x3 / transposed convs on flat pixel rows through the im2col tensor map (single CTAs, pairs, odd tile counts)
-    Case a = {"IM2COL 3x3 256->256 relu 23x23 n64", CONV_3x3, 3, 23, 23, 256, 256, 256, 64, EPI_TMA, true, false, 256, 0};
-    Case b = {"IM2COL PAIR 3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256, 0};
-    Case c = {"IM2COL PAIR 3x3 512->512 relu 23x23 (odd tile count)", CONV_3x3, 5, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512, 0};
-    Case d = {"IM2COL 3x3 64->64 relu 13x9 n64", CONV_3x3, 2, 13, 9, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-    Case e = {"IM2COL deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 3, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    Case g = {"IM2COL PAIR deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 3, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128, 0};
-    b.cg = c.cg = g.cg = 2;
-    for (Case* k : {&a, &b, &c, &d, &e, &g}) {
-      k->im2col = 1;
-      fails += run_case(*k, sms, true);
-    }
+    Case a = {"IM2COL 3x3 256->256 relu 23x23 n64", CONV_3x3, 3, 23, 23, 256, 256, 256, 64, EPI_TMA, true, false, 256};
+    Case b = {"IM2COL PAIR 3x3 256->256 relu 23x23", CONV_3x3, 3, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256};
+    Case c = {"IM2COL PAIR 3x3 512->512 relu 23x23 (odd tile count)", CONV_3x3, 5, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512};
+    Case d = {"IM2COL 3x3 128->128 relu 13x9 n64", CONV_3x3, 2, 13, 9, 128, 128, 128, 64, EPI_TMA, true, false, 128};
+    Case g = {"IM2COL PAIR deconv4x4s2 256->192 head 23x23", CONV_DECONV4, 3, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128};
+    for (Case* k : {&a, &b, &c, &d, &g}) fails += run_case(*k, sms, true);
   }
   fails += run_stem_pool(2, 368, sms);
   fails += run_stem_pool(2, 448, sms);
@@ -717,72 +618,30 @@ int main(int argc, char** argv) {
     fails += run_stem_pool(32, 368, sms);
     fails += run_stem_pool(128, 368, sms);
     std::vector<Case> bigc = {
-        {"BIG 1x1 1024->1024 23x23 nb128", CONV_1x1, 128, 23, 23, 1024, 1024, 1024, 256, EPI_NHWC_F16, true, false,
-         1024, 0},
-        {"BIG 3x3 512->512 23x23 nb64", CONV_3x3, 64, 23, 23, 512, 512, 512, 256, EPI_NHWC_F16, true, false, 512, 0},
-        {"BIG 3x3 64->64 92x92 nb32", CONV_3x3, 32, 92, 92, 64, 64, 64, 64, EPI_NHWC_F16, true, false, 64, 0},
-        {"BIG 1x1 256->64 92x92 nb32", CONV_1x1, 32, 92, 92, 256, 64, 64, 64, EPI_NHWC_F16, true, false, 64, 0},
-        {"BIG TMARES 1x1 64->256 +res 92x92 nb32", CONV_1x1, 32, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0},
-        {"BIG TMA 1x1 64->256 92x92 nb32", CONV_1x1, 32, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 0, 0},
-        {"BIG TMA 3x3 64->64 92x92 nb32", CONV_3x3, 32, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-        {"BIG TMA stem nb32", CONV_STEM7, 32, 184, 184, 0, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-        {"BIG TMARES 1x1 256->1024 +res 23x23 nb128", CONV_1x1, 128, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0},
+        {"BIG TMARES 1x1 64->256 +res 92x92 nb32", CONV_1x1, 32, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256},
+        {"BIG TMA 1x1 64->256 92x92 nb32", CONV_1x1, 32, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 0},
+        {"BIG TMA 3x3 64->64 92x92 nb32", CONV_3x3, 32, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64},
+        {"BIG TMARES 1x1 256->1024 +res 23x23 nb128", CONV_1x1, 128, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024},
+        {"BIG TMA 1x1 1024->256 23x23 nb128", CONV_1x1, 128, 23, 23, 1024, 256, 256, 256, EPI_TMA, true, false, 256},
+        {"BIG TMA 1x1 512->128 46x46 nb128", CONV_1x1, 128, 46, 46, 512, 128, 128, 128, EPI_TMA, true, false, 128},
+        {"BIG TMARES 1x1 128->512 +res 46x46 nb128", CONV_1x1, 128, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512},
+        {"BIG TMARES 1x1 64->256 +res 92x92 nb128", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256},
+        {"BRES BIG 1x1 256->64 92x92 nb128", CONV_1x1, 128, 92, 92, 256, 64, 64, 64, EPI_TMA, true, false, 64},
+        // fused block tails at full batch (compare: the unfused 2c kernels above + the stand-alone reduce convs)
+        {"BIG TAIL 1x1 128->512 +res 46x46 nb128 > 128", CONV_1x1, 128, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 1, 1, 0, 128},
+        {"BIG TAIL FOLD 1x1 64(+64)->256 92x92 nb128 > 64", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 256, 1, 1, 64, 64},
+        // halo patches, full batch
+        {"BIG HALO BRES 3x3 64->64 92x92 nb128", CONV_3x3, 128, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64},
+        {"BIG HALO PAIR 3x3 128->128 46x46 nb128", CONV_3x3, 128, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128},
+        {"BIG HALO PAIR 3x3 256->128 46x46 nb128 (head)", CONV_3x3, 128, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128},
+        // resident weights on spatial tiles and im2col, full batch
+        {"BIG BRES S2 3x3 64->64 92->46 nb128", CONV_3x3, 128, 46, 46, 64, 64, 64, 64, EPI_TMA, true, false, 64, 2, 1},
+        {"BIG IM2COL PAIR 3x3 256->256 23x23 nb128", CONV_3x3, 128, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256},
+        {"BIG IM2COL PAIR 3x3 512->512 23x23 nb128", CONV_3x3, 128, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512},
+        {"BIG IM2COL S2 PAIR 3x3 128->128 46->23 nb128", CONV_3x3, 128, 23, 23, 128, 128, 128, 128, EPI_TMA, true, false, 128, 2, 1},
+        {"BIG IM2COL PAIR deconv4x4s2 256->192 head 23x23 nb128", CONV_DECONV4, 128, 23, 23, 256, 192, 191, 192, EPI_DECONV_HEAD, true, false, 128},
     };
     for (const auto& c : bigc) fails += run_case(c, sms, true);
-    std::vector<Case> pairc = {
-        {"BIG TMA 3x3 512->512 23x23 nb64", CONV_3x3, 64, 23, 23, 512, 512, 512, 256, EPI_TMA, true, false, 512, 0},
-        {"BIG TMA 3x3 256->256 23x23 nb128", CONV_3x3, 128, 23, 23, 256, 256, 256, 256, EPI_TMA, true, false, 256, 0},
-        {"BIG TMA 3x3 128->128 46x46 nb128", CONV_3x3, 128, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0},
-        {"BIG TMA 3x3 64->64 92x92 nb128", CONV_3x3, 128, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0},
-        {"BIG TMA 1x1 1024->256 23x23 nb128", CONV_1x1, 128, 23, 23, 1024, 256, 256, 256, EPI_TMA, true, false, 256, 0},
-        {"BIG TMA 1x1 512->128 46x46 nb128", CONV_1x1, 128, 46, 46, 512, 128, 128, 128, EPI_TMA, true, false, 128, 0},
-        {"BIG TMARES 1x1 256->1024 +res 23x23 nb128", CONV_1x1, 128, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0},
-        {"BIG TMARES 1x1 128->512 +res 46x46 nb128", CONV_1x1, 128, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0},
-        {"BIG TMARES 1x1 64->256 +res 92x92 nb128", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0},
-    };
-    {
-      Case b1 = {"BRES BIG TMA 3x3 64->64 92x92 nb128", CONV_3x3, 128, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-      Case b2 = {"BRES BIG TMA 1x1 256->64 92x92 nb128", CONV_1x1, 128, 92, 92, 256, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-      Case b3 = b2;
-      b3.name = "BIG TMA 1x1 256->64 92x92 nb128";
-      b1.bres = b2.bres = 1;
-      fails += run_case(b1, sms, true);
-      fails += run_case(b2, sms, true);
-      fails += run_case(b3, sms, true);
-    }
-    {  // fused block tails at full batch (compare: the unfused 2c kernels above + the stand-alone reduce convs)
-      Case a = {"BIG TAIL 1x1 64->256 +res 92x92 nb128 > 64", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA_RES, true, true, 256, 0};
-      Case b = {"BIG TAIL 1x1 128->512 +res 46x46 nb128 > 128", CONV_1x1, 128, 46, 46, 128, 512, 512, 256, EPI_TMA_RES, true, true, 512, 0};
-      Case c = {"BIG TAIL 1x1 256->1024 +res 23x23 nb128 > 256", CONV_1x1, 128, 23, 23, 256, 1024, 1024, 256, EPI_TMA_RES, true, true, 1024, 0};
-      Case d = {"BIG TAIL FOLD 1x1 64(+64)->256 92x92 nb128 > 64", CONV_1x1, 128, 92, 92, 64, 256, 256, 256, EPI_TMA, true, false, 256, 0, 1, 1, 64};
-      a.n2 = d.n2 = 64; b.n2 = 128; c.n2 = 256;
-      a.cg = b.cg = c.cg = d.cg = 2;
-      fails += run_case(a, sms, true);
-      fails += run_case(b, sms, true);
-      fails += run_case(c, sms, true);
-      fails += run_case(d, sms, true);
-    }
-    {  // halo patches against the nine-box path, full batch
-      Case a = {"BIG HALO BRES 3x3 64->64 92x92 nb128", CONV_3x3, 128, 92, 92, 64, 64, 64, 64, EPI_TMA, true, false, 64, 0};
-      Case b = {"BIG HALO PAIR 3x3 128->128 46x46 nb128", CONV_3x3, 128, 46, 46, 128, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-      Case c = {"BIG HALO PAIR 3x3 256->128 46x46 nb128 (head)", CONV_3x3, 128, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-      Case d = {"BIG PAIR 3x3 256->128 46x46 nb128 (head, nine boxes)", CONV_3x3, 128, 46, 46, 256, 128, 128, 128, EPI_TMA, true, false, 128, 0};
-      a.bres = 1;
-      b.cg = c.cg = d.cg = 2;
-      a.halo = b.halo = c.halo = 1;
-      fails += run_case(a, sms, true);
-      fails += run_case(b, sms, true);
-      fails += run_case(c, sms, true);
-      fails += run_case(d, sms, true);
-    }
-    for (const auto& c : pairc) {  // same layer on single CTAs and on CTA pairs, timings side by side
-      fails += run_case(c, sms, true);
-      Case c2 = c;
-      std::string nm = std::string("PAIR ") + c.name;
-      c2.name = nm.c_str();
-      c2.cg = 2;
-      fails += run_case(c2, sms, true);
-    }
   }
   printf("SELFTEST %s (%d failing cases)\n", fails == 0 ? "PASSED" : "FAILED", fails);
   return fails == 0 ? 0 : 1;

@@ -313,13 +313,6 @@ struct ConvOpts {
   int chain_cout = 0;
 };
 
-// The block tail is fused with the next block's reduce conv on the throughput plans (256-column tiles on CTA pairs);
-// VNECT_B200_CHAIN=0 turns it off (A/B measurement)
-static bool chain_enabled() {
-  static const bool on = [] { const char* e = getenv("VNECT_B200_CHAIN"); return !(e && atoi(e) == 0); }();
-  return on;
-}
-
 // uploads the chained conv's weights ([n2][cout] K-major fp16) and bias, creates its output activation
 static int attach_chain(vnect_t* h, ConvSpec& s, const ConvOpts& o, int cout, int OH, int OW) {
   const HostVar& w = h->vars.at(o.chain_scope + "/weights");
@@ -337,14 +330,13 @@ static int attach_chain(vnect_t* h, ConvSpec& s, const ConvOpts& o, int cout, in
   return VNECT_OK;
 }
 
+// The block tail is fused with the next block's reduce conv on the throughput plans (256-column tiles on CTA pairs).
 // Measured at batch 128 (profiles/r02_gpu_check_tail.log): the fused tail beats the two kernels it replaces where the
 // pair is HBM-bound -- res2a (224 vs 262 us), res2c (78 vs 101), res3b / res3c (137 vs 172) -- and loses where the
 // second accumulator is 256 wide (single-buffered TMEM, res3d / res4* / res5a: 120 vs 107 us) or the main GEMM carries a
-// folded projection with a 128-wide second conv (res3a: 165 vs 161).  VNECT_B200_CHAIN=all forces it everywhere.
+// folded projection with a 128-wide second conv (res3a: 165 vs 161).
 static bool can_chain(const ConvSpec& s, const ConvOpts& o, int cout) {
-  if (!chain_enabled() || o.chain_scope.empty() || s.block_n != kTailBlockN || s.cg != 2 || cout % kTailBlockN != 0) return false;
-  static const bool all = [] { const char* e = getenv("VNECT_B200_CHAIN"); return e && strcmp(e, "all") == 0; }();
-  if (all) return o.chain_cout == 64 || o.chain_cout == 128 || o.chain_cout == 256;
+  if (o.chain_scope.empty() || s.block_n != kTailBlockN || cout % kTailBlockN != 0) return false;
   return o.chain_cout == 64 || (o.chain_cout == 128 && s.residual != nullptr);
 }
 
@@ -353,16 +345,6 @@ static bool can_chain(const ConvSpec& s, const ConvOpts& o, int cout) {
 static int pick_block_n(int n, int cap_fw) {
   if (cap_fw <= 8) return 64;
   return n >= 256 ? 256 : n >= 128 ? 128 : 64;
-}
-
-// CTA pairs (tcgen05 cta_group::2) pay off where the MMA's smem operand reads are the limit: N >= 128 tiles
-// (measured 5-8 % on the tensor-bound layers, nothing at N = 64).  VNECT_B200_PAIRS=0 / 64 moves the threshold (A/B).
-static int pick_cg(int block_n) {
-  static const int min_n = [] {
-    const char* e = getenv("VNECT_B200_PAIRS");
-    return e ? (atoi(e) > 0 ? atoi(e) : 1 << 30) : 128;
-  }();
-  return block_n >= min_n ? 2 : 1;
 }
 
 static int add_conv(vnect_t* h, const std::string& scope, int k, const std::string& in, const std::string& out,
@@ -384,7 +366,7 @@ static int add_conv(vnect_t* h, const std::string& scope, int k, const std::stri
   s.kind = k == 1 ? CONV_1x1 : CONV_3x3;
   s.NB = h->cap_fw; s.H = OH; s.W = OW;
   s.in = ai.p; s.cin_pad = cin_pad; s.in_stride = o.in_stride;
-  s.w = dw; s.n_pad = cout; s.n_valid = cout; s.block_n = pick_block_n(cout, h->cap_fw); s.cg = pick_cg(s.block_n);
+  s.w = dw; s.n_pad = cout; s.n_valid = cout; s.block_n = pick_block_n(cout, h->cap_fw);
   s.bias = db; s.relu_cols = o.relu ? cout : 0;
   if (!o.residual.empty()) {
     const Act& r = h->acts.at(o.residual);
@@ -394,24 +376,7 @@ static int add_conv(vnect_t* h, const std::string& scope, int k, const std::stri
   }
   // outputs leave through swizzled smem + TMA tensor stores; residual tiles are prefetched by TMA
   s.out = h->acts.at(out).p; s.ldc = cout;
-  s.epi = s.residual ? EPI_TMA_RES : EPI_TMA;
-  // 64-channel convs whose whole weight matrix fits 9 K blocks keep it resident in smem: the 3x3s of res2 are bound
-  // by L2->SM traffic (158 -> 135 us), the 1x1 256->64 convs gain a few percent
-  static const bool bres_on = [] { const char* e = getenv("VNECT_B200_BRES"); return !(e && atoi(e) == 0); }();
-  if (bres_on && cout == 64 && s.block_n == 64 && s.cg == 1 && s.epi == EPI_TMA && k * k * cin_pad / 64 <= kMaxResidentKBlocks)
-    s.b_resident = 1;
-  // stride-1 3x3 convs on the larger grids read one halo patch per channel block instead of nine shifted boxes
-  // (conv_gemm.cuh HALO); VNECT_B200_HALO=0 turns it off (A/B measurement)
-  static const bool halo_on = [] { const char* e = getenv("VNECT_B200_HALO"); return !(e && atoi(e) == 0); }();
-  if (halo_on && k == 3 && o.in_stride == 1 && s.epi == EPI_TMA && halo_tiling_ok(OH, OW) &&
-      (s.block_n == 64 ? s.cg == 1 : (s.block_n == 128)))
-    s.halo = 1;
-  // the other stride-1 3x3 convs (23 x 23 at box size 368: five 23 x 5 tiles fill 529 of 640 GEMM rows) run on flat pixel
-  // rows through an im2col tensor map: every row of a 128-row tile is a real pixel.  Same K order, so the same results.
-  // VNECT_B200_IM2COL=0 turns it off (A/B measurement)
-  static const bool im2col_on = [] { const char* e = getenv("VNECT_B200_IM2COL"); return !(e && atoi(e) == 0); }();
-  // (stride-2 convs included: res3d's 3x3 at 46 -> 23, 31 -> 27 us; the resident-weight 64-channel ones gain nothing)
-  if (im2col_on && k == 3 && !s.halo && !s.b_resident && cin_pad % 64 == 0) s.im2col = 1;
+  s.epi = s.residual ? EPI_TMA_RES : EPI_TMA;  // resident weights, halo patches or im2col: conv_path() in build_conv
   Step st;
   st.kind = 0; st.name = scope;
   if (k == 1 && can_chain(s, o, cout)) {
@@ -455,7 +420,7 @@ static int add_proj_tail(vnect_t* h, const std::string& scope2c, const std::stri
   s.kind = CONV_1x1;
   s.NB = h->cap_fw; s.H = ab.H; s.W = ab.W;
   s.in = ab.p; s.cin_pad = mid; s.in2 = ax.p; s.cin2_pad = cin;
-  s.w = dw; s.n_pad = cout; s.n_valid = cout; s.block_n = pick_block_n(cout, h->cap_fw); s.cg = pick_cg(s.block_n);
+  s.w = dw; s.n_pad = cout; s.n_valid = cout; s.block_n = pick_block_n(cout, h->cap_fw);
   s.bias = db; s.relu_cols = cout;
   s.out = h->acts.at(out).p; s.ldc = cout; s.epi = EPI_TMA;
   Step st;
@@ -819,12 +784,8 @@ int vnect_finalize(vnect_t* h) {
     ConvSpec s;
     s.kind = CONV_DECONV4;
     s.NB = nb; s.H = ai.H; s.W = ai.W; s.in = ai.p; s.cin_pad = 256;
-    s.w = dw; s.n_pad = 192; s.n_valid = 191; s.block_n = 192; s.bias = db; s.relu_cols = 128; s.cg = pick_cg(192);
+    s.w = dw; s.n_pad = 192; s.n_valid = 191; s.block_n = 192; s.bias = db; s.relu_cols = 128;
     s.out = h->acts.at("res5c_branch2a_feat").p; s.ldc = 256; s.epi = EPI_DECONV_HEAD;
-    {  // flat pixel rows through the im2col tensor map (see add_conv): 114 -> 103 us per 128 forwards
-      const char* e = getenv("VNECT_B200_IM2COL");
-      if (!(e && atoi(e) == 0)) s.im2col = 1;
-    }
     Step st;
     st.kind = 0; st.name = "res5c_deconv_head";
     std::string err;
@@ -841,7 +802,7 @@ int vnect_finalize(vnect_t* h) {
     ConvSpec s;
     s.kind = CONV_1x1;
     s.NB = nb; s.H = ai.H; s.W = ai.W; s.in = ai.p; s.cin_pad = 128;
-    s.w = dw; s.n_pad = 96; s.n_valid = 84; s.block_n = 96; s.bias = nullptr; s.relu_cols = 0; s.cg = pick_cg(96);
+    s.w = dw; s.n_pad = 96; s.n_valid = 84; s.block_n = 96; s.bias = nullptr; s.relu_cols = 0;
     s.out = h->maps; s.ldc = 0; s.epi = EPI_PLANAR_F32;
     Step st;
     st.kind = 0; st.name = "res5c_branch2c";
@@ -853,10 +814,8 @@ int vnect_finalize(vnect_t* h) {
   h->conv_steps = (int)h->steps.size();
   // ping-pong tile order: layer i walks its tiles in the opposite direction of layer i-1, so it starts on the data
   // that is still in the 126 MB L2 (the pyramid kernel writes forwards in ascending order, hence the stem reverses)
-  const char* order = getenv("VNECT_B200_TILE_ORDER");  // "forward" turns the ping-pong off (profiling A/B only)
-  const bool pingpong = !(order && strcmp(order, "forward") == 0);
   for (size_t i = 0; i < h->steps.size(); ++i) {
-    const int rev = (pingpong && i % 2 == 0) ? 1 : 0;
+    const int rev = i % 2 == 0 ? 1 : 0;
     if (h->steps[i].kind == 0) h->steps[i].launch.p.reverse = rev;
     else h->steps[i].stem_pool.r.reverse = rev;
   }
@@ -1048,12 +1007,8 @@ static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, i
   if (guard) CU(h, cudaHostGetDevicePointer(reinterpret_cast<void**>(&p.nonfinite_flag), h->cur->h_nonfinite, 0));
   // Threads per (frame, joint) block = the cells of `rows` heat-map rows.  A full batch is bound by instruction issue
   // summed over all blocks (two rows: every lane busy at hs = 46); a few frames leave most SMs empty, so wider blocks
-  // shorten each block's own chain instead.  VNECT_B200_POST_ROWS overrides for A/B runs.
-  static const int rows_env = [] {
-    const char* e = getenv("VNECT_B200_POST_ROWS");
-    return e ? atoi(e) : 0;
-  }();
-  const int rows = rows_env > 0 ? rows_env : n_frames >= 48 ? 2 : n_frames >= 12 ? 4 : 8;
+  // shorten each block's own chain instead.
+  const int rows = n_frames >= 48 ? 2 : n_frames >= 12 ? 4 : 8;
   const int threads = post_threads(h->hs, rows);
   const int rpp = threads / h->hs;
   post_smem_plan(p, h->h_tables.data(), (h->hs / 2 / rpp) * rpp);
@@ -1723,55 +1678,6 @@ int vnect_time_prepost(vnect_t* h, int32_t n_frames, int32_t reps, float* pre_ms
     CU(h, cudaEventSynchronize(e1));
     CU(h, cudaEventElapsedTime(&ms, e0, e1));
     if (r >= 0) post += ms;
-  }
-  if (h->d_post_trace) {  // developer diagnostics: where a (frame, joint) block of the last launch spent its time
-    const int nb = n_frames * kJoints;
-    std::vector<unsigned long long> tr((size_t)nb * 16);
-    CU(h, cudaMemcpy(tr.data(), h->d_post_trace, tr.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    unsigned long long t0 = ~0ull, t1 = 0;
-    for (int b = 0; b < nb; ++b) { t0 = std::min(t0, tr[(size_t)b * 16]); for (int k = 0; k <= 10; ++k) t1 = std::max(t1, tr[(size_t)b * 16 + k]); }
-    static const char* names[] = {"start", "pdl_wait", "staged", "sum pass", "reduced", "marked", "exact+reduce", "2D filter", "gather", "fence+atomic", "tail"};
-    fprintf(stderr, "post-process trace (%d blocks, kernel span %.2f us): phase end relative to the block's start, mean / max us; block start spread %.2f us\n",
-            nb, (t1 - t0) * 1e-3, 0.0);
-    double start_max = 0;
-    for (int b = 0; b < nb; ++b) start_max = std::max(start_max, (tr[(size_t)b * 16] - t0) * 1e-3);
-    fprintf(stderr, "  last block started %.2f us after the first\n", start_max);
-    for (int b = 0; b < nb; ++b)
-      if (tr[(size_t)b * 16 + 10] > tr[(size_t)b * 16]) {  // a block that ran the tail: SM cycles per ns over its lifetime
-        fprintf(stderr, "  SM clock during the kernel: %.0f MHz\n",
-                1e3 * (double)(tr[(size_t)b * 16 + 12] - tr[(size_t)b * 16 + 11]) / (double)(tr[(size_t)b * 16 + 10] - tr[(size_t)b * 16]));
-        break;
-      }
-    {  // survivors per block and the spread of the blocks' own durations (start -> fence + counter)
-      std::vector<double> dur;
-      std::vector<unsigned long long> nqs;
-      for (int b = 0; b < nb; ++b) {
-        dur.push_back((tr[(size_t)b * 16 + 9] - tr[(size_t)b * 16]) * 1e-3);
-        nqs.push_back(tr[(size_t)b * 16 + 13]);
-      }
-      std::sort(dur.begin(), dur.end());
-      std::sort(nqs.begin(), nqs.end());
-      fprintf(stderr, "  block duration p50 %.2f p90 %.2f p99 %.2f max %.2f us; surviving quads per block p50 %llu p90 %llu p99 %llu max %llu\n",
-              dur[nb / 2], dur[nb * 9 / 10], dur[nb * 99 / 100], dur[nb - 1], nqs[nb / 2], nqs[nb * 9 / 10], nqs[nb * 99 / 100], nqs[nb - 1]);
-    }
-    {  // inside "exact+reduce": the exact cells are in shared memory (blocks on the few-quads path only)
-      double sum = 0; int cnt = 0;
-      for (int b = 0; b < nb; ++b) {
-        const unsigned long long v = tr[(size_t)b * 16 + 14], s0 = tr[(size_t)b * 16 + 5];
-        if (v >= s0 && v <= t1) { sum += (v - s0) * 1e-3; ++cnt; }
-      }
-      fprintf(stderr, "  exact cells ready %.2f us after the marking barrier (%d blocks)\n", cnt ? sum / cnt : 0.0, cnt);
-    }
-    for (int k = 1; k <= 10; ++k) {
-      double sum = 0, mx = 0; int cnt = 0;
-      for (int b = 0; b < nb; ++b) {
-        const unsigned long long v = tr[(size_t)b * 16 + k], s0 = tr[(size_t)b * 16];
-        if (v < s0 || v > t1) continue;  // stale slot (tail runs in one block per frame)
-        if (k == 10 && v < tr[(size_t)b * 16 + 9]) continue;
-        sum += (v - s0) * 1e-3; mx = std::max(mx, (v - s0) * 1e-3); ++cnt;
-      }
-      fprintf(stderr, "  %-14s %7.2f / %7.2f us  (%d blocks)\n", names[k], cnt ? sum / cnt : 0.0, mx, cnt);
-    }
   }
   if (h->d_post_trace) {  // developer diagnostics: where a (frame, joint) block of the last launch spent its time
     const int nb = n_frames * kJoints;
