@@ -101,6 +101,46 @@ int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, 
                           int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d,
                           double* dev_joints2d, float* dev_joints3d);
 
+/* YUV 4:2:0 frames, as video decoders write them.  A YUV frame gives exactly the results of the BGR frame
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12) (or COLOR_YUV2BGR_I420) fed to the BGR entry point: BT.601 limited range,
+ * one chroma pair per 2x2 luma block, no chroma interpolation.  The conversion is fused into the pre-processing; no
+ * BGR copy of the frame is ever made.  H and W must be even.  All offsets are in bytes from the start of each frame
+ * (frame i starts at frames + i * frame_stride); planes may carry row padding and the chroma plane may start after
+ * padding rows, as in a hardware decoder's surface (u_offset = y_pitch * aligned_height).
+ * cv2's contiguous layout of a [3H/2][W] array:
+ *   NV12: y_pitch = uv_pitch = W, u_offset = H*W, v_offset = H*W + 1 (U and V interleaved)
+ *   I420: y_pitch = W, uv_pitch = W/2, u_offset = H*W, v_offset = H*W + (H/2)*(W/2)
+ * Refused with VNECT_E_INVALID before anything runs: an unknown format, reserved != 0, odd or too small / large H or W,
+ * pitches smaller than a row, a negative offset, a chroma plane that starts inside the luma plane, NV12 with
+ * v_offset != u_offset + 1. */
+#define VNECT_FMT_NV12 1
+#define VNECT_FMT_I420 2
+typedef struct vnect_yuv_layout {
+  int32_t format;        /* VNECT_FMT_NV12 or VNECT_FMT_I420 */
+  int32_t reserved;      /* 0 */
+  int64_t y_pitch;       /* bytes between luma rows, >= W */
+  int64_t uv_pitch;      /* bytes between chroma rows: >= W (NV12), >= W/2 (I420) */
+  int64_t u_offset;      /* bytes from a frame's start to its first U sample */
+  int64_t v_offset;      /* bytes from a frame's start to its first V sample (NV12: u_offset + 1) */
+  int64_t frame_stride;  /* bytes between frames */
+} vnect_yuv_layout;
+
+/* replaces cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420) followed by VNectEstimator.__call__: vnect_submit for
+ * HOST YUV frames (H x W pixels each; staged to the device at 1.5 bytes per pixel).  Completes with vnect_wait. */
+int vnect_submit_yuv(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_frames, int32_t H, int32_t W,
+                     const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                     double* joints2d, float* joints3d);
+/* replaces cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420) followed by VNectEstimator.__call__, like
+ * vnect_estimate_device: DEVICE frames (e.g. a decoder's output surfaces) and DEVICE results, asynchronous. */
+int vnect_estimate_device_yuv(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
+                              const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d,
+                              const double* t3d, double* dev_joints2d, float* dev_joints3d);
+/* replaces cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420) followed by the loop body of run_estimator.py:98-119, like
+ * vnect_track: HOST full frames of FH x FW pixels, cropped by each stream's tracked box. */
+int vnect_track_yuv(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW,
+                    const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                    double* joints2d, float* joints3d, int32_t* boxes_used);
+
 /* replaces VNectEstimator.gen_input_batch (src/estimator.py:70-81): out float32 [n_frames*n_scales][S][S][3]
  * (fp16-rounded values of the network input), scaler_offsets float64 [3] = {scaler, offset_x, offset_y} */
 int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,

@@ -27,8 +27,25 @@ class Config(C.Structure):
     ]
 
 
+FMT_NV12, FMT_I420 = 1, 2
+
+
+class YuvLayout(C.Structure):
+    """vnect_yuv_layout: where the planes of each YUV 4:2:0 frame are (bytes, relative to the frame's start)."""
+    _fields_ = [
+        ("format", C.c_int32),
+        ("reserved", C.c_int32),
+        ("y_pitch", C.c_int64),
+        ("uv_pitch", C.c_int64),
+        ("u_offset", C.c_int64),
+        ("v_offset", C.c_int64),
+        ("frame_stride", C.c_int64),
+    ]
+
+
 # every symbol include/vnect_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
+_YL = C.POINTER(YuvLayout)
 SIGNATURES = {
     "vnect_create": (C.c_int, [C.POINTER(_P), C.POINTER(Config)]),
     "vnect_set_weight": (C.c_int, [_P, C.c_char_p, _P, C.POINTER(C.c_int64), C.c_int32]),
@@ -42,6 +59,9 @@ SIGNATURES = {
     "vnect_track_get_box": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
     "vnect_track": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P, _P, _P, _P, _P]),
     "vnect_estimate_device": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P, _P, _P, _P]),
+    "vnect_submit_yuv": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P]),
+    "vnect_estimate_device_yuv": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P]),
+    "vnect_track_yuv": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P, _P]),
     "vnect_preprocess": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P]),
     "vnect_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32, C.c_int32, _P, _P, _P]),
     "vnect_filter": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P]),

@@ -40,9 +40,10 @@ __device__ __forceinline__ void cv_linear_coord(int d, double inv_scale, int src
 __device__ __forceinline__ int cv_coef(float f) { return __float2int_rn(__fmul_rn(f, 2048.f)); }
 
 // One output pixel (3 channels) of cv2.resize(u8, INTER_LINEAR): 11-bit fixed point, vertical pass
-// (((b0*(T0>>4))>>16) + ((b1*(T1>>4))>>16) + 2) >> 2.   src rows are `pitch` bytes apart, 3 bytes per pixel.
-__device__ __forceinline__ void cv_resize_u8_px(const uint8_t* __restrict__ src, int64_t pitch, int sh, int sw, int dy,
-                                                int dx, double inv_scale, int out[3]) {
+// (((b0*(T0>>4))>>16) + ((b1*(T1>>4))>>16) + 2) >> 2.   `src` reads the source pixels (BgrSrc / Yuv420Src below).
+template <class Src>
+__device__ __forceinline__ void cv_resize_u8_px(const Src& src, int sh, int sw, int dy, int dx, double inv_scale,
+                                                int out[3]) {
   int ix, iy;
   float fx, fy;
   cv_linear_coord(dx, inv_scale, sw, true, &ix, &fx);
@@ -51,14 +52,23 @@ __device__ __forceinline__ void cv_resize_u8_px(const uint8_t* __restrict__ src,
   const int b0 = cv_coef(__fsub_rn(1.f, fy)), b1 = cv_coef(fy);
   const int ix1 = min(ix + 1, sw - 1);
   const int y0 = min(max(iy, 0), sh - 1), y1 = min(max(iy + 1, 0), sh - 1);
-  const uint8_t* r0 = src + (int64_t)y0 * pitch;
-  const uint8_t* r1 = src + (int64_t)y1 * pitch;
+  const auto r0 = src.at(y0, 0);
+  const auto r1 = src.at(y1, 0);
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
-    const int t0 = r0[ix * 3 + c] * a0 + r0[ix1 * 3 + c] * a1;
-    const int t1 = r1[ix * 3 + c] * a0 + r1[ix1 * 3 + c] * a1;
+    const int t0 = src.get(r0, ix, c) * a0 + src.get(r0, ix1, c) * a1;
+    const int t1 = src.get(r1, ix, c) * a0 + src.get(r1, ix1, c) * a1;
     out[c] = (((b0 * (t0 >> 4)) >> 16) + ((b1 * (t1 >> 4)) >> 16) + 2) >> 2;
   }
+}
+
+// Channel c (0 B, 1 G, 2 R) of cv2.cvtColor(COLOR_YUV2BGR_NV12 / _I420) of one pixel: BT.601 limited range in OpenCV's
+// 20-bit fixed point.  Every intermediate stays below 6e8 in magnitude, so int32 is exact.
+__device__ __forceinline__ int yuv_to_bgr(int Y, int U, int V, int c) {
+  const int uu = U - 128, vv = V - 128, half = 1 << 19;
+  const int y = max(0, Y - 16) * 1220542;
+  const int uv = c == 0 ? half + 2116026 * uu : c == 1 ? half - 852492 * vv - 409993 * uu : half + 1673527 * vv;
+  return min(max((y + uv) >> 20, 0), 255);
 }
 
 // Per-frame crop + squarify geometry of the tracked-stream path (run_estimator.py:100 crop, utils.py:107-120 squarify).
@@ -80,6 +90,43 @@ struct SquarifyParams {
   double inv_scale;         // 1 / scaler
   int mode;                 // 0 = bilinear, 1 = exact 2x decimation (OpenCV switches INTER_LINEAR to INTER_AREA)
   const FrameGeom* geoms;   // optional per-frame geometry (tracked streams); overrides the uniform fields above
+  // YUV 4:2:0 sources only (`pitch` is then the luma pitch): chroma planes relative to a frame's start
+  int64_t uv_pitch, u_offset, v_offset;
+  int uv_step;              // bytes between horizontally adjacent chroma samples: 2 (NV12) or 1 (I420)
+};
+
+// Source pixels of squarify_kernel, one type per input format.  Coordinates count from the crop origin set by crop()
+// (the frame's top-left corner when there is none):
+//   at(y, x)         a handle on pixel (y, x)
+//   below(q, step)   the handle one row below q when step is true, q otherwise
+//   get(q, dx, c)    channel c (0 B, 1 G, 2 R) of the pixel dx columns right of q
+struct BgrSrc {
+  const uint8_t* p;
+  int64_t pitch;
+  __device__ __forceinline__ BgrSrc(const uint8_t* frame, const SquarifyParams& sp) : p(frame), pitch(sp.pitch) {}
+  __device__ __forceinline__ void crop(int x, int y) { p += (int64_t)y * pitch + (int64_t)x * 3; }
+  __device__ __forceinline__ const uint8_t* at(int y, int x) const { return p + (int64_t)y * pitch + (int64_t)x * 3; }
+  __device__ __forceinline__ const uint8_t* below(const uint8_t* q, bool step) const { return q + (step ? pitch : 0); }
+  __device__ __forceinline__ int get(const uint8_t* q, int dx, int c) const { return q[dx * 3 + c]; }
+};
+
+// NV12 (uv_step 2) and I420 (uv_step 1), converted per tap.  One chroma pair covers a 2x2 luma block of the FULL frame,
+// so the chroma row and column come from full-frame coordinates, not crop-relative ones (a crop box may be odd).
+struct Yuv420Src {
+  const uint8_t *luma, *u, *v;
+  int64_t pitch, uv_pitch;
+  int uv_step, x0, y0;
+  __device__ __forceinline__ Yuv420Src(const uint8_t* frame, const SquarifyParams& sp)
+      : luma(frame), u(frame + sp.u_offset), v(frame + sp.v_offset), pitch(sp.pitch), uv_pitch(sp.uv_pitch),
+        uv_step(sp.uv_step), x0(0), y0(0) {}
+  __device__ __forceinline__ void crop(int x, int y) { x0 = x; y0 = y; }
+  __device__ __forceinline__ int2 at(int y, int x) const { return make_int2(x0 + x, y0 + y); }  // full-frame (x, y)
+  __device__ __forceinline__ int2 below(int2 q, bool step) const { return make_int2(q.x, q.y + (step ? 1 : 0)); }
+  __device__ __forceinline__ int get(int2 q, int dx, int c) const {
+    const int fx = q.x + dx;
+    const int64_t ci = (int64_t)(q.y >> 1) * uv_pitch + (int64_t)(fx >> 1) * uv_step;
+    return yuv_to_bgr(luma[(int64_t)q.y * pitch + fx], u[ci], v[ci], c);
+  }
 };
 
 // utils.img_scale_squarify geometry (utils.py:107-120) for box (x, y, w, h) -- same arithmetic as the host version
@@ -114,6 +161,8 @@ __global__ void track_geometry_kernel(const int4* __restrict__ boxes, const int*
 }
 
 // utils.img_scale_squarify (utils.py:107-120): resize so the longer side is S, centre on black.  out: u8 [n,S,S,3].
+// Src is the source format: BgrSrc, or Yuv420Src, which makes this cv2.cvtColor(YUV2BGR) followed by the squarify.
+template <class Src>
 __global__ void squarify_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, SquarifyParams p) {
   const int64_t total = (int64_t)p.n_frames * p.S * p.S;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -122,35 +171,35 @@ __global__ void squarify_kernel(const uint8_t* __restrict__ in, uint8_t* __restr
     const int n = (int)(i / ((int64_t)p.S * p.S));
     int H = p.H, W = p.W, dh = p.dh, dw = p.dw, off_x = p.off_x, off_y = p.off_y, mode = p.mode;
     double inv_scale = p.inv_scale;
-    const uint8_t* src = in + (int64_t)n * p.frame_stride;
+    Src src(in + (int64_t)n * p.frame_stride, p);
     if (p.geoms != nullptr) {
       const FrameGeom g = p.geoms[n];
       H = g.h; W = g.w; dh = g.dh; dw = g.dw; off_x = g.off_x; off_y = g.off_y; mode = g.mode; inv_scale = g.inv_scale;
-      src += (int64_t)g.y * p.pitch + (int64_t)g.x * 3;
+      src.crop(g.x, g.y);
     }
     int v[3] = {0, 0, 0};
     const int sy = y - off_y, sx = x - off_x;
     if (sy >= 0 && sy < dh && sx >= 0 && sx < dw) {
       if (mode == 0) {
-        cv_resize_u8_px(src, p.pitch, H, W, sy, sx, inv_scale, v);
+        cv_resize_u8_px(src, H, W, sy, sx, inv_scale, v);
       } else {
         // OpenCV resizeAreaFast (exact 2x): full 2x2 blocks are (sum + 2) >> 2; where an odd source side leaves a
         // partial block (e.g. 736x735 -> dw = cvRound(367.5) = 368), only the in-range pixels are averaged:
         // saturate_cast<uchar>((float)sum / count), i.e. float division then round-half-even.
-        const uint8_t* r0 = src + (int64_t)(2 * sy) * p.pitch + (int64_t)(2 * sx) * 3;
+        const auto r0 = src.at(2 * sy, 2 * sx);
         const bool col2 = 2 * sx + 1 < W, row2 = 2 * sy + 1 < H;
-        const uint8_t* r1 = r0 + (row2 ? p.pitch : 0);
-        const int dxo = col2 ? 3 : 0;
+        const auto r1 = src.below(r0, row2);
         if (col2 && row2) {
 #pragma unroll
-          for (int c = 0; c < 3; ++c) v[c] = (r0[c] + r0[3 + c] + r1[c] + r1[3 + c] + 2) >> 2;
+          for (int c = 0; c < 3; ++c)
+            v[c] = (src.get(r0, 0, c) + src.get(r0, 1, c) + src.get(r1, 0, c) + src.get(r1, 1, c) + 2) >> 2;
         } else {
           const int count = (col2 ? 2 : 1) * (row2 ? 2 : 1);
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
-            int sum = r0[c];
-            if (col2) sum += r0[dxo + c];
-            if (row2) sum += r1[c];
+            int sum = src.get(r0, 0, c);
+            if (col2) sum += src.get(r0, 1, c);
+            if (row2) sum += src.get(r1, 0, c);
             v[c] = __float2int_rn(__fdiv_rn((float)sum, (float)count));
           }
         }

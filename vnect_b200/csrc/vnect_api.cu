@@ -102,7 +102,9 @@ struct vnect_handle {
   int* d_boxes_used = nullptr;     // [max_frames][4]
   // CUDA graphs of the kernel sequence of one estimate call, keyed by everything baked into the kernel parameters.
   // First use of a key runs directly (warm-up), the second captures, later ones replay: ~50 launches -> 1.
-  typedef std::tuple<int, int, int, int, long long, long long, const void*, const void*, const void*> GraphKey;
+  // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset)
+  typedef std::tuple<int, int, int, int, long long, long long, const void*, const void*, const void*, int, long long,
+                     long long, long long> GraphKey;
   struct GraphEntry {
     cudaGraphExec_t exec = nullptr;
     long long launches = 0;
@@ -846,14 +848,54 @@ static int run_forward(vnect_t* h, int n, cudaEvent_t* layer_events = nullptr) {
   return VNECT_OK;
 }
 
+constexpr int kFmtBGR = 0;  // packed BGR24; the YUV formats are VNECT_FMT_NV12 / VNECT_FMT_I420
+
+// Where the pixels of each frame of a batch are, in device memory, for any input format.
+struct FrameSource {
+  int format = kFmtBGR;
+  int64_t pitch = 0;         // bytes between BGR rows, or between luma rows
+  int64_t frame_stride = 0;  // bytes between frames
+  int64_t uv_pitch = 0, u_offset = 0, v_offset = 0;  // YUV: chroma rows, chroma planes relative to a frame's start
+};
+
+static FrameSource bgr_source(int64_t pitch, int64_t frame_stride) {
+  FrameSource s;
+  s.pitch = pitch;
+  s.frame_stride = frame_stride;
+  return s;
+}
+
+static FrameSource yuv_source(const vnect_yuv_layout& l) {
+  FrameSource s;
+  s.format = l.format;
+  s.pitch = l.y_pitch;
+  s.frame_stride = l.frame_stride;
+  s.uv_pitch = l.uv_pitch;
+  s.u_offset = l.u_offset;
+  s.v_offset = l.v_offset;
+  return s;
+}
+
+// cv2's contiguous layout of a [3H/2][W] YUV 4:2:0 frame (what the host paths stage on the device)
+static vnect_yuv_layout packed_yuv_layout(int format, int H, int W) {
+  vnect_yuv_layout l{};
+  l.format = format;
+  l.y_pitch = W;
+  l.uv_pitch = format == VNECT_FMT_NV12 ? W : W / 2;
+  l.u_offset = (int64_t)H * W;
+  l.v_offset = format == VNECT_FMT_NV12 ? l.u_offset + 1 : l.u_offset + (int64_t)(H / 2) * (W / 2);
+  l.frame_stride = (int64_t)H * W * 3 / 2;
+  return l;
+}
+
 struct Geometry {
   double scaler;
   int dh, dw, off_x, off_y, mode;
-  bool alias;  // frames already are S x S: the pyramid reads them directly
+  bool alias;  // BGR frames already are S x S: the pyramid reads them directly
 };
 
-// utils.img_scale_squarify geometry (utils.py:82-120)
-static Geometry squarify_geometry(int S, int H, int W) {
+// utils.img_scale_squarify geometry (utils.py:82-120).  YUV frames never alias: the squarify stage converts them.
+static Geometry squarify_geometry(int S, int H, int W, int format = kFmtBGR) {
   Geometry g;
   g.scaler = (double)S / (double)std::max(H, W);
   g.dw = cv_round_host(W * g.scaler);
@@ -862,7 +904,7 @@ static Geometry squarify_geometry(int S, int H, int W) {
   if (g.dh > g.dw) g.off_x = S / 2 - g.dw / 2;
   else g.off_y = S / 2 - g.dh / 2;
   g.mode = (1.0 / g.scaler == 2.0) ? 1 : 0;  // OpenCV turns exact 2x INTER_LINEAR decimation into INTER_AREA
-  g.alias = (H == S && W == S);
+  g.alias = (format == kFmtBGR && H == S && W == S);
   return g;
 }
 
@@ -893,13 +935,13 @@ static int ensure_surround(vnect_t* h) {
   return VNECT_OK;
 }
 
-static int run_preprocess(vnect_t* h, const uint8_t* dev_bgr, int n_frames, int H, int W, int64_t pitch,
-                          int64_t frame_stride, const Geometry& g, bool tracked = false) {
+static int run_preprocess(vnect_t* h, const uint8_t* dev_frames, int n_frames, int H, int W, const FrameSource& src,
+                          const Geometry& g, bool tracked = false) {
   const int S = h->S;
   int rc0 = ensure_surround(h);
   if (rc0) return rc0;
-  const uint8_t* sq = dev_bgr;
-  int64_t sq_pitch = pitch, sq_stride = frame_stride;
+  const uint8_t* sq = dev_frames;
+  int64_t sq_pitch = src.pitch, sq_stride = src.frame_stride;
   if (tracked) {
     track_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(h->d_boxes, h->cur->d_stream_ids, n_frames, S, H, W,
                                                                       h->d_geoms, h->d_boxes_used);
@@ -909,10 +951,15 @@ static int run_preprocess(vnect_t* h, const uint8_t* dev_bgr, int n_frames, int 
   if (!g.alias || tracked) {
     SquarifyParams sp;
     sp.geoms = tracked ? h->d_geoms : nullptr;
-    sp.n_frames = n_frames; sp.H = H; sp.W = W; sp.pitch = pitch; sp.frame_stride = frame_stride; sp.S = S;
+    sp.n_frames = n_frames; sp.H = H; sp.W = W; sp.pitch = src.pitch; sp.frame_stride = src.frame_stride; sp.S = S;
     sp.dh = g.dh; sp.dw = g.dw; sp.off_x = g.off_x; sp.off_y = g.off_y; sp.inv_scale = 1.0 / g.scaler; sp.mode = g.mode;
+    sp.uv_pitch = src.uv_pitch; sp.u_offset = src.u_offset; sp.v_offset = src.v_offset;
+    sp.uv_step = src.format == VNECT_FMT_NV12 ? 2 : 1;
     const int64_t total = (int64_t)n_frames * S * S;
-    squarify_kernel<<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(dev_bgr, h->d_sq, sp);
+    if (src.format == kFmtBGR)
+      squarify_kernel<BgrSrc><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(dev_frames, h->d_sq, sp);
+    else
+      squarify_kernel<Yuv420Src><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(dev_frames, h->d_sq, sp);
     CU(h, cudaGetLastError());
     ++h->launches;
     sq = h->d_sq; sq_pitch = (int64_t)S * 3; sq_stride = (int64_t)S * S * 3;
@@ -1072,13 +1119,13 @@ int vnect_forward(vnect_t* h, const float* nhwc, int32_t n, float* hm, float* xm
 }
 
 // pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
-static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_bgr, int n_frames, int H, int W, int64_t pitch,
-                        int64_t frame_stride, double* out2d, float* out3d, bool tracked = false) {
-  const Geometry g = squarify_geometry(h->S, H, W);
+static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
+                        const FrameSource& src, double* out2d, float* out3d, bool tracked = false) {
+  const Geometry g = squarify_geometry(h->S, H, W, src.format);
   if (int rc = ensure_surround(h)) return rc;
   auto direct = [&]() -> int {
     int rc;
-    if ((rc = run_preprocess(h, dev_bgr, n_frames, H, W, pitch, frame_stride, g, tracked))) return rc;
+    if ((rc = run_preprocess(h, dev_frames, n_frames, H, W, src, g, tracked))) return rc;
     if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
     if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, out2d, out3d, tracked))) return rc;
     if (tracked) {
@@ -1089,7 +1136,10 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_bgr, int n_fram
     return VNECT_OK;
   };
   if (!h->use_graphs) return direct();
-  const vnect_handle::GraphKey key(lane + (tracked ? 2 : 0), n_frames, H, W, (long long)pitch, (long long)frame_stride, dev_bgr, out2d, out3d);
+  // the format and the chroma layout are baked into the squarify launch as much as the pointers are
+  const vnect_handle::GraphKey key(lane + (tracked ? 2 : 0), n_frames, H, W, (long long)src.pitch,
+                                   (long long)src.frame_stride, dev_frames, out2d, out3d, src.format,
+                                   (long long)src.uv_pitch, (long long)src.u_offset, (long long)src.v_offset);
   auto it = h->graphs.find(key);
   if (it == h->graphs.end()) {
     if (h->graphs.size() >= vnect_handle::kMaxGraphs) {  // evict the least recently used entry
@@ -1137,13 +1187,72 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_bgr, int n_fram
   return VNECT_OK;
 }
 
-int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
-                          int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                          double* dev_joints2d, float* dev_joints3d) {
-  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
-  ON_DEVICE(h);
-  if (!dev_bgr || !dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
-  if (H < 2 || W < 2 || pitch < (int64_t)W * 3) return fail(h, VNECT_E_INVALID, "bad frame geometry %dx%d pitch %lld", H, W, (long long)pitch);
+// Checks a YUV 4:2:0 layout of H x W frames (include/vnect_b200.h) before anything is launched or staged.
+static int check_yuv_layout(vnect_t* h, const vnect_yuv_layout* l, int H, int W) {
+  if (!l) return fail(h, VNECT_E_INVALID, "null layout");
+  if ((l->format != VNECT_FMT_NV12 && l->format != VNECT_FMT_I420) || l->reserved != 0)
+    return fail(h, VNECT_E_INVALID, "unknown YUV format %d (reserved %d)", l->format, l->reserved);
+  if (H < 2 || W < 2 || (H & 1) || (W & 1))
+    return fail(h, VNECT_E_INVALID, "YUV 4:2:0 frame %dx%d: H and W must be even and at least 2", H, W);
+  const bool nv12 = l->format == VNECT_FMT_NV12;
+  if (l->y_pitch < W || l->uv_pitch < (nv12 ? W : W / 2))
+    return fail(h, VNECT_E_INVALID, "pitch smaller than a row (y_pitch %lld, uv_pitch %lld, W %d)", (long long)l->y_pitch,
+                (long long)l->uv_pitch, W);
+  if (l->u_offset < 0 || l->v_offset < 0) return fail(h, VNECT_E_INVALID, "negative chroma offset");
+  const int64_t luma_end = (int64_t)(H - 1) * l->y_pitch + W;
+  if (l->u_offset < luma_end || l->v_offset < luma_end)
+    return fail(h, VNECT_E_INVALID, "chroma plane overlaps the luma plane (offsets %lld / %lld, luma ends at %lld)",
+                (long long)l->u_offset, (long long)l->v_offset, (long long)luma_end);
+  if (nv12 && l->v_offset != l->u_offset + 1) return fail(h, VNECT_E_INVALID, "NV12 needs v_offset == u_offset + 1");
+  return VNECT_OK;
+}
+
+static int check_host_frame_size(vnect_t* h, int H, int W) {
+  if (H < 2 || W < 2 || H > h->cfg.max_input_h || W > h->cfg.max_input_w)
+    return fail(h, VNECT_E_INVALID, "frame %dx%d outside [2, max_input %dx%d]", H, W, h->cfg.max_input_h, h->cfg.max_input_w);
+  return VNECT_OK;
+}
+
+// host frames described by `src` -> the current lane's d_frames, tightly packed (BGR: 3 bytes per pixel, YUV: cv2's
+// contiguous layout, 1.5), on the copy stream; `packed` describes them there
+static int stage_frames(vnect_t* h, const uint8_t* frames, int n_frames, int H, int W, const FrameSource& src,
+                        FrameSource* packed) {
+  uint8_t* d = h->cur->d_frames;
+  if (src.format == kFmtBGR) {
+    const int64_t dpitch = (int64_t)W * 3, dstride = dpitch * H;
+    *packed = bgr_source(dpitch, dstride);
+    if (src.pitch == dpitch && src.frame_stride == dstride) {
+      CU(h, cudaMemcpyAsync(d, frames, (size_t)dstride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
+    } else {
+      for (int i = 0; i < n_frames; ++i)
+        CU(h, cudaMemcpy2DAsync(d + (size_t)i * dstride, dpitch, frames + (size_t)i * src.frame_stride, src.pitch, dpitch, H, cudaMemcpyHostToDevice, h->copy_stream));
+    }
+    return VNECT_OK;
+  }
+  const vnect_yuv_layout l = packed_yuv_layout(src.format, H, W);
+  *packed = yuv_source(l);
+  if (src.pitch == l.y_pitch && src.uv_pitch == l.uv_pitch && src.u_offset == l.u_offset && src.v_offset == l.v_offset &&
+      (n_frames == 1 || src.frame_stride == l.frame_stride)) {
+    CU(h, cudaMemcpyAsync(d, frames, (size_t)l.frame_stride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
+    return VNECT_OK;
+  }
+  // per plane: luma, then the interleaved U/V plane (NV12) or the U and the V plane (I420)
+  const int64_t uv_row = src.format == VNECT_FMT_NV12 ? W : W / 2;
+  for (int i = 0; i < n_frames; ++i) {
+    const uint8_t* f = frames + (size_t)i * src.frame_stride;
+    uint8_t* o = d + (size_t)i * l.frame_stride;
+    CU(h, cudaMemcpy2DAsync(o, l.y_pitch, f, src.pitch, W, H, cudaMemcpyHostToDevice, h->copy_stream));
+    CU(h, cudaMemcpy2DAsync(o + l.u_offset, l.uv_pitch, f + src.u_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
+    if (src.format == VNECT_FMT_I420)
+      CU(h, cudaMemcpy2DAsync(o + l.v_offset, l.uv_pitch, f + src.v_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
+  }
+  return VNECT_OK;
+}
+
+// vnect_estimate_device / vnect_estimate_device_yuv once the frame description is validated
+static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
+                           const FrameSource& src, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                           double* dev_joints2d, float* dev_joints3d) {
   // alternate lanes for the per-call meta so the host can run one call ahead of the GPU
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
@@ -1152,11 +1261,76 @@ int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, 
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
-  if ((rc = run_pipeline(h, lane, dev_bgr, n_frames, H, W, pitch, frame_stride, dev_joints2d, dev_joints3d))) return rc;
+  if ((rc = run_pipeline(h, lane, dev_frames, n_frames, H, W, src, dev_joints2d, dev_joints3d))) return rc;
   if ((rc = snapshot_nonfinite(h))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
   return VNECT_OK;
+}
+
+// vnect_submit / vnect_submit_yuv once the arguments are validated
+static int submit(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_frames, int32_t H, int32_t W,
+                  const FrameSource& src, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                  double* joints2d, float* joints3d) {
+  int rc = lane_acquire(h, lane);
+  if (rc) return rc;
+  // host -> device on the copy stream (tightly packed on the device), overlapping the previous lane's kernels
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
+  FrameSource packed;
+  if ((rc = stage_frames(h, frames, n_frames, H, W, src, &packed))) return rc;
+  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
+  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
+  if ((rc = run_pipeline(h, lane, h->cur->d_frames, n_frames, H, W, packed, h->cur->d_out2d, h->cur->d_out3d))) return rc;
+  CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = snapshot_nonfinite(h))) return rc;
+  CU(h, cudaEventRecord(h->cur->done, h->stream));
+  h->cur->pending = true;
+  return VNECT_OK;
+}
+
+// vnect_track / vnect_track_yuv once the arguments are validated
+static int track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW, const FrameSource& src,
+                 const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d, float* joints3d,
+                 int32_t* boxes_used) {
+  int rc = lane_acquire(h, 0);
+  if (rc) return rc;
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
+  FrameSource packed;
+  if ((rc = stage_frames(h, frames, n_frames, FH, FW, src, &packed))) return rc;
+  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
+  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
+  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW, packed, h->cur->d_out2d, h->cur->d_out3d, true))) return rc;
+  CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if (boxes_used)
+    CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = snapshot_nonfinite(h))) return rc;
+  CU(h, cudaEventRecord(h->cur->done, h->stream));
+  h->cur->pending = true;
+  return lane_acquire(h, 0);  // synchronises and reports non-finite maps
+}
+
+int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
+                          int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                          double* dev_joints2d, float* dev_joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!dev_bgr || !dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (H < 2 || W < 2 || pitch < (int64_t)W * 3) return fail(h, VNECT_E_INVALID, "bad frame geometry %dx%d pitch %lld", H, W, (long long)pitch);
+  return estimate_device(h, dev_bgr, n_frames, H, W, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d,
+                         dev_joints2d, dev_joints3d);
+}
+
+int vnect_estimate_device_yuv(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
+                              const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d,
+                              const double* t3d, double* dev_joints2d, float* dev_joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!dev_frames || !dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_yuv_layout(h, layout, H, W)) return rc;
+  return estimate_device(h, dev_frames, n_frames, H, W, yuv_source(*layout), stream_ids, t2d, t3d, dev_joints2d,
+                         dev_joints3d);
 }
 
 int vnect_submit(vnect_t* h, int32_t lane, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
@@ -1167,29 +1341,22 @@ int vnect_submit(vnect_t* h, int32_t lane, const uint8_t* bgr, int32_t n_frames,
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
   if (!bgr || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
-  if (H < 2 || W < 2 || H > h->cfg.max_input_h || W > h->cfg.max_input_w)
-    return fail(h, VNECT_E_INVALID, "frame %dx%d outside [2, max_input %dx%d]", H, W, h->cfg.max_input_h, h->cfg.max_input_w);
+  if (int rc = check_host_frame_size(h, H, W)) return rc;
   if (pitch < (int64_t)W * 3) return fail(h, VNECT_E_INVALID, "pitch smaller than a row");
-  int rc = lane_acquire(h, lane);
-  if (rc) return rc;
-  // host -> device on the copy stream (tightly packed on the device), overlapping the previous lane's kernels
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
-  const int64_t dpitch = (int64_t)W * 3, dstride = dpitch * H;
-  if (pitch == dpitch && frame_stride == dstride) {
-    CU(h, cudaMemcpyAsync(h->cur->d_frames, bgr, (size_t)dstride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
-  } else {
-    for (int i = 0; i < n_frames; ++i)
-      CU(h, cudaMemcpy2DAsync(h->cur->d_frames + (size_t)i * dstride, dpitch, bgr + (size_t)i * frame_stride, pitch, dpitch, H, cudaMemcpyHostToDevice, h->copy_stream));
-  }
-  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
-  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, lane, h->cur->d_frames, n_frames, H, W, dpitch, dstride, h->cur->d_out2d, h->cur->d_out3d))) return rc;
-  CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  if ((rc = snapshot_nonfinite(h))) return rc;
-  CU(h, cudaEventRecord(h->cur->done, h->stream));
-  h->cur->pending = true;
-  return VNECT_OK;
+  return submit(h, lane, bgr, n_frames, H, W, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d, joints2d, joints3d);
+}
+
+int vnect_submit_yuv(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_frames, int32_t H, int32_t W,
+                     const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                     double* joints2d, float* joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
+  if (!frames || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
+  if (int rc = check_host_frame_size(h, H, W)) return rc;
+  if (int rc = check_yuv_layout(h, layout, H, W)) return rc;
+  return submit(h, lane, frames, n_frames, H, W, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d);
 }
 
 int vnect_track_set_box(vnect_t* h, int32_t stream_id, int32_t x, int32_t y, int32_t w, int32_t hh) {
@@ -1221,26 +1388,22 @@ int vnect_track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH,
   ON_DEVICE(h);
   if (!frames || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
-  if (FH < 2 || FW < 2 || FH > h->cfg.max_input_h || FW > h->cfg.max_input_w)
-    return fail(h, VNECT_E_INVALID, "frame %dx%d outside [2, max_input %dx%d]", FH, FW, h->cfg.max_input_h, h->cfg.max_input_w);
+  if (int rc = check_host_frame_size(h, FH, FW)) return rc;
   if (pitch < (int64_t)FW * 3) return fail(h, VNECT_E_INVALID, "pitch smaller than a row");
-  int rc = lane_acquire(h, 0);
-  if (rc) return rc;
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
-  const int64_t dpitch = (int64_t)FW * 3, dstride = dpitch * FH;
-  for (int i = 0; i < n_frames; ++i)
-    CU(h, cudaMemcpy2DAsync(h->cur->d_frames + (size_t)i * dstride, dpitch, frames + (size_t)i * frame_stride, pitch, dpitch, FH, cudaMemcpyHostToDevice, h->copy_stream));
-  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
-  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW, dpitch, dstride, h->cur->d_out2d, h->cur->d_out3d, true))) return rc;
-  CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  if (boxes_used)
-    CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  if ((rc = snapshot_nonfinite(h))) return rc;
-  CU(h, cudaEventRecord(h->cur->done, h->stream));
-  h->cur->pending = true;
-  return lane_acquire(h, 0);  // synchronises and reports non-finite maps
+  return track(h, frames, n_frames, FH, FW, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d, joints2d, joints3d,
+               boxes_used);
+}
+
+int vnect_track_yuv(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW,
+                    const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                    double* joints2d, float* joints3d, int32_t* boxes_used) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!frames || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
+  if (int rc = check_host_frame_size(h, FH, FW)) return rc;
+  if (int rc = check_yuv_layout(h, layout, FH, FW)) return rc;
+  return track(h, frames, n_frames, FH, FW, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d, boxes_used);
 }
 
 int vnect_wait(vnect_t* h, int32_t lane) {
@@ -1269,7 +1432,7 @@ int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H
   for (int i = 0; i < n_frames; ++i)
     CU(h, cudaMemcpy2DAsync(h->cur->d_frames + (size_t)i * dstride, dpitch, bgr + (size_t)i * frame_stride, pitch, dpitch, H, cudaMemcpyHostToDevice, h->stream));
   const Geometry g = squarify_geometry(h->S, H, W);
-  int rc = run_preprocess(h, h->cur->d_frames, n_frames, H, W, dpitch, dstride, g);
+  int rc = run_preprocess(h, h->cur->d_frames, n_frames, H, W, bgr_source(dpitch, dstride), g);
   if (rc) return rc;
   const int n = n_frames * h->n_scales, S = h->S;
   stem_to_f32_kernel<<<grid_for((int64_t)n * S * S, 256, h->num_sms), 256, 0, h->stream>>>(h->x1, h->d_f32_in, n, S, h->stem_rpp, h->stem_pitch);
@@ -1667,7 +1830,7 @@ int vnect_time_prepost(vnect_t* h, int32_t n_frames, int32_t reps, float* pre_ms
     if ((rc = stage_frame_meta(h, n_frames, ids.data(), t2.data(), t3.data(), h->stream))) return rc;
     float ms = 0;
     CU(h, cudaEventRecord(e0, h->stream));
-    if ((rc = run_preprocess(h, h->cur->d_frames, n_frames, S, S, (int64_t)S * 3, (int64_t)S * S * 3, g))) return rc;
+    if ((rc = run_preprocess(h, h->cur->d_frames, n_frames, S, S, bgr_source((int64_t)S * 3, (int64_t)S * S * 3), g))) return rc;
     CU(h, cudaEventRecord(e1, h->stream));
     CU(h, cudaEventSynchronize(e1));
     CU(h, cudaEventElapsedTime(&ms, e0, e1));

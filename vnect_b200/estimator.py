@@ -22,6 +22,28 @@ def _ptr(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
+_YUV_FORMATS = {"nv12": _capi.FMT_NV12, "i420": _capi.FMT_I420}
+
+
+def yuv_layout(pixel_format, h, w, y_pitch=None, uv_pitch=None, u_offset=None, v_offset=None, frame_stride=None):
+    """``vnect_yuv_layout`` of h x w YUV 4:2:0 frames ("nv12" or "i420"); byte offsets relative to each frame's start.
+    Fields left out follow the planes from ``y_pitch`` (default w) on without gaps, i.e. cv2's contiguous
+    [3h/2, w] layout.  A decoder surface whose chroma plane starts after padding rows gives ``u_offset``
+    (``y_pitch * aligned_height``) and, for several frames, ``frame_stride``."""
+    if pixel_format not in _YUV_FORMATS:
+        raise ValueError(f"pixel_format must be 'bgr', 'nv12' or 'i420', got {pixel_format!r}")
+    nv12 = pixel_format == "nv12"
+    lay = _capi.YuvLayout()
+    lay.format = _YUV_FORMATS[pixel_format]
+    lay.y_pitch = w if y_pitch is None else y_pitch
+    lay.uv_pitch = (lay.y_pitch if nv12 else lay.y_pitch // 2) if uv_pitch is None else uv_pitch
+    lay.u_offset = lay.y_pitch * h if u_offset is None else u_offset
+    chroma_rows = (h // 2) * lay.uv_pitch
+    lay.v_offset = (lay.u_offset + 1 if nv12 else lay.u_offset + chroma_rows) if v_offset is None else v_offset
+    lay.frame_stride = ((lay.u_offset if nv12 else lay.v_offset) + chroma_rows) if frame_stride is None else frame_stride
+    return lay
+
+
 class VNectEngine:
     """Batched estimator: ``estimate(frames[n,H,W,3] uint8 BGR) -> (joints_2d [n,21,2] f64, joints_3d [n,21,3] f32)``.
 
@@ -110,6 +132,26 @@ class VNectEngine:
             st = frames.strides
         return frames, st
 
+    def _source(self, frames, pixel_format):
+        """Frames of any accepted pixel format -> (host array, n, H, W, the C entry point's frame-description
+        arguments).  BGR: uint8 [n,H,W,3]; "nv12" / "i420": uint8 [n,3H/2,W] or [3H/2,W] in cv2's layout."""
+        if pixel_format == "bgr":
+            frames, st = self._frames(frames)
+            n, h, w = frames.shape[:3]
+            return frames, n, h, w, (st[1], st[0] if n > 1 else st[1] * h)
+        yuv_layout(pixel_format, 2, 2)  # rejects an unknown format before the frames are looked at
+        frames = np.asarray(frames)
+        if frames.ndim == 2:
+            frames = frames[None]
+        if frames.dtype != np.uint8 or frames.ndim != 3 or frames.shape[1] % 3 or frames.shape[1] == 0:
+            raise ValueError(f"{pixel_format} frames must be uint8 [n,3H/2,W] or [3H/2,W], got {frames.dtype} "
+                             f"{frames.shape}")
+        n, h, w = frames.shape[0], frames.shape[1] // 3 * 2, frames.shape[2]
+        if h % 2 or w % 2:
+            raise ValueError(f"{pixel_format} frames need an even height and width, got {h}x{w}")
+        frames = np.ascontiguousarray(frames)
+        return frames, n, h, w, (C.byref(yuv_layout(pixel_format, h, w)),)
+
     def _meta(self, n, stream_ids, t2d, t3d):
         ids = np.arange(n, dtype=np.int32) if stream_ids is None else np.ascontiguousarray(stream_ids, dtype=np.int32)
         if t2d is None:
@@ -122,8 +164,14 @@ class VNectEngine:
             raise ValueError("stream_ids must have one entry per frame")
         return ids, t2d, t3d
 
-    def estimate(self, frames, stream_ids=None, t2d=None, t3d=None, out=None):
-        """VNectEstimator.__call__ for n independent frames (host arrays in, host arrays out)."""
+    def estimate(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """VNectEstimator.__call__ for n independent frames (host arrays in, host arrays out).  ``pixel_format``
+        "nv12" / "i420" takes YUV 4:2:0 frames (uint8 [n,3H/2,W]) and gives exactly the results of the BGR frames
+        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420); the conversion runs inside the pre-processing."""
+        if pixel_format != "bgr":
+            j2, j3 = self.submit(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+            self.wait(0)
+            return j2, j3
         frames, st = self._frames(frames)
         n, h, w = frames.shape[:3]
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
@@ -132,17 +180,16 @@ class VNectEngine:
                                              _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
         return j2, j3
 
-    def submit(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None):
+    def submit(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
         """Pipelined estimate(): enqueue a batch on lane 0/1 and return (joints_2d, joints_3d) arrays that are filled
         once wait(lane) returns.  `frames` and the result arrays must stay alive until then (pinned memory makes the
-        copies truly asynchronous)."""
-        frames, st = self._frames(frames)
-        n, h, w = frames.shape[:3]
+        copies truly asynchronous).  ``pixel_format`` as in estimate()."""
+        frames, n, h, w, layout = self._source(frames, pixel_format)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
-        self._check(self._lib.vnect_submit(self._h, int(lane), _ptr(frames), n, h, w, st[1],
-                                           st[0] if n > 1 else st[1] * h, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2),
-                                           _ptr(j3)))
+        fn = self._lib.vnect_submit if pixel_format == "bgr" else self._lib.vnect_submit_yuv
+        self._check(fn(self._h, int(lane), _ptr(frames), n, h, w, *layout, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2),
+                       _ptr(j3)))
         self._inflight = getattr(self, "_inflight", {})
         self._inflight[int(lane)] = (frames, j2, j3)  # keep the buffers alive
         return j2, j3
@@ -161,23 +208,34 @@ class VNectEngine:
         self._check(self._lib.vnect_track_get_box(self._h, int(stream_id), out))
         return tuple(out)
 
-    def track(self, frames, stream_ids=None, t2d=None, t3d=None):
+    def track(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr"):
         """One step of the reference's video loop (run_estimator.py:98-119) for n streams: crop each full frame by
         its stream's box, estimate, shift joints_2d to full-frame coordinates, update the box on the device.
-        Returns (joints_2d [n,21,2], joints_3d [n,21,3], boxes_used [n,4])."""
-        frames, st = self._frames(frames)
-        n, h, w = frames.shape[:3]
+        Returns (joints_2d [n,21,2], joints_3d [n,21,3], boxes_used [n,4]).  ``pixel_format`` as in estimate()."""
+        frames, n, h, w, layout = self._source(frames, pixel_format)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         boxes = np.empty((n, 4), np.int32)
-        self._check(self._lib.vnect_track(self._h, _ptr(frames), n, h, w, st[1], st[0] if n > 1 else st[1] * h,
-                                          _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
+        fn = self._lib.vnect_track if pixel_format == "bgr" else self._lib.vnect_track_yuv
+        self._check(fn(self._h, _ptr(frames), n, h, w, *layout, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3),
+                       _ptr(boxes)))
         return j2, j3, boxes
 
     def estimate_device(self, dev_frames_ptr, n, h, w, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
-                        pitch=None, frame_stride=None):
-        """Same path with frames / results resident in device memory (raw device pointers, e.g. tensor.data_ptr())."""
+                        pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
+        """Same path with frames / results resident in device memory (raw device pointers, e.g. tensor.data_ptr()).
+        For "nv12" / "i420" frames of h x w pixels, ``layout`` is a dict of yuv_layout() fields (y_pitch, uv_pitch,
+        u_offset, v_offset, frame_stride) describing e.g. a padded decoder surface; by default cv2's contiguous
+        layout.  ``pitch`` and ``frame_stride`` describe BGR frames only."""
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        if pixel_format != "bgr":
+            if pitch is not None or frame_stride is not None:
+                raise ValueError("YUV frames are described by `layout`, not by pitch / frame_stride")
+            lay = yuv_layout(pixel_format, h, w, **(layout or {}))
+            self._check(self._lib.vnect_estimate_device_yuv(self._h, C.c_void_p(dev_frames_ptr), n, h, w, C.byref(lay),
+                                                            _ptr(ids), _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
+                                                            C.c_void_p(dev_j3_ptr)))
+            return
         pitch = pitch or w * 3
         frame_stride = frame_stride or pitch * h
         self._check(self._lib.vnect_estimate_device(self._h, C.c_void_p(dev_frames_ptr), n, h, w, pitch, frame_stride,
