@@ -141,6 +141,41 @@ int vnect_track_yuv(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t
                     const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
                     double* joints2d, float* joints3d, int32_t* boxes_used);
 
+/* Mixed-size batches: frames of different sizes, pitches and addresses in one call, one vnect_frame each (a HOST
+ * array, copied by the call).  One pixel format per call: VNECT_FMT_BGR, VNECT_FMT_NV12 or VNECT_FMT_I420.  Frame i
+ * gives bit-for-bit what the uniform entry point gives for that frame alone (joints, raw argmax, tracked box, filter
+ * state), so a multi-camera server can fill one batch from cameras of any resolution, and device frames need not be
+ * gathered into one strided buffer.  CUDA graphs are keyed by the frame count and format only: every composition of
+ * a batch replays the same graph.
+ * Refused with VNECT_E_INVALID before anything is staged or launched and before any filter state is touched: n_frames
+ * outside [1, max_frames], a null table or null data, an unknown format, a side below 2, a BGR pitch below 3 * width,
+ * a YUV entry that fails the vnect_yuv_layout rules above (frame_stride does not apply), and for the HOST entry points
+ * a frame larger than max_input.  Duplicate stream ids and repeated or earlier timestamps are refused as elsewhere. */
+#define VNECT_FMT_BGR 0
+typedef struct vnect_frame {
+  const uint8_t* data;                   /* first byte of the frame (BGR) or of its luma plane (YUV) */
+  int32_t height, width;                 /* this frame's size (the FULL frame for vnect_track_frames) */
+  int64_t pitch;                         /* BGR row pitch, or luma pitch */
+  int64_t uv_pitch, u_offset, v_offset;  /* YUV only, bytes relative to data, as in vnect_yuv_layout; 0 for BGR */
+} vnect_frame;                           /* 48 bytes */
+
+/* replaces VNectEstimator.__call__ (src/estimator.py:97-142), or cv2.cvtColor(YUV2BGR) followed by it, for n_frames
+ * frames of any sizes: vnect_submit(_yuv) with one descriptor per HOST frame.  The frames are staged one after another
+ * into the lane's device buffer.  Completes with vnect_wait. */
+int vnect_submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                        const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                        float* joints3d);
+/* the same on DEVICE frames (e.g. one decoder surface or one tensor per camera) with DEVICE results, like
+ * vnect_estimate_device(_yuv); asynchronous on the handle's stream.  The frames' pointers are used as they are. */
+int vnect_estimate_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                                 const int32_t* stream_ids, const double* t2d, const double* t3d,
+                                 double* dev_joints2d, float* dev_joints3d);
+/* replaces the loop body of run_estimator.py:98-119 for streams whose full frames differ in size, like
+ * vnect_track(_yuv): HOST full frames, each cropped by its stream's box clipped to that frame. */
+int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                       const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                       float* joints3d, int32_t* boxes_used);
+
 /* replaces VNectEstimator.gen_input_batch (src/estimator.py:70-81): out float32 [n_frames*n_scales][S][S][3]
  * (fp16-rounded values of the network input), scaler_offsets float64 [3] = {scaler, offset_x, offset_y} */
 int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
@@ -203,7 +238,8 @@ int vnect_get_raw_argmax(vnect_t* h, int32_t n_frames, int32_t* raw_argmax);
  * saturated (|x| >= 65504); counts has one entry per launch (vnect_step_name order). */
 int vnect_check_finite(vnect_t* h, int32_t n, int64_t* counts);
 int64_t vnect_launch_count(vnect_t* h);      /* kernels launched by this handle so far */
-double vnect_info(vnect_t* h, const char* key); /* "flops_per_forward", "num_sms", "conv_launches_per_forward", ... */
+double vnect_info(vnect_t* h, const char* key); /* "flops_per_forward", "num_sms", "conv_launches_per_forward", ...,
+                                                   "cached_graphs" (live CUDA-graph cache entries) */
 /* device time of `reps` back-to-back forwards of n images already in device memory (CUDA events on the handle's
  * stream); per_layer_ms may be NULL or float[conv_launches_per_forward + 1] (pool is the last entry) */
 int vnect_time_forward(vnect_t* h, int32_t n, int32_t reps, float* total_ms, float* per_layer_ms);

@@ -27,7 +27,7 @@ class Config(C.Structure):
     ]
 
 
-FMT_NV12, FMT_I420 = 1, 2
+FMT_BGR, FMT_NV12, FMT_I420 = 0, 1, 2
 
 
 class YuvLayout(C.Structure):
@@ -43,9 +43,23 @@ class YuvLayout(C.Structure):
     ]
 
 
+class Frame(C.Structure):
+    """vnect_frame: one frame of a mixed-size batch -- its address, full size, row pitch and (YUV) chroma layout."""
+    _fields_ = [
+        ("data", C.c_void_p),
+        ("height", C.c_int32),
+        ("width", C.c_int32),
+        ("pitch", C.c_int64),
+        ("uv_pitch", C.c_int64),
+        ("u_offset", C.c_int64),
+        ("v_offset", C.c_int64),
+    ]
+
+
 # every symbol include/vnect_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _YL = C.POINTER(YuvLayout)
+_FR = C.POINTER(Frame)
 SIGNATURES = {
     "vnect_create": (C.c_int, [C.POINTER(_P), C.POINTER(Config)]),
     "vnect_set_weight": (C.c_int, [_P, C.c_char_p, _P, C.POINTER(C.c_int64), C.c_int32]),
@@ -62,6 +76,9 @@ SIGNATURES = {
     "vnect_submit_yuv": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P]),
     "vnect_estimate_device_yuv": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P]),
     "vnect_track_yuv": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _YL, _P, _P, _P, _P, _P, _P]),
+    "vnect_submit_frames": (C.c_int, [_P, C.c_int32, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "vnect_estimate_device_frames": (C.c_int, [_P, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "vnect_track_frames": (C.c_int, [_P, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "vnect_preprocess": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P]),
     "vnect_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32, C.c_int32, _P, _P, _P]),
     "vnect_filter": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P]),

@@ -95,6 +95,15 @@ struct SquarifyParams {
   int uv_step;              // bytes between horizontally adjacent chroma samples: 2 (NV12) or 1 (I420)
 };
 
+// One frame of a mixed-size batch: the device copy of a vnect_frame (include/vnect_b200.h; same layout, 48 bytes).
+// `data` is the frame's first byte (BGR) or the first byte of its luma plane (YUV), height x width its FULL size,
+// `pitch` the BGR or luma row pitch; YUV chroma planes are addressed relative to `data`.
+struct FrameDesc {
+  const uint8_t* data;
+  int height, width;
+  int64_t pitch, uv_pitch, u_offset, v_offset;
+};
+
 // Source pixels of squarify_kernel, one type per input format.  Coordinates count from the crop origin set by crop()
 // (the frame's top-left corner when there is none):
 //   at(y, x)         a handle on pixel (y, x)
@@ -104,6 +113,7 @@ struct BgrSrc {
   const uint8_t* p;
   int64_t pitch;
   __device__ __forceinline__ BgrSrc(const uint8_t* frame, const SquarifyParams& sp) : p(frame), pitch(sp.pitch) {}
+  __device__ __forceinline__ BgrSrc(const FrameDesc& f, const SquarifyParams&) : p(f.data), pitch(f.pitch) {}
   __device__ __forceinline__ void crop(int x, int y) { p += (int64_t)y * pitch + (int64_t)x * 3; }
   __device__ __forceinline__ const uint8_t* at(int y, int x) const { return p + (int64_t)y * pitch + (int64_t)x * 3; }
   __device__ __forceinline__ const uint8_t* below(const uint8_t* q, bool step) const { return q + (step ? pitch : 0); }
@@ -119,6 +129,9 @@ struct Yuv420Src {
   __device__ __forceinline__ Yuv420Src(const uint8_t* frame, const SquarifyParams& sp)
       : luma(frame), u(frame + sp.u_offset), v(frame + sp.v_offset), pitch(sp.pitch), uv_pitch(sp.uv_pitch),
         uv_step(sp.uv_step), x0(0), y0(0) {}
+  __device__ __forceinline__ Yuv420Src(const FrameDesc& f, const SquarifyParams& sp)
+      : luma(f.data), u(f.data + f.u_offset), v(f.data + f.v_offset), pitch(f.pitch), uv_pitch(f.uv_pitch),
+        uv_step(sp.uv_step), x0(0), y0(0) {}
   __device__ __forceinline__ void crop(int x, int y) { x0 = x; y0 = y; }
   __device__ __forceinline__ int2 at(int y, int x) const { return make_int2(x0 + x, y0 + y); }  // full-frame (x, y)
   __device__ __forceinline__ int2 below(int2 q, bool step) const { return make_int2(q.x, q.y + (step ? 1 : 0)); }
@@ -127,6 +140,15 @@ struct Yuv420Src {
     const int64_t ci = (int64_t)(q.y >> 1) * uv_pitch + (int64_t)(fx >> 1) * uv_step;
     return yuv_to_bgr(luma[(int64_t)q.y * pitch + fx], u[ci], v[ci], c);
   }
+};
+
+// Source of a frame of a mixed-size batch.  squarify_kernel's frame pointer `in + n * frame_stride` is then entry n of
+// the device frame table (in = the table, frame_stride = sizeof(FrameDesc)), which gives the frame's own address,
+// pitches and chroma layout; its crop and size come from SquarifyParams::geoms (frame_geometry_kernel).
+template <class Base>
+struct FrameTableSrc : Base {
+  __device__ __forceinline__ FrameTableSrc(const uint8_t* entry, const SquarifyParams& sp)
+      : Base(*reinterpret_cast<const FrameDesc*>(entry), sp) {}
 };
 
 // utils.img_scale_squarify geometry (utils.py:107-120) for box (x, y, w, h) -- same arithmetic as the host version
@@ -145,19 +167,40 @@ __device__ __forceinline__ FrameGeom make_frame_geom(int x, int y, int w, int h,
   return g;
 }
 
+// numpy slicing frame[y:y+h, x:x+w] clips a tracked box to the FH x FW frame (run_estimator.py:100); keep at least
+// 2x2 pixels
+__device__ __forceinline__ int4 clip_box(int4 b, int FH, int FW) {
+  b.x = min(max(b.x, 0), FW - 2);
+  b.y = min(max(b.y, 0), FH - 2);
+  b.z = max(min(b.z, FW - b.x), 2);
+  b.w = max(min(b.w, FH - b.y), 2);
+  return b;
+}
+
 // boxes: [max_streams] int4 (x, y, w, h); one thread per frame
 __global__ void track_geometry_kernel(const int4* __restrict__ boxes, const int* __restrict__ stream_ids, int n, int S,
                                       int FH, int FW, FrameGeom* __restrict__ geoms, int* __restrict__ boxes_used) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  int4 b = boxes[stream_ids[i]];
-  // numpy slicing frame[y:y+h, x:x+w] clips to the frame (run_estimator.py:100); keep at least 2x2 pixels
-  b.x = min(max(b.x, 0), FW - 2);
-  b.y = min(max(b.y, 0), FH - 2);
-  b.z = max(min(b.z, FW - b.x), 2);
-  b.w = max(min(b.w, FH - b.y), 2);
+  const int4 b = clip_box(boxes[stream_ids[i]], FH, FW);
   geoms[i] = make_frame_geom(b.x, b.y, b.z, b.w, S);
   boxes_used[4 * i + 0] = b.x; boxes_used[4 * i + 1] = b.y; boxes_used[4 * i + 2] = b.z; boxes_used[4 * i + 3] = b.w;
+}
+
+// Geometry of a mixed-size batch, one thread per frame, from each frame's own size: the stream's tracked box clipped
+// to that frame when `boxes` is set (boxes_used records it), otherwise the whole frame, box (0, 0, W_i, H_i).
+__global__ void frame_geometry_kernel(const FrameDesc* __restrict__ frames, const int4* __restrict__ boxes,
+                                      const int* __restrict__ stream_ids, int n, int S, FrameGeom* __restrict__ geoms,
+                                      int* __restrict__ boxes_used) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int FH = frames[i].height, FW = frames[i].width;
+  int4 b = make_int4(0, 0, FW, FH);
+  if (boxes != nullptr) {
+    b = clip_box(boxes[stream_ids[i]], FH, FW);
+    boxes_used[4 * i + 0] = b.x; boxes_used[4 * i + 1] = b.y; boxes_used[4 * i + 2] = b.z; boxes_used[4 * i + 3] = b.w;
+  }
+  geoms[i] = make_frame_geom(b.x, b.y, b.z, b.w, S);
 }
 
 // utils.img_scale_squarify (utils.py:107-120): resize so the longer side is S, centre on black.  out: u8 [n,S,S,3].
@@ -1128,9 +1171,8 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
 //   x, y = max(int(x_min - buffer_x / 2), 0), max(int(y_min - buffer_y / 2), 0)
 //   w, h = int(min(x_max - x_min + buffer_x, W_img - x)), int(min(y_max - y_min + buffer_y, H_img - y))
 // joints2d are full-frame (row, col) coordinates; float64 arithmetic without FMA, int() truncates toward zero.
-__global__ void track_update_kernel(const double* __restrict__ joints2d, const int* __restrict__ stream_ids, int n,
-                                    int FH, int FW, int4* __restrict__ boxes) {
-  const int frame = blockIdx.x;
+__device__ __forceinline__ void track_box_update(const double* __restrict__ joints2d, const int* __restrict__ stream_ids,
+                                                 int frame, int FH, int FW, int4* __restrict__ boxes) {
   const int lane = threadIdx.x;
   double ymin = INFINITY, ymax = -INFINITY, xmin = INFINITY, xmax = -INFINITY;
   if (lane < kJoints) {
@@ -1153,6 +1195,18 @@ __global__ void track_update_kernel(const double* __restrict__ joints2d, const i
     const int h = (int)fmin(__dadd_rn(__dsub_rn(ymax, ymin), buffer_y), (double)(FH - y));
     boxes[stream_ids[frame]] = make_int4(x, y, w, h);
   }
+}
+
+__global__ void track_update_kernel(const double* __restrict__ joints2d, const int* __restrict__ stream_ids, int n,
+                                    int FH, int FW, int4* __restrict__ boxes) {
+  track_box_update(joints2d, stream_ids, blockIdx.x, FH, FW, boxes);
+}
+
+// the same for a mixed-size batch: frame f's box is clipped to its own full-frame size frames[f]
+__global__ void track_update_frames_kernel(const double* __restrict__ joints2d, const int* __restrict__ stream_ids,
+                                           const FrameDesc* __restrict__ frames, int4* __restrict__ boxes) {
+  const int f = blockIdx.x;
+  track_box_update(joints2d, stream_ids, f, frames[f].height, frames[f].width, boxes);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -3,7 +3,9 @@
 
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdlib>
+#include <cstring>
 #include <tuple>
 #include <map>
 #include <algorithm>
@@ -86,7 +88,13 @@ struct vnect_handle {
     int* h_stream_ids = nullptr;
     double *h_t2d = nullptr, *h_t3d = nullptr;
     void* h_meta = nullptr;               // pinned block behind h_stream_ids / h_t2d / h_t3d (one H2D copy per call)
-    size_t meta_bytes = 0;
+    size_t meta_bytes = 0;                // ids | t2d | t3d: what a uniform call copies
+    // mixed-size calls: [max_frames] frame descriptors after the ids and timestamps in the same block (copied with
+    // them), and the per-frame geometry the device derives from them.  Per lane: lane 1's table is written on the
+    // copy stream while lane 0's kernels still read theirs.
+    size_t table_off = 0;
+    FrameDesc *h_table = nullptr, *d_table = nullptr;
+    FrameGeom* d_geoms = nullptr;         // [max_frames]
     unsigned int* h_nonfinite = nullptr;  // pinned + device-visible: set by the post-process when a batch of this lane met NaN / Inf maps
     cudaEvent_t copy_done = nullptr, done = nullptr;
     bool pending = false;
@@ -102,7 +110,9 @@ struct vnect_handle {
   int* d_boxes_used = nullptr;     // [max_frames][4]
   // CUDA graphs of the kernel sequence of one estimate call, keyed by everything baked into the kernel parameters.
   // First use of a key runs directly (warm-up), the second captures, later ones replay: ~50 launches -> 1.
-  // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset)
+  // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset).
+  // Mixed-size calls read sizes and addresses from the lane's device table, so only (4 + lane + tracked, n_frames,
+  // out2d, out3d, format) is set in their key: one graph serves every composition of a batch.
   typedef std::tuple<int, int, int, int, long long, long long, const void*, const void*, const void*, int, long long,
                      long long, long long> GraphKey;
   struct GraphEntry {
@@ -553,17 +563,22 @@ static int alloc_prepost(vnect_t* h) {
     {  // ids | t2d | t3d in one block on both sides: one H2D copy per call
       const size_t off_t2 = ((size_t)mf * sizeof(int) + 15) & ~size_t(15), off_t3 = off_t2 + (size_t)mf * sizeof(double);
       L.meta_bytes = off_t3 + (size_t)mf * sizeof(double);
+      L.table_off = (L.meta_bytes + 15) & ~size_t(15);
+      const size_t block = L.table_off + (size_t)mf * sizeof(FrameDesc);
       uint8_t* d_meta = nullptr;
-      if ((rc = dev_alloc(h, &d_meta, L.meta_bytes))) return rc;
+      if ((rc = dev_alloc(h, &d_meta, block))) return rc;
       L.d_stream_ids = reinterpret_cast<int*>(d_meta);
       L.d_t2d = reinterpret_cast<double*>(d_meta + off_t2);
       L.d_t3d = reinterpret_cast<double*>(d_meta + off_t3);
-      CU(h, cudaMallocHost(&L.h_meta, L.meta_bytes));
-      memset(L.h_meta, 0, L.meta_bytes);
+      L.d_table = reinterpret_cast<FrameDesc*>(d_meta + L.table_off);
+      CU(h, cudaMallocHost(&L.h_meta, block));
+      memset(L.h_meta, 0, block);
       L.h_stream_ids = reinterpret_cast<int*>(L.h_meta);
       L.h_t2d = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + off_t2);
       L.h_t3d = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + off_t3);
+      L.h_table = reinterpret_cast<FrameDesc*>(static_cast<uint8_t*>(L.h_meta) + L.table_off);
     }
+    if ((rc = dev_alloc(h, &L.d_geoms, mf))) return rc;
     if ((rc = dev_alloc(h, &L.d_out2d, (size_t)mf * kJoints * 2))) return rc;
     if ((rc = dev_alloc(h, &L.d_out3d, (size_t)mf * kJoints * 3))) return rc;
     CU(h, cudaHostAlloc(&L.h_nonfinite, sizeof(unsigned int), cudaHostAllocMapped));
@@ -856,7 +871,15 @@ struct FrameSource {
   int64_t pitch = 0;         // bytes between BGR rows, or between luma rows
   int64_t frame_stride = 0;  // bytes between frames
   int64_t uv_pitch = 0, u_offset = 0, v_offset = 0;  // YUV: chroma rows, chroma planes relative to a frame's start
+  bool table = false;  // mixed sizes: every frame's address, size and layout come from the current lane's d_table
 };
+
+static FrameSource table_source(int format) {
+  FrameSource s;
+  s.format = format;
+  s.table = true;
+  return s;
+}
 
 static FrameSource bgr_source(int64_t pitch, int64_t frame_stride) {
   FrameSource s;
@@ -940,6 +963,28 @@ static int run_preprocess(vnect_t* h, const uint8_t* dev_frames, int n_frames, i
   const int S = h->S;
   int rc0 = ensure_surround(h);
   if (rc0) return rc0;
+  if (src.table) {  // per-frame geometry from each frame's own size, then squarify through the lane's table
+    vnect_handle::Lane* L = h->cur;
+    frame_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(L->d_table, tracked ? h->d_boxes : nullptr,
+                                                                      L->d_stream_ids, n_frames, S, L->d_geoms,
+                                                                      h->d_boxes_used);
+    CU(h, cudaGetLastError());
+    ++h->launches;
+    SquarifyParams sp{};  // nothing size- or address-dependent: one captured graph serves every composition
+    sp.geoms = L->d_geoms;
+    sp.n_frames = n_frames; sp.S = S;
+    sp.frame_stride = sizeof(FrameDesc);
+    sp.uv_step = src.format == VNECT_FMT_NV12 ? 2 : 1;
+    const int64_t total = (int64_t)n_frames * S * S;
+    const uint8_t* table = reinterpret_cast<const uint8_t*>(L->d_table);
+    if (src.format == kFmtBGR)
+      squarify_kernel<FrameTableSrc<BgrSrc>><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(table, h->d_sq, sp);
+    else
+      squarify_kernel<FrameTableSrc<Yuv420Src>><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(table, h->d_sq, sp);
+    CU(h, cudaGetLastError());
+    ++h->launches;
+    return launch_pyramid(h, h->d_sq, (int64_t)S * 3, (int64_t)S * S * 3, n_frames, false);
+  }
   const uint8_t* sq = dev_frames;
   int64_t sq_pitch = src.pitch, sq_stride = src.frame_stride;
   if (tracked) {
@@ -992,8 +1037,9 @@ static int lane_acquire(vnect_t* h, int lane) {
 // it meets NaN / Inf maps, so no device -> host copy of a counter sits in the stream after every batch.
 static int snapshot_nonfinite(vnect_t*) { return VNECT_OK; }
 
+// table_frames > 0: the lane's frame table (already written to its pinned block) travels in the same copy
 static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                            cudaStream_t copy_on) {
+                            cudaStream_t copy_on, int table_frames = 0) {
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   h->seen_stamp.resize(h->cfg.max_streams, 0);
   const unsigned int stamp = ++h->seen_epoch;
@@ -1028,14 +1074,16 @@ static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids,
       h->last_t3d[sid] = t3d[i];
     }
   }
-  CU(h, cudaMemcpyAsync(h->cur->d_stream_ids, h->cur->h_meta, h->cur->meta_bytes, cudaMemcpyHostToDevice, copy_on));
+  const size_t bytes = table_frames > 0 ? h->cur->table_off + (size_t)table_frames * sizeof(FrameDesc) : h->cur->meta_bytes;
+  CU(h, cudaMemcpyAsync(h->cur->d_stream_ids, h->cur->h_meta, bytes, cudaMemcpyHostToDevice, copy_on));
   return VNECT_OK;
 }
 
+// geoms: per-frame geometry (tracked streams, mixed sizes), which overrides scaler and the offsets
 static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, int off_y, double* dev_out2d,
-                           float* dev_out3d, bool tracked = false, bool guard = true) {
+                           float* dev_out3d, const FrameGeom* geoms = nullptr, bool guard = true) {
   PostParams p;
-  p.geoms = tracked ? h->d_geoms : nullptr;
+  p.geoms = geoms;
   p.n_frames = n_frames; p.n_scales = h->n_scales; p.hs = h->hs; p.S = h->S;
   p.maps = h->maps; p.tables = h->d_tables;
   p.stream_ids = h->cur->d_stream_ids; p.t2d = h->cur->d_t2d; p.t3d = h->cur->d_t3d;
@@ -1118,28 +1166,12 @@ int vnect_forward(vnect_t* h, const float* nhwc, int32_t n, float* hm, float* xm
   return VNECT_OK;
 }
 
-// pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
-static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
-                        const FrameSource& src, double* out2d, float* out3d, bool tracked = false) {
-  const Geometry g = squarify_geometry(h->S, H, W, src.format);
-  if (int rc = ensure_surround(h)) return rc;
-  auto direct = [&]() -> int {
-    int rc;
-    if ((rc = run_preprocess(h, dev_frames, n_frames, H, W, src, g, tracked))) return rc;
-    if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
-    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, out2d, out3d, tracked))) return rc;
-    if (tracked) {
-      track_update_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, n_frames, H, W, h->d_boxes);
-      CU(h, cudaGetLastError());
-      ++h->launches;
-    }
-    return VNECT_OK;
-  };
-  if (!h->use_graphs) return direct();
-  // the format and the chroma layout are baked into the squarify launch as much as the pointers are
-  const vnect_handle::GraphKey key(lane + (tracked ? 2 : 0), n_frames, H, W, (long long)src.pitch,
-                                   (long long)src.frame_stride, dev_frames, out2d, out3d, src.format,
-                                   (long long)src.uv_pitch, (long long)src.u_offset, (long long)src.v_offset);
+}  // extern "C"
+
+// Runs direct() -- the kernel sequence of one batch -- as a CUDA graph cached under `key`: the first use of a key runs
+// directly (warm-up), the second captures, later ones replay.
+template <class F>
+static int run_graphed(vnect_t* h, const vnect_handle::GraphKey& key, F direct) {
   auto it = h->graphs.find(key);
   if (it == h->graphs.end()) {
     if (h->graphs.size() >= vnect_handle::kMaxGraphs) {  // evict the least recently used entry
@@ -1187,6 +1219,52 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
   return VNECT_OK;
 }
 
+extern "C" {
+
+// pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
+static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
+                        const FrameSource& src, double* out2d, float* out3d, bool tracked = false) {
+  if (src.table) {  // sizes, addresses and geometry live in the lane's device tables, not in kernel parameters
+    if (int rc = ensure_surround(h)) return rc;
+    auto direct = [&]() -> int {
+      int rc;
+      if ((rc = run_preprocess(h, nullptr, n_frames, 0, 0, src, Geometry{}, tracked))) return rc;
+      if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
+      if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, out2d, out3d, h->cur->d_geoms))) return rc;
+      if (tracked) {
+        track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table, h->d_boxes);
+        CU(h, cudaGetLastError());
+        ++h->launches;
+      }
+      return VNECT_OK;
+    };
+    if (!h->use_graphs) return direct();
+    const vnect_handle::GraphKey key(4 + lane + (tracked ? 2 : 0), n_frames, 0, 0, 0, 0, nullptr, out2d, out3d,
+                                     src.format, 0, 0, 0);
+    return run_graphed(h, key, direct);
+  }
+  const Geometry g = squarify_geometry(h->S, H, W, src.format);
+  if (int rc = ensure_surround(h)) return rc;
+  auto direct = [&]() -> int {
+    int rc;
+    if ((rc = run_preprocess(h, dev_frames, n_frames, H, W, src, g, tracked))) return rc;
+    if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
+    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, out2d, out3d, tracked ? h->d_geoms : nullptr))) return rc;
+    if (tracked) {
+      track_update_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, n_frames, H, W, h->d_boxes);
+      CU(h, cudaGetLastError());
+      ++h->launches;
+    }
+    return VNECT_OK;
+  };
+  if (!h->use_graphs) return direct();
+  // the format and the chroma layout are baked into the squarify launch as much as the pointers are
+  const vnect_handle::GraphKey key(lane + (tracked ? 2 : 0), n_frames, H, W, (long long)src.pitch,
+                                   (long long)src.frame_stride, dev_frames, out2d, out3d, src.format,
+                                   (long long)src.uv_pitch, (long long)src.u_offset, (long long)src.v_offset);
+  return run_graphed(h, key, direct);
+}
+
 // Checks a YUV 4:2:0 layout of H x W frames (include/vnect_b200.h) before anything is launched or staged.
 static int check_yuv_layout(vnect_t* h, const vnect_yuv_layout* l, int H, int W) {
   if (!l) return fail(h, VNECT_E_INVALID, "null layout");
@@ -1213,6 +1291,23 @@ static int check_host_frame_size(vnect_t* h, int H, int W) {
   return VNECT_OK;
 }
 
+// one host frame described by `src` -> dst in the layout stage_frames packs it in (BGR: 3W-byte rows, YUV: cv2's
+// contiguous [3H/2][W] layout), on the copy stream
+static int stage_frame(vnect_t* h, uint8_t* dst, const uint8_t* f, int H, int W, const FrameSource& src) {
+  if (src.format == kFmtBGR) {
+    CU(h, cudaMemcpy2DAsync(dst, (size_t)W * 3, f, src.pitch, (size_t)W * 3, H, cudaMemcpyHostToDevice, h->copy_stream));
+    return VNECT_OK;
+  }
+  // per plane: luma, then the interleaved U/V plane (NV12) or the U and the V plane (I420)
+  const vnect_yuv_layout l = packed_yuv_layout(src.format, H, W);
+  const int64_t uv_row = src.format == VNECT_FMT_NV12 ? W : W / 2;
+  CU(h, cudaMemcpy2DAsync(dst, l.y_pitch, f, src.pitch, W, H, cudaMemcpyHostToDevice, h->copy_stream));
+  CU(h, cudaMemcpy2DAsync(dst + l.u_offset, l.uv_pitch, f + src.u_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
+  if (src.format == VNECT_FMT_I420)
+    CU(h, cudaMemcpy2DAsync(dst + l.v_offset, l.uv_pitch, f + src.v_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
+  return VNECT_OK;
+}
+
 // host frames described by `src` -> the current lane's d_frames, tightly packed (BGR: 3 bytes per pixel, YUV: cv2's
 // contiguous layout, 1.5), on the copy stream; `packed` describes them there
 static int stage_frames(vnect_t* h, const uint8_t* frames, int n_frames, int H, int W, const FrameSource& src,
@@ -1223,29 +1318,20 @@ static int stage_frames(vnect_t* h, const uint8_t* frames, int n_frames, int H, 
     *packed = bgr_source(dpitch, dstride);
     if (src.pitch == dpitch && src.frame_stride == dstride) {
       CU(h, cudaMemcpyAsync(d, frames, (size_t)dstride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
-    } else {
-      for (int i = 0; i < n_frames; ++i)
-        CU(h, cudaMemcpy2DAsync(d + (size_t)i * dstride, dpitch, frames + (size_t)i * src.frame_stride, src.pitch, dpitch, H, cudaMemcpyHostToDevice, h->copy_stream));
+      return VNECT_OK;
     }
-    return VNECT_OK;
+  } else {
+    const vnect_yuv_layout l = packed_yuv_layout(src.format, H, W);
+    *packed = yuv_source(l);
+    if (src.pitch == l.y_pitch && src.uv_pitch == l.uv_pitch && src.u_offset == l.u_offset && src.v_offset == l.v_offset &&
+        (n_frames == 1 || src.frame_stride == l.frame_stride)) {
+      CU(h, cudaMemcpyAsync(d, frames, (size_t)l.frame_stride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
+      return VNECT_OK;
+    }
   }
-  const vnect_yuv_layout l = packed_yuv_layout(src.format, H, W);
-  *packed = yuv_source(l);
-  if (src.pitch == l.y_pitch && src.uv_pitch == l.uv_pitch && src.u_offset == l.u_offset && src.v_offset == l.v_offset &&
-      (n_frames == 1 || src.frame_stride == l.frame_stride)) {
-    CU(h, cudaMemcpyAsync(d, frames, (size_t)l.frame_stride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
-    return VNECT_OK;
-  }
-  // per plane: luma, then the interleaved U/V plane (NV12) or the U and the V plane (I420)
-  const int64_t uv_row = src.format == VNECT_FMT_NV12 ? W : W / 2;
-  for (int i = 0; i < n_frames; ++i) {
-    const uint8_t* f = frames + (size_t)i * src.frame_stride;
-    uint8_t* o = d + (size_t)i * l.frame_stride;
-    CU(h, cudaMemcpy2DAsync(o, l.y_pitch, f, src.pitch, W, H, cudaMemcpyHostToDevice, h->copy_stream));
-    CU(h, cudaMemcpy2DAsync(o + l.u_offset, l.uv_pitch, f + src.u_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
-    if (src.format == VNECT_FMT_I420)
-      CU(h, cudaMemcpy2DAsync(o + l.v_offset, l.uv_pitch, f + src.v_offset, src.uv_pitch, uv_row, H / 2, cudaMemcpyHostToDevice, h->copy_stream));
-  }
+  for (int i = 0; i < n_frames; ++i)
+    if (int rc = stage_frame(h, d + (size_t)i * packed->frame_stride, frames + (size_t)i * src.frame_stride, H, W, src))
+      return rc;
   return VNECT_OK;
 }
 
@@ -1309,6 +1395,147 @@ static int track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
   return lane_acquire(h, 0);  // synchronises and reports non-finite maps
+}
+
+// ------------------------------------------------------------------------------------------------ mixed-size batches
+static_assert(sizeof(vnect_frame) == sizeof(FrameDesc) && sizeof(FrameDesc) == 48 &&
+                  offsetof(vnect_frame, data) == offsetof(FrameDesc, data) &&
+                  offsetof(vnect_frame, height) == offsetof(FrameDesc, height) &&
+                  offsetof(vnect_frame, width) == offsetof(FrameDesc, width) &&
+                  offsetof(vnect_frame, pitch) == offsetof(FrameDesc, pitch) &&
+                  offsetof(vnect_frame, uv_pitch) == offsetof(FrameDesc, uv_pitch) &&
+                  offsetof(vnect_frame, u_offset) == offsetof(FrameDesc, u_offset) &&
+                  offsetof(vnect_frame, v_offset) == offsetof(FrameDesc, v_offset),
+              "the device frame table is a copy of the caller's vnect_frame array");
+
+static FrameSource frame_source(const vnect_frame& f, int format) {
+  FrameSource s = bgr_source(f.pitch, 0);
+  s.format = format;
+  s.uv_pitch = f.uv_pitch;
+  s.u_offset = f.u_offset;
+  s.v_offset = f.v_offset;
+  return s;
+}
+
+// Checks every entry of a mixed-size call's frame table before anything is staged or launched and before any filter
+// state or timestamp mirror is touched; `host`: the frames are staged into the lane's buffer, so each must fit max_input.
+static int check_frames(vnect_t* h, const vnect_frame* frames, int n_frames, int format, bool host) {
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
+  if (!frames) return fail(h, VNECT_E_INVALID, "null frame table");
+  if (format != kFmtBGR && format != VNECT_FMT_NV12 && format != VNECT_FMT_I420)
+    return fail(h, VNECT_E_INVALID, "unknown pixel format %d", format);
+  for (int i = 0; i < n_frames; ++i) {
+    const vnect_frame& f = frames[i];
+    int rc = VNECT_OK;
+    if (!f.data) {
+      rc = fail(h, VNECT_E_INVALID, "null data");
+    } else if (f.height < 2 || f.width < 2) {
+      rc = fail(h, VNECT_E_INVALID, "frame %dx%d smaller than 2x2", f.height, f.width);
+    } else if (host && (rc = check_host_frame_size(h, f.height, f.width))) {
+    } else if (format == kFmtBGR) {
+      if (f.pitch < (int64_t)f.width * 3) rc = fail(h, VNECT_E_INVALID, "pitch %lld smaller than a row", (long long)f.pitch);
+    } else {
+      vnect_yuv_layout l{};
+      l.format = format;
+      l.y_pitch = f.pitch;
+      l.uv_pitch = f.uv_pitch;
+      l.u_offset = f.u_offset;
+      l.v_offset = f.v_offset;
+      rc = check_yuv_layout(h, &l, f.height, f.width);
+    }
+    if (rc) {
+      h->err = "frame " + std::to_string(i) + ": " + h->err;
+      return rc;
+    }
+  }
+  return VNECT_OK;
+}
+
+// vnect_submit_frames / vnect_track_frames once the table is validated: the frames are staged into the lane's buffer
+// one after another (BGR packed tight, YUV in cv2's layout) and the table points at the staged copies
+static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                         const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                         float* joints3d, bool tracked, int32_t* boxes_used) {
+  int rc = lane_acquire(h, lane);
+  if (rc) return rc;
+  uint8_t* d = h->cur->d_frames;
+  for (int i = 0; i < n_frames; ++i) {  // each frame is within max_input, so the sum fits d_frames_bytes
+    const int H = frames[i].height, W = frames[i].width;
+    FrameDesc& t = h->cur->h_table[i];
+    t.data = d;
+    t.height = H;
+    t.width = W;
+    if (format == kFmtBGR) {
+      t.pitch = (int64_t)W * 3;
+      t.uv_pitch = t.u_offset = t.v_offset = 0;
+      d += (size_t)H * W * 3;
+    } else {
+      const vnect_yuv_layout l = packed_yuv_layout(format, H, W);
+      t.pitch = l.y_pitch;
+      t.uv_pitch = l.uv_pitch;
+      t.u_offset = l.u_offset;
+      t.v_offset = l.v_offset;
+      d += (size_t)l.frame_stride;
+    }
+  }
+  // ids, timestamps and the table in one copy; a refused id or timestamp returns before any frame copy is queued
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
+  for (int i = 0; i < n_frames; ++i)
+    if ((rc = stage_frame(h, const_cast<uint8_t*>(h->cur->h_table[i].data), frames[i].data, frames[i].height,
+                          frames[i].width, frame_source(frames[i], format))))
+      return rc;
+  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
+  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
+  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), h->cur->d_out2d, h->cur->d_out3d, tracked)))
+    return rc;
+  CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if (boxes_used)
+    CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaEventRecord(h->cur->done, h->stream));
+  h->cur->pending = true;
+  return tracked ? lane_acquire(h, lane) : VNECT_OK;  // tracked: synchronises and reports non-finite maps
+}
+
+int vnect_submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                        const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                        float* joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
+  if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
+  return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr);
+}
+
+int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                       const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                       float* joints3d, int32_t* boxes_used) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
+  return submit_frames(h, 0, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used);
+}
+
+int vnect_estimate_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                                 const int32_t* stream_ids, const double* t2d, const double* t3d,
+                                 double* dev_joints2d, float* dev_joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
+  int rc = lane_acquire(h, (int)(h->device_calls++ & 1));  // alternate lanes like vnect_estimate_device
+  if (rc) return rc;
+  memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));  // the caller's device pointers as they are
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
+  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
+  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
+  const int lane = (int)(h->cur - h->lanes);
+  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d))) return rc;
+  CU(h, cudaEventRecord(h->cur->done, h->stream));
+  h->cur->pending = true;
+  return VNECT_OK;
 }
 
 int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
@@ -1469,7 +1696,7 @@ int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float*
         for (size_t px = 0; px < plane; ++px) dst[px] = src[px * kJoints];
       }
   CU(h, cudaMemcpyAsync(h->maps, planar.data(), planar.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, false, false))) return rc;
+  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false))) return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (raw_argmax)
@@ -1761,6 +1988,7 @@ double vnect_info(vnect_t* h, const char* key) {
   }
   if (k == "hm_size") return h->hs;
   if (k == "max_forwards") return h->cap_fw;
+  if (k == "cached_graphs") return (double)h->graphs.size();
   return NAN;
 }
 
@@ -1836,7 +2064,7 @@ int vnect_time_prepost(vnect_t* h, int32_t n_frames, int32_t reps, float* pre_ms
     CU(h, cudaEventElapsedTime(&ms, e0, e1));
     if (r >= 0) pre += ms;
     CU(h, cudaEventRecord(e0, h->stream));
-    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, h->cur->d_out2d, h->cur->d_out3d, false, false))) return rc;
+    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false))) return rc;
     CU(h, cudaEventRecord(e1, h->stream));
     CU(h, cudaEventSynchronize(e1));
     CU(h, cudaEventElapsedTime(&ms, e0, e1));

@@ -44,6 +44,72 @@ def yuv_layout(pixel_format, h, w, y_pitch=None, uv_pitch=None, u_offset=None, v
     return lay
 
 
+_FORMATS = {"bgr": _capi.FMT_BGR, **_YUV_FORMATS}
+
+
+def _format_code(pixel_format):
+    if pixel_format not in _FORMATS:
+        raise ValueError(f"pixel_format must be 'bgr', 'nv12' or 'i420', got {pixel_format!r}")
+    return _FORMATS[pixel_format]
+
+
+def frame_table(frames, pixel_format="bgr"):
+    """Host frames of any sizes -> (``vnect_frame`` table as a ctypes array, the arrays it points into, which must
+    stay alive while the call uses them).  "bgr": uint8 [H_i, W_i, 3] arrays with any row pitch; "nv12" / "i420":
+    uint8 [3H_i/2, W_i] arrays in cv2's layout with even sides.  Raises ValueError on anything else."""
+    _format_code(pixel_format)
+    frames = list(frames)
+    if not frames:
+        raise ValueError("no frames")
+    table, keep = (_capi.Frame * len(frames))(), []
+    for i, f in enumerate(frames):
+        f = np.asarray(f)
+        if pixel_format == "bgr":
+            if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3:
+                raise ValueError(f"frame {i}: BGR frames must be uint8 [H,W,3], got {f.dtype} {f.shape}")
+            st = f.strides
+            if not (st[2] == 1 and st[1] == 3 and st[0] >= f.shape[1] * 3):
+                f = np.ascontiguousarray(f)
+            h, w = f.shape[:2]
+            table[i] = _capi.Frame(f.ctypes.data, h, w, f.strides[0], 0, 0, 0)
+        else:
+            if f.dtype != np.uint8 or f.ndim != 2 or f.shape[0] % 3 or f.shape[0] == 0:
+                raise ValueError(f"frame {i}: {pixel_format} frames must be uint8 [3H/2,W], got {f.dtype} {f.shape}")
+            h, w = f.shape[0] // 3 * 2, f.shape[1]
+            if h % 2 or w % 2:
+                raise ValueError(f"frame {i}: {pixel_format} frames need an even height and width, got {h}x{w}")
+            f = np.ascontiguousarray(f)
+            lay = yuv_layout(pixel_format, h, w)
+            table[i] = _capi.Frame(f.ctypes.data, h, w, lay.y_pitch, lay.uv_pitch, lay.u_offset, lay.v_offset)
+        keep.append(f)
+    return table, keep
+
+
+def device_frame_table(frames, pixel_format="bgr"):
+    """Device frames -> ``vnect_frame`` table.  Each frame is a dict {ptr, h, w} plus, for BGR, an optional ``pitch``
+    (default 3w) or, for "nv12" / "i420", optional yuv_layout() fields (y_pitch, uv_pitch, u_offset, v_offset;
+    default cv2's contiguous layout)."""
+    _format_code(pixel_format)
+    frames = list(frames)
+    if not frames:
+        raise ValueError("no frames")
+    table = (_capi.Frame * len(frames))()
+    for i, d in enumerate(frames):
+        d = dict(d)
+        ptr, h, w = int(d.pop("ptr")), int(d.pop("h")), int(d.pop("w"))
+        if pixel_format == "bgr":
+            pitch = d.pop("pitch", None)
+            if d:
+                raise ValueError(f"frame {i}: unknown BGR frame fields {sorted(d)}")
+            table[i] = _capi.Frame(ptr, h, w, w * 3 if pitch is None else pitch, 0, 0, 0)
+        else:
+            if set(d) - {"y_pitch", "uv_pitch", "u_offset", "v_offset", "frame_stride"}:
+                raise ValueError(f"frame {i}: unknown YUV frame fields {sorted(d)}")
+            lay = yuv_layout(pixel_format, h, w, **d)
+            table[i] = _capi.Frame(ptr, h, w, lay.y_pitch, lay.uv_pitch, lay.u_offset, lay.v_offset)
+    return table
+
+
 class VNectEngine:
     """Batched estimator: ``estimate(frames[n,H,W,3] uint8 BGR) -> (joints_2d [n,21,2] f64, joints_3d [n,21,3] f32)``.
 
@@ -194,6 +260,25 @@ class VNectEngine:
         self._inflight[int(lane)] = (frames, j2, j3)  # keep the buffers alive
         return j2, j3
 
+    def estimate_frames(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """estimate() for frames of different sizes in one batch: ``frames`` is a sequence of host arrays as
+        frame_table() takes them.  Frame i gives exactly what estimate() gives for that frame alone."""
+        j2, j3 = self.submit_frames(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+        self.wait(0)
+        return j2, j3
+
+    def submit_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """submit() for frames of different sizes (see estimate_frames); completes with wait(lane)."""
+        table, keep = frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        self._check(self._lib.vnect_submit_frames(self._h, int(lane), table, n, _format_code(pixel_format), _ptr(ids),
+                                                  _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[int(lane)] = (keep, j2, j3)  # keep the buffers alive
+        return j2, j3
+
     def wait(self, lane):
         self._check(self._lib.vnect_wait(self._h, int(lane)))
         return self.__dict__.get("_inflight", {}).pop(int(lane), (None, None, None))[1:]
@@ -220,6 +305,29 @@ class VNectEngine:
         self._check(fn(self._h, _ptr(frames), n, h, w, *layout, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3),
                        _ptr(boxes)))
         return j2, j3, boxes
+
+    def track_frames(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr"):
+        """track() for streams whose full frames differ in size: each frame is cropped by its stream's box clipped to
+        that frame.  Returns (joints_2d [n,21,2], joints_3d [n,21,3], boxes_used [n,4])."""
+        table, keep = frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
+        boxes = np.empty((n, 4), np.int32)
+        self._check(self._lib.vnect_track_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids), _ptr(t2d),
+                                                 _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
+        return j2, j3, boxes
+
+    def estimate_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
+                               pixel_format="bgr"):
+        """estimate_device() for device frames of different sizes, each at its own address (e.g. one tensor or
+        decoder surface per camera): ``frames`` as device_frame_table() takes them.  Asynchronous."""
+        table = device_frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        self._check(self._lib.vnect_estimate_device_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids),
+                                                           _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
+                                                           C.c_void_p(dev_j3_ptr)))
 
     def estimate_device(self, dev_frames_ptr, n, h, w, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
                         pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
