@@ -176,6 +176,41 @@ int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, 
                        const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                        float* joints3d, int32_t* boxes_used);
 
+/* Pipelined and device-resident tracking: the loop body of run_estimator.py:98-119 without waiting for the GPU.
+ * vnect_track / vnect_track_frames synchronise, so the upload of the next step's full frames cannot overlap this
+ * step's kernels, and frames already in device memory would have to round-trip through the host.  The calls below
+ * take the vnect_frame table of vnect_track_frames (same validation, same errors, in the same order) and return
+ * once the work is enqueued.  Every tracked call runs on the handle's stream in submission order, so frame i of an
+ * asynchronous call gives bit for bit what vnect_track_frames gives for the same submission order -- joints_2d,
+ * joints_3d, boxes_used, the raw argmax, the box left behind, the filter state, the timestamps and the packed
+ * results -- also when consecutive frames of one stream go to different lanes and when lane 1 is submitted before
+ * lane 0 has been waited on.  A refused call stages and launches nothing and touches no box, filter state or
+ * timestamp.  CUDA graphs are keyed by lane, frame count, format and output pointers, as for the other table calls:
+ * a moving crop, a decoder's rotating surfaces and changing camera sizes replay the same graph.
+ * vnect_track_set_box, vnect_track_get_box, vnect_reset_stream, vnect_get_raw_argmax and vnect_export /
+ * import_stream_state keep their synchronous meaning: they act after everything already submitted.  Waiting for
+ * the GPU there does not complete a lane: NaN / Inf maps of its batch are still reported by its vnect_wait. */
+
+/* vnect_track_frames on submission lane 0 or 1, completed by vnect_wait(h, lane) like vnect_submit: HOST frames
+ * (staged into the lane's buffer), HOST results (boxes_used optional).  frames' pixels, joints2d, joints3d and
+ * boxes_used must stay valid until the wait (pinned memory makes the copies truly asynchronous); NaN / Inf maps are
+ * reported by the wait or by the next use of the lane. */
+int vnect_submit_track_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                              const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                              float* joints3d, int32_t* boxes_used);
+/* vnect_track_frames on DEVICE full frames (e.g. a decoder's surfaces or one tensor per camera, pointers used as they
+ * are) with DEVICE results: dev_joints2d float64 [n][21][2], dev_joints3d float32 [n][21][3], dev_boxes_used
+ * (optional) int32 [n][4].  Asynchronous on the handle's stream, like vnect_estimate_device_frames. */
+int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                              const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
+                              float* dev_joints3d, int32_t* dev_boxes_used);
+/* vnect_track_set_box for n streams at once, in submission order: after every call already submitted and before
+ * every later one, without the host waiting for the GPU.  stream_ids int32 [n] and xywh int32 [n][4] are HOST arrays,
+ * copied by the call; n = 0 does nothing.  Refused before anything is enqueued: n below 0, a null array, and as
+ * vnect_track_set_box refuses one box, an id outside [0, max_streams), an id given twice, x or y below 0, w or h
+ * below 2. */
+int vnect_track_set_boxes(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* xywh);
+
 /* replaces VNectEstimator.gen_input_batch (src/estimator.py:70-81): out float32 [n_frames*n_scales][S][S][3]
  * (fp16-rounded values of the network input), scaler_offsets float64 [3] = {scaler, offset_x, offset_y} */
 int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,

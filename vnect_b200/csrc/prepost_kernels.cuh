@@ -1209,6 +1209,21 @@ __global__ void track_update_frames_kernel(const double* __restrict__ joints2d, 
   track_box_update(joints2d, stream_ids, f, frames[f].height, frames[f].width, boxes);
 }
 
+// vnect_track_set_boxes: up to kSeedBoxes seeded boxes travel in the kernel's parameters, so the caller's arrays are
+// free once the launch returns and the write lands in stream order between the tracked calls around it.  Ids are
+// distinct (checked on the host), so one thread per box writes without conflicts.
+constexpr int kSeedBoxes = 64;
+struct BoxSeeds {
+  int4 box[kSeedBoxes];  // (x, y, w, h)
+  int stream_id[kSeedBoxes];
+  int n;
+};
+
+__global__ void track_seed_boxes_kernel(const __grid_constant__ BoxSeeds s, int4* __restrict__ boxes) {
+  const int i = threadIdx.x;
+  if (i < s.n) boxes[s.stream_id[i]] = s.box[i];
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Joints2Angles (reference: src/joints2angles.py:60-110): eight arm angles of a robot from the 3D joints -- the step
 // right after the hot path for the robot use case (SURVEY.md section 8f row 4).  One thread per frame.  The reference

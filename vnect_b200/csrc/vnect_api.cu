@@ -111,7 +111,7 @@ struct vnect_handle {
   // CUDA graphs of the kernel sequence of one estimate call, keyed by everything baked into the kernel parameters.
   // First use of a key runs directly (warm-up), the second captures, later ones replay: ~50 launches -> 1.
   // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset).
-  // Mixed-size calls read sizes and addresses from the lane's device table, so only (4 + lane + tracked, n_frames,
+  // Mixed-size calls read sizes and addresses from the lane's device table, so only (4 + lane + 2 * tracked, n_frames,
   // out2d, out3d, format) is set in their key: one graph serves every composition of a batch.
   typedef std::tuple<int, int, int, int, long long, long long, const void*, const void*, const void*, int, long long,
                      long long, long long> GraphKey;
@@ -1451,11 +1451,12 @@ static int check_frames(vnect_t* h, const vnect_frame* frames, int n_frames, int
   return VNECT_OK;
 }
 
-// vnect_submit_frames / vnect_track_frames once the table is validated: the frames are staged into the lane's buffer
-// one after another (BGR packed tight, YUV in cv2's layout) and the table points at the staged copies
+// vnect_submit_frames / vnect_track_frames / vnect_submit_track_frames once the table is validated: the frames are
+// staged into the lane's buffer one after another (BGR packed tight, YUV in cv2's layout) and the table points at the
+// staged copies.  `synchronous`: wait for the lane before returning (vnect_track_frames).
 static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
-                         float* joints3d, bool tracked, int32_t* boxes_used) {
+                         float* joints3d, bool tracked, int32_t* boxes_used, bool synchronous) {
   int rc = lane_acquire(h, lane);
   if (rc) return rc;
   uint8_t* d = h->cur->d_frames;
@@ -1494,7 +1495,29 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
     CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
-  return tracked ? lane_acquire(h, lane) : VNECT_OK;  // tracked: synchronises and reports non-finite maps
+  return synchronous ? lane_acquire(h, lane) : VNECT_OK;  // synchronises and reports non-finite maps
+}
+
+// vnect_estimate_device_frames / vnect_track_device_frames once the table is validated: the caller's device pointers
+// are used as they are; the lanes alternate for the per-call meta so the host can run one call ahead of the GPU
+static int device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                         const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
+                         float* dev_joints3d, bool tracked, int32_t* dev_boxes_used) {
+  int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
+  if (rc) return rc;
+  memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
+  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
+  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
+  const int lane = (int)(h->cur - h->lanes);
+  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d, tracked)))
+    return rc;
+  if (dev_boxes_used)  // outside the graph, so the caller's pointer stays out of its key
+    CU(h, cudaMemcpyAsync(dev_boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToDevice,
+                          h->stream));
+  CU(h, cudaEventRecord(h->cur->done, h->stream));
+  h->cur->pending = true;
+  return VNECT_OK;
 }
 
 int vnect_submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
@@ -1505,7 +1528,8 @@ int vnect_submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
-  return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr);
+  return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr,
+                       false);
 }
 
 int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
@@ -1515,7 +1539,30 @@ int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, 
   ON_DEVICE(h);
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
-  return submit_frames(h, 0, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used);
+  return submit_frames(h, 0, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used,
+                       true);
+}
+
+// Pipelined and device-resident tracking.  A tracked call no longer has to wait for its results: every kernel that
+// reads or writes tracking state runs on the handle's stream in submission order, whichever lane carried the call.
+//   d_boxes         frame_geometry_kernel of call k+1 reads the box track_update_frames_kernel of call k wrote.
+//   d_boxes_used    written by call k's geometry kernel, read by call k's copy-out; both on the handle's stream, and
+//                   call k+1's geometry kernel is enqueued after that copy.
+//   d_raw_argmax    written by every call's post-process; vnect_get_raw_argmax waits for all lanes, so it reads the
+//                   most recent call's.
+//   d_geoms         the uniform tracked path's geometry; the table path uses the lane's own L.d_geoms.
+// What a lane stages (meta, table, frames) is only rewritten after lane_acquire has waited for that lane's previous
+// call, as for vnect_submit.
+int vnect_submit_track_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                              const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                              float* joints3d, int32_t* boxes_used) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
+  if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
+  return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used,
+                       false);
 }
 
 int vnect_estimate_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
@@ -1525,17 +1572,18 @@ int vnect_estimate_device_frames(vnect_t* h, const vnect_frame* frames, int32_t 
   ON_DEVICE(h);
   if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
-  int rc = lane_acquire(h, (int)(h->device_calls++ & 1));  // alternate lanes like vnect_estimate_device
-  if (rc) return rc;
-  memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));  // the caller's device pointers as they are
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
-  CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
-  CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  const int lane = (int)(h->cur - h->lanes);
-  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d))) return rc;
-  CU(h, cudaEventRecord(h->cur->done, h->stream));
-  h->cur->pending = true;
-  return VNECT_OK;
+  return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, false, nullptr);
+}
+
+int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                              const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
+                              float* dev_joints3d, int32_t* dev_boxes_used) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
+  return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, true,
+                       dev_boxes_used);
 }
 
 int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
@@ -1594,6 +1642,38 @@ int vnect_track_set_box(vnect_t* h, int32_t stream_id, int32_t x, int32_t y, int
   const int4 b = make_int4(x, y, w, hh);
   CU(h, cudaStreamSynchronize(h->stream));
   CU(h, cudaMemcpy(h->d_boxes + stream_id, &b, sizeof b, cudaMemcpyHostToDevice));
+  return VNECT_OK;
+}
+
+int vnect_track_set_boxes(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* xywh) {
+  if (!h || !h->d_boxes) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (n < 0) return fail(h, VNECT_E_INVALID, "n %d below 0", n);
+  if (n == 0) return VNECT_OK;
+  if (!stream_ids || !xywh) return fail(h, VNECT_E_INVALID, "null buffer");
+  h->seen_stamp.resize(h->cfg.max_streams, 0);
+  const unsigned int stamp = ++h->seen_epoch;
+  for (int i = 0; i < n; ++i) {  // everything is checked before the first launch
+    const int sid = stream_ids[i];
+    const int32_t* b = xywh + 4 * i;
+    if (sid < 0 || sid >= h->cfg.max_streams) return fail(h, VNECT_E_INVALID, "stream id %d not in [0, %d)", sid, h->cfg.max_streams);
+    if (h->seen_stamp[sid] == stamp) return fail(h, VNECT_E_INVALID, "stream id %d appears twice", sid);
+    h->seen_stamp[sid] = stamp;
+    if (b[0] < 0 || b[1] < 0 || b[2] < 2 || b[3] < 2)
+      return fail(h, VNECT_E_INVALID, "box %d of stream %d must have x, y >= 0 and w, h >= 2", i, sid);
+  }
+  for (int i0 = 0; i0 < n; i0 += kSeedBoxes) {
+    BoxSeeds s;
+    s.n = std::min(kSeedBoxes, n - i0);
+    for (int i = 0; i < s.n; ++i) {
+      const int32_t* b = xywh + 4 * (i0 + i);
+      s.box[i] = make_int4(b[0], b[1], b[2], b[3]);
+      s.stream_id[i] = stream_ids[i0 + i];
+    }
+    track_seed_boxes_kernel<<<1, kSeedBoxes, 0, h->stream>>>(s, h->d_boxes);
+    CU(h, cudaGetLastError());
+    ++h->launches;
+  }
   return VNECT_OK;
 }
 
@@ -1759,13 +1839,11 @@ int vnect_filter(vnect_t* h, int32_t stream_id, int32_t dim, int32_t values_are_
   return VNECT_OK;
 }
 
-// waits for every submitted batch: the per-call scratch (raw argmax) and the per-stream state are then at rest
+// waits for every submitted batch: the per-call scratch (raw argmax) and the per-stream state are then at rest.  A lane
+// stays pending, so that its vnect_wait (or its next use) still reports NaN / Inf maps of the batch it carried.
 static int quiesce(vnect_t* h) {
   for (auto& L : h->lanes)
-    if (L.pending) {
-      CU(h, cudaEventSynchronize(L.done));
-      L.pending = false;
-    }
+    if (L.pending) CU(h, cudaEventSynchronize(L.done));
   CU(h, cudaStreamSynchronize(h->stream));
   return VNECT_OK;
 }

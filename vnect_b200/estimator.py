@@ -110,6 +110,61 @@ def device_frame_table(frames, pixel_format="bgr"):
     return table
 
 
+def uniform_frame_table(frames, pixel_format="bgr"):
+    """A batch of equal-size host frames as track() takes it -> (``vnect_frame`` table, the array it points into).
+    Entry i is a view of frame i: its address, the array's row pitch and, between entries, the array's frame stride.
+    Nothing is copied unless the rows are not byte-packed, or for I420 not contiguous (its chroma planes then have no
+    single pitch).  "bgr": uint8 [n,H,W,3] or [H,W,3]; "nv12" / "i420": uint8 [n,3H/2,W] or [3H/2,W].  Raises
+    ValueError on anything else."""
+    _format_code(pixel_format)
+    if pixel_format == "bgr":
+        frames, st = VNectEngine._frames(frames)
+        n, h, w = frames.shape[:3]
+        table = (_capi.Frame * n)()
+        for i in range(n):
+            table[i] = _capi.Frame(frames.ctypes.data + i * st[0], h, w, st[1], 0, 0, 0)
+        return table, frames
+    frames = np.asarray(frames)
+    if frames.ndim == 2:
+        frames = frames[None]
+    if frames.dtype != np.uint8 or frames.ndim != 3 or frames.shape[1] % 3 or 0 in frames.shape:
+        raise ValueError(f"{pixel_format} frames must be uint8 [n,3H/2,W] or [3H/2,W], got {frames.dtype} "
+                         f"{frames.shape}")
+    n, h, w = frames.shape[0], frames.shape[1] // 3 * 2, frames.shape[2]
+    if h % 2 or w % 2:
+        raise ValueError(f"{pixel_format} frames need an even height and width, got {h}x{w}")
+    st = frames.strides
+    if not (st[2] == 1 and st[1] >= w and st[0] >= 0 and (pixel_format == "nv12" or st[1] == w)):
+        frames = np.ascontiguousarray(frames)
+        st = frames.strides
+    lay = yuv_layout(pixel_format, h, w, y_pitch=st[1])
+    table = (_capi.Frame * n)()
+    for i in range(n):
+        table[i] = _capi.Frame(frames.ctypes.data + i * st[0], h, w, lay.y_pitch, lay.uv_pitch, lay.u_offset,
+                               lay.v_offset)
+    return table, frames
+
+
+def strided_device_frames(dev_frames_ptr, n, h, w, pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
+    """The n frames estimate_device() describes (frame i at ``dev_frames_ptr + i * frame_stride``) as the list of
+    frames device_frame_table() takes.  BGR: ``pitch`` (default 3w) and ``frame_stride`` (default pitch * h); YUV:
+    ``layout``, a dict of yuv_layout() fields (default cv2's contiguous layout)."""
+    _format_code(pixel_format)
+    if n < 1:
+        raise ValueError(f"n must be at least 1, got {n}")
+    if pixel_format == "bgr":
+        if layout is not None:
+            raise ValueError("BGR frames are described by pitch / frame_stride, not by `layout`")
+        pitch = w * 3 if pitch is None else int(pitch)
+        stride = pitch * h if frame_stride is None else int(frame_stride)
+        return [dict(ptr=int(dev_frames_ptr) + i * stride, h=h, w=w, pitch=pitch) for i in range(n)]
+    if pitch is not None or frame_stride is not None:
+        raise ValueError("YUV frames are described by `layout`, not by pitch / frame_stride")
+    lay = yuv_layout(pixel_format, h, w, **(layout or {}))
+    planes = dict(y_pitch=lay.y_pitch, uv_pitch=lay.uv_pitch, u_offset=lay.u_offset, v_offset=lay.v_offset)
+    return [dict(ptr=int(dev_frames_ptr) + i * lay.frame_stride, h=h, w=w, **planes) for i in range(n)]
+
+
 class VNectEngine:
     """Batched estimator: ``estimate(frames[n,H,W,3] uint8 BGR) -> (joints_2d [n,21,2] f64, joints_3d [n,21,3] f32)``.
 
@@ -280,6 +335,8 @@ class VNectEngine:
         return j2, j3
 
     def wait(self, lane):
+        """Completes the lane's submission: (joints_2d, joints_3d), or (joints_2d, joints_3d, boxes_used) after
+        submit_track / submit_track_frames."""
         self._check(self._lib.vnect_wait(self._h, int(lane)))
         return self.__dict__.get("_inflight", {}).pop(int(lane), (None, None, None))[1:]
 
@@ -317,6 +374,59 @@ class VNectEngine:
         self._check(self._lib.vnect_track_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids), _ptr(t2d),
                                                  _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
         return j2, j3, boxes
+
+    def submit_track(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """Pipelined track(): enqueue one tracked step on lane 0/1 and return (joints_2d, joints_3d, boxes_used)
+        arrays that are filled once wait(lane) returns.  Same frames as track(); the call reads them in place
+        (uniform_frame_table), so they, and ``out`` if given, must stay alive until the wait (pinned memory makes the
+        copies truly asynchronous).  Steps of one stream may alternate between the lanes."""
+        table, keep = uniform_frame_table(frames, pixel_format)
+        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format)
+
+    def submit_track_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """submit_track() for streams whose full frames differ in size, as track_frames() takes them."""
+        table, keep = frame_table(frames, pixel_format)
+        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format)
+
+    def _submit_track(self, lane, table, keep, stream_ids, t2d, t3d, out, pixel_format):
+        n = len(table)
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        j2, j3, boxes = out if out is not None else (np.empty((n, JOINTS, 2), np.float64),
+                                                     np.empty((n, JOINTS, 3), np.float32), np.empty((n, 4), np.int32))
+        self._check(self._lib.vnect_submit_track_frames(self._h, int(lane), table, n, _format_code(pixel_format),
+                                                        _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3),
+                                                        _ptr(boxes)))
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[int(lane)] = (keep, j2, j3, boxes)  # keep the buffers alive
+        return j2, j3, boxes
+
+    def track_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr=None, stream_ids=None, t2d=None,
+                            t3d=None, pixel_format="bgr"):
+        """track_frames() on device full frames (``frames`` as device_frame_table() takes them) with device results:
+        joints_2d float64 [n,21,2], joints_3d float32 [n,21,3] and, when ``dev_boxes_ptr`` is given, boxes_used int32
+        [n,4].  Asynchronous on the engine's stream."""
+        table = device_frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        self._check(self._lib.vnect_track_device_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids),
+                                                        _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
+                                                        C.c_void_p(dev_j3_ptr),
+                                                        C.c_void_p(dev_boxes_ptr) if dev_boxes_ptr else None))
+
+    def track_device(self, dev_frames_ptr, n, h, w, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr=None, stream_ids=None,
+                     t2d=None, t3d=None, pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
+        """track_device_frames() on n equal-size device frames described as estimate_device() takes them."""
+        frames = strided_device_frames(dev_frames_ptr, n, h, w, pitch, frame_stride, pixel_format, layout)
+        self.track_device_frames(frames, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr, stream_ids, t2d, t3d, pixel_format)
+
+    def set_boxes(self, stream_ids, rects):
+        """set_box() for several streams, in submission order: after every call already submitted and before every
+        later one, without waiting for the GPU."""
+        ids = np.ascontiguousarray(stream_ids, dtype=np.int32).reshape(-1)
+        rects = np.ascontiguousarray(rects, dtype=np.int32)
+        if rects.shape != (len(ids), 4):
+            raise ValueError(f"expected one (x, y, w, h) per stream id: {len(ids)} ids, rects {rects.shape}")
+        self._check(self._lib.vnect_track_set_boxes(self._h, len(ids), _ptr(ids), _ptr(rects)))
 
     def estimate_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
                                pixel_format="bgr"):
