@@ -56,6 +56,8 @@ def resize_u8_int(img, fx, fy):
     """Integer restatement of cv2.resize(u8, (0,0), fx, fy, INTER_LINEAR); bit-exact (utils.py:13-21 call site)."""
     h, w = img.shape[:2]
     dw, dh = cv_round(w * fx), cv_round(h * fy)
+    if (dh, dw) == (h, w):  # cv::resize copies when dsize == ssize, whatever fx and fy are
+        return img.copy()
     ix, ffx = linear_coords(dw, w, 1.0 / fx, True)
     iy, ffy = linear_coords(dh, h, 1.0 / fy, False)
     one, sc = np.float32(1), np.float32(2048)
@@ -77,6 +79,8 @@ def resize_f32_np(img, fx, fy):
     assert img.dtype == np.float32
     h, w = img.shape[:2]
     dw, dh = cv_round(w * fx), cv_round(h * fy)
+    if (dh, dw) == (h, w):  # cv::resize copies when dsize == ssize (a scale s > hs / (hs + 0.5) of a heat-map)
+        return img.copy()
     ix, ffx = linear_coords(dw, w, 1.0 / fx, True)
     iy, ffy = linear_coords(dh, h, 1.0 / fy, False)
     ix1 = np.minimum(ix + 1, w - 1)

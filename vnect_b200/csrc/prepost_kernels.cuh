@@ -638,9 +638,11 @@ __device__ __forceinline__ float scaled_cell(const float* __restrict__ m, int hs
 }
 
 // Candidate k (0 .. 2*hs-1) of the x8 upsample along one axis: destination index d, source cell i, fraction f.
-// Between two source cell centres the upsample is monotonic, so its maximum over the 8 samples of a segment sits at
-// the first (f = 1/16) or last (f = 15/16) one; d = 0 stands for the exactly-tied samples 0..3 and d = 8*(hs-1)+4 for
-// the last four (SURVEY.md App. C.4), where the first index wins like np.argmax.
+// Between two source cell centres the EXACT bilinear upsample is affine, so its maximum over the 8 samples of a segment
+// sits at the first (f = 1/16) or last (f = 15/16) one; d = 0 stands for the exactly-tied samples 0..3 and
+// d = 8*(hs-1)+4 for the last four (SURVEY.md App. C.4), where the first index wins like np.argmax.  The ROUNDED
+// upsample is not monotonic on a quad whose corners agree to ~1e-11 relative: an interior sample can then beat or tie
+// (at an earlier index) both ends, so step D rescans every sample of the quads near the best candidate.
 __device__ __forceinline__ void upsample_candidate(int k, int hs, int* d, int* i, double* f) {
   if (k == 0) { *d = 0; *i = 0; *f = 0.0; return; }
   if (k == 2 * hs - 1) { *d = 8 * (hs - 1) + 4; *i = hs - 1; *f = 0.0; return; }
@@ -649,11 +651,36 @@ __device__ __forceinline__ void upsample_candidate(int k, int hs, int* d, int* i
   else             { *d = 8 * r + 4;  *i = r; *f = 0.0625; }
 }
 
+// Sample j along one axis of the quad whose first cell is q: the samples with source cell q (d = 8q+4 .. 8q+11,
+// f = 1/16 .. 15/16), plus d = 0 (f = 0) ahead of them for q = 0; the last cell has the one sample d = 8(hs-1)+4.
+// An axis has 9, 8 or 1 of them (upsample_axis_len); together the quads cover every sample exactly once.
+__device__ __forceinline__ int upsample_axis_len(int q, int hs) { return q == hs - 1 ? 1 : q == 0 ? 9 : 8; }
+__device__ __forceinline__ void upsample_sample(int q, int j, int hs, int* d, double* f) {
+  if (q == hs - 1) { *d = 8 * q + 4; *f = 0.0; return; }
+  if (q == 0) {
+    if (j == 0) { *d = 0; *f = 0.0; return; }
+    --j;
+  }
+  *d = 8 * q + 4 + j;
+  *f = (double)(2 * j + 1) * 0.0625;
+}
+
 // OpenCV+IPP's float64 x8 upsample at fractions (fy, fx) inside the source quad (s00 s01 / s10 s11): fma per axis
 __device__ __forceinline__ double upsample_quad(double s00, double s01, double s10, double s11, double fy, double fx) {
   const double h0 = __fma_rn(__dsub_rn(s01, s00), fx, s00);
   const double h1 = __fma_rn(__dsub_rn(s11, s10), fx, s10);
   return __fma_rn(__dsub_rn(h1, h0), fy, h0);
+}
+
+// Rounding of upsample_quad against the exact bilinear value, relative to M = the largest |corner|: each difference
+// errs by <= u * 2M (u = 2^-53), each row fma by <= 2uM + u(M + 2uM), the column step adds <= 2uM + uM: in all
+// < 6.01 uM.  The window 2e = 2^-49 M (e = 8uM) keeps a further ~4uM for the rounding of `best - 2e` itself.
+// A sample's exact value is at most its quad's best exact candidate (the exact upsample is affine per axis), so a
+// sample that ties or beats the best COMPUTED candidate B lies in a quad whose best computed candidate is >= B - 2e.
+// A quad with four equal corners rounds every sample to that value; its first sample is a candidate already.
+__device__ __forceinline__ bool quad_needs_scan(double e00, double e01, double e10, double e11, double cand, double b) {
+  const double m = fmax(fmax(fabs(e00), fabs(e01)), fmax(fabs(e10), fabs(e11)));
+  return !(e00 == e01 && e00 == e10 && e00 == e11) && cand >= b - m * 0x1p-49;
 }
 
 __device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gsrc) {
@@ -707,9 +734,11 @@ __device__ __forceinline__ double oef_finish(FilterState& st, const FilterCfg& c
 //     cell below (bound - 1e-6 * largest |sum|) provably cannot belong to the source quad of the argmax (an upsampled
 //     value is a convex combination of its quad), so only the quads around the few remaining cells survive;
 //  D. the survivors are evaluated EXACTLY as the reference does (float64 accumulation over the scales, /= n,
-//     OpenCV+IPP's fma upsample), ties to the first index like np.argmax.  Pruning only removes candidates that
-//     cannot win, so the result equals the exhaustive float64 scan bit for bit; if more than kQuadCap quads survive
-//     (flat or saturated maps) every quad that passes the same test is scanned in place;
+//     OpenCV+IPP's fma upsample), ties to the first index like np.argmax: first their candidates (upsample_candidate),
+//     then every sample of the quads whose best candidate is within the rounding window of the block's best one
+//     (quad_needs_scan; usually just the winning quad).  Pruning only removes samples that cannot win, so the result
+//     equals the exhaustive float64 scan bit for bit; if more than kQuadCap quads survive (flat or saturated maps)
+//     every quad that passes the same test is evaluated in place;
 //  E. 2D 1-euro filters, location-map gather at the FILTERED point, and -- in the last block of the frame to arrive --
 //     root subtraction, 3D filters and the rescale to input pixels.
 #define POST_TRACE(i) do { if (p.trace != nullptr && threadIdx.x == 0) p.trace[(size_t)blockIdx.x * 16 + (i)] = globaltimer_ns(); } while (0)
@@ -960,9 +989,34 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
   };
   double best = -INFINITY;
   int best_idx = 0x7fffffff;
+  auto take = [&](double v, int idx) {
+    if (v > best || (v == best && idx < best_idx)) { best = v; best_idx = idx; }
+  };
+  auto warp_best = [&]() {  // (best, best_idx) of the warp in every lane
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double ov = __shfl_xor_sync(0xffffffffu, best, o);
+      const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
+      if (ov > best || (ov == best && oi < best_idx)) { best = ov; best_idx = oi; }
+    }
+  };
+  // samples first, first + step, ... (row-major) of every sample of quad (qy, qx)
+  auto scan_quad = [&](int qy, int qx, double e00, double e01, double e10, double e11, int first, int step) {
+    const int nx = upsample_axis_len(qx, hs), n = upsample_axis_len(qy, hs) * nx;
+    for (int i = first; i < n; i += step) {
+      const int jy = i / nx;
+      int dy, dx;
+      double fy, fx;
+      upsample_sample(qy, jy, hs, &dy, &fy);
+      upsample_sample(qx, i - jy * nx, hs, &dx, &fx);
+      take(upsample_quad(e00, e01, e10, e11, fy, fx), dy * S + dx);
+    }
+  };
   // quad = cells (qy, qy+1) x (qx, qx+1), clamped; its axis candidates: cell 0: k = 0..2, cell i: k = 2i+1, 2i+2, the
-  // last cell: k = 2*hs-1
-  auto eval_quad = [&](int qy, int qx) {
+  // last cell: k = 2*hs-1.  First look (b = -INFINITY): the candidates; returns whether the quad is within the window
+  // of this thread's best so far, a superset of the quads within the window of the block's best.  Second look (b = the
+  // block's best candidate): the candidates again, and every sample if the quad is within the window of b.
+  auto eval_quad = [&](int qy, int qx, double b) -> bool {
     const int qy1 = min(qy + 1, hs - 1), qx1 = min(qx + 1, hs - 1);
     const double e00 = exact_cell(qy, qx);
     const double e01 = qx1 == qx ? e00 : exact_cell(qy, qx1);
@@ -970,6 +1024,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
     const double e11 = qy1 == qy ? e01 : (qx1 == qx ? e10 : exact_cell(qy1, qx1));
     const int ky_lo = qy == 0 ? 0 : 2 * qy + 1, ky_hi = qy == hs - 1 ? nc - 1 : 2 * qy + 2;
     const int kx_lo = qx == 0 ? 0 : 2 * qx + 1, kx_hi = qx == hs - 1 ? nc - 1 : 2 * qx + 2;
+    double cand = -INFINITY;
     for (int ky = ky_lo; ky <= ky_hi; ++ky) {
       int dy, iy;
       double fy;
@@ -979,10 +1034,13 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
         double fx;
         upsample_candidate(kx, hs, &dx, &ix, &fx);
         const double v = upsample_quad(e00, e01, e10, e11, fy, fx);
-        const int idx = dy * S + dx;
-        if (v > best || (v == best && idx < best_idx)) { best = v; best_idx = idx; }
+        cand = fmax(cand, v);
+        take(v, dy * S + dx);
       }
     }
+    if (b == -INFINITY) return quad_needs_scan(e00, e01, e10, e11, cand, best);
+    if (quad_needs_scan(e00, e01, e10, e11, cand, b)) scan_quad(qy, qx, e00, e01, e10, e11, 0, 1);
+    return false;
   };
   const int nq = s_nq;
   const bool one_warp = nq <= kQuadPar;  // the usual case: a handful of quads
@@ -1000,6 +1058,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
       o[0] = f.freq; o[1] = f.te; o[2] = f.a_d;
     }
   }
+  unsigned second = 0;  // bit k: the k-th quad this thread evaluated needs a second look (k < hs / rpp <= 32)
   if (one_warp) {
     // every cell of every surviving quad on its own thread, then every candidate on its own lane of warp 0
     for (int i = tid; i < nq * 4; i += nthreads) {
@@ -1010,44 +1069,87 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
     __syncthreads();
     if (p.trace != nullptr && tid == 0) p.trace[(size_t)blockIdx.x * 16 + 14] = globaltimer_ns();
     if (warp_id == 0) {
-      for (int i = lane_id; i < nq * 9; i += 32) {
+      // candidate slot -> its value; returns false for the slots a border quad does not have
+      auto candidate = [&](int i, double* v, int* idx) -> bool {
         const int qi = i / 9, slot = i - qi * 9;
         const int q = s_quads[qi];
         const int qy = q / hs, qx = q - qy * hs;
         const int ky = (qy == 0 ? 0 : 2 * qy + 1) + slot / 3, kx = (qx == 0 ? 0 : 2 * qx + 1) + slot % 3;
-        if (ky > (qy == hs - 1 ? nc - 1 : 2 * qy + 2) || kx > (qx == hs - 1 ? nc - 1 : 2 * qx + 2)) continue;
+        if (ky > (qy == hs - 1 ? nc - 1 : 2 * qy + 2) || kx > (qx == hs - 1 ? nc - 1 : 2 * qx + 2)) return false;
         int dy, dx, iy, ix;
         double fy, fx;
         upsample_candidate(ky, hs, &dy, &iy, &fy);
         upsample_candidate(kx, hs, &dx, &ix, &fx);
-        const double v = upsample_quad(s_exact[qi * 4], s_exact[qi * 4 + 1], s_exact[qi * 4 + 2], s_exact[qi * 4 + 3], fy, fx);
-        const int idx = dy * S + dx;
-        if (v > best || (v == best && idx < best_idx)) { best = v; best_idx = idx; }
+        *v = upsample_quad(s_exact[qi * 4], s_exact[qi * 4 + 1], s_exact[qi * 4 + 2], s_exact[qi * 4 + 3], fy, fx);
+        *idx = dy * S + dx;
+        return true;
+      };
+      for (int i = lane_id; i < nq * 9; i += 32) {
+        double v;
+        int idx;
+        if (candidate(i, &v, &idx)) take(v, idx);
+      }
+      warp_best();
+      // the quads within the window of the best candidate (bit qi), then all their samples on the lanes of the warp
+      unsigned scan = 0;
+      for (int i = lane_id; i < nq * 9; i += 32) {
+        double v;
+        int idx;
+        const int qi = i / 9;
+        if (candidate(i, &v, &idx) &&
+            quad_needs_scan(s_exact[qi * 4], s_exact[qi * 4 + 1], s_exact[qi * 4 + 2], s_exact[qi * 4 + 3], v, best))
+          scan |= 1u << qi;
+      }
+      scan = __reduce_or_sync(0xffffffffu, scan);
+      if (scan) {
+        do {
+          const int qi = __ffs(scan) - 1;
+          scan &= scan - 1;
+          const int q = s_quads[qi];
+          const int qy = q / hs;
+          scan_quad(qy, q - qy * hs, s_exact[qi * 4], s_exact[qi * 4 + 1], s_exact[qi * 4 + 2], s_exact[qi * 4 + 3],
+                    lane_id, 32);
+        } while (scan);
+        warp_best();
+      }
+      if (lane_id == 0) { s_bval[0] = best; s_bidx[0] = best_idx; }
+    }
+  } else {
+    if (nq <= kQuadCap) {
+      for (int i = tid, k = 0; i < nq; i += nthreads, ++k) {
+        const int q = s_quads[i];
+        const int qy = q / hs;
+        if (eval_quad(qy, q - qy * hs, -INFINITY)) second |= 1u << k;
+      }
+    } else if (act) {
+      for (int y = ro, k = 0; y < hs; y += rpp, ++k) {
+        const int y1 = min(y + 1, hs - 1), x1 = min(x + 1, hs - 1);
+        const float m4 = fmaxf(fmaxf(s_sum[y * hs + x], s_sum[y * hs + x1]), fmaxf(s_sum[y1 * hs + x], s_sum[y1 * hs + x1]));
+        if (m4 >= thr && eval_quad(y, x, -INFINITY)) second |= 1u << k;
       }
     }
-  } else if (nq <= kQuadCap) {
-    for (int i = tid; i < nq; i += nthreads) {
-      const int q = s_quads[i];
-      const int qy = q / hs;
-      eval_quad(qy, q - qy * hs);
-    }
-  } else if (act) {
-    for (int y = ro; y < hs; y += rpp) {
-      const int y1 = min(y + 1, hs - 1), x1 = min(x + 1, hs - 1);
-      const float m4 = fmaxf(fmaxf(s_sum[y * hs + x], s_sum[y * hs + x1]), fmaxf(s_sum[y1 * hs + x], s_sum[y1 * hs + x1]));
-      if (m4 >= thr) eval_quad(y, x);
-    }
-  }
-  if (!one_warp || warp_id == 0) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const double ov = __shfl_xor_sync(0xffffffffu, best, o);
-      const int oi = __shfl_xor_sync(0xffffffffu, best_idx, o);
-      if (ov > best || (ov == best && oi < best_idx)) { best = ov; best_idx = oi; }
-    }
+    warp_best();
     if (lane_id == 0) { s_bval[warp_id] = best; s_bidx[warp_id] = best_idx; }
+    if (__syncthreads_or(second != 0)) {  // block-uniform
+      double b = s_bval[0];
+      for (int w = 1; w < nwarps; ++w) b = fmax(b, s_bval[w]);
+      __syncthreads();  // every warp has read s_bval
+      while (second) {
+        const int k = __ffs(second) - 1;
+        second &= second - 1;
+        if (nq <= kQuadCap) {
+          const int q = s_quads[tid + k * nthreads];
+          const int qy = q / hs;
+          eval_quad(qy, q - qy * hs, b);
+        } else {
+          eval_quad(ro + k * rpp, x, b);
+        }
+      }
+      warp_best();
+      if (lane_id == 0) { s_bval[warp_id] = best; s_bidx[warp_id] = best_idx; }
+      __syncthreads();
+    }
   }
-  if (!one_warp) __syncthreads();  // block-uniform
   POST_TRACE(6);
 
   // ---- E. 2D filters, then the location-map gather at the FILTERED point (estimator.py:132-134)

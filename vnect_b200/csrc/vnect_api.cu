@@ -508,13 +508,15 @@ static int build_tables(vnect_t* h) {
     ScaleTable& T = t[s];
     memset(&T, 0, sizeof T);
     const double sc = h->cfg.scales[s];
-    if (sc == 1.0) {
-      T.identity = 1;
-      continue;
-    }
     // estimator.py:112-120: rescale = 1.0 / s; cv2.resize(fx = fy = rescale); centre crop of hs cells
     const double rescale = 1.0 / sc;
     const int R = cv_round_host(hs * rescale);
+    // cv::resize copies the source when the destination size equals the source size, so every scale whose resized
+    // map keeps hs cells (s > hs / (hs + 0.5), not only s = 1) is a plain copy, not a resample with inv = s
+    if (R == hs) {
+      T.identity = 1;
+      continue;
+    }
     const double inv = 1.0 / rescale;
     const int crop0 = R / 2 - hs / 2;
     for (int c = 0; c < hs; ++c) {
