@@ -283,6 +283,11 @@ int vnect_time_forward(vnect_t* h, int32_t n, int32_t reps, float* total_ms, flo
  * of streams 0..n_frames-1 advances by one step per repetition */
 int vnect_time_prepost(vnect_t* h, int32_t n_frames, int32_t reps, float* pre_ms, float* post_ms);
 const char* vnect_step_name(vnect_t* h, int32_t i); /* name of launch i of one forward, NULL past the end */
+/* how launch i of one forward runs, as the plan built it (tests check their coverage with it): out = int32[12].
+ * Implicit-GEMM conv: {block_n, epilogue, cg (CTAs per MMA), b_resident, halo, im2col, mode (0 flat rows, 1 spatial
+ * tiles), n2 (second conv of a fused block tail, 0 = none), tw, th (pixel tile), H, W (GEMM-row grid)}.
+ * conv1 + pool1 (the step named "conv1+pool1"): {cg, n_xt (x tiles per row segment), 0, ...}. */
+int vnect_step_path(vnect_t* h, int32_t i, int32_t* out);
 
 const char* vnect_last_error(vnect_t* h);
 const char* vnect_version(void);

@@ -100,6 +100,7 @@ SIGNATURES = {
     "vnect_time_forward": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_float), _P]),
     "vnect_time_prepost": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "vnect_step_name": (C.c_char_p, [_P, C.c_int32]),
+    "vnect_step_path": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
     "vnect_last_error": (C.c_char_p, [_P]),
     "vnect_version": (C.c_char_p, []),
     "vnect_destroy": (None, [_P]),

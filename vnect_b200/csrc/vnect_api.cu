@@ -2053,6 +2053,22 @@ const char* vnect_step_name(vnect_t* h, int32_t i) {
   return h->steps[i].name.c_str();
 }
 
+int vnect_step_path(vnect_t* h, int32_t i, int32_t* out) {
+  if (!h || !h->finalized || !out) return fail(h, VNECT_E_INVALID, "handle not finalized / null buffer");
+  if (i < 0 || i >= (int)h->steps.size()) return fail(h, VNECT_E_INVALID, "step %d not in [0, %zu)", i, h->steps.size());
+  const Step& st = h->steps[i];
+  for (int k = 0; k < 12; ++k) out[k] = 0;
+  if (st.kind != 0) {
+    out[0] = st.stem_pool.cg;
+    out[1] = st.stem_pool.r.n_xt;
+    return VNECT_OK;
+  }
+  const ConvLaunch& L = st.launch;
+  const int32_t v[12] = {L.block_n, L.epi, L.cg, L.b_resident, L.halo, L.p.im2col, L.p.mode, L.n2, L.p.tw, L.p.th, L.p.H, L.p.W};
+  for (int k = 0; k < 12; ++k) out[k] = v[k];
+  return VNECT_OK;
+}
+
 double vnect_info(vnect_t* h, const char* key) {
   if (!h || !key) return NAN;
   const std::string k = key;

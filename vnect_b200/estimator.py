@@ -571,6 +571,22 @@ class VNectEngine:
             out.append(s.decode())
             i += 1
 
+    _CONV_PATH_FIELDS = ("block_n", "epi", "cg", "b_resident", "halo", "im2col", "mode", "n2", "tw", "th", "H", "W")
+
+    def step_paths(self):
+        """How each launch of one forward runs (vnect_step_path), in step_names() order: {"kind": "stem", "cg", "n_xt"}
+        for conv1+pool1, {"kind": "conv", block_n, epi, cg, b_resident, halo, im2col, mode, n2, tw, th, H, W} for the
+        implicit-GEMM convs."""
+        out = []
+        for i, name in enumerate(self.step_names()):
+            v = (C.c_int32 * 12)()
+            self._check(self._lib.vnect_step_path(self._h, i, v))
+            if name == "conv1+pool1":
+                out.append({"kind": "stem", "cg": v[0], "n_xt": v[1]})
+            else:
+                out.append({"kind": "conv", **dict(zip(self._CONV_PATH_FIELDS, v))})
+        return out
+
     def time_forward(self, n, reps=5, per_layer=False):
         """Device time (ms) of one forward of n images already resident; optionally per launch."""
         total = C.c_float()
