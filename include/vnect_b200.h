@@ -262,6 +262,11 @@ int vnect_synchronize(vnect_t* h);
 /* introspection for tests and benchmarks */
 int vnect_get_tap(vnect_t* h, const char* name, int32_t n, float* out_nhwc, int64_t capacity_elems,
                   int32_t* dims4 /* n, H, W, C */);
+/* the network input of the most recent call, as the stem reads it: the raw fp16 bits of the first n forwards,
+ * uint16 [n][2 parities][S/2 + 3 rows][(S + 6) * 4], zero border and 4th channel included (pixel (y, x) of forward f
+ * is at parity (y + 2) & 1, row (y + 2) >> 1, column (x + 2) * 4).  Synchronises the handle's stream.  A null `out`
+ * only fills dims4. */
+int vnect_get_input(vnect_t* h, int32_t n, uint16_t* out, int64_t capacity, int32_t* dims4 /* n, 2, rows, halves */);
 /* unfiltered (row, col) argmax in box pixels of the frames of the most recent estimate / submit / track call
  * (what utils.extract_2d_joints returns, src/utils.py:153-175, before joint_filter): int32 [n_frames][21][2].
  * Waits for that call to complete.  Parity tests use it to prove that an argmax difference is a near-tie. */

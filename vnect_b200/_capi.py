@@ -94,6 +94,7 @@ SIGNATURES = {
     "vnect_set_packed_results": (C.c_int, [_P, _P]),
     "vnect_synchronize": (C.c_int, [_P]),
     "vnect_get_tap": (C.c_int, [_P, C.c_char_p, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32)]),
+    "vnect_get_input": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32)]),
     "vnect_check_finite": (C.c_int, [_P, C.c_int32, _P]),
     "vnect_launch_count": (C.c_int64, [_P]),
     "vnect_info": (C.c_double, [_P, C.c_char_p]),

@@ -548,7 +548,47 @@ static int build_tables(vnect_t* h) {
   return upload(h, t, &h->d_tables);
 }
 
-static int alloc_prepost(vnect_t* h) {
+constexpr size_t kPyrMaxSmem = 160 * 1024;  // dynamic shared memory of pyramid_kernel's staged source rows
+
+// The pyramid's per-scale geometry (h->pyr: R, pad0, 1 / s, the magic divisors) and resize tables, and the most source
+// rows one block stages (h->pyr_src_rows).  Host arithmetic only: vnect_create refuses a scale list whose staged rows
+// do not fit in kPyrMaxSmem before anything is allocated.
+static void pyramid_tables(vnect_t* h, std::vector<PyramidTable>* ptab_out) {
+  const int S = h->S;
+  PyramidParams& py = h->pyr;
+  py.S = S; py.n_scales = h->n_scales;
+  std::vector<PyramidTable>& ptab = *ptab_out;
+  ptab.assign(h->n_scales, PyramidTable{});
+  h->pyr_src_rows = 1;
+  for (int i = 0; i < h->n_scales; ++i) {
+    const double sc = h->cfg.scales[i];
+    py.R[i] = sc < 1.0 ? cv_round_host(S * sc) : S;  // estimator.py:77: only scales < 1 are resized
+    py.pad0[i] = (S - py.R[i]) / 2;
+    py.inv_scale[i] = 1.0 / sc;
+    for (int d = 0; d < py.R[i] && py.R[i] != S; ++d) {  // same arithmetic as cv_linear_coord / cv_coef on the device
+      int ix, iy;
+      float fx, fy;
+      host_linear_coord(d, py.inv_scale[i], S, true, &ix, &fx);
+      host_linear_coord(d, py.inv_scale[i], S, false, &iy, &fy);
+      const unsigned int a0 = (unsigned int)std::nearbyint((1.f - fx) * 2048.f), a1 = (unsigned int)std::nearbyint(fx * 2048.f);
+      ptab[i].xt[d].x = (unsigned int)(4 * ix) | ((unsigned int)(4 * std::min(ix + 1, S - 1)) << 16);
+      ptab[i].xt[d].y = a0 | (a1 << 16);
+      ptab[i].yt[d].x = (short)std::min(std::max(iy, 0), S - 1);
+      ptab[i].yt[d].y = (short)std::min(std::max(iy + 1, 0), S - 1);
+      ptab[i].yt[d].z = (short)std::nearbyint((1.f - fy) * 2048.f);
+      ptab[i].yt[d].w = (short)std::nearbyint(fy * 2048.f);
+    }
+    py.r_magic[i] = (unsigned int)((1ull << 32) / (unsigned long long)py.R[i]) + 1u;
+    // source rows one block of kPyrRows output rows samples
+    for (int y0 = 0; y0 < py.R[i] && py.R[i] != S; y0 += 1) {
+      const int y1 = std::min(y0 + kPyrRows, py.R[i]) - 1;
+      h->pyr_src_rows = std::max(h->pyr_src_rows, ptab[i].yt[y1].y - ptab[i].yt[y0].x + 1);
+    }
+  }
+  py.q_magic = (unsigned int)((1ull << 32) / (unsigned long long)(S / 4)) + 1u;
+}
+
+static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
   const int S = h->S, nb = h->cap_fw;
   int rc;
   // stem input: parity-split, zero-padded NHWC4 (zeros are written once here and never touched again)
@@ -614,35 +654,7 @@ static int alloc_prepost(vnect_t* h) {
   h->last_t2d.assign(ms, NAN);
   h->last_t3d.assign(ms, NAN);
   PyramidParams& py = h->pyr;
-  py.S = S; py.n_scales = h->n_scales;
   py.rows_per_parity = h->stem_rpp; py.row_pitch = h->stem_pitch;
-  std::vector<PyramidTable> ptab(h->n_scales);
-  for (int i = 0; i < h->n_scales; ++i) {
-    const double sc = h->cfg.scales[i];
-    py.R[i] = sc < 1.0 ? cv_round_host(S * sc) : S;  // estimator.py:77: only scales < 1 are resized
-    py.pad0[i] = (S - py.R[i]) / 2;
-    py.inv_scale[i] = 1.0 / sc;
-    memset(&ptab[i], 0, sizeof(PyramidTable));
-    for (int d = 0; d < py.R[i] && py.R[i] != S; ++d) {  // same arithmetic as cv_linear_coord / cv_coef on the device
-      int ix, iy;
-      float fx, fy;
-      host_linear_coord(d, py.inv_scale[i], S, true, &ix, &fx);
-      host_linear_coord(d, py.inv_scale[i], S, false, &iy, &fy);
-      const unsigned int a0 = (unsigned int)std::nearbyint((1.f - fx) * 2048.f), a1 = (unsigned int)std::nearbyint(fx * 2048.f);
-      ptab[i].xt[d].x = (unsigned int)(4 * ix) | ((unsigned int)(4 * std::min(ix + 1, S - 1)) << 16);
-      ptab[i].xt[d].y = a0 | (a1 << 16);
-      ptab[i].yt[d].x = (short)std::min(std::max(iy, 0), S - 1);
-      ptab[i].yt[d].y = (short)std::min(std::max(iy + 1, 0), S - 1);
-      ptab[i].yt[d].z = (short)std::nearbyint((1.f - fy) * 2048.f);
-      ptab[i].yt[d].w = (short)std::nearbyint(fy * 2048.f);
-    }
-    py.r_magic[i] = (unsigned int)((1ull << 32) / (unsigned long long)py.R[i]) + 1u;
-    // source rows one block of kPyrRows output rows samples
-    for (int y0 = 0; y0 < py.R[i] && py.R[i] != S; y0 += 1) {
-      const int y1 = std::min(y0 + kPyrRows, py.R[i]) - 1;
-      h->pyr_src_rows = std::max(h->pyr_src_rows, ptab[i].yt[y1].y - ptab[i].yt[y0].x + 1);
-    }
-  }
   if ((rc = upload(h, ptab, &h->d_pyr_tables))) return rc;
   py.tables = h->d_pyr_tables;
   // float32(v) / 255 - 0.4 -> fp16 (estimator.py:81 in float32, then the operand precision of the stem)
@@ -655,7 +667,6 @@ static int alloc_prepost(vnect_t* h) {
   }
   if ((rc = upload(h, lut, &h->d_norm_lut))) return rc;
   py.lut = h->d_norm_lut;
-  py.q_magic = (unsigned int)((1ull << 32) / (unsigned long long)(S / 4)) + 1u;
   py.full = 0;
   return VNECT_OK;
 }
@@ -684,6 +695,11 @@ int vnect_create(vnect_t** out, const vnect_config* cfg) {
   h->hs = h->S / 8;
   h->n_scales = cfg->n_scales;
   h->cap_fw = cfg->max_frames * cfg->n_scales;
+  std::vector<PyramidTable> ptab;
+  pyramid_tables(h, &ptab);
+  if ((size_t)h->pyr_src_rows * h->S * 4 > kPyrMaxSmem)
+    return fail(h, VNECT_E_INVALID, "pyramid scale too small: a block stages %d source rows (%zu bytes, at most %zu)",
+                h->pyr_src_rows, (size_t)h->pyr_src_rows * h->S * 4, kPyrMaxSmem);
   if (h->cfg.max_input_h <= 0) h->cfg.max_input_h = h->S;
   if (h->cfg.max_input_w <= 0) h->cfg.max_input_w = h->S;
   int ndev = 0;
@@ -698,7 +714,7 @@ int vnect_create(vnect_t** out, const vnect_config* cfg) {
   CU(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   h->own_stream = true;
   h->use_graphs = getenv("VNECT_B200_NO_GRAPH") == nullptr;
-  int rc = alloc_prepost(h);
+  int rc = alloc_prepost(h, ptab);
   if (rc) return rc;
   return vnect_reset_stream(h, -1);
 }
@@ -939,10 +955,9 @@ static int launch_pyramid(vnect_t* h, const uint8_t* sq, int64_t sq_pitch, int64
   PyramidParams py = h->pyr;
   py.n_frames = n_frames; py.sq_pitch = sq_pitch; py.sq_frame_stride = sq_stride;
   py.full = full_surround ? 1 : 0;
-  const size_t smem = (size_t)h->pyr_src_rows * S * 4;  // staged source rows, one word per pixel
+  const size_t smem = (size_t)h->pyr_src_rows * S * 4;  // staged source rows, one word per pixel (vnect_create: <= kPyrMaxSmem)
   static unsigned long long done = 0;
-  CU(h, ensure_dyn_smem(pyramid_kernel, 160 * 1024, &done));
-  if (smem > 160 * 1024) return fail(h, VNECT_E_INVALID, "pyramid scale too small for the staged rows (%zu bytes)", smem);
+  CU(h, ensure_dyn_smem(pyramid_kernel, kPyrMaxSmem, &done));
   CU(h, launch_pdl(pyramid_kernel, dim3((S + kPyrRows - 1) / kPyrRows, n_frames * h->n_scales), dim3(kPyrThreads), smem,
                    h->stream, sq, h->x1, py));
   ++h->launches;
@@ -1988,6 +2003,19 @@ int vnect_get_tap(vnect_t* h, const char* name, int32_t n, float* out_nhwc, int6
         const __half* src = tmp.data() + ((size_t)i * a.img_px + (size_t)y * a.row_px + x) * a.C;
         for (int c = 0; c < a.C; ++c) out_nhwc[o++] = __half2float(src[c]);
       }
+  return VNECT_OK;
+}
+
+int vnect_get_input(vnect_t* h, int32_t n, uint16_t* out, int64_t capacity, int32_t* dims4) {
+  if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (n < 1 || n > h->cap_fw) return fail(h, VNECT_E_INVALID, "n out of range");
+  if (dims4) { dims4[0] = n; dims4[1] = 2; dims4[2] = h->stem_rpp; dims4[3] = h->stem_pitch; }
+  const size_t elems = (size_t)n * 2 * h->stem_rpp * h->stem_pitch;
+  if (!out) return VNECT_OK;
+  if ((int64_t)elems > capacity) return fail(h, VNECT_E_INVALID, "buffer too small for the network input");
+  CU(h, cudaStreamSynchronize(h->stream));
+  CU(h, cudaMemcpy(out, h->x1, elems * sizeof(__half), cudaMemcpyDeviceToHost));
   return VNECT_OK;
 }
 

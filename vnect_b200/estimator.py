@@ -535,6 +535,15 @@ class VNectEngine:
         self._check(self._lib.vnect_get_tap(self._h, name.encode(), n, _ptr(out), out.size, dims))
         return out
 
+    def stem_input(self, n=1):
+        """The network input of the first n forwards of the last call as the stem reads it: the raw fp16 bits, uint16
+        [n, 2 parities, S/2 + 3, (S + 6) * 4], zero border and 4th channel included."""
+        dims = (C.c_int32 * 4)()
+        self._check(self._lib.vnect_get_input(self._h, int(n), None, 0, dims))
+        out = np.empty(tuple(dims), np.uint16)
+        self._check(self._lib.vnect_get_input(self._h, int(n), _ptr(out), out.size, dims))
+        return out
+
     def check_finite(self, n=1):
         """{launch name: count of NaN / Inf / saturated fp16 values in its output} for the first n forwards of the last
         batch -- names the layer where un-normalised weights overflow fp16 (65504)."""
