@@ -222,6 +222,16 @@ int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H
 int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm, int32_t n_frames,
                       const int32_t* stream_ids, const double* t2d, const double* t3d, double scaler, int32_t offset_x,
                       int32_t offset_y, double* joints2d, float* joints3d, int32_t* raw_argmax);
+/* the tracked tail of vnect_track_frames (src/estimator.py:105-142 and run_estimator.py:100-119 after the CNN) fed
+ * with given maps, laid out as for vnect_postprocess: each frame's geometry from its stream's box clipped to the frame,
+ * the post-process with that geometry (joints2d in full-frame pixels), then the box update.  frame_hw: host int32
+ * [n_frames][2] full-frame (height, width); boxes_used (optional): int32 [n_frames][4].  Validated like
+ * vnect_track_frames (sides below 2, ids, duplicate ids, repeated or earlier timestamps); a refused call touches no
+ * box, filter state or timestamp.  Not graphed; synchronises before returning.  The raw argmax is read with
+ * vnect_get_raw_argmax. */
+int vnect_track_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm,
+                            int32_t n_frames, const int32_t* frame_hw, const int32_t* stream_ids, const double* t2d,
+                            const double* t3d, double* joints2d, float* joints3d, int32_t* boxes_used);
 
 /* replaces VNectEstimator.joint_filter (src/estimator.py:83-95) on explicit values: one step of the 21*dim scalar
  * filters of a stream at clock reading t.  values: host float64 [21*dim], filtered in place.  values_are_f32 = 1 when
@@ -267,6 +277,10 @@ int vnect_get_tap(vnect_t* h, const char* name, int32_t n, float* out_nhwc, int6
  * is at parity (y + 2) & 1, row (y + 2) >> 1, column (x + 2) * 4).  Synchronises the handle's stream.  A null `out`
  * only fills dims4. */
 int vnect_get_input(vnect_t* h, int32_t n, uint16_t* out, int64_t capacity, int32_t* dims4 /* n, 2, rows, halves */);
+/* the CNN output maps of the most recent call (or the maps vnect_postprocess / vnect_track_postprocess were given) as
+ * the post-process reads them: planar float32 [n_frames*n_scales][84][S/8][S/8], channels hm 0..20, xm 21..41, ym
+ * 42..62, zm 63..83.  Synchronises the handle's stream.  A null `out` only fills dims4. */
+int vnect_get_maps(vnect_t* h, int32_t n_frames, float* out, int64_t capacity, int32_t* dims4 /* n, 84, hs, hs */);
 /* unfiltered (row, col) argmax in box pixels of the frames of the most recent estimate / submit / track call
  * (what utils.extract_2d_joints returns, src/utils.py:153-175, before joint_filter): int32 [n_frames][21][2].
  * Waits for that call to complete.  Parity tests use it to prove that an argmax difference is a near-tie. */

@@ -84,6 +84,7 @@ SIGNATURES = {
     "vnect_track_set_boxes": (C.c_int, [_P, C.c_int32, _P, _P]),
     "vnect_preprocess": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P]),
     "vnect_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32, C.c_int32, _P, _P, _P]),
+    "vnect_track_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "vnect_filter": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P]),
     "vnect_export_stream_state": (C.c_int, [_P, C.c_int32, _P]),
     "vnect_import_stream_state": (C.c_int, [_P, C.c_int32, _P]),
@@ -95,6 +96,7 @@ SIGNATURES = {
     "vnect_synchronize": (C.c_int, [_P]),
     "vnect_get_tap": (C.c_int, [_P, C.c_char_p, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32)]),
     "vnect_get_input": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32)]),
+    "vnect_get_maps": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32)]),
     "vnect_check_finite": (C.c_int, [_P, C.c_int32, _P]),
     "vnect_launch_count": (C.c_int64, [_P]),
     "vnect_info": (C.c_double, [_P, C.c_char_p]),

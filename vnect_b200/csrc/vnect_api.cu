@@ -1772,15 +1772,9 @@ int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H
   return VNECT_OK;
 }
 
-int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm, int32_t n_frames,
-                      const int32_t* stream_ids, const double* t2d, const double* t3d, double scaler, int32_t offset_x,
-                      int32_t offset_y, double* joints2d, float* joints3d, int32_t* raw_argmax) {
-  if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
-  ON_DEVICE(h);
-  if (!hm || !xm || !ym || !zm || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
-  int rc = lane_acquire(h, 0);
-  if (rc) return rc;
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream))) return rc;
+// caller-supplied NHWC maps [n_frames*n_scales][hs][hs][21] -> the planar fp32 maps the CNN writes, then to h->maps on
+// the handle's stream.  A copy from pageable memory has read its source when it returns, so the vector may go.
+static int stage_maps(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm, int n_frames) {
   const int n = n_frames * h->n_scales, hs = h->hs;
   const size_t plane = (size_t)hs * hs;
   std::vector<float> planar((size_t)n * 84 * plane);
@@ -1793,11 +1787,64 @@ int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float*
         for (size_t px = 0; px < plane; ++px) dst[px] = src[px * kJoints];
       }
   CU(h, cudaMemcpyAsync(h->maps, planar.data(), planar.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  return VNECT_OK;
+}
+
+int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm, int32_t n_frames,
+                      const int32_t* stream_ids, const double* t2d, const double* t3d, double scaler, int32_t offset_x,
+                      int32_t offset_y, double* joints2d, float* joints3d, int32_t* raw_argmax) {
+  if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (!hm || !xm || !ym || !zm || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  int rc = lane_acquire(h, 0);
+  if (rc) return rc;
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream))) return rc;
+  if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
   if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false))) return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (raw_argmax)
     CU(h, cudaMemcpyAsync(raw_argmax, h->d_raw_argmax, (size_t)n_frames * kJoints * 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  return VNECT_OK;
+}
+
+// The tracked tail of vnect_track_frames on caller-supplied maps: the three launches of run_pipeline's table path after
+// the CNN (frame geometry from the stream boxes, post-process with per-frame geometry, box update), on lane 0's table.
+// Only the frame sizes of the table are read, so its entries carry no data pointer.
+int vnect_track_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm,
+                            int32_t n_frames, const int32_t* frame_hw, const int32_t* stream_ids, const double* t2d,
+                            const double* t3d, double* joints2d, float* joints3d, int32_t* boxes_used) {
+  if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (!hm || !xm || !ym || !zm || !frame_hw || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
+  for (int i = 0; i < n_frames; ++i)  // before the ids and timestamps are checked and recorded, as check_frames does
+    if (frame_hw[2 * i] < 2 || frame_hw[2 * i + 1] < 2)
+      return fail(h, VNECT_E_INVALID, "frame %d: frame %dx%d smaller than 2x2", i, frame_hw[2 * i], frame_hw[2 * i + 1]);
+  int rc = lane_acquire(h, 0);
+  if (rc) return rc;
+  vnect_handle::Lane* L = h->cur;
+  for (int i = 0; i < n_frames; ++i) {
+    FrameDesc& t = L->h_table[i];
+    memset(&t, 0, sizeof t);
+    t.height = frame_hw[2 * i];
+    t.width = frame_hw[2 * i + 1];
+  }
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream, n_frames))) return rc;
+  if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
+  frame_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(L->d_table, h->d_boxes, L->d_stream_ids, n_frames,
+                                                                    h->S, L->d_geoms, h->d_boxes_used);
+  CU(h, cudaGetLastError());
+  ++h->launches;
+  if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, L->d_out2d, L->d_out3d, L->d_geoms, false))) return rc;
+  track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(L->d_out2d, L->d_stream_ids, L->d_table, h->d_boxes);
+  CU(h, cudaGetLastError());
+  ++h->launches;
+  CU(h, cudaMemcpyAsync(joints2d, L->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaMemcpyAsync(joints3d, L->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if (boxes_used)
+    CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaStreamSynchronize(h->stream));
   return VNECT_OK;
 }
@@ -2016,6 +2063,20 @@ int vnect_get_input(vnect_t* h, int32_t n, uint16_t* out, int64_t capacity, int3
   if ((int64_t)elems > capacity) return fail(h, VNECT_E_INVALID, "buffer too small for the network input");
   CU(h, cudaStreamSynchronize(h->stream));
   CU(h, cudaMemcpy(out, h->x1, elems * sizeof(__half), cudaMemcpyDeviceToHost));
+  return VNECT_OK;
+}
+
+int vnect_get_maps(vnect_t* h, int32_t n_frames, float* out, int64_t capacity, int32_t* dims4) {
+  if (!h || !h->maps) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames out of range");
+  const int n = n_frames * h->n_scales;
+  if (dims4) { dims4[0] = n; dims4[1] = 4 * kJoints; dims4[2] = h->hs; dims4[3] = h->hs; }
+  const size_t elems = (size_t)n * 4 * kJoints * h->hs * h->hs;
+  if (!out) return VNECT_OK;
+  if ((int64_t)elems > capacity) return fail(h, VNECT_E_INVALID, "buffer too small for the maps");
+  CU(h, cudaStreamSynchronize(h->stream));
+  CU(h, cudaMemcpy(out, h->maps, elems * sizeof(float), cudaMemcpyDeviceToHost));
   return VNECT_OK;
 }
 

@@ -165,6 +165,38 @@ def strided_device_frames(dev_frames_ptr, n, h, w, pitch=None, frame_stride=None
     return [dict(ptr=int(dev_frames_ptr) + i * lay.frame_stride, h=h, w=w, **planes) for i in range(n)]
 
 
+def planar_to_nhwc(planar):
+    """Planar maps float32 [n][84][hs][hs] (what the CNN writes and vnect_get_maps returns: channel 21 * m + j is joint
+    j of map m = hm, xm, ym, zm) -> the 4-tuple (hm, xm, ym, zm) of NHWC [n][hs][hs][21] arrays that postprocess(),
+    track_postprocess() and the reference's sess.run (src/estimator.py:100-104) use."""
+    planar = np.asarray(planar, dtype=np.float32)
+    n, c, hs = planar.shape[:3]
+    if c != 4 * JOINTS or planar.shape != (n, c, hs, hs):
+        raise ValueError(f"expected planar maps [n,{4 * JOINTS},hs,hs], got {planar.shape}")
+    nhwc = planar.reshape(n, 4, JOINTS, hs, hs).transpose(1, 0, 3, 4, 2)
+    return tuple(np.ascontiguousarray(m) for m in nhwc)
+
+
+def nhwc_to_planar(maps):
+    """Inverse of planar_to_nhwc: the transposition vnect_postprocess / vnect_track_postprocess apply to their maps."""
+    maps = np.stack([np.asarray(m, dtype=np.float32) for m in maps])  # [4][n][hs][hs][21]
+    if maps.ndim != 5 or maps.shape[4] != JOINTS or maps.shape[2] != maps.shape[3]:
+        raise ValueError(f"expected 4 maps [n,hs,hs,{JOINTS}], got {maps.shape[1:]}")
+    return np.ascontiguousarray(maps.transpose(1, 0, 4, 2, 3).reshape(maps.shape[1], 4 * JOINTS, *maps.shape[2:4]))
+
+
+def check_maps(maps, n_scales, hs):
+    """(hm, xm, ym, zm), each [n*n_scales, hs, hs, 21] -> (contiguous float32 maps, n).  vnect_postprocess and
+    vnect_track_postprocess read exactly that many floats from each, so any other shape is refused here."""
+    maps = [np.ascontiguousarray(m, dtype=np.float32) for m in maps]
+    n = maps[0].shape[0] // n_scales if maps and maps[0].ndim == 4 else 0
+    want = (n * n_scales, hs, hs, JOINTS)
+    if len(maps) != 4 or n < 1 or any(m.shape != want for m in maps):
+        raise ValueError(f"expected 4 maps [n*{n_scales}, {hs}, {hs}, {JOINTS}] with n >= 1, got "
+                         f"{[m.shape for m in maps]}")
+    return maps, n
+
+
 class VNectEngine:
     """Batched estimator: ``estimate(frames[n,H,W,3] uint8 BGR) -> (joints_2d [n,21,2] f64, joints_3d [n,21,3] f32)``.
 
@@ -474,8 +506,7 @@ class VNectEngine:
     def postprocess(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None):
         """src/estimator.py:105-142 on given (hm, xm, ym, zm) maps, each [n*n_scales, S/8, S/8, 21] float32.
         Returns (joints_2d, joints_3d, raw_argmax)."""
-        maps = [np.ascontiguousarray(m, dtype=np.float32) for m in maps]
-        n = maps[0].shape[0] // len(self.scales)
+        maps, n = check_maps(maps, len(self.scales), self.hm_size)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         raw = np.empty((n, JOINTS, 2), np.int32)
@@ -483,6 +514,31 @@ class VNectEngine:
                                                 float(scaler), int(offsets[0]), int(offsets[1]), _ptr(j2), _ptr(j3),
                                                 _ptr(raw)))
         return j2, j3, raw
+
+    def track_postprocess(self, maps, frame_hw, stream_ids=None, t2d=None, t3d=None):
+        """The tracked tail of track_frames() on given (hm, xm, ym, zm) maps, each [n*n_scales, S/8, S/8, 21] float32:
+        frame f of stream stream_ids[f] is a full frame of frame_hw[f] = (height, width), cropped by the stream's box.
+        Returns (joints_2d [n,21,2] in full-frame pixels, joints_3d [n,21,3], boxes_used [n,4]); the box update runs on
+        the device as in track_frames().  The raw argmax comes from raw_argmax()."""
+        maps, n = check_maps(maps, len(self.scales), self.hm_size)
+        hw = np.ascontiguousarray(frame_hw, dtype=np.int32).reshape(-1)
+        if hw.shape != (2 * n,):
+            raise ValueError(f"frame_hw must give (height, width) for each of the {n} frames")
+        ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
+        boxes = np.empty((n, 4), np.int32)
+        self._check(self._lib.vnect_track_postprocess(self._h, *[_ptr(m) for m in maps], n, _ptr(hw), _ptr(ids),
+                                                      _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
+        return j2, j3, boxes
+
+    def maps(self, n_frames=1):
+        """The CNN output maps of the first n_frames frames of the last call (all their scales) as the 4-tuple
+        (hm, xm, ym, zm) of NHWC [n_frames*n_scales, S/8, S/8, 21] float32 arrays that postprocess() takes."""
+        dims = (C.c_int32 * 4)()
+        self._check(self._lib.vnect_get_maps(self._h, int(n_frames), None, 0, dims))
+        out = np.empty(tuple(dims), np.float32)
+        self._check(self._lib.vnect_get_maps(self._h, int(n_frames), _ptr(out), out.size, dims))
+        return planar_to_nhwc(out)
 
     def filter(self, values, dim, t, stream_id=0, is_f32=None):
         """One joint_filter step (src/estimator.py:83-95) on explicit values [21, dim].  ``is_f32`` says whether the
