@@ -211,6 +211,40 @@ int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_f
  * below 2. */
 int vnect_track_set_boxes(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* xywh);
 
+/* Sequence calls: consecutive frames of one stream in one batch (offline video: annotating a dataset, re-processing a
+ * recording, motion capture from footage).  Up to max_frames frames in which a stream id may appear more than once;
+ * the frames of one stream are consecutive in time in the order they appear in the call, and may be interleaved with
+ * other streams' frames.  Frame i gets bit for bit what the untracked entry points give when the frames go in one
+ * at a time in call order: joints2d, joints3d, the raw argmax, the packed results, and afterwards every stream's
+ * filter state and timestamp mirror.  The CNN runs over the whole call at batch size; each stream's 2D filters, the
+ * location-map gather at the filtered points and the 3D filters are then walked in frame order on the GPU.  Tracked
+ * streams cannot be batched this way: frame k+1's crop depends on frame k's joints.
+ * stream_ids is required; with filters on, so are t2d and t3d (one reading per frame).  Validation runs before
+ * anything is staged or launched: the vnect_frame table as for vnect_submit_frames, ids in [0, max_streams), and each
+ * stream's readings walked in call order against its previous reading (before the call, then the call's own earlier
+ * frames) with the rules of the other calls -- a repeated 2D or 3D reading is VNECT_E_ZERO_DT, an earlier one
+ * VNECT_E_INVALID, a reading of 0 is never compared.  A refused call touches no filter state and no timestamp mirror:
+ * unlike a frame-by-frame loop, which would already have processed the frames before the bad one, it processes none.
+ * A stream may continue across sequence calls on either lane and across ordinary calls, in submission order.  CUDA
+ * graphs are keyed by lane, frame count, format and output pointers: every composition of a batch replays the same
+ * graph. */
+/* vnect_submit_frames with repeated stream ids: HOST frames of any sizes (BGR, NV12 or I420), HOST results;
+ * completes with vnect_wait(h, lane). */
+int vnect_submit_sequence(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                          float* joints3d);
+/* vnect_estimate_device_frames with repeated stream ids: DEVICE frames, DEVICE results, asynchronous on the handle's
+ * stream. */
+int vnect_estimate_device_sequence(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                                   const int32_t* stream_ids, const double* t2d, const double* t3d,
+                                   double* dev_joints2d, float* dev_joints3d);
+/* vnect_postprocess with repeated stream ids, a diagnostic on given maps (same layout and arguments as
+ * vnect_postprocess, same validation as the sequence calls above).  Not graphed; synchronises before returning. */
+int vnect_postprocess_sequence(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm,
+                               int32_t n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                               double scaler, int32_t offset_x, int32_t offset_y, double* joints2d, float* joints3d,
+                               int32_t* raw_argmax);
+
 /* replaces VNectEstimator.gen_input_batch (src/estimator.py:70-81): out float32 [n_frames*n_scales][S][S][3]
  * (fp16-rounded values of the network input), scaler_offsets float64 [3] = {scaler, offset_x, offset_y} */
 int vnect_preprocess(vnect_t* h, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,

@@ -82,6 +82,10 @@ SIGNATURES = {
     "vnect_submit_track_frames": (C.c_int, [_P, C.c_int32, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "vnect_track_device_frames": (C.c_int, [_P, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "vnect_track_set_boxes": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "vnect_submit_sequence": (C.c_int, [_P, C.c_int32, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "vnect_estimate_device_sequence": (C.c_int, [_P, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
+    "vnect_postprocess_sequence": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32,
+                                             C.c_int32, _P, _P, _P]),
     "vnect_preprocess": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, _P, _P]),
     "vnect_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32, C.c_int32, _P, _P, _P]),
     "vnect_track_postprocess": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),

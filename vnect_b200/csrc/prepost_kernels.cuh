@@ -724,6 +724,76 @@ __device__ __forceinline__ double oef_finish(FilterState& st, const FilterCfg& c
   return sm;
 }
 
+// ---- step E's location-map gather and rescale, shared by postprocess_kernel and sequence_filter_kernel
+// utils.hm_pt_interp_bilinear (utils.py:58-79) at a filtered joint (py, px) in box pixels: the heat-map cells around it
+// and the UNCLAMPED bilinear weights (a point below 3.5 extrapolates, one at or above 8(hs-1)+3.5 gives exactly 0).
+struct GatherPoint {
+  double sx, sy;
+  int x0, y0, x1, y1;
+};
+__device__ __forceinline__ GatherPoint gather_point(double py, double px, int hs) {
+  GatherPoint g;
+  g.sx = __dsub_rn(__dmul_rn(__dadd_rn(px, 0.5), 0.125), 0.5);  // / 8 exactly
+  g.sy = __dsub_rn(__dmul_rn(__dadd_rn(py, 0.5), 0.125), 0.5);
+  int x0 = (int)g.sx, y0 = (int)g.sy;  // truncation toward zero, like int()
+  x0 = min(max(x0, 0), hs - 1);        // memory safety only: filtered joints stay inside the box
+  y0 = min(max(y0, 0), hs - 1);
+  g.x0 = x0; g.y0 = y0;
+  g.x1 = min(x0 + 1, hs - 1); g.y1 = min(y0 + 1, hs - 1);
+  return g;
+}
+
+// gather_value and gather_combine are sequence_filter_kernel's; postprocess_kernel keeps the same arithmetic inline,
+// since routing it through them changes that kernel's SASS at MASK = -1.
+// Item i (0 .. 12*NS-1) of a joint's gather: scale i % NS of cell (i / NS) & 3 (bit 1: row y1, bit 0: column x1) of
+// location map i / (4*NS) (x, y, z), resampled like the heat maps.
+template <int NS>
+__device__ __forceinline__ float gather_value(const PostParams& p, int hs, int cells, int frame, int joint, int i,
+                                             const GatherPoint& g) {
+  const int sc = i % NS;
+  const int cell = (i / NS) & 3;
+  const int map = i / (4 * NS);
+  const float* m = p.maps + ((size_t)(frame * NS + sc) * 84 + kJoints * (1 + map) + joint) * cells;
+  return scaled_cell(m, hs, p.tables[sc], (cell & 2) ? g.y1 : g.y0, (cell & 1) ? g.x1 : g.x0);
+}
+
+// Map `map`'s 4 cells x NS scales (items[(map * 4 + cell) * NS + sc], as gather_value numbers them) -> the x100 sample in mm:
+// float64 sum over the scales in order, / NS, bilinear with the weights of `g`, float32 store.
+template <int NS>
+__device__ __forceinline__ float gather_combine(const float* items, int map, const GatherPoint& g) {
+  double v[4];
+#pragma unroll
+  for (int cell = 0; cell < 4; ++cell) {
+    double acc = 0.0;
+    for (int sc = 0; sc < NS; ++sc) acc = __dadd_rn(acc, (double)items[(map * 4 + cell) * NS + sc]);
+    // an exact scaling for 1, 2 or 4 scales, bit-identical to the division
+    v[cell] = NS == 1 ? acc : NS == 2 ? __dmul_rn(acc, 0.5) : NS == 4 ? __dmul_rn(acc, 0.25) : __ddiv_rn(acc, (double)NS);
+  }
+  const double wx1 = __dsub_rn((double)g.x1, g.sx), wx0 = __dsub_rn(g.sx, (double)g.x0);
+  const double wy1 = __dsub_rn((double)g.y1, g.sy), wy0 = __dsub_rn(g.sy, (double)g.y0);
+  const double value0 = __dadd_rn(__dmul_rn(wx1, v[0]), __dmul_rn(wx0, v[1]));
+  const double value1 = __dadd_rn(__dmul_rn(wx1, v[2]), __dmul_rn(wx0, v[3]));
+  const double val = __dadd_rn(__dmul_rn(wy1, value0), __dmul_rn(wy0, value1));
+  return __double2float_rn(__dmul_rn(val, 100.0));
+}
+
+// Coordinate c (0 row, 1 col) of a filtered joint in box pixels -> input pixels (estimator.py:138-139; + the crop
+// origin for tracked streams, run_estimator.py:104-105).
+__device__ __forceinline__ double rescale_joint(const PostParams& p, int frame, int c, double jb) {
+  double off = (c == 0) ? (double)p.off_y : (double)p.off_x, scaler = p.scaler;
+  double v2;
+  if (p.geoms != nullptr) {
+    const FrameGeom g = p.geoms[frame];
+    off = (c == 0) ? (double)g.off_y : (double)g.off_x;
+    scaler = g.scaler;
+    v2 = __ddiv_rn(__dsub_rn(jb, off), scaler);
+    v2 = __dadd_rn(v2, (c == 0) ? (double)g.y : (double)g.x);
+  } else {
+    v2 = __ddiv_rn(__dsub_rn(jb, off), scaler);
+  }
+  return v2;
+}
+
 // grid = n_frames * 21 blocks; block (frame, joint), thread = one cell of the `rpp` heat-map rows a pass covers.
 //
 //  A. the raw heat-map planes of every scale go to shared memory with 16-byte cp.async (the only HBM traffic that
@@ -742,7 +812,9 @@ __device__ __forceinline__ double oef_finish(FilterState& st, const FilterCfg& c
 //  E. 2D 1-euro filters, location-map gather at the FILTERED point, and -- in the last block of the frame to arrive --
 //     root subtraction, 3D filters and the rescale to input pixels.
 #define POST_TRACE(i) do { if (p.trace != nullptr && threadIdx.x == 0) p.trace[(size_t)blockIdx.x * 16 + (i)] = globaltimer_ns(); } while (0)
-template <int NS, int MASK>  // MASK >= 0: the identity mask (PostParams::identity_mask) is this compile-time constant
+// RAW_ONLY: steps A-D only, ending with raw_argmax (the argmax launch of a sequence call, sequence_filter_kernel does
+// the rest); no filter state, scratch or frame counter is touched.
+template <int NS, int MASK, bool RAW_ONLY = false>  // MASK >= 0: the identity mask (PostParams::identity_mask) is this compile-time constant
 __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const __grid_constant__ PostParams p) {
   extern __shared__ float4 s_dyn4[];
   float* s_dyn = reinterpret_cast<float*>(s_dyn4);
@@ -823,12 +895,12 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
     if (part == 0) {
       // the two 2D filters of this joint: state fetched now, used after the argmax
       static_assert(sizeof(FilterState) == 48, "three 16-byte pieces per filter state");
-      if (tid < 6 && p.filters_on) {
+      if (tid < 6 && !RAW_ONLY && p.filters_on) {
         const int sid = p.stream_ids[frame];
         cp_async_16(reinterpret_cast<char*>(s_st2) + tid * 16,
                     reinterpret_cast<const char*>(p.st2d + ((size_t)sid * kJoints + joint) * 2) + tid * 16);
         if (tid == 0) { s_sid = sid; s_t2 = p.t2d[frame]; s_t3 = p.t3d[frame]; }
-      } else if (tid < 15 && p.filters_on) {  // this joint's three 3D filter states (144 contiguous bytes)
+      } else if (tid < 15 && !RAW_ONLY && p.filters_on) {  // this joint's three 3D filter states (144 contiguous bytes)
         const int sid = p.stream_ids[frame];
         cp_async_16(reinterpret_cast<char*>(s_st3) + (tid - 6) * 16,
                     reinterpret_cast<const char*>(p.st3d + ((size_t)sid * kJoints + joint) * 3) + (tid - 6) * 16);
@@ -1047,7 +1119,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
   if (p.trace != nullptr && tid == 0) p.trace[(size_t)blockIdx.x * 16 + 13] = (unsigned long long)nq;
   // Five lanes of warp 1 advance the clock-only part (four dependent divisions, ~0.5 us each here) of this joint's two 2D
   // and three 3D filter steps while warp 0 evaluates the quads; the 3D ones go to global scratch for the frame's tail.
-  if (p.filters_on && tid >= 32 && tid < 37) {
+  if (!RAW_ONLY && p.filters_on && tid >= 32 && tid < 37) {
     const int k = tid - 32;
     if (k < 2) {
       const FilterPrep f = oef_prepare(s_st2[k], p.cfg2d, s_t2);
@@ -1163,46 +1235,30 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
     double coord = (tid == 0) ? (double)row : (double)col;
     if (tid < 2) {
       p.raw_argmax[(frame * kJoints + joint) * 2 + tid] = (tid == 0) ? row : col;
-      if (p.filters_on) {
+      if (!RAW_ONLY && p.filters_on) {
         FilterState st2 = s_st2[tid];
         const FilterPrep f = {s_prep[tid][0], s_prep[tid][1], s_prep[tid][2]};
         coord = oef_finish(st2, p.cfg2d, f, coord, s_t2, false);
         p.st2d[((size_t)s_sid * kJoints + joint) * 2 + tid] = st2;
       }
-      p.j2_box[(frame * kJoints + joint) * 2 + tid] = coord;
+      if (!RAW_ONLY) p.j2_box[(frame * kJoints + joint) * 2 + tid] = coord;
     }
     const double py = __shfl_sync(0xffffffffu, coord, 0), px = __shfl_sync(0xffffffffu, coord, 1);
     if (tid == 0) { s_pt[0] = py; s_pt[1] = px; }
     POST_TRACE(7);
   }
+  if (RAW_ONLY) return;
   __syncthreads();
   // utils.hm_pt_interp_bilinear (utils.py:58-79) on the three averaged location maps.  The 3 maps x 4 cells x n_scales
   // resampled values are fetched by 12*n_scales threads at once (the first version walked them serially in 3 threads
   // and the dependent global loads dominated the kernel); the float64 arithmetic and its order are unchanged.
   {
     const double py = s_pt[0], px = s_pt[1];
-    const double sx = __dsub_rn(__dmul_rn(__dadd_rn(px, 0.5), 0.125), 0.5);  // / 8 exactly
-    const double sy = __dsub_rn(__dmul_rn(__dadd_rn(py, 0.5), 0.125), 0.5);
-    int x0 = (int)sx, y0 = (int)sy;  // truncation toward zero, like int()
-    x0 = min(max(x0, 0), hs - 1);    // memory safety only: filtered joints stay inside the box
-    y0 = min(max(y0, 0), hs - 1);
-    const int x1 = min(x0 + 1, hs - 1), y1 = min(y0 + 1, hs - 1);
-    // rescale to input pixels (estimator.py:138-139; + the crop origin for tracked streams, run_estimator.py:104-105):
-    // two lanes of warp 1, beside the gather of warp 0
+    const GatherPoint g = gather_point(py, px, hs);
+    // rescale to input pixels: two lanes of warp 1, beside the gather of warp 0
     if (tid >= 32 && tid < 34) {
       const int c = tid - 32;
-      const double jb = c == 0 ? py : px;
-      double off = (c == 0) ? (double)p.off_y : (double)p.off_x, scaler = p.scaler;
-      double v2;
-      if (p.geoms != nullptr) {
-        const FrameGeom g = p.geoms[frame];
-        off = (c == 0) ? (double)g.off_y : (double)g.off_x;
-        scaler = g.scaler;
-        v2 = __ddiv_rn(__dsub_rn(jb, off), scaler);
-        v2 = __dadd_rn(v2, (c == 0) ? (double)g.y : (double)g.x);
-      } else {
-        v2 = __ddiv_rn(__dsub_rn(jb, off), scaler);
-      }
+      const double v2 = rescale_joint(p, frame, c, c == 0 ? py : px);
       p.out2d[(frame * kJoints + joint) * 2 + c] = v2;
       if (p.packed != nullptr) p.packed[(frame * kJoints + joint) * 5 + c] = v2;
     }
@@ -1212,7 +1268,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
       const int cell = (tid / ns) & 3;
       const int map = tid / (4 * ns);
       const float* m = p.maps + ((size_t)(frame * ns + sc) * 84 + kJoints * (1 + map) + joint) * cells;
-      const float gv = scaled_cell(m, hs, p.tables[sc], (cell & 2) ? y1 : y0, (cell & 1) ? x1 : x0);
+      const float gv = scaled_cell(m, hs, p.tables[sc], (cell & 2) ? g.y1 : g.y0, (cell & 1) ? g.x1 : g.x0);
       s_gather[tid] = gv;
       if (!(fabsf(gv) <= 3.4028234e38f) && p.nonfinite != nullptr) {
         atomicAdd(p.nonfinite, 1u);
@@ -1220,7 +1276,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
       }
     }
     __syncthreads();
-    if (tid < 3) {
+    if (tid < 3) {  // gather_combine's arithmetic, kept inline: through the function the MASK = -1 SASS changes
       double v[4];
 #pragma unroll
       for (int cell = 0; cell < 4; ++cell) {
@@ -1229,8 +1285,8 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
         // an exact scaling for 1, 2 or 4 scales, bit-identical to the division
         v[cell] = ns == 1 ? acc : ns == 2 ? __dmul_rn(acc, 0.5) : ns == 4 ? __dmul_rn(acc, 0.25) : __ddiv_rn(acc, (double)ns);
       }
-      const double wx1 = __dsub_rn((double)x1, sx), wx0 = __dsub_rn(sx, (double)x0);
-      const double wy1 = __dsub_rn((double)y1, sy), wy0 = __dsub_rn(sy, (double)y0);
+      const double wx1 = __dsub_rn((double)g.x1, g.sx), wx0 = __dsub_rn(g.sx, (double)g.x0);
+      const double wy1 = __dsub_rn((double)g.y1, g.sy), wy0 = __dsub_rn(g.sy, (double)g.y0);
       const double value0 = __dadd_rn(__dmul_rn(wx1, v[0]), __dmul_rn(wx0, v[1]));
       const double value1 = __dadd_rn(__dmul_rn(wx1, v[2]), __dmul_rn(wx0, v[3]));
       const double val = __dadd_rn(__dmul_rn(wy1, value0), __dmul_rn(wy0, value1));
@@ -1267,6 +1323,110 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
   if (p.trace != nullptr && tid == 0) p.trace[(size_t)blockIdx.x * 16 + 12] = (unsigned long long)clock64();
 }
 #undef POST_TRACE
+
+// ---------------------------------------------------------------------------------------------------------------
+// Sequence calls: a stream id may appear several times in one call, its frames consecutive in time in call order.
+// postprocess_kernel<NS, MASK, true> gives every frame's raw argmax (it depends on no other frame); this kernel then
+// walks each stream's frames in order through everything that carries state from one frame to the next.  Segment
+// table (host: stage_sequence_meta): seg[0] = number of distinct streams n_seg, seg[1 .. n_seg+1] = where each stream's
+// frames start in the frame list seg[n_seg + 2 ..], which holds the frame indices of every stream in call order.
+// grid = n_frames blocks (the surplus ones return), so the launch does not depend on the composition; block b = the
+// b-th distinct stream.  Same arithmetic as postprocess_kernel's step E and frame tail:
+//   1. 42 threads, one per (joint, axis), walk the 2D filters and write j2_box, out2d (and packed); 63 other threads
+//      walk the clock-only part (FilterPrep) of the 3D filters ahead, into prep3;
+//   2. all threads gather the three location maps at the filtered points of every (frame, joint), into j3_raw;
+//   3. 63 threads, one per (joint, axis), subtract the root and walk the 3D filters: out3d (and packed).
+constexpr int kSeqThreads = 512;
+template <int NS>
+__global__ void __launch_bounds__(kSeqThreads) sequence_filter_kernel(const __grid_constant__ PostParams p,
+                                                                      const int* __restrict__ seg) {
+  const int n_seg = seg[0];
+  if ((int)blockIdx.x >= n_seg) return;
+  const int lo = seg[1 + blockIdx.x], hi = seg[2 + blockIdx.x];
+  const int* fr = seg + 2 + n_seg;
+  const int sid = p.stream_ids[fr[lo]];
+  const int tid = threadIdx.x;
+  if (tid < 2 * kJoints) {
+    const int joint = tid >> 1, c = tid & 1;
+    FilterState st;
+    FilterPrep pr;
+    if (p.filters_on) {
+      st = p.st2d[((size_t)sid * kJoints + joint) * 2 + c];
+      pr = oef_prepare(st, p.cfg2d, p.t2d[fr[lo]]);
+    }
+    for (int k = lo; k < hi; ++k) {
+      const int f = fr[k], i = (f * kJoints + joint) * 2 + c;
+      double coord = (double)p.raw_argmax[i];
+      if (p.filters_on) {
+        const double t = p.t2d[f];
+        FilterPrep nx = pr;
+        if (k + 1 < hi) {  // the next step's clock-only part: independent of this step's value chain
+          FilterState clk = st;
+          clk.freq = pr.freq; clk.lasttime = t; clk.has_time = 1;
+          nx = oef_prepare(clk, p.cfg2d, p.t2d[fr[k + 1]]);
+        }
+        coord = oef_finish(st, p.cfg2d, pr, coord, t, false);
+        pr = nx;
+      }
+      p.j2_box[i] = coord;
+      const double v2 = rescale_joint(p, f, c, coord);
+      p.out2d[i] = v2;
+      if (p.packed != nullptr) p.packed[(f * kJoints + joint) * 5 + c] = v2;
+    }
+    if (p.filters_on) p.st2d[((size_t)sid * kJoints + joint) * 2 + c] = st;
+  } else if (tid >= 64 && tid < 64 + 3 * kJoints && p.filters_on) {
+    const int k3 = tid - 64, joint = k3 / 3, c = k3 - joint * 3;
+    FilterState clk = p.st3d[((size_t)sid * kJoints + joint) * 3 + c];
+    for (int k = lo; k < hi; ++k) {
+      const int f = fr[k];
+      const double t = p.t3d[f];
+      const FilterPrep pr = oef_prepare(clk, p.cfg3d, t);
+      double* o = p.prep3 + ((size_t)(f * kJoints + joint) * 3 + c) * 3;
+      o[0] = pr.freq; o[1] = pr.te; o[2] = pr.a_d;
+      clk.freq = pr.freq; clk.lasttime = t; clk.has_time = 1;
+    }
+  }
+  __syncthreads();
+  // 2. gather: one thread per (frame, joint, map), its 4 cells x NS scales loaded at once
+  for (int item = tid; item < (hi - lo) * kJoints * 3; item += blockDim.x) {
+    const int k = lo + item / (kJoints * 3), r = item - (k - lo) * (kJoints * 3);
+    const int joint = r / 3, map = r - joint * 3;
+    const int f = fr[k];
+    const GatherPoint g = gather_point(p.j2_box[(f * kJoints + joint) * 2], p.j2_box[(f * kJoints + joint) * 2 + 1], p.hs);
+    float v4[4 * NS];
+    bool bad = false;
+#pragma unroll
+    for (int i = 0; i < 4 * NS; ++i) {
+      v4[i] = gather_value<NS>(p, p.hs, p.hs * p.hs, f, joint, map * 4 * NS + i, g);
+      bad |= !(fabsf(v4[i]) <= 3.4028234e38f);
+    }
+    if (bad && p.nonfinite != nullptr) {
+      atomicAdd(p.nonfinite, 1u);
+      if (p.nonfinite_flag != nullptr) *reinterpret_cast<volatile unsigned int*>(p.nonfinite_flag) = 1u;
+    }
+    p.j3_raw[(f * kJoints + joint) * 3 + map] = gather_combine<NS>(v4, 0, g);
+  }
+  __syncthreads();
+  // 3. root subtraction (utils.py:218) and the 3D filters in frame order
+  if (tid < 3 * kJoints) {
+    const int joint = tid / 3, c = tid - joint * 3;
+    FilterState st;
+    if (p.filters_on) st = p.st3d[((size_t)sid * kJoints + joint) * 3 + c];
+    for (int k = lo; k < hi; ++k) {
+      const int f = fr[k];
+      const float* raw = p.j3_raw + f * kJoints * 3;
+      float v = __fsub_rn(raw[joint * 3 + c], raw[kRootJoint * 3 + c]);
+      if (p.filters_on) {
+        const double* pr = p.prep3 + ((size_t)(f * kJoints + joint) * 3 + c) * 3;
+        const FilterPrep fp = {pr[0], pr[1], pr[2]};
+        v = __double2float_rn(oef_finish(st, p.cfg3d, fp, (double)v, p.t3d[f], true));
+      }
+      p.out3d[(f * kJoints + joint) * 3 + c] = v;
+      if (p.packed != nullptr) p.packed[(f * kJoints + joint) * 5 + 2 + c] = (double)v;
+    }
+    if (p.filters_on) p.st3d[((size_t)sid * kJoints + joint) * 3 + c] = st;
+  }
+}
 
 // Bounding-box tracker of the reference's video loop (run_estimator.py:110-119), one warp per frame:
 //   buffer_x = 0.8 * (x_max - x_min + 1);  buffer_y = 0.2 * (y_max - y_min + 1)

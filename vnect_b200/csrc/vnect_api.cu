@@ -95,6 +95,10 @@ struct vnect_handle {
     size_t table_off = 0;
     FrameDesc *h_table = nullptr, *d_table = nullptr;
     FrameGeom* d_geoms = nullptr;         // [max_frames]
+    // sequence calls: the segment table of sequence_filter_kernel (n_seg, [max_frames + 1] starts, [max_frames] frame
+    // indices) after the frame table, copied with it
+    size_t seg_off = 0;
+    int *h_seg = nullptr, *d_seg = nullptr;
     unsigned int* h_nonfinite = nullptr;  // pinned + device-visible: set by the post-process when a batch of this lane met NaN / Inf maps
     cudaEvent_t copy_done = nullptr, done = nullptr;
     bool pending = false;
@@ -103,6 +107,8 @@ struct vnect_handle {
   cudaStream_t copy_stream = nullptr;
   std::vector<unsigned int> seen_stamp;  // duplicate stream ids within a call (stage_frame_meta)
   unsigned int seen_epoch = 0;
+  std::vector<int> seq_slot;             // stage_sequence_meta: a stream's segment in the current call
+  std::vector<double> seq_t2d, seq_t3d;  // stage_sequence_meta: a stream's last timestamps as the call's frames advance
   unsigned device_calls = 0;
   // tracked streams (run_estimator.py:100-119): per-stream crop box on the device, per-call frame geometry
   int4* d_boxes = nullptr;         // [max_streams] (x, y, w, h)
@@ -606,19 +612,22 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       const size_t off_t2 = ((size_t)mf * sizeof(int) + 15) & ~size_t(15), off_t3 = off_t2 + (size_t)mf * sizeof(double);
       L.meta_bytes = off_t3 + (size_t)mf * sizeof(double);
       L.table_off = (L.meta_bytes + 15) & ~size_t(15);
-      const size_t block = L.table_off + (size_t)mf * sizeof(FrameDesc);
+      L.seg_off = L.table_off + (size_t)mf * sizeof(FrameDesc);
+      const size_t block = L.seg_off + (size_t)(2 * mf + 2) * sizeof(int);
       uint8_t* d_meta = nullptr;
       if ((rc = dev_alloc(h, &d_meta, block))) return rc;
       L.d_stream_ids = reinterpret_cast<int*>(d_meta);
       L.d_t2d = reinterpret_cast<double*>(d_meta + off_t2);
       L.d_t3d = reinterpret_cast<double*>(d_meta + off_t3);
       L.d_table = reinterpret_cast<FrameDesc*>(d_meta + L.table_off);
+      L.d_seg = reinterpret_cast<int*>(d_meta + L.seg_off);
       CU(h, cudaMallocHost(&L.h_meta, block));
       memset(L.h_meta, 0, block);
       L.h_stream_ids = reinterpret_cast<int*>(L.h_meta);
       L.h_t2d = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + off_t2);
       L.h_t3d = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + off_t3);
       L.h_table = reinterpret_cast<FrameDesc*>(static_cast<uint8_t*>(L.h_meta) + L.table_off);
+      L.h_seg = reinterpret_cast<int*>(static_cast<uint8_t*>(L.h_meta) + L.seg_off);
     }
     if ((rc = dev_alloc(h, &L.d_geoms, mf))) return rc;
     if ((rc = dev_alloc(h, &L.d_out2d, (size_t)mf * kJoints * 2))) return rc;
@@ -1096,9 +1105,85 @@ static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids,
   return VNECT_OK;
 }
 
-// geoms: per-frame geometry (tracked streams, mixed sizes), which overrides scaler and the offsets
+// stage_frame_meta for a sequence call: a stream id may repeat, its frames being consecutive in time in call order.
+// Every frame's timestamps are checked against its stream's previous reading -- the one before the call, then the
+// call's own earlier frames -- with stage_frame_meta's rules and messages, and only once the whole call has passed is
+// anything recorded.  The segment table of sequence_filter_kernel goes to the lane's pinned block after the frame
+// table, and ids, timestamps, table and segments travel in one copy.
+static int stage_sequence_meta(vnect_t* h, int n_frames, const int32_t* stream_ids, const double* t2d,
+                               const double* t3d, cudaStream_t copy_on) {
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
+  if (!stream_ids) return fail(h, VNECT_E_INVALID, "a sequence call needs stream ids");
+  if (h->cfg.filters && (!t2d || !t3d)) return fail(h, VNECT_E_INVALID, "timestamps required when filters are on");
+  const int ms = h->cfg.max_streams;
+  h->seen_stamp.resize(ms, 0);
+  h->seq_slot.resize(ms, 0);
+  h->seq_t2d.resize(ms, NAN);
+  h->seq_t3d.resize(ms, NAN);
+  const unsigned int stamp = ++h->seen_epoch;
+  vnect_handle::Lane* L = h->cur;
+  int* starts = L->h_seg + 1;
+  int n_seg = 0;
+  for (int i = 0; i < n_frames; ++i) {
+    const int sid = stream_ids[i];
+    if (sid < 0 || sid >= ms) return fail(h, VNECT_E_INVALID, "stream id %d not in [0, %d)", sid, ms);
+    if (h->seen_stamp[sid] != stamp) {
+      h->seen_stamp[sid] = stamp;
+      h->seq_slot[sid] = n_seg;
+      starts[n_seg++] = 0;
+      h->seq_t2d[sid] = h->last_t2d[sid];
+      h->seq_t3d[sid] = h->last_t3d[sid];
+    }
+    ++starts[h->seq_slot[sid]];
+    if (h->cfg.filters) {
+      const double l2 = h->seq_t2d[sid], l3 = h->seq_t3d[sid];
+      if (l2 == l2 && l2 != 0.0 && t2d[i] != 0.0 && t2d[i] == l2)
+        return fail(h, VNECT_E_ZERO_DT, "float division by zero (stream %d: repeated 2D timestamp %.17g)", sid, t2d[i]);
+      if (l3 == l3 && l3 != 0.0 && t3d[i] != 0.0 && t3d[i] == l3)
+        return fail(h, VNECT_E_ZERO_DT, "float division by zero (stream %d: repeated 3D timestamp %.17g)", sid, t3d[i]);
+      if (l2 == l2 && l2 != 0.0 && t2d[i] != 0.0 && t2d[i] < l2)
+        return fail(h, VNECT_E_INVALID, "alpha should be in (0.0, 1.0] (stream %d: 2D timestamp %.17g earlier than the previous %.17g)", sid, t2d[i], l2);
+      if (l3 == l3 && l3 != 0.0 && t3d[i] != 0.0 && t3d[i] < l3)
+        return fail(h, VNECT_E_INVALID, "alpha should be in (0.0, 1.0] (stream %d: 3D timestamp %.17g earlier than the previous %.17g)", sid, t3d[i], l3);
+      h->seq_t2d[sid] = t2d[i];
+      h->seq_t3d[sid] = t3d[i];
+    }
+  }
+  // counts -> starts (exclusive prefix sum), then the frame list, each stream's frames in call order
+  L->h_seg[0] = n_seg;
+  for (int b = 0, acc = 0; b <= n_seg; ++b) {
+    const int c = b < n_seg ? starts[b] : 0;
+    starts[b] = acc;
+    acc += c;
+  }
+  int* list = L->h_seg + 2 + n_seg;
+  for (int i = 0; i < n_frames; ++i) {
+    const int sid = stream_ids[i];
+    list[starts[h->seq_slot[sid]]++] = i;
+  }
+  for (int b = n_seg; b > 0; --b) starts[b] = starts[b - 1];  // the fill advanced each start to the next one's
+  starts[0] = 0;
+  for (int i = 0; i < n_frames; ++i) {
+    const int sid = stream_ids[i];
+    L->h_stream_ids[i] = sid;
+    L->h_t2d[i] = t2d ? t2d[i] : 0.0;
+    L->h_t3d[i] = t3d ? t3d[i] : 0.0;
+    if (h->cfg.filters) {
+      h->last_t2d[sid] = h->seq_t2d[sid];
+      h->last_t3d[sid] = h->seq_t3d[sid];
+    }
+  }
+  const size_t bytes = L->seg_off + (size_t)(2 + n_seg + n_frames) * sizeof(int);
+  CU(h, cudaMemcpyAsync(L->d_stream_ids, L->h_meta, bytes, cudaMemcpyHostToDevice, copy_on));
+  return VNECT_OK;
+}
+
+// geoms: per-frame geometry (tracked streams, mixed sizes), which overrides scaler and the offsets.
+// seq_seg: a sequence call's device segment table (stage_sequence_meta): the argmax-only instantiation, then
+// sequence_filter_kernel walks each stream's frames in order.
 static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, int off_y, double* dev_out2d,
-                           float* dev_out3d, const FrameGeom* geoms = nullptr, bool guard = true) {
+                           float* dev_out3d, const FrameGeom* geoms = nullptr, bool guard = true,
+                           const int* seq_seg = nullptr) {
   PostParams p;
   p.geoms = geoms;
   p.n_frames = n_frames; p.n_scales = h->n_scales; p.hs = h->hs; p.S = h->S;
@@ -1133,6 +1218,35 @@ static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, i
   };
   // the usual pyramid (scale 1.0 first, smaller ones after) gets its identity mask as a compile-time constant
   static unsigned long long done1[kMaxScales] = {0, 0, 0, 0};
+  if (seq_seg != nullptr) {
+    static unsigned long long done_raw[2][kMaxScales] = {{0, 0, 0, 0}, {0, 0, 0, 0}};
+    if (p.identity_mask == 1) {
+      switch (h->n_scales) {
+        case 1: CU(h, launch(postprocess_kernel<1, 1, true>, &done_raw[0][0])); break;
+        case 2: CU(h, launch(postprocess_kernel<2, 1, true>, &done_raw[0][1])); break;
+        case 3: CU(h, launch(postprocess_kernel<3, 1, true>, &done_raw[0][2])); break;
+        default: CU(h, launch(postprocess_kernel<4, 1, true>, &done_raw[0][3])); break;
+      }
+    } else {
+      switch (h->n_scales) {
+        case 1: CU(h, launch(postprocess_kernel<1, -1, true>, &done_raw[1][0])); break;
+        case 2: CU(h, launch(postprocess_kernel<2, -1, true>, &done_raw[1][1])); break;
+        case 3: CU(h, launch(postprocess_kernel<3, -1, true>, &done_raw[1][2])); break;
+        default: CU(h, launch(postprocess_kernel<4, -1, true>, &done_raw[1][3])); break;
+      }
+    }
+    ++h->launches;
+    // one block per distinct stream; n_frames blocks whatever the composition, so one graph serves them all
+    switch (h->n_scales) {
+      case 1: sequence_filter_kernel<1><<<n_frames, kSeqThreads, 0, h->stream>>>(p, seq_seg); break;
+      case 2: sequence_filter_kernel<2><<<n_frames, kSeqThreads, 0, h->stream>>>(p, seq_seg); break;
+      case 3: sequence_filter_kernel<3><<<n_frames, kSeqThreads, 0, h->stream>>>(p, seq_seg); break;
+      default: sequence_filter_kernel<4><<<n_frames, kSeqThreads, 0, h->stream>>>(p, seq_seg); break;
+    }
+    CU(h, cudaGetLastError());
+    ++h->launches;
+    return VNECT_OK;
+  }
   if (p.identity_mask == 1) {
     switch (h->n_scales) {
       case 1: CU(h, launch(postprocess_kernel<1, 1>, &done1[0])); break;
@@ -1240,14 +1354,17 @@ extern "C" {
 
 // pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
 static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
-                        const FrameSource& src, double* out2d, float* out3d, bool tracked = false) {
+                        const FrameSource& src, double* out2d, float* out3d, bool tracked = false,
+                        bool sequence = false) {
   if (src.table) {  // sizes, addresses and geometry live in the lane's device tables, not in kernel parameters
     if (int rc = ensure_surround(h)) return rc;
     auto direct = [&]() -> int {
       int rc;
       if ((rc = run_preprocess(h, nullptr, n_frames, 0, 0, src, Geometry{}, tracked))) return rc;
       if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
-      if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, out2d, out3d, h->cur->d_geoms))) return rc;
+      if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, out2d, out3d, h->cur->d_geoms, true,
+                                sequence ? h->cur->d_seg : nullptr)))
+        return rc;
       if (tracked) {
         track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table, h->d_boxes);
         CU(h, cudaGetLastError());
@@ -1256,8 +1373,9 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
       return VNECT_OK;
     };
     if (!h->use_graphs) return direct();
-    const vnect_handle::GraphKey key(4 + lane + (tracked ? 2 : 0), n_frames, 0, 0, 0, 0, nullptr, out2d, out3d,
-                                     src.format, 0, 0, 0);
+    // sequence calls (8 + lane) read their segment table from the lane's device block as well
+    const vnect_handle::GraphKey key(sequence ? 8 + lane : 4 + lane + (tracked ? 2 : 0), n_frames, 0, 0, 0, 0, nullptr,
+                                     out2d, out3d, src.format, 0, 0, 0);
     return run_graphed(h, key, direct);
   }
   const Geometry g = squarify_geometry(h->S, H, W, src.format);
@@ -1470,10 +1588,12 @@ static int check_frames(vnect_t* h, const vnect_frame* frames, int n_frames, int
 
 // vnect_submit_frames / vnect_track_frames / vnect_submit_track_frames once the table is validated: the frames are
 // staged into the lane's buffer one after another (BGR packed tight, YUV in cv2's layout) and the table points at the
-// staged copies.  `synchronous`: wait for the lane before returning (vnect_track_frames).
+// staged copies.  `synchronous`: wait for the lane before returning (vnect_track_frames).  `sequence`: a stream id
+// may repeat (vnect_submit_sequence).
 static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
-                         float* joints3d, bool tracked, int32_t* boxes_used, bool synchronous) {
+                         float* joints3d, bool tracked, int32_t* boxes_used, bool synchronous,
+                         bool sequence = false) {
   int rc = lane_acquire(h, lane);
   if (rc) return rc;
   uint8_t* d = h->cur->d_frames;
@@ -1497,14 +1617,17 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
     }
   }
   // ids, timestamps and the table in one copy; a refused id or timestamp returns before any frame copy is queued
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
+  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream)
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames);
+  if (rc) return rc;
   for (int i = 0; i < n_frames; ++i)
     if ((rc = stage_frame(h, const_cast<uint8_t*>(h->cur->h_table[i].data), frames[i].data, frames[i].height,
                           frames[i].width, frame_source(frames[i], format))))
       return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), h->cur->d_out2d, h->cur->d_out3d, tracked)))
+  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), h->cur->d_out2d, h->cur->d_out3d, tracked,
+                         sequence)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
@@ -1519,15 +1642,18 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
 // are used as they are; the lanes alternate for the per-call meta so the host can run one call ahead of the GPU
 static int device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
-                         float* dev_joints3d, bool tracked, int32_t* dev_boxes_used) {
+                         float* dev_joints3d, bool tracked, int32_t* dev_boxes_used, bool sequence = false) {
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
   memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames))) return rc;
+  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream)
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames);
+  if (rc) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
-  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d, tracked)))
+  if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d, tracked,
+                         sequence)))
     return rc;
   if (dev_boxes_used)  // outside the graph, so the caller's pointer stays out of its key
     CU(h, cudaMemcpyAsync(dev_boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToDevice,
@@ -1601,6 +1727,32 @@ int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_f
   if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
   return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, true,
                        dev_boxes_used);
+}
+
+// Sequence calls (include/vnect_b200.h): the table paths above with a stream id allowed to repeat.  Filter state is
+// read and written only by sequence_filter_kernel on the handle's stream, so a stream continues across sequence calls
+// on either lane and across ordinary calls in submission order.
+int vnect_submit_sequence(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
+                          float* joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
+  if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
+  return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr,
+                       false, true);
+}
+
+int vnect_estimate_device_sequence(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
+                                   const int32_t* stream_ids, const double* t2d, const double* t3d,
+                                   double* dev_joints2d, float* dev_joints3d) {
+  if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
+  ON_DEVICE(h);
+  if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
+  return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, false, nullptr,
+                       true);
 }
 
 int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
@@ -1803,6 +1955,29 @@ int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float*
   if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false))) return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if (raw_argmax)
+    CU(h, cudaMemcpyAsync(raw_argmax, h->d_raw_argmax, (size_t)n_frames * kJoints * 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaStreamSynchronize(h->stream));
+  return VNECT_OK;
+}
+
+// vnect_postprocess for a sequence call: the argmax launch and sequence_filter_kernel on the given maps, lane 0.
+int vnect_postprocess_sequence(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm,
+                               int32_t n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
+                               double scaler, int32_t offset_x, int32_t offset_y, double* joints2d, float* joints3d,
+                               int32_t* raw_argmax) {
+  if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
+  ON_DEVICE(h);
+  if (!hm || !xm || !ym || !zm || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
+  int rc = lane_acquire(h, 0);
+  if (rc) return rc;
+  vnect_handle::Lane* L = h->cur;
+  if ((rc = stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->stream))) return rc;
+  if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
+  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, L->d_out2d, L->d_out3d, nullptr, false, L->d_seg)))
+    return rc;
+  CU(h, cudaMemcpyAsync(joints2d, L->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(h, cudaMemcpyAsync(joints3d, L->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (raw_argmax)
     CU(h, cudaMemcpyAsync(raw_argmax, h->d_raw_argmax, (size_t)n_frames * kJoints * 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaStreamSynchronize(h->stream));

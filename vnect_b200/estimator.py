@@ -215,6 +215,7 @@ class VNectEngine:
         self.max_streams = int(max_streams if max_streams is not None else max_frames)
         self.max_input = tuple(max_input) if max_input else (self.box_size, self.box_size)
         self.device = int(device)
+        self.filters = bool(filters)
         cfg = _capi.Config()
         cfg.device = self.device
         cfg.box_size = self.box_size
@@ -366,6 +367,46 @@ class VNectEngine:
         self._inflight[int(lane)] = (keep, j2, j3)  # keep the buffers alive
         return j2, j3
 
+    def _sequence_meta(self, n, stream_ids, t2d, t3d):
+        """_meta for a sequence call: ids are required and, with filters on, one 2D and one 3D reading per frame (a
+        default clock reading would repeat within the call)."""
+        if stream_ids is None:
+            raise ValueError("a sequence call needs stream_ids")
+        if self.filters and (t2d is None or t3d is None):
+            raise ValueError("a sequence call with filters on needs t2d and t3d for every frame")
+        return self._meta(n, stream_ids, 0.0 if t2d is None else t2d, 0.0 if t3d is None else t3d)
+
+    def estimate_sequence(self, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """estimate_frames() where a stream id may appear several times: the frames of one stream are consecutive in
+        time in call order (they may be interleaved with other streams' frames).  Frame i gets bit for bit what
+        estimate_frames() gives when the frames go in one per call in call order; the CNN runs over the whole call at
+        batch size.  A call refused for its ids or timestamps processes none of its frames."""
+        j2, j3 = self.submit_sequence(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+        self.wait(0)
+        return j2, j3
+
+    def submit_sequence(self, lane, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+        """submit_frames() for a sequence call (see estimate_sequence); completes with wait(lane)."""
+        table, keep = frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
+        j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        self._check(self._lib.vnect_submit_sequence(self._h, int(lane), table, n, _format_code(pixel_format),
+                                                    _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[int(lane)] = (keep, j2, j3)  # keep the buffers alive
+        return j2, j3
+
+    def estimate_device_sequence(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids, t2d=None, t3d=None,
+                                 pixel_format="bgr"):
+        """estimate_device_frames() for a sequence call (see estimate_sequence).  Asynchronous."""
+        table = device_frame_table(frames, pixel_format)
+        n = len(table)
+        ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
+        self._check(self._lib.vnect_estimate_device_sequence(self._h, table, n, _format_code(pixel_format), _ptr(ids),
+                                                             _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
+                                                             C.c_void_p(dev_j3_ptr)))
+
     def wait(self, lane):
         """Completes the lane's submission: (joints_2d, joints_3d), or (joints_2d, joints_3d, boxes_used) after
         submit_track / submit_track_frames."""
@@ -513,6 +554,18 @@ class VNectEngine:
         self._check(self._lib.vnect_postprocess(self._h, *[_ptr(m) for m in maps], n, _ptr(ids), _ptr(t2d), _ptr(t3d),
                                                 float(scaler), int(offsets[0]), int(offsets[1]), _ptr(j2), _ptr(j3),
                                                 _ptr(raw)))
+        return j2, j3, raw
+
+    def postprocess_sequence(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None):
+        """postprocess() for a sequence call (see estimate_sequence) on given maps.  Returns (joints_2d, joints_3d,
+        raw_argmax)."""
+        maps, n = check_maps(maps, len(self.scales), self.hm_size)
+        ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
+        j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
+        raw = np.empty((n, JOINTS, 2), np.int32)
+        self._check(self._lib.vnect_postprocess_sequence(self._h, *[_ptr(m) for m in maps], n, _ptr(ids), _ptr(t2d),
+                                                         _ptr(t3d), float(scaler), int(offsets[0]), int(offsets[1]),
+                                                         _ptr(j2), _ptr(j3), _ptr(raw)))
         return j2, j3, raw
 
     def track_postprocess(self, maps, frame_hw, stream_ids=None, t2d=None, t3d=None):
