@@ -211,6 +211,36 @@ int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_f
  * below 2. */
 int vnect_track_set_boxes(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* xywh);
 
+/* Frame orientation of a stream: a camera mounted sideways, upside down or mirrored.  A stream with orientation o
+ * that is given stored frame F produces bit for bit what a stream with VNECT_ORIENT_IDENTITY produces for the
+ * materialised frame orient(F, o): joints2d, joints3d, the raw argmax, the packed results, boxes_used, the box left
+ * behind, the filter state and the timestamp mirror.  Every coordinate the caller sees is in the oriented frame
+ * (joints2d, boxes of vnect_track_set_box(es) / vnect_track_get_box, boxes_used, frame_hw of vnect_track_postprocess);
+ * a frame's data, height, width, pitches and chroma layout describe it as stored, and max_input and the YUV layout
+ * rules apply to the stored frame.  The tracked box is clamped to the oriented frame's sides.
+ * The codes, with the numpy definition that is the contract, for a stored frame f of H x W and oriented pixel (yo, xo)
+ * read from stored pixel (ys, xs).  Codes 1, 3, 6 and 7 swap the frame's sides.  A YUV 4:2:0 frame is oriented as
+ * the BGR image cv2.cvtColor gives (the same as converting oriented planes, H and W being even). */
+#define VNECT_ORIENT_IDENTITY 0   /* f                                     (ys, xs) = (yo, xo)             */
+#define VNECT_ORIENT_ROT90_CW 1   /* np.rot90(f, 3)                        (ys, xs) = (H-1-xo, yo)         */
+#define VNECT_ORIENT_ROT180 2     /* np.rot90(f, 2)                        (ys, xs) = (H-1-yo, W-1-xo)     */
+#define VNECT_ORIENT_ROT90_CCW 3  /* np.rot90(f, 1)                        (ys, xs) = (xo, W-1-yo)         */
+#define VNECT_ORIENT_FLIP_H 4     /* f[:, ::-1] (mirror)                   (ys, xs) = (yo, W-1-xo)         */
+#define VNECT_ORIENT_FLIP_V 5     /* f[::-1]                               (ys, xs) = (H-1-yo, xo)         */
+#define VNECT_ORIENT_TRANSPOSE 6  /* f.transpose(1, 0, 2)                  (ys, xs) = (xo, yo)             */
+#define VNECT_ORIENT_TRANSVERSE 7 /* np.rot90(f, 2).transpose(1, 0, 2)     (ys, xs) = (H-1-xo, W-1-yo)     */
+/* Sets the orientation of n streams (HOST arrays stream_ids int32 [n] and codes int32 [n], copied by the call;
+ * n = 0 does nothing).  Host-only, nothing is enqueued: every call submitted after it, on either lane, uses the new
+ * codes, and calls already submitted keep the ones they were submitted with.  Orientation is configuration, not
+ * temporal state: vnect_reset_stream keeps it and vnect_export / import_stream_state do not carry it, so a stream
+ * moved to another handle needs its orientation set there too.  A call in which every frame's stream has
+ * VNECT_ORIENT_IDENTITY runs exactly as before (same launches, graphs and kernels).
+ * Refused with VNECT_E_INVALID, changing nothing: n below 0, a null array, an id outside [0, max_streams), an id
+ * given twice, a code outside [0, 8). */
+int vnect_set_orientations(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* codes);
+/* the orientation of one stream */
+int vnect_get_orientation(vnect_t* h, int32_t stream_id, int32_t* code);
+
 /* Sequence calls: consecutive frames of one stream in one batch (offline video: annotating a dataset, re-processing a
  * recording, motion capture from footage).  Up to max_frames frames in which a stream id may appear more than once;
  * the frames of one stream are consecutive in time in the order they appear in the call, and may be interleaved with

@@ -4,7 +4,7 @@ Public surface: ``VNectEstimator`` (drop-in for the reference class, src/estimat
 batched multi-stream form).  The compute lives in ``lib/libvnect_b200.so`` (hand-written CUDA: tcgen05/TMEM/TMA
 implicit-GEMM convolutions, fused pre- and post-processing); this package only marshals pointers through ctypes.
 """
-from .estimator import Joints2Angles, VNectEngine, VNectEstimator  # noqa: F401
+from .estimator import ORIENTATIONS, Joints2Angles, VNectEngine, VNectEstimator  # noqa: F401
 from .hog_box import HOGBox  # noqa: F401
 
-__all__ = ["VNectEstimator", "VNectEngine", "Joints2Angles", "HOGBox"]
+__all__ = ["VNectEstimator", "VNectEngine", "Joints2Angles", "HOGBox", "ORIENTATIONS"]

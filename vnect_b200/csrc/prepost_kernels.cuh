@@ -77,7 +77,7 @@ struct FrameGeom {
   int dh, dw;               // scaled content size (cvRound(h*scaler), cvRound(w*scaler))
   int off_x, off_y;         // placement inside the S x S box (utils.py:82-104)
   int mode;                 // 0 bilinear, 1 exact 2x decimation (INTER_AREA)
-  int pad_;
+  int orient;               // VNECT_ORIENT_* of the frame (frame_geometry_oriented_kernel; 0 elsewhere)
   double scaler, inv_scale;
 };
 
@@ -115,6 +115,7 @@ struct BgrSrc {
   __device__ __forceinline__ BgrSrc(const uint8_t* frame, const SquarifyParams& sp) : p(frame), pitch(sp.pitch) {}
   __device__ __forceinline__ BgrSrc(const FrameDesc& f, const SquarifyParams&) : p(f.data), pitch(f.pitch) {}
   __device__ __forceinline__ void crop(int x, int y) { p += (int64_t)y * pitch + (int64_t)x * 3; }
+  __device__ __forceinline__ void crop(const FrameGeom& g) { crop(g.x, g.y); }
   __device__ __forceinline__ const uint8_t* at(int y, int x) const { return p + (int64_t)y * pitch + (int64_t)x * 3; }
   __device__ __forceinline__ const uint8_t* below(const uint8_t* q, bool step) const { return q + (step ? pitch : 0); }
   __device__ __forceinline__ int get(const uint8_t* q, int dx, int c) const { return q[dx * 3 + c]; }
@@ -133,6 +134,7 @@ struct Yuv420Src {
       : luma(f.data), u(f.data + f.u_offset), v(f.data + f.v_offset), pitch(f.pitch), uv_pitch(f.uv_pitch),
         uv_step(sp.uv_step), x0(0), y0(0) {}
   __device__ __forceinline__ void crop(int x, int y) { x0 = x; y0 = y; }
+  __device__ __forceinline__ void crop(const FrameGeom& g) { crop(g.x, g.y); }
   __device__ __forceinline__ int2 at(int y, int x) const { return make_int2(x0 + x, y0 + y); }  // full-frame (x, y)
   __device__ __forceinline__ int2 below(int2 q, bool step) const { return make_int2(q.x, q.y + (step ? 1 : 0)); }
   __device__ __forceinline__ int get(int2 q, int dx, int c) const {
@@ -151,6 +153,70 @@ struct FrameTableSrc : Base {
       : Base(*reinterpret_cast<const FrameDesc*>(entry), sp) {}
 };
 
+// Frame orientation VNECT_ORIENT_* (include/vnect_b200.h) as an index map.  Oriented pixel (yo, xo) of a stored H x W
+// frame is stored pixel (ys, xs): ys comes from xo for the codes that swap the sides (1, 3, 6, 7), from yo otherwise,
+// and is H-1-(that) for codes 1, 2, 5, 7; xs comes from the other one and is W-1-(that) for codes 2, 3, 4, 7.  The map
+// is affine, stored = origin + yo * (step per oriented row) + xo * (step per oriented column), and sends every 2x2
+// block of an even-sided frame to a 2x2 block, so 4:2:0 chroma at (ys >> 1, xs >> 1) is that of the oriented frame.
+__device__ __forceinline__ bool orient_swaps(int o) { return (0xCA >> o) & 1; }
+__device__ __forceinline__ bool orient_rev_y(int o) { return (0xA6 >> o) & 1; }
+__device__ __forceinline__ bool orient_rev_x(int o) { return (0x9C >> o) & 1; }
+
+// squarify_kernel source of an oriented frame of a mixed-size batch (through FrameTableSrc): the crop box and the
+// pixel coordinates are the oriented frame's, FrameGeom::orient is the code, the FrameDesc the frame as stored.
+template <class Base>
+struct Oriented;
+
+// BGR: a handle is the stored pixel's byte pointer; one oriented row / column is `sy` / `sx` bytes (signed), e.g.
+// (pitch, 3) for identity and (3, -pitch) for ROT90_CW.
+template <>
+struct Oriented<BgrSrc> {
+  const uint8_t *frame, *p;
+  int64_t pitch, sy, sx;
+  int H, W;
+  __device__ __forceinline__ Oriented(const FrameDesc& f, const SquarifyParams&)
+      : frame(f.data), p(f.data), pitch(f.pitch), sy(f.pitch), sx(3), H(f.height), W(f.width) {}
+  __device__ __forceinline__ void crop(const FrameGeom& g) {
+    const int o = g.orient;
+    const bool ry = orient_rev_y(o), rx = orient_rev_x(o);
+    const int64_t dy = ry ? -pitch : pitch, dx = rx ? -3 : 3;
+    if (orient_swaps(o)) { sy = dx; sx = dy; } else { sy = dy; sx = dx; }
+    p = frame + (ry ? (int64_t)(H - 1) * pitch : 0) + (rx ? (int64_t)(W - 1) * 3 : 0) + (int64_t)g.y * sy +
+        (int64_t)g.x * sx;
+  }
+  __device__ __forceinline__ const uint8_t* at(int y, int x) const { return p + (int64_t)y * sy + (int64_t)x * sx; }
+  __device__ __forceinline__ const uint8_t* below(const uint8_t* q, bool step) const { return q + (step ? sy : 0); }
+  __device__ __forceinline__ int get(const uint8_t* q, int dx, int c) const { return q[dx * sx + c]; }
+};
+
+// YUV 4:2:0: a handle is the stored full-frame (x, y); `ey` / `ex` are the stored (x, y) steps of one oriented row /
+// column.  Luma and chroma are read at the stored coordinates, like Yuv420Src.
+template <>
+struct Oriented<Yuv420Src> : Yuv420Src {
+  int H, W;
+  int2 org, ey, ex;
+  __device__ __forceinline__ Oriented(const FrameDesc& f, const SquarifyParams& sp)
+      : Yuv420Src(f, sp), H(f.height), W(f.width), org(make_int2(0, 0)), ey(make_int2(0, 1)), ex(make_int2(1, 0)) {}
+  __device__ __forceinline__ void crop(const FrameGeom& g) {
+    const int o = g.orient;
+    const bool ry = orient_rev_y(o), rx = orient_rev_x(o);
+    const int2 dy = make_int2(0, ry ? -1 : 1), dx = make_int2(rx ? -1 : 1, 0);
+    if (orient_swaps(o)) { ey = dx; ex = dy; } else { ey = dy; ex = dx; }
+    org = make_int2((rx ? W - 1 : 0) + g.y * ey.x + g.x * ex.x, (ry ? H - 1 : 0) + g.y * ey.y + g.x * ex.y);
+  }
+  __device__ __forceinline__ int2 at(int y, int x) const {
+    return make_int2(org.x + y * ey.x + x * ex.x, org.y + y * ey.y + x * ex.y);
+  }
+  __device__ __forceinline__ int2 below(int2 q, bool step) const {
+    return step ? make_int2(q.x + ey.x, q.y + ey.y) : q;
+  }
+  __device__ __forceinline__ int get(int2 q, int dx, int c) const {
+    const int xs = q.x + dx * ex.x, ys = q.y + dx * ex.y;
+    const int64_t ci = (int64_t)(ys >> 1) * uv_pitch + (int64_t)(xs >> 1) * uv_step;
+    return yuv_to_bgr(luma[(int64_t)ys * pitch + xs], u[ci], v[ci], c);
+  }
+};
+
 // utils.img_scale_squarify geometry (utils.py:107-120) for box (x, y, w, h) -- same arithmetic as the host version
 __device__ __forceinline__ FrameGeom make_frame_geom(int x, int y, int w, int h, int S) {
   FrameGeom g;
@@ -163,7 +229,7 @@ __device__ __forceinline__ FrameGeom make_frame_geom(int x, int y, int w, int h,
   else g.off_y = S / 2 - g.dh / 2;
   g.inv_scale = __ddiv_rn(1.0, g.scaler);
   g.mode = (g.inv_scale == 2.0) ? 1 : 0;
-  g.pad_ = 0;
+  g.orient = 0;
   return g;
 }
 
@@ -203,8 +269,76 @@ __global__ void frame_geometry_kernel(const FrameDesc* __restrict__ frames, cons
   geoms[i] = make_frame_geom(b.x, b.y, b.z, b.w, S);
 }
 
+// frame_geometry_kernel for a batch with oriented frames (orient[i]: frame i's VNECT_ORIENT_* code): box, clip and
+// geometry are those of the oriented frame, whose sides are the stored ones swapped for codes 1, 3, 6 and 7.
+__global__ void frame_geometry_oriented_kernel(const FrameDesc* __restrict__ frames, const int* __restrict__ orient,
+                                               const int4* __restrict__ boxes, const int* __restrict__ stream_ids,
+                                               int n, int S, FrameGeom* __restrict__ geoms,
+                                               int* __restrict__ boxes_used) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int o = orient[i];
+  const bool swap = orient_swaps(o);
+  const int FH = swap ? frames[i].width : frames[i].height, FW = swap ? frames[i].height : frames[i].width;
+  int4 b = make_int4(0, 0, FW, FH);
+  if (boxes != nullptr) {
+    b = clip_box(boxes[stream_ids[i]], FH, FW);
+    boxes_used[4 * i + 0] = b.x; boxes_used[4 * i + 1] = b.y; boxes_used[4 * i + 2] = b.z; boxes_used[4 * i + 3] = b.w;
+  }
+  FrameGeom g = make_frame_geom(b.x, b.y, b.z, b.w, S);
+  g.orient = o;
+  geoms[i] = g;
+}
+
 // utils.img_scale_squarify (utils.py:107-120): resize so the longer side is S, centre on black.  out: u8 [n,S,S,3].
 // Src is the source format: BgrSrc, or Yuv420Src, which makes this cv2.cvtColor(YUV2BGR) followed by the squarify.
+// Output pixel (n, y, x) of squarify_tiled_kernel, element i = (n * S + y) * S + x of `out`: squarify_kernel's loop
+// body, restated because routing squarify_kernel through it changes that kernel's SASS.
+template <class Src>
+__device__ __forceinline__ void squarify_px(const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
+                                            const SquarifyParams& p, int n, int y, int x, int64_t i) {
+  int H = p.H, W = p.W, dh = p.dh, dw = p.dw, off_x = p.off_x, off_y = p.off_y, mode = p.mode;
+  double inv_scale = p.inv_scale;
+  Src src(in + (int64_t)n * p.frame_stride, p);
+  if (p.geoms != nullptr) {
+    const FrameGeom g = p.geoms[n];
+    H = g.h; W = g.w; dh = g.dh; dw = g.dw; off_x = g.off_x; off_y = g.off_y; mode = g.mode; inv_scale = g.inv_scale;
+    src.crop(g);
+  }
+  int v[3] = {0, 0, 0};
+  const int sy = y - off_y, sx = x - off_x;
+  if (sy >= 0 && sy < dh && sx >= 0 && sx < dw) {
+    if (mode == 0) {
+      cv_resize_u8_px(src, H, W, sy, sx, inv_scale, v);
+    } else {
+      // OpenCV resizeAreaFast (exact 2x): full 2x2 blocks are (sum + 2) >> 2; where an odd source side leaves a
+      // partial block (e.g. 736x735 -> dw = cvRound(367.5) = 368), only the in-range pixels are averaged:
+      // saturate_cast<uchar>((float)sum / count), i.e. float division then round-half-even.
+      const auto r0 = src.at(2 * sy, 2 * sx);
+      const bool col2 = 2 * sx + 1 < W, row2 = 2 * sy + 1 < H;
+      const auto r1 = src.below(r0, row2);
+      if (col2 && row2) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+          v[c] = (src.get(r0, 0, c) + src.get(r0, 1, c) + src.get(r1, 0, c) + src.get(r1, 1, c) + 2) >> 2;
+      } else {
+        const int count = (col2 ? 2 : 1) * (row2 ? 2 : 1);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          int sum = src.get(r0, 0, c);
+          if (col2) sum += src.get(r0, 1, c);
+          if (row2) sum += src.get(r1, 0, c);
+          v[c] = __float2int_rn(__fdiv_rn((float)sum, (float)count));
+        }
+      }
+    }
+  }
+  uint8_t* o = out + i * 3;
+  o[0] = (uint8_t)v[0];
+  o[1] = (uint8_t)v[1];
+  o[2] = (uint8_t)v[2];
+}
+
 template <class Src>
 __global__ void squarify_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, SquarifyParams p) {
   const int64_t total = (int64_t)p.n_frames * p.S * p.S;
@@ -218,7 +352,7 @@ __global__ void squarify_kernel(const uint8_t* __restrict__ in, uint8_t* __restr
     if (p.geoms != nullptr) {
       const FrameGeom g = p.geoms[n];
       H = g.h; W = g.w; dh = g.dh; dw = g.dw; off_x = g.off_x; off_y = g.off_y; mode = g.mode; inv_scale = g.inv_scale;
-      src.crop(g.x, g.y);
+      src.crop(g);
     }
     int v[3] = {0, 0, 0};
     const int sy = y - off_y, sx = x - off_x;
@@ -252,6 +386,23 @@ __global__ void squarify_kernel(const uint8_t* __restrict__ in, uint8_t* __restr
     o[0] = (uint8_t)v[0];
     o[1] = (uint8_t)v[1];
     o[2] = (uint8_t)v[2];
+  }
+}
+
+// squarify_kernel with each warp on an 8 x 4 (rows x columns) tile of output pixels instead of 32 consecutive pixels
+// of one row.  For the orientations that swap the sides, one oriented column is one stored row: a warp's taps then
+// fall on 4 stored rows, 8 adjacent pixels each, instead of 32 stored rows one pixel each.  S is a multiple of 16, so
+// the tiles cover the box exactly.
+template <class Src>
+__global__ void squarify_tiled_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, SquarifyParams p) {
+  const int tx = p.S / 4, per_frame = tx * (p.S / 8);
+  const int64_t tiles = (int64_t)p.n_frames * per_frame;
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x / 32);
+  for (int64_t t = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / 32; t < tiles; t += warps) {
+    const int n = (int)(t / per_frame), r = (int)(t - (int64_t)n * per_frame);
+    const int y = (r / tx) * 8 + (lane >> 2), x = (r % tx) * 4 + (lane & 3);
+    squarify_px<Src>(in, out, p, n, y, x, ((int64_t)n * p.S + y) * p.S + x);
   }
 }
 
@@ -1469,6 +1620,18 @@ __global__ void track_update_frames_kernel(const double* __restrict__ joints2d, 
                                            const FrameDesc* __restrict__ frames, int4* __restrict__ boxes) {
   const int f = blockIdx.x;
   track_box_update(joints2d, stream_ids, f, frames[f].height, frames[f].width, boxes);
+}
+
+// the same with oriented frames: the box is clamped to the oriented frame's sides (W_img, H_img of the frame the
+// joints are in)
+__global__ void track_update_frames_oriented_kernel(const double* __restrict__ joints2d,
+                                                    const int* __restrict__ stream_ids,
+                                                    const FrameDesc* __restrict__ frames,
+                                                    const int* __restrict__ orient, int4* __restrict__ boxes) {
+  const int f = blockIdx.x;
+  const bool swap = orient_swaps(orient[f]);
+  track_box_update(joints2d, stream_ids, f, swap ? frames[f].width : frames[f].height,
+                   swap ? frames[f].height : frames[f].width, boxes);
 }
 
 // vnect_track_set_boxes: up to kSeedBoxes seeded boxes travel in the kernel's parameters, so the caller's arrays are

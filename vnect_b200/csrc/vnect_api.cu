@@ -99,6 +99,10 @@ struct vnect_handle {
     // indices) after the frame table, copied with it
     size_t seg_off = 0;
     int *h_seg = nullptr, *d_seg = nullptr;
+    // calls with oriented frames: each frame's VNECT_ORIENT_* code ([max_frames]) after the segment table, copied with
+    // the rest (a call takes its streams' codes at submission)
+    size_t orient_off = 0;
+    int *h_orient = nullptr, *d_orient = nullptr;
     unsigned int* h_nonfinite = nullptr;  // pinned + device-visible: set by the post-process when a batch of this lane met NaN / Inf maps
     cudaEvent_t copy_done = nullptr, done = nullptr;
     bool pending = false;
@@ -114,6 +118,7 @@ struct vnect_handle {
   int4* d_boxes = nullptr;         // [max_streams] (x, y, w, h)
   FrameGeom* d_geoms = nullptr;    // [max_frames]
   int* d_boxes_used = nullptr;     // [max_frames][4]
+  std::vector<int32_t> orient;     // [max_streams] VNECT_ORIENT_* per stream (vnect_set_orientations), host only
   // CUDA graphs of the kernel sequence of one estimate call, keyed by everything baked into the kernel parameters.
   // First use of a key runs directly (warm-up), the second captures, later ones replay: ~50 launches -> 1.
   // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset).
@@ -613,7 +618,8 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.meta_bytes = off_t3 + (size_t)mf * sizeof(double);
       L.table_off = (L.meta_bytes + 15) & ~size_t(15);
       L.seg_off = L.table_off + (size_t)mf * sizeof(FrameDesc);
-      const size_t block = L.seg_off + (size_t)(2 * mf + 2) * sizeof(int);
+      L.orient_off = L.seg_off + (size_t)(2 * mf + 2) * sizeof(int);
+      const size_t block = L.orient_off + (size_t)mf * sizeof(int);
       uint8_t* d_meta = nullptr;
       if ((rc = dev_alloc(h, &d_meta, block))) return rc;
       L.d_stream_ids = reinterpret_cast<int*>(d_meta);
@@ -621,6 +627,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.d_t3d = reinterpret_cast<double*>(d_meta + off_t3);
       L.d_table = reinterpret_cast<FrameDesc*>(d_meta + L.table_off);
       L.d_seg = reinterpret_cast<int*>(d_meta + L.seg_off);
+      L.d_orient = reinterpret_cast<int*>(d_meta + L.orient_off);
       CU(h, cudaMallocHost(&L.h_meta, block));
       memset(L.h_meta, 0, block);
       L.h_stream_ids = reinterpret_cast<int*>(L.h_meta);
@@ -628,6 +635,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.h_t3d = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + off_t3);
       L.h_table = reinterpret_cast<FrameDesc*>(static_cast<uint8_t*>(L.h_meta) + L.table_off);
       L.h_seg = reinterpret_cast<int*>(static_cast<uint8_t*>(L.h_meta) + L.seg_off);
+      L.h_orient = reinterpret_cast<int*>(static_cast<uint8_t*>(L.h_meta) + L.orient_off);
     }
     if ((rc = dev_alloc(h, &L.d_geoms, mf))) return rc;
     if ((rc = dev_alloc(h, &L.d_out2d, (size_t)mf * kJoints * 2))) return rc;
@@ -660,6 +668,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
   if ((rc = dev_alloc(h, &h->d_boxes, ms))) return rc;
   if ((rc = dev_alloc(h, &h->d_geoms, mf))) return rc;
   if ((rc = dev_alloc(h, &h->d_boxes_used, (size_t)mf * 4))) return rc;
+  h->orient.assign(ms, VNECT_ORIENT_IDENTITY);
   h->last_t2d.assign(ms, NAN);
   h->last_t3d.assign(ms, NAN);
   PyramidParams& py = h->pyr;
@@ -985,15 +994,20 @@ static int ensure_surround(vnect_t* h) {
 }
 
 static int run_preprocess(vnect_t* h, const uint8_t* dev_frames, int n_frames, int H, int W, const FrameSource& src,
-                          const Geometry& g, bool tracked = false) {
+                          const Geometry& g, bool tracked = false, bool oriented = false) {
   const int S = h->S;
   int rc0 = ensure_surround(h);
   if (rc0) return rc0;
   if (src.table) {  // per-frame geometry from each frame's own size, then squarify through the lane's table
     vnect_handle::Lane* L = h->cur;
-    frame_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(L->d_table, tracked ? h->d_boxes : nullptr,
-                                                                      L->d_stream_ids, n_frames, S, L->d_geoms,
-                                                                      h->d_boxes_used);
+    if (oriented)
+      frame_geometry_oriented_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(
+          L->d_table, L->d_orient, tracked ? h->d_boxes : nullptr, L->d_stream_ids, n_frames, S, L->d_geoms,
+          h->d_boxes_used);
+    else
+      frame_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(L->d_table, tracked ? h->d_boxes : nullptr,
+                                                                        L->d_stream_ids, n_frames, S, L->d_geoms,
+                                                                        h->d_boxes_used);
     CU(h, cudaGetLastError());
     ++h->launches;
     SquarifyParams sp{};  // nothing size- or address-dependent: one captured graph serves every composition
@@ -1003,10 +1017,15 @@ static int run_preprocess(vnect_t* h, const uint8_t* dev_frames, int n_frames, i
     sp.uv_step = src.format == VNECT_FMT_NV12 ? 2 : 1;
     const int64_t total = (int64_t)n_frames * S * S;
     const uint8_t* table = reinterpret_cast<const uint8_t*>(L->d_table);
-    if (src.format == kFmtBGR)
-      squarify_kernel<FrameTableSrc<BgrSrc>><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(table, h->d_sq, sp);
+    const int grid = grid_for(total, 256, h->num_sms);
+    if (oriented && src.format == kFmtBGR)
+      squarify_tiled_kernel<FrameTableSrc<Oriented<BgrSrc>>><<<grid, 256, 0, h->stream>>>(table, h->d_sq, sp);
+    else if (oriented)
+      squarify_tiled_kernel<FrameTableSrc<Oriented<Yuv420Src>>><<<grid, 256, 0, h->stream>>>(table, h->d_sq, sp);
+    else if (src.format == kFmtBGR)
+      squarify_kernel<FrameTableSrc<BgrSrc>><<<grid, 256, 0, h->stream>>>(table, h->d_sq, sp);
     else
-      squarify_kernel<FrameTableSrc<Yuv420Src>><<<grid_for(total, 256, h->num_sms), 256, 0, h->stream>>>(table, h->d_sq, sp);
+      squarify_kernel<FrameTableSrc<Yuv420Src>><<<grid, 256, 0, h->stream>>>(table, h->d_sq, sp);
     CU(h, cudaGetLastError());
     ++h->launches;
     return launch_pyramid(h, h->d_sq, (int64_t)S * 3, (int64_t)S * S * 3, n_frames, false);
@@ -1063,9 +1082,11 @@ static int lane_acquire(vnect_t* h, int lane) {
 // it meets NaN / Inf maps, so no device -> host copy of a counter sits in the stream after every batch.
 static int snapshot_nonfinite(vnect_t*) { return VNECT_OK; }
 
-// table_frames > 0: the lane's frame table (already written to its pinned block) travels in the same copy
+// table_frames > 0: the lane's frame table (already written to its pinned block) travels in the same copy.
+// oriented: so do the frames' orientation codes, taken from their streams now (a call with oriented frames always
+// carries its table)
 static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                            cudaStream_t copy_on, int table_frames = 0) {
+                            cudaStream_t copy_on, int table_frames = 0, bool oriented = false) {
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   h->seen_stamp.resize(h->cfg.max_streams, 0);
   const unsigned int stamp = ++h->seen_epoch;
@@ -1095,12 +1116,15 @@ static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids,
     h->cur->h_stream_ids[i] = sid;
     h->cur->h_t2d[i] = t2d ? t2d[i] : 0.0;
     h->cur->h_t3d[i] = t3d ? t3d[i] : 0.0;
+    if (oriented) h->cur->h_orient[i] = h->orient[sid];
     if (h->cfg.filters) {
       h->last_t2d[sid] = t2d[i];
       h->last_t3d[sid] = t3d[i];
     }
   }
-  const size_t bytes = table_frames > 0 ? h->cur->table_off + (size_t)table_frames * sizeof(FrameDesc) : h->cur->meta_bytes;
+  const size_t bytes = oriented ? h->cur->orient_off + (size_t)n_frames * sizeof(int)
+                       : table_frames > 0 ? h->cur->table_off + (size_t)table_frames * sizeof(FrameDesc)
+                                          : h->cur->meta_bytes;
   CU(h, cudaMemcpyAsync(h->cur->d_stream_ids, h->cur->h_meta, bytes, cudaMemcpyHostToDevice, copy_on));
   return VNECT_OK;
 }
@@ -1111,7 +1135,7 @@ static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids,
 // anything recorded.  The segment table of sequence_filter_kernel goes to the lane's pinned block after the frame
 // table, and ids, timestamps, table and segments travel in one copy.
 static int stage_sequence_meta(vnect_t* h, int n_frames, const int32_t* stream_ids, const double* t2d,
-                               const double* t3d, cudaStream_t copy_on) {
+                               const double* t3d, cudaStream_t copy_on, bool oriented = false) {
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   if (!stream_ids) return fail(h, VNECT_E_INVALID, "a sequence call needs stream ids");
   if (h->cfg.filters && (!t2d || !t3d)) return fail(h, VNECT_E_INVALID, "timestamps required when filters are on");
@@ -1168,12 +1192,14 @@ static int stage_sequence_meta(vnect_t* h, int n_frames, const int32_t* stream_i
     L->h_stream_ids[i] = sid;
     L->h_t2d[i] = t2d ? t2d[i] : 0.0;
     L->h_t3d[i] = t3d ? t3d[i] : 0.0;
+    if (oriented) L->h_orient[i] = h->orient[sid];
     if (h->cfg.filters) {
       h->last_t2d[sid] = h->seq_t2d[sid];
       h->last_t3d[sid] = h->seq_t3d[sid];
     }
   }
-  const size_t bytes = L->seg_off + (size_t)(2 + n_seg + n_frames) * sizeof(int);
+  const size_t bytes = oriented ? L->orient_off + (size_t)n_frames * sizeof(int)
+                                : L->seg_off + (size_t)(2 + n_seg + n_frames) * sizeof(int);
   CU(h, cudaMemcpyAsync(L->d_stream_ids, L->h_meta, bytes, cudaMemcpyHostToDevice, copy_on));
   return VNECT_OK;
 }
@@ -1353,29 +1379,35 @@ static int run_graphed(vnect_t* h, const vnect_handle::GraphKey& key, F direct) 
 extern "C" {
 
 // pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
+// oriented (table calls only): the lane carries its frames' orientation codes
 static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
                         const FrameSource& src, double* out2d, float* out3d, bool tracked = false,
-                        bool sequence = false) {
+                        bool sequence = false, bool oriented = false) {
   if (src.table) {  // sizes, addresses and geometry live in the lane's device tables, not in kernel parameters
     if (int rc = ensure_surround(h)) return rc;
     auto direct = [&]() -> int {
       int rc;
-      if ((rc = run_preprocess(h, nullptr, n_frames, 0, 0, src, Geometry{}, tracked))) return rc;
+      if ((rc = run_preprocess(h, nullptr, n_frames, 0, 0, src, Geometry{}, tracked, oriented))) return rc;
       if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
       if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, out2d, out3d, h->cur->d_geoms, true,
                                 sequence ? h->cur->d_seg : nullptr)))
         return rc;
       if (tracked) {
-        track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table, h->d_boxes);
+        if (oriented)
+          track_update_frames_oriented_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table,
+                                                                              h->cur->d_orient, h->d_boxes);
+        else
+          track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table, h->d_boxes);
         CU(h, cudaGetLastError());
         ++h->launches;
       }
       return VNECT_OK;
     };
     if (!h->use_graphs) return direct();
-    // sequence calls (8 + lane) read their segment table from the lane's device block as well
-    const vnect_handle::GraphKey key(sequence ? 8 + lane : 4 + lane + (tracked ? 2 : 0), n_frames, 0, 0, 0, 0, nullptr,
-                                     out2d, out3d, src.format, 0, 0, 0);
+    // sequence calls (8 + lane) read their segment table from the lane's device block as well; so do calls with
+    // oriented frames their codes (the third field), so every composition of orientations replays one graph
+    const vnect_handle::GraphKey key(sequence ? 8 + lane : 4 + lane + (tracked ? 2 : 0), n_frames, oriented ? 1 : 0, 0,
+                                     0, 0, nullptr, out2d, out3d, src.format, 0, 0, 0);
     return run_graphed(h, key, direct);
   }
   const Geometry g = squarify_geometry(h->S, H, W, src.format);
@@ -1445,19 +1477,22 @@ static int stage_frame(vnect_t* h, uint8_t* dst, const uint8_t* f, int H, int W,
 
 // host frames described by `src` -> the current lane's d_frames, tightly packed (BGR: 3 bytes per pixel, YUV: cv2's
 // contiguous layout, 1.5), on the copy stream; `packed` describes them there
+// how stage_frames packs H x W frames of `format` on the device
+static FrameSource packed_source(int format, int H, int W) {
+  return format == kFmtBGR ? bgr_source((int64_t)W * 3, (int64_t)W * 3 * H) : yuv_source(packed_yuv_layout(format, H, W));
+}
+
 static int stage_frames(vnect_t* h, const uint8_t* frames, int n_frames, int H, int W, const FrameSource& src,
                         FrameSource* packed) {
   uint8_t* d = h->cur->d_frames;
+  *packed = packed_source(src.format, H, W);
   if (src.format == kFmtBGR) {
-    const int64_t dpitch = (int64_t)W * 3, dstride = dpitch * H;
-    *packed = bgr_source(dpitch, dstride);
-    if (src.pitch == dpitch && src.frame_stride == dstride) {
-      CU(h, cudaMemcpyAsync(d, frames, (size_t)dstride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
+    if (src.pitch == packed->pitch && src.frame_stride == packed->frame_stride) {
+      CU(h, cudaMemcpyAsync(d, frames, (size_t)packed->frame_stride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
       return VNECT_OK;
     }
   } else {
     const vnect_yuv_layout l = packed_yuv_layout(src.format, H, W);
-    *packed = yuv_source(l);
     if (src.pitch == l.y_pitch && src.uv_pitch == l.uv_pitch && src.u_offset == l.u_offset && src.v_offset == l.v_offset &&
         (n_frames == 1 || src.frame_stride == l.frame_stride)) {
       CU(h, cudaMemcpyAsync(d, frames, (size_t)l.frame_stride * n_frames, cudaMemcpyHostToDevice, h->copy_stream));
@@ -1470,6 +1505,32 @@ static int stage_frames(vnect_t* h, const uint8_t* frames, int n_frames, int H, 
   return VNECT_OK;
 }
 
+// Whether a call's frames need the oriented path: some frame's stream has a non-identity orientation.  Ids that
+// stage_frame_meta refuses are skipped here, and so is a frame count it refuses.
+static bool any_oriented(vnect_t* h, int n_frames, const int32_t* stream_ids) {
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return false;
+  for (int i = 0; i < n_frames; ++i) {
+    const int sid = stream_ids ? stream_ids[i] : i;
+    if (sid >= 0 && sid < h->cfg.max_streams && h->orient[sid] != VNECT_ORIENT_IDENTITY) return true;
+  }
+  return false;
+}
+
+// The current lane's frame table for n_frames uniform frames at `frames` (device), laid out as `src` describes:
+// a uniform call with oriented frames runs the table pipeline on it.
+static void uniform_table(vnect_t* h, const uint8_t* frames, int n_frames, int H, int W, const FrameSource& src) {
+  for (int i = 0; i < n_frames; ++i) {
+    FrameDesc& t = h->cur->h_table[i];
+    t.data = frames + (size_t)i * src.frame_stride;
+    t.height = H;
+    t.width = W;
+    t.pitch = src.pitch;
+    t.uv_pitch = src.uv_pitch;
+    t.u_offset = src.u_offset;
+    t.v_offset = src.v_offset;
+  }
+}
+
 // vnect_estimate_device / vnect_estimate_device_yuv once the frame description is validated
 static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
                            const FrameSource& src, const int32_t* stream_ids, const double* t2d, const double* t3d,
@@ -1477,12 +1538,16 @@ static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_fram
   // alternate lanes for the per-call meta so the host can run one call ahead of the GPU
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
+  const bool oriented = any_oriented(h, n_frames, stream_ids);
+  if (oriented) uniform_table(h, dev_frames, n_frames, H, W, src);
   // the per-call meta travels on the copy stream, under the previous call's kernels
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, 0, oriented))) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
-  if ((rc = run_pipeline(h, lane, dev_frames, n_frames, H, W, src, dev_joints2d, dev_joints3d))) return rc;
+  if ((rc = run_pipeline(h, lane, dev_frames, n_frames, H, W, oriented ? table_source(src.format) : src, dev_joints2d,
+                         dev_joints3d, false, false, oriented)))
+    return rc;
   if ((rc = snapshot_nonfinite(h))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
@@ -1495,13 +1560,17 @@ static int submit(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_fra
                   double* joints2d, float* joints3d) {
   int rc = lane_acquire(h, lane);
   if (rc) return rc;
+  const bool oriented = any_oriented(h, n_frames, stream_ids);
+  if (oriented) uniform_table(h, h->cur->d_frames, n_frames, H, W, packed_source(src.format, H, W));
   // host -> device on the copy stream (tightly packed on the device), overlapping the previous lane's kernels
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, 0, oriented))) return rc;
   FrameSource packed;
   if ((rc = stage_frames(h, frames, n_frames, H, W, src, &packed))) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, lane, h->cur->d_frames, n_frames, H, W, packed, h->cur->d_out2d, h->cur->d_out3d))) return rc;
+  if ((rc = run_pipeline(h, lane, h->cur->d_frames, n_frames, H, W, oriented ? table_source(src.format) : packed,
+                         h->cur->d_out2d, h->cur->d_out3d, false, false, oriented)))
+    return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if ((rc = snapshot_nonfinite(h))) return rc;
@@ -1516,12 +1585,16 @@ static int track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH
                  int32_t* boxes_used) {
   int rc = lane_acquire(h, 0);
   if (rc) return rc;
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream))) return rc;
+  const bool oriented = any_oriented(h, n_frames, stream_ids);
+  if (oriented) uniform_table(h, h->cur->d_frames, n_frames, FH, FW, packed_source(src.format, FH, FW));
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, 0, oriented))) return rc;
   FrameSource packed;
   if ((rc = stage_frames(h, frames, n_frames, FH, FW, src, &packed))) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW, packed, h->cur->d_out2d, h->cur->d_out3d, true))) return rc;
+  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW, oriented ? table_source(src.format) : packed,
+                         h->cur->d_out2d, h->cur->d_out3d, true, false, oriented)))
+    return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (boxes_used)
@@ -1616,9 +1689,11 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
       d += (size_t)l.frame_stride;
     }
   }
-  // ids, timestamps and the table in one copy; a refused id or timestamp returns before any frame copy is queued
-  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream)
-                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames);
+  // ids, timestamps, the table and any orientation codes in one copy; a refused id or timestamp returns before any
+  // frame copy is queued
+  const bool oriented = any_oriented(h, n_frames, stream_ids);
+  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, oriented)
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented);
   if (rc) return rc;
   for (int i = 0; i < n_frames; ++i)
     if ((rc = stage_frame(h, const_cast<uint8_t*>(h->cur->h_table[i].data), frames[i].data, frames[i].height,
@@ -1627,7 +1702,7 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), h->cur->d_out2d, h->cur->d_out3d, tracked,
-                         sequence)))
+                         sequence, oriented)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
@@ -1646,14 +1721,15 @@ static int device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
   memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));
-  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream)
-                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames);
+  const bool oriented = any_oriented(h, n_frames, stream_ids);
+  rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, oriented)
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented);
   if (rc) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
   if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d, tracked,
-                         sequence)))
+                         sequence, oriented)))
     return rc;
   if (dev_boxes_used)  // outside the graph, so the caller's pointer stays out of its key
     CU(h, cudaMemcpyAsync(dev_boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToDevice,
@@ -1854,6 +1930,32 @@ int vnect_track_get_box(vnect_t* h, int32_t stream_id, int32_t* xywh) {
   int4 b;
   CU(h, cudaMemcpy(&b, h->d_boxes + stream_id, sizeof b, cudaMemcpyDeviceToHost));
   xywh[0] = b.x; xywh[1] = b.y; xywh[2] = b.z; xywh[3] = b.w;
+  return VNECT_OK;
+}
+
+int vnect_set_orientations(vnect_t* h, int32_t n, const int32_t* stream_ids, const int32_t* codes) {
+  if (!h || h->orient.empty()) return fail(h, VNECT_E_INVALID, "handle not created");
+  if (n < 0) return fail(h, VNECT_E_INVALID, "n %d below 0", n);
+  if (n == 0) return VNECT_OK;
+  if (!stream_ids || !codes) return fail(h, VNECT_E_INVALID, "null buffer");
+  h->seen_stamp.resize(h->cfg.max_streams, 0);
+  const unsigned int stamp = ++h->seen_epoch;
+  for (int i = 0; i < n; ++i) {  // everything is checked before the first change
+    const int sid = stream_ids[i];
+    if (sid < 0 || sid >= h->cfg.max_streams) return fail(h, VNECT_E_INVALID, "stream id %d not in [0, %d)", sid, h->cfg.max_streams);
+    if (h->seen_stamp[sid] == stamp) return fail(h, VNECT_E_INVALID, "stream id %d appears twice", sid);
+    h->seen_stamp[sid] = stamp;
+    if (codes[i] < VNECT_ORIENT_IDENTITY || codes[i] > VNECT_ORIENT_TRANSVERSE)
+      return fail(h, VNECT_E_INVALID, "orientation %d of stream %d not in [0, 8)", codes[i], sid);
+  }
+  for (int i = 0; i < n; ++i) h->orient[stream_ids[i]] = codes[i];
+  return VNECT_OK;
+}
+
+int vnect_get_orientation(vnect_t* h, int32_t stream_id, int32_t* code) {
+  if (!h || h->orient.empty() || !code) return fail(h, VNECT_E_INVALID, "handle not created / null buffer");
+  if (stream_id < 0 || stream_id >= h->cfg.max_streams) return fail(h, VNECT_E_INVALID, "stream id out of range");
+  *code = h->orient[stream_id];
   return VNECT_OK;
 }
 

@@ -46,6 +46,13 @@ def yuv_layout(pixel_format, h, w, y_pitch=None, uv_pitch=None, u_offset=None, v
 
 _FORMATS = {"bgr": _capi.FMT_BGR, **_YUV_FORMATS}
 
+# VNECT_ORIENT_* (include/vnect_b200.h): how a stream's camera is mounted.  The name gives the numpy form of the
+# oriented frame the engine sees for a stored frame f: rot90_cw = np.rot90(f, 3) (cv2.ROTATE_90_CLOCKWISE),
+# rot180 = np.rot90(f, 2), rot90_ccw = np.rot90(f, 1), flip_h = f[:, ::-1] (a mirror), flip_v = f[::-1],
+# transpose = f.transpose(1, 0, 2), transverse = np.rot90(f, 2).transpose(1, 0, 2).
+ORIENTATIONS = {"identity": 0, "rot90_cw": 1, "rot180": 2, "rot90_ccw": 3, "flip_h": 4, "flip_v": 5, "transpose": 6,
+                "transverse": 7}
+
 
 def _format_code(pixel_format):
     if pixel_format not in _FORMATS:
@@ -500,6 +507,27 @@ class VNectEngine:
         if rects.shape != (len(ids), 4):
             raise ValueError(f"expected one (x, y, w, h) per stream id: {len(ids)} ids, rects {rects.shape}")
         self._check(self._lib.vnect_track_set_boxes(self._h, len(ids), _ptr(ids), _ptr(rects)))
+
+    def set_orientations(self, stream_ids, orientations):
+        """Set how each stream's camera is mounted: a code or a name of ``ORIENTATIONS`` per stream id.  Every later
+        call, on either lane, reads that stream's frames as stored and sees them oriented; joints, boxes and
+        ``boxes_used`` are in the oriented frame.  Calls already submitted keep their orientation; reset() keeps it
+        and export_stream_state() does not carry it."""
+        ids = np.ascontiguousarray(stream_ids, dtype=np.int32).reshape(-1)
+        codes = [ORIENTATIONS[o] if isinstance(o, str) and o in ORIENTATIONS else o
+                 for o in np.asarray(orientations, dtype=object).reshape(-1)]
+        if any(isinstance(o, str) for o in codes):
+            raise ValueError(f"unknown orientation name in {orientations!r}: expected one of {list(ORIENTATIONS)}")
+        codes = np.ascontiguousarray(codes, dtype=np.int32)
+        if codes.shape != ids.shape:
+            raise ValueError(f"expected one orientation per stream id: {len(ids)} ids, {len(codes)} orientations")
+        self._check(self._lib.vnect_set_orientations(self._h, len(ids), _ptr(ids), _ptr(codes)))
+
+    def orientation(self, stream_id):
+        """The orientation code of a stream (see ``ORIENTATIONS``)."""
+        out = C.c_int32()
+        self._check(self._lib.vnect_get_orientation(self._h, int(stream_id), C.byref(out)))
+        return out.value
 
     def estimate_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
                                pixel_format="bgr"):
