@@ -241,6 +241,36 @@ int vnect_set_orientations(vnect_t* h, int32_t n, const int32_t* stream_ids, con
 /* the orientation of one stream */
 int vnect_get_orientation(vnect_t* h, int32_t stream_id, int32_t* code);
 
+/* Joint confidence.  score[f][j] of frame f and joint j is the float64 value the reference takes its argmax of in
+ * utils.extract_2d_joints (src/utils.py:153-175): up = cv2.resize(hm_avg[:, :, j], (0, 0), fx=8, fy=8, INTER_LINEAR)
+ * on the multi-scale float64 average hm_avg of src/estimator.py:105-129, score = up.flat[np.argmax(up)] == up.max().
+ * Bit for bit the reference's value, unfiltered, in heat-map units; it depends only on the CNN maps, not on filters,
+ * orientation, tracking or the order of a sequence.  A confidence, not a probability.
+ * The NEXT call of vnect_estimate, vnect_submit(_yuv), vnect_estimate_device(_yuv), vnect_track(_yuv),
+ * vnect_submit_frames, vnect_estimate_device_frames, vnect_track_frames, vnect_submit_track_frames,
+ * vnect_track_device_frames, vnect_submit_sequence, vnect_estimate_device_sequence, vnect_postprocess,
+ * vnect_postprocess_sequence or vnect_track_postprocess also writes float64 [n_frames][21] scores to `scores`: a HOST
+ * pointer, filled when the call completes (vnect_wait for the submit calls), except for the *_device* calls, where it
+ * is a DEVICE pointer written in stream order.  That call consumes the request whether it is accepted or refused; a
+ * refused call writes nothing.  NULL cancels a pending request.  Each call carries its own buffer, so two lanes in
+ * flight never share one, and a rotating pool of buffers replays the same CUDA graphs.  A call with no pending request
+ * (and no recovering stream, below) runs exactly as before: same launches, graphs and kernels. */
+int vnect_request_scores(vnect_t* h, double* scores);
+/* Lost-person recovery of tracked streams.  Sets the least mean score min_mean_score[i] (HOST arrays, copied; n = 0
+ * does nothing) of n streams; 0 = off, the default and the reference's behaviour.  When a tracked call processes
+ * frame f of a stream whose threshold tau > 0, it computes m = (((s0 + s1) + s2) + ... + s20) / 21 over the frame's
+ * scores in float64 without FMA (Python's sum(scores[f]) / 21).  If m < tau, the box left behind is the one
+ * vnect_reset_stream leaves, (0, 0, 1 << 30, 1 << 30), so the stream's next frame is cropped to its whole (oriented)
+ * frame; otherwise the box update of run_estimator.py:110-119 runs unchanged.  Frame f's joints, filters and
+ * timestamps are untouched.  Configuration like the orientation: host-only, a call reads its streams' thresholds at
+ * submission, vnect_reset_stream keeps them and the stream-state export / import does not carry them.  A tracked call
+ * with a recovering stream runs the table pipeline (uniform calls build their frame table on the host).
+ * Refused with VNECT_E_INVALID, changing nothing: n below 0, a null array, an id outside [0, max_streams), an id
+ * given twice, a threshold that is negative, NaN or infinite. */
+int vnect_set_track_recovery(vnect_t* h, int32_t n, const int32_t* stream_ids, const double* min_mean_score);
+/* the recovery threshold of one stream (0 = off) */
+int vnect_get_track_recovery(vnect_t* h, int32_t stream_id, double* min_mean_score);
+
 /* Sequence calls: consecutive frames of one stream in one batch (offline video: annotating a dataset, re-processing a
  * recording, motion capture from footage).  Up to max_frames frames in which a stream id may appear more than once;
  * the frames of one stream are consecutive in time in the order they appear in the call, and may be interleaved with

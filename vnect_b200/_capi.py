@@ -84,6 +84,9 @@ SIGNATURES = {
     "vnect_track_set_boxes": (C.c_int, [_P, C.c_int32, _P, _P]),
     "vnect_set_orientations": (C.c_int, [_P, C.c_int32, _P, _P]),
     "vnect_get_orientation": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
+    "vnect_request_scores": (C.c_int, [_P, _P]),
+    "vnect_set_track_recovery": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "vnect_get_track_recovery": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_double)]),
     "vnect_submit_sequence": (C.c_int, [_P, C.c_int32, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "vnect_estimate_device_sequence": (C.c_int, [_P, _FR, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "vnect_postprocess_sequence": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_double, C.c_int32,

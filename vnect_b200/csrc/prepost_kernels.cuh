@@ -691,6 +691,8 @@ struct PostParams {
   FilterState* st3d;              // [max_streams][21][3]
   FilterCfg cfg2d, cfg3d;
   int filters_on;
+  int scores_off;                 // SCORES: the [n_frames][21] float64 scores start this many ints after raw_argmax (in
+                                  // the padding before `scaler`, so the parameter block is that of the other kernels)
   double scaler;                  // box px per input px (S / max(H, W))
   int off_x, off_y;
   const FrameGeom* geoms;         // optional per-frame geometry (tracked streams): scaler, offsets and the crop origin
@@ -965,7 +967,9 @@ __device__ __forceinline__ double rescale_joint(const PostParams& p, int frame, 
 #define POST_TRACE(i) do { if (p.trace != nullptr && threadIdx.x == 0) p.trace[(size_t)blockIdx.x * 16 + (i)] = globaltimer_ns(); } while (0)
 // RAW_ONLY: steps A-D only, ending with raw_argmax (the argmax launch of a sequence call, sequence_filter_kernel does
 // the rest); no filter state, scratch or frame counter is touched.
-template <int NS, int MASK, bool RAW_ONLY = false>  // MASK >= 0: the identity mask (PostParams::identity_mask) is this compile-time constant
+// SCORES: step D's best value -- the reference's upsampled float64 heat-map at the raw argmax, i.e. the joint's
+// confidence -- goes to p.scores as well.
+template <int NS, int MASK, bool RAW_ONLY = false, bool SCORES = false>  // MASK >= 0: the identity mask (PostParams::identity_mask) is this compile-time constant
 __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const __grid_constant__ PostParams p) {
   extern __shared__ float4 s_dyn4[];
   float* s_dyn = reinterpret_cast<float*>(s_dyn4);
@@ -1384,6 +1388,7 @@ __global__ void __launch_bounds__(kPostMaxThreads, 2) postprocess_kernel(const _
     }
     const int row = best_idx / S, col = best_idx - row * S;
     double coord = (tid == 0) ? (double)row : (double)col;
+    if (SCORES && tid == 0) reinterpret_cast<double*>(p.raw_argmax + p.scores_off)[frame * kJoints + joint] = best;
     if (tid < 2) {
       p.raw_argmax[(frame * kJoints + joint) * 2 + tid] = (tid == 0) ? row : col;
       if (!RAW_ONLY && p.filters_on) {
@@ -1630,6 +1635,33 @@ __global__ void track_update_frames_oriented_kernel(const double* __restrict__ j
                                                     const int* __restrict__ orient, int4* __restrict__ boxes) {
   const int f = blockIdx.x;
   const bool swap = orient_swaps(orient[f]);
+  track_box_update(joints2d, stream_ids, f, swap ? frames[f].width : frames[f].height,
+                   swap ? frames[f].height : frames[f].width, boxes);
+}
+
+// The box update of a call in which some stream recovers lost people (vnect_set_track_recovery), with or without
+// oriented frames (orient == nullptr: all identity).  Frame f's mean score m = (((s0 + s1) + s2) + ... + s20) / 21, in
+// float64 without FMA (Python's sum(scores) / 21), against the stream's threshold min_mean[f] taken at submission:
+// below a positive threshold the stream's next crop is its whole frame, the box vnect_reset_stream leaves; otherwise
+// the reference's box update runs unchanged.
+__global__ void track_update_frames_recover_kernel(const double* __restrict__ joints2d,
+                                                   const int* __restrict__ stream_ids,
+                                                   const FrameDesc* __restrict__ frames,
+                                                   const int* __restrict__ orient, const double* __restrict__ scores,
+                                                   const double* __restrict__ min_mean, int4* __restrict__ boxes) {
+  const int f = blockIdx.x;
+  int lost = 0;
+  if (threadIdx.x == 0) {
+    const double tau = min_mean[f];
+    double acc = 0.0;
+    for (int j = 0; j < kJoints; ++j) acc = __dadd_rn(acc, scores[f * kJoints + j]);
+    lost = tau > 0.0 && __ddiv_rn(acc, (double)kJoints) < tau;
+  }
+  if (__shfl_sync(0xffffffffu, lost, 0)) {
+    if (threadIdx.x == 0) boxes[stream_ids[f]] = make_int4(0, 0, 1 << 30, 1 << 30);
+    return;
+  }
+  const bool swap = orient != nullptr && orient_swaps(orient[f]);
   track_box_update(joints2d, stream_ids, f, swap ? frames[f].width : frames[f].height,
                    swap ? frames[f].height : frames[f].width, boxes);
 }

@@ -74,6 +74,7 @@ struct vnect_handle {
   double* d_j2_box = nullptr;
   float* d_j3_raw = nullptr;
   int* d_raw_argmax = nullptr;
+  double* d_scores = nullptr;  // [max_frames][21] after d_raw_argmax's [max_frames][21][2] (PostParams::scores_off)
   unsigned int* d_counter = nullptr;
   double* d_prep3 = nullptr;   // [max_frames][21][3][3]: see PostParams::prep3
   double* d_filter_scratch = nullptr;
@@ -103,6 +104,10 @@ struct vnect_handle {
     // the rest (a call takes its streams' codes at submission)
     size_t orient_off = 0;
     int *h_orient = nullptr, *d_orient = nullptr;
+    // tracked calls with a recovering stream: each frame's threshold ([max_frames], vnect_set_track_recovery) after the
+    // orientation codes, copied with the rest (a call takes its streams' thresholds at submission)
+    size_t recover_off = 0;
+    double *h_recover = nullptr, *d_recover = nullptr;
     unsigned int* h_nonfinite = nullptr;  // pinned + device-visible: set by the post-process when a batch of this lane met NaN / Inf maps
     cudaEvent_t copy_done = nullptr, done = nullptr;
     bool pending = false;
@@ -119,6 +124,8 @@ struct vnect_handle {
   FrameGeom* d_geoms = nullptr;    // [max_frames]
   int* d_boxes_used = nullptr;     // [max_frames][4]
   std::vector<int32_t> orient;     // [max_streams] VNECT_ORIENT_* per stream (vnect_set_orientations), host only
+  std::vector<double> recover;     // [max_streams] least mean score of a tracked frame (vnect_set_track_recovery), 0 = off
+  double* score_req = nullptr;     // vnect_request_scores: where the next result-producing call writes its scores
   // CUDA graphs of the kernel sequence of one estimate call, keyed by everything baked into the kernel parameters.
   // First use of a key runs directly (warm-up), the second captures, later ones replay: ~50 launches -> 1.
   // (lane + tracked, n_frames, H, W, pitch, frame_stride, frames, out2d, out3d, format, uv_pitch, u_offset, v_offset).
@@ -619,7 +626,8 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.table_off = (L.meta_bytes + 15) & ~size_t(15);
       L.seg_off = L.table_off + (size_t)mf * sizeof(FrameDesc);
       L.orient_off = L.seg_off + (size_t)(2 * mf + 2) * sizeof(int);
-      const size_t block = L.orient_off + (size_t)mf * sizeof(int);
+      L.recover_off = (L.orient_off + (size_t)mf * sizeof(int) + 7) & ~size_t(7);
+      const size_t block = L.recover_off + (size_t)mf * sizeof(double);
       uint8_t* d_meta = nullptr;
       if ((rc = dev_alloc(h, &d_meta, block))) return rc;
       L.d_stream_ids = reinterpret_cast<int*>(d_meta);
@@ -628,6 +636,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.d_table = reinterpret_cast<FrameDesc*>(d_meta + L.table_off);
       L.d_seg = reinterpret_cast<int*>(d_meta + L.seg_off);
       L.d_orient = reinterpret_cast<int*>(d_meta + L.orient_off);
+      L.d_recover = reinterpret_cast<double*>(d_meta + L.recover_off);
       CU(h, cudaMallocHost(&L.h_meta, block));
       memset(L.h_meta, 0, block);
       L.h_stream_ids = reinterpret_cast<int*>(L.h_meta);
@@ -636,6 +645,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
       L.h_table = reinterpret_cast<FrameDesc*>(static_cast<uint8_t*>(L.h_meta) + L.table_off);
       L.h_seg = reinterpret_cast<int*>(static_cast<uint8_t*>(L.h_meta) + L.seg_off);
       L.h_orient = reinterpret_cast<int*>(static_cast<uint8_t*>(L.h_meta) + L.orient_off);
+      L.h_recover = reinterpret_cast<double*>(static_cast<uint8_t*>(L.h_meta) + L.recover_off);
     }
     if ((rc = dev_alloc(h, &L.d_geoms, mf))) return rc;
     if ((rc = dev_alloc(h, &L.d_out2d, (size_t)mf * kJoints * 2))) return rc;
@@ -652,7 +662,9 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
   if ((rc = dev_alloc(h, &h->d_st3d, (size_t)ms * kJoints * 3))) return rc;
   if ((rc = dev_alloc(h, &h->d_j2_box, (size_t)mf * kJoints * 2))) return rc;
   if ((rc = dev_alloc(h, &h->d_j3_raw, (size_t)mf * kJoints * 3))) return rc;
-  if ((rc = dev_alloc(h, &h->d_raw_argmax, (size_t)mf * kJoints * 2))) return rc;
+  // the raw argmax, then the scores of a SCORES post-process; both are per call and ordered on the handle's stream
+  if ((rc = dev_alloc(h, &h->d_raw_argmax, (size_t)mf * kJoints * 4))) return rc;
+  h->d_scores = reinterpret_cast<double*>(h->d_raw_argmax + (size_t)mf * kJoints * 2);
   if ((rc = dev_alloc(h, &h->d_counter, mf))) return rc;
   if ((rc = dev_alloc(h, &h->d_prep3, (size_t)mf * kJoints * 9))) return rc;
   if (getenv("VNECT_B200_POST_TRACE") && (rc = dev_alloc(h, &h->d_post_trace, (size_t)mf * kJoints * 16))) return rc;
@@ -669,6 +681,7 @@ static int alloc_prepost(vnect_t* h, const std::vector<PyramidTable>& ptab) {
   if ((rc = dev_alloc(h, &h->d_geoms, mf))) return rc;
   if ((rc = dev_alloc(h, &h->d_boxes_used, (size_t)mf * 4))) return rc;
   h->orient.assign(ms, VNECT_ORIENT_IDENTITY);
+  h->recover.assign(ms, 0.0);
   h->last_t2d.assign(ms, NAN);
   h->last_t3d.assign(ms, NAN);
   PyramidParams& py = h->pyr;
@@ -1084,9 +1097,10 @@ static int snapshot_nonfinite(vnect_t*) { return VNECT_OK; }
 
 // table_frames > 0: the lane's frame table (already written to its pinned block) travels in the same copy.
 // oriented: so do the frames' orientation codes, taken from their streams now (a call with oriented frames always
+// carries its table); recover: so do the frames' recovery thresholds (a tracked call with a recovering stream always
 // carries its table)
 static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                            cudaStream_t copy_on, int table_frames = 0, bool oriented = false) {
+                            cudaStream_t copy_on, int table_frames = 0, bool oriented = false, bool recover = false) {
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   h->seen_stamp.resize(h->cfg.max_streams, 0);
   const unsigned int stamp = ++h->seen_epoch;
@@ -1117,12 +1131,14 @@ static int stage_frame_meta(vnect_t* h, int n_frames, const int32_t* stream_ids,
     h->cur->h_t2d[i] = t2d ? t2d[i] : 0.0;
     h->cur->h_t3d[i] = t3d ? t3d[i] : 0.0;
     if (oriented) h->cur->h_orient[i] = h->orient[sid];
+    if (recover) h->cur->h_recover[i] = h->recover[sid];
     if (h->cfg.filters) {
       h->last_t2d[sid] = t2d[i];
       h->last_t3d[sid] = t3d[i];
     }
   }
-  const size_t bytes = oriented ? h->cur->orient_off + (size_t)n_frames * sizeof(int)
+  const size_t bytes = recover ? h->cur->recover_off + (size_t)n_frames * sizeof(double)
+                       : oriented ? h->cur->orient_off + (size_t)n_frames * sizeof(int)
                        : table_frames > 0 ? h->cur->table_off + (size_t)table_frames * sizeof(FrameDesc)
                                           : h->cur->meta_bytes;
   CU(h, cudaMemcpyAsync(h->cur->d_stream_ids, h->cur->h_meta, bytes, cudaMemcpyHostToDevice, copy_on));
@@ -1204,12 +1220,29 @@ static int stage_sequence_meta(vnect_t* h, int n_frames, const int32_t* stream_i
   return VNECT_OK;
 }
 
+// The SCORES instantiations of postprocess_kernel: `launch` as run_postprocess defines it.
+template <bool RAW_ONLY, class Launch>
+static cudaError_t launch_post_scores(Launch& launch, int n_scales, bool mask1) {
+  static unsigned long long done[2][kMaxScales] = {{0, 0, 0, 0}, {0, 0, 0, 0}};
+  switch (n_scales) {
+    case 1: return mask1 ? launch(postprocess_kernel<1, 1, RAW_ONLY, true>, &done[0][0])
+                         : launch(postprocess_kernel<1, -1, RAW_ONLY, true>, &done[1][0]);
+    case 2: return mask1 ? launch(postprocess_kernel<2, 1, RAW_ONLY, true>, &done[0][1])
+                         : launch(postprocess_kernel<2, -1, RAW_ONLY, true>, &done[1][1]);
+    case 3: return mask1 ? launch(postprocess_kernel<3, 1, RAW_ONLY, true>, &done[0][2])
+                         : launch(postprocess_kernel<3, -1, RAW_ONLY, true>, &done[1][2]);
+    default: return mask1 ? launch(postprocess_kernel<4, 1, RAW_ONLY, true>, &done[0][3])
+                          : launch(postprocess_kernel<4, -1, RAW_ONLY, true>, &done[1][3]);
+  }
+}
+
 // geoms: per-frame geometry (tracked streams, mixed sizes), which overrides scaler and the offsets.
 // seq_seg: a sequence call's device segment table (stage_sequence_meta): the argmax-only instantiation, then
 // sequence_filter_kernel walks each stream's frames in order.
+// scores: the SCORES instantiation, which also writes every joint's score to d_scores.
 static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, int off_y, double* dev_out2d,
                            float* dev_out3d, const FrameGeom* geoms = nullptr, bool guard = true,
-                           const int* seq_seg = nullptr) {
+                           const int* seq_seg = nullptr, bool scores = false) {
   PostParams p;
   p.geoms = geoms;
   p.n_frames = n_frames; p.n_scales = h->n_scales; p.hs = h->hs; p.S = h->S;
@@ -1236,6 +1269,7 @@ static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, i
   const int rpp = threads / h->hs;
   post_smem_plan(p, h->h_tables.data(), (h->hs / 2 / rpp) * rpp);
   p.trace = h->d_post_trace;
+  p.scores_off = h->cfg.max_frames * kJoints * 2;
   const size_t smem = (size_t)p.smem_floats * sizeof(float);
   static unsigned long long done[kMaxScales] = {0, 0, 0, 0};
   auto launch = [&](auto kern, unsigned long long* mask) -> cudaError_t {
@@ -1246,7 +1280,9 @@ static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, i
   static unsigned long long done1[kMaxScales] = {0, 0, 0, 0};
   if (seq_seg != nullptr) {
     static unsigned long long done_raw[2][kMaxScales] = {{0, 0, 0, 0}, {0, 0, 0, 0}};
-    if (p.identity_mask == 1) {
+    if (scores) {
+      CU(h, launch_post_scores<true>(launch, h->n_scales, p.identity_mask == 1));
+    } else if (p.identity_mask == 1) {
       switch (h->n_scales) {
         case 1: CU(h, launch(postprocess_kernel<1, 1, true>, &done_raw[0][0])); break;
         case 2: CU(h, launch(postprocess_kernel<2, 1, true>, &done_raw[0][1])); break;
@@ -1273,7 +1309,9 @@ static int run_postprocess(vnect_t* h, int n_frames, double scaler, int off_x, i
     ++h->launches;
     return VNECT_OK;
   }
-  if (p.identity_mask == 1) {
+  if (scores) {
+    CU(h, launch_post_scores<false>(launch, h->n_scales, p.identity_mask == 1));
+  } else if (p.identity_mask == 1) {
     switch (h->n_scales) {
       case 1: CU(h, launch(postprocess_kernel<1, 1>, &done1[0])); break;
       case 2: CU(h, launch(postprocess_kernel<2, 1>, &done1[1])); break;
@@ -1380,9 +1418,15 @@ extern "C" {
 
 // pre-process -> CNN -> post-process for one batch, as a replayed CUDA graph when possible
 // oriented (table calls only): the lane carries its frames' orientation codes
+// scores: the post-process writes every joint's score to d_scores (the caller copies them out)
+// recover (tracked table calls only): the lane carries its frames' recovery thresholds, and the box update checks
+// each frame's mean score against them (it implies scores)
 static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_frames, int H, int W,
                         const FrameSource& src, double* out2d, float* out3d, bool tracked = false,
-                        bool sequence = false, bool oriented = false) {
+                        bool sequence = false, bool oriented = false, bool scores = false, bool recover = false) {
+  scores = scores || recover;
+  // the kernel choices the key does not otherwise carry: the SCORES post-process and the recovering box update
+  const int variant = (scores ? 16 : 0) + (recover ? 32 : 0);
   if (src.table) {  // sizes, addresses and geometry live in the lane's device tables, not in kernel parameters
     if (int rc = ensure_surround(h)) return rc;
     auto direct = [&]() -> int {
@@ -1390,10 +1434,14 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
       if ((rc = run_preprocess(h, nullptr, n_frames, 0, 0, src, Geometry{}, tracked, oriented))) return rc;
       if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
       if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, out2d, out3d, h->cur->d_geoms, true,
-                                sequence ? h->cur->d_seg : nullptr)))
+                                sequence ? h->cur->d_seg : nullptr, scores)))
         return rc;
       if (tracked) {
-        if (oriented)
+        if (recover)
+          track_update_frames_recover_kernel<<<n_frames, 32, 0, h->stream>>>(
+              out2d, h->cur->d_stream_ids, h->cur->d_table, oriented ? h->cur->d_orient : nullptr, h->d_scores,
+              h->cur->d_recover, h->d_boxes);
+        else if (oriented)
           track_update_frames_oriented_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, h->cur->d_table,
                                                                               h->cur->d_orient, h->d_boxes);
         else
@@ -1406,8 +1454,8 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
     if (!h->use_graphs) return direct();
     // sequence calls (8 + lane) read their segment table from the lane's device block as well; so do calls with
     // oriented frames their codes (the third field), so every composition of orientations replays one graph
-    const vnect_handle::GraphKey key(sequence ? 8 + lane : 4 + lane + (tracked ? 2 : 0), n_frames, oriented ? 1 : 0, 0,
-                                     0, 0, nullptr, out2d, out3d, src.format, 0, 0, 0);
+    const vnect_handle::GraphKey key(variant + (sequence ? 8 + lane : 4 + lane + (tracked ? 2 : 0)), n_frames,
+                                     oriented ? 1 : 0, 0, 0, 0, nullptr, out2d, out3d, src.format, 0, 0, 0);
     return run_graphed(h, key, direct);
   }
   const Geometry g = squarify_geometry(h->S, H, W, src.format);
@@ -1416,7 +1464,9 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
     int rc;
     if ((rc = run_preprocess(h, dev_frames, n_frames, H, W, src, g, tracked))) return rc;
     if ((rc = run_forward(h, n_frames * h->n_scales))) return rc;
-    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, out2d, out3d, tracked ? h->d_geoms : nullptr))) return rc;
+    if ((rc = run_postprocess(h, n_frames, g.scaler, g.off_x, g.off_y, out2d, out3d, tracked ? h->d_geoms : nullptr, true,
+                              nullptr, scores)))
+      return rc;
     if (tracked) {
       track_update_kernel<<<n_frames, 32, 0, h->stream>>>(out2d, h->cur->d_stream_ids, n_frames, H, W, h->d_boxes);
       CU(h, cudaGetLastError());
@@ -1426,7 +1476,7 @@ static int run_pipeline(vnect_t* h, int lane, const uint8_t* dev_frames, int n_f
   };
   if (!h->use_graphs) return direct();
   // the format and the chroma layout are baked into the squarify launch as much as the pointers are
-  const vnect_handle::GraphKey key(lane + (tracked ? 2 : 0), n_frames, H, W, (long long)src.pitch,
+  const vnect_handle::GraphKey key(variant + lane + (tracked ? 2 : 0), n_frames, H, W, (long long)src.pitch,
                                    (long long)src.frame_stride, dev_frames, out2d, out3d, src.format,
                                    (long long)src.uv_pitch, (long long)src.u_offset, (long long)src.v_offset);
   return run_graphed(h, key, direct);
@@ -1516,6 +1566,32 @@ static bool any_oriented(vnect_t* h, int n_frames, const int32_t* stream_ids) {
   return false;
 }
 
+// Whether a tracked call recovers lost people: some frame's stream has a recovery threshold (vnect_set_track_recovery).
+// Ids that stage_frame_meta refuses are skipped here, and so is a frame count it refuses.
+static bool any_recovering(vnect_t* h, int n_frames, const int32_t* stream_ids) {
+  if (n_frames < 1 || n_frames > h->cfg.max_frames) return false;
+  for (int i = 0; i < n_frames; ++i) {
+    const int sid = stream_ids ? stream_ids[i] : i;
+    if (sid >= 0 && sid < h->cfg.max_streams && h->recover[sid] > 0.0) return true;
+  }
+  return false;
+}
+
+// The pending vnect_request_scores buffer, consumed by the result-producing call that takes it, accepted or refused.
+static double* take_scores(vnect_t* h) {
+  if (!h) return nullptr;
+  double* s = h->score_req;
+  h->score_req = nullptr;
+  return s;
+}
+
+// The scores of the call's n_frames frames -> the caller's buffer, on the handle's stream after the call's kernels
+// (outside any graph, so the pointer is not part of a graph key)
+static int copy_scores(vnect_t* h, double* scores, int n_frames, cudaMemcpyKind kind) {
+  if (scores) CU(h, cudaMemcpyAsync(scores, h->d_scores, (size_t)n_frames * kJoints * sizeof(double), kind, h->stream));
+  return VNECT_OK;
+}
+
 // The current lane's frame table for n_frames uniform frames at `frames` (device), laid out as `src` describes:
 // a uniform call with oriented frames runs the table pipeline on it.
 static void uniform_table(vnect_t* h, const uint8_t* frames, int n_frames, int H, int W, const FrameSource& src) {
@@ -1534,7 +1610,7 @@ static void uniform_table(vnect_t* h, const uint8_t* frames, int n_frames, int H
 // vnect_estimate_device / vnect_estimate_device_yuv once the frame description is validated
 static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
                            const FrameSource& src, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                           double* dev_joints2d, float* dev_joints3d) {
+                           double* dev_joints2d, float* dev_joints3d, double* dev_scores) {
   // alternate lanes for the per-call meta so the host can run one call ahead of the GPU
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
@@ -1546,8 +1622,9 @@ static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_fram
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
   if ((rc = run_pipeline(h, lane, dev_frames, n_frames, H, W, oriented ? table_source(src.format) : src, dev_joints2d,
-                         dev_joints3d, false, false, oriented)))
+                         dev_joints3d, false, false, oriented, dev_scores != nullptr)))
     return rc;
+  if ((rc = copy_scores(h, dev_scores, n_frames, cudaMemcpyDeviceToDevice))) return rc;
   if ((rc = snapshot_nonfinite(h))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
@@ -1557,7 +1634,7 @@ static int estimate_device(vnect_t* h, const uint8_t* dev_frames, int32_t n_fram
 // vnect_submit / vnect_submit_yuv once the arguments are validated
 static int submit(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_frames, int32_t H, int32_t W,
                   const FrameSource& src, const int32_t* stream_ids, const double* t2d, const double* t3d,
-                  double* joints2d, float* joints3d) {
+                  double* joints2d, float* joints3d, double* scores) {
   int rc = lane_acquire(h, lane);
   if (rc) return rc;
   const bool oriented = any_oriented(h, n_frames, stream_ids);
@@ -1569,10 +1646,11 @@ static int submit(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_fra
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   if ((rc = run_pipeline(h, lane, h->cur->d_frames, n_frames, H, W, oriented ? table_source(src.format) : packed,
-                         h->cur->d_out2d, h->cur->d_out3d, false, false, oriented)))
+                         h->cur->d_out2d, h->cur->d_out3d, false, false, oriented, scores != nullptr)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   if ((rc = snapshot_nonfinite(h))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
@@ -1582,23 +1660,26 @@ static int submit(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_fra
 // vnect_track / vnect_track_yuv once the arguments are validated
 static int track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW, const FrameSource& src,
                  const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d, float* joints3d,
-                 int32_t* boxes_used) {
+                 int32_t* boxes_used, double* scores) {
   int rc = lane_acquire(h, 0);
   if (rc) return rc;
-  const bool oriented = any_oriented(h, n_frames, stream_ids);
-  if (oriented) uniform_table(h, h->cur->d_frames, n_frames, FH, FW, packed_source(src.format, FH, FW));
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, 0, oriented))) return rc;
+  // oriented frames or a recovering stream: the table pipeline, on a table of the staged frames
+  const bool oriented = any_oriented(h, n_frames, stream_ids), recover = any_recovering(h, n_frames, stream_ids);
+  if (oriented || recover) uniform_table(h, h->cur->d_frames, n_frames, FH, FW, packed_source(src.format, FH, FW));
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, 0, oriented, recover))) return rc;
   FrameSource packed;
   if ((rc = stage_frames(h, frames, n_frames, FH, FW, src, &packed))) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
-  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW, oriented ? table_source(src.format) : packed,
-                         h->cur->d_out2d, h->cur->d_out3d, true, false, oriented)))
+  if ((rc = run_pipeline(h, 0, h->cur->d_frames, n_frames, FH, FW,
+                         oriented || recover ? table_source(src.format) : packed, h->cur->d_out2d, h->cur->d_out3d,
+                         true, false, oriented, scores != nullptr, recover)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (boxes_used)
     CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   if ((rc = snapshot_nonfinite(h))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
@@ -1665,7 +1746,7 @@ static int check_frames(vnect_t* h, const vnect_frame* frames, int n_frames, int
 // may repeat (vnect_submit_sequence).
 static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
-                         float* joints3d, bool tracked, int32_t* boxes_used, bool synchronous,
+                         float* joints3d, bool tracked, int32_t* boxes_used, bool synchronous, double* scores,
                          bool sequence = false) {
   int rc = lane_acquire(h, lane);
   if (rc) return rc;
@@ -1692,8 +1773,9 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
   // ids, timestamps, the table and any orientation codes in one copy; a refused id or timestamp returns before any
   // frame copy is queued
   const bool oriented = any_oriented(h, n_frames, stream_ids);
+  const bool recover = tracked && any_recovering(h, n_frames, stream_ids);
   rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, oriented)
-                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented);
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented, recover);
   if (rc) return rc;
   for (int i = 0; i < n_frames; ++i)
     if ((rc = stage_frame(h, const_cast<uint8_t*>(h->cur->h_table[i].data), frames[i].data, frames[i].height,
@@ -1702,12 +1784,13 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), h->cur->d_out2d, h->cur->d_out3d, tracked,
-                         sequence, oriented)))
+                         sequence, oriented, scores != nullptr, recover)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (boxes_used)
     CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
   return synchronous ? lane_acquire(h, lane) : VNECT_OK;  // synchronises and reports non-finite maps
@@ -1717,23 +1800,26 @@ static int submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, in
 // are used as they are; the lanes alternate for the per-call meta so the host can run one call ahead of the GPU
 static int device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                          const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
-                         float* dev_joints3d, bool tracked, int32_t* dev_boxes_used, bool sequence = false) {
+                         float* dev_joints3d, bool tracked, int32_t* dev_boxes_used, double* dev_scores,
+                         bool sequence = false) {
   int rc = lane_acquire(h, (int)(h->device_calls++ & 1));
   if (rc) return rc;
   memcpy(h->cur->h_table, frames, (size_t)n_frames * sizeof(FrameDesc));
   const bool oriented = any_oriented(h, n_frames, stream_ids);
+  const bool recover = tracked && any_recovering(h, n_frames, stream_ids);
   rc = sequence ? stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, oriented)
-                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented);
+                : stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->copy_stream, n_frames, oriented, recover);
   if (rc) return rc;
   CU(h, cudaEventRecord(h->cur->copy_done, h->copy_stream));
   CU(h, cudaStreamWaitEvent(h->stream, h->cur->copy_done, 0));
   const int lane = (int)(h->cur - h->lanes);
   if ((rc = run_pipeline(h, lane, nullptr, n_frames, 0, 0, table_source(format), dev_joints2d, dev_joints3d, tracked,
-                         sequence, oriented)))
+                         sequence, oriented, dev_scores != nullptr, recover)))
     return rc;
   if (dev_boxes_used)  // outside the graph, so the caller's pointer stays out of its key
     CU(h, cudaMemcpyAsync(dev_boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToDevice,
                           h->stream));
+  if ((rc = copy_scores(h, dev_scores, n_frames, cudaMemcpyDeviceToDevice))) return rc;
   CU(h, cudaEventRecord(h->cur->done, h->stream));
   h->cur->pending = true;
   return VNECT_OK;
@@ -1742,24 +1828,26 @@ static int device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames
 int vnect_submit_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                         const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                         float* joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
   return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr,
-                       false);
+                       false, scores);
 }
 
 int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                        const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                        float* joints3d, int32_t* boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
   return submit_frames(h, 0, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used,
-                       true);
+                       true, scores);
 }
 
 // Pipelined and device-resident tracking.  A tracked call no longer has to wait for its results: every kernel that
@@ -1775,34 +1863,38 @@ int vnect_track_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, 
 int vnect_submit_track_frames(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                               const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                               float* joints3d, int32_t* boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
   return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, true, boxes_used,
-                       false);
+                       false, scores);
 }
 
 int vnect_estimate_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                                  const int32_t* stream_ids, const double* t2d, const double* t3d,
                                  double* dev_joints2d, float* dev_joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
-  return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, false, nullptr);
+  return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, false, nullptr,
+                       scores);
 }
 
 int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                               const int32_t* stream_ids, const double* t2d, const double* t3d, double* dev_joints2d,
                               float* dev_joints3d, int32_t* dev_boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
   return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, true,
-                       dev_boxes_used);
+                       dev_boxes_used, scores);
 }
 
 // Sequence calls (include/vnect_b200.h): the table paths above with a stream id allowed to repeat.  Filter state is
@@ -1811,51 +1903,56 @@ int vnect_track_device_frames(vnect_t* h, const vnect_frame* frames, int32_t n_f
 int vnect_submit_sequence(vnect_t* h, int32_t lane, const vnect_frame* frames, int32_t n_frames, int32_t format,
                           const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                           float* joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
   if (!joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, true)) return rc;
   return submit_frames(h, lane, frames, n_frames, format, stream_ids, t2d, t3d, joints2d, joints3d, false, nullptr,
-                       false, true);
+                       false, scores, true);
 }
 
 int vnect_estimate_device_sequence(vnect_t* h, const vnect_frame* frames, int32_t n_frames, int32_t format,
                                    const int32_t* stream_ids, const double* t2d, const double* t3d,
                                    double* dev_joints2d, float* dev_joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_frames(h, frames, n_frames, format, false)) return rc;
   return device_frames(h, frames, n_frames, format, stream_ids, t2d, t3d, dev_joints2d, dev_joints3d, false, nullptr,
-                       true);
+                       scores, true);
 }
 
 int vnect_estimate_device(vnect_t* h, const uint8_t* dev_bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
                           int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d,
                           double* dev_joints2d, float* dev_joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!dev_bgr || !dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (H < 2 || W < 2 || pitch < (int64_t)W * 3) return fail(h, VNECT_E_INVALID, "bad frame geometry %dx%d pitch %lld", H, W, (long long)pitch);
   return estimate_device(h, dev_bgr, n_frames, H, W, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d,
-                         dev_joints2d, dev_joints3d);
+                         dev_joints2d, dev_joints3d, scores);
 }
 
 int vnect_estimate_device_yuv(vnect_t* h, const uint8_t* dev_frames, int32_t n_frames, int32_t H, int32_t W,
                               const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d,
                               const double* t3d, double* dev_joints2d, float* dev_joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!dev_frames || !dev_joints2d || !dev_joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (int rc = check_yuv_layout(h, layout, H, W)) return rc;
   return estimate_device(h, dev_frames, n_frames, H, W, yuv_source(*layout), stream_ids, t2d, t3d, dev_joints2d,
-                         dev_joints3d);
+                         dev_joints3d, scores);
 }
 
 int vnect_submit(vnect_t* h, int32_t lane, const uint8_t* bgr, int32_t n_frames, int32_t H, int32_t W, int64_t pitch,
                  int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                  float* joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
@@ -1863,12 +1960,14 @@ int vnect_submit(vnect_t* h, int32_t lane, const uint8_t* bgr, int32_t n_frames,
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   if (int rc = check_host_frame_size(h, H, W)) return rc;
   if (pitch < (int64_t)W * 3) return fail(h, VNECT_E_INVALID, "pitch smaller than a row");
-  return submit(h, lane, bgr, n_frames, H, W, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d, joints2d, joints3d);
+  return submit(h, lane, bgr, n_frames, H, W, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d, joints2d, joints3d,
+                scores);
 }
 
 int vnect_submit_yuv(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_frames, int32_t H, int32_t W,
                      const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
                      double* joints2d, float* joints3d) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (lane < 0 || lane > 1) return fail(h, VNECT_E_INVALID, "lane must be 0 or 1");
@@ -1876,7 +1975,8 @@ int vnect_submit_yuv(vnect_t* h, int32_t lane, const uint8_t* frames, int32_t n_
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   if (int rc = check_host_frame_size(h, H, W)) return rc;
   if (int rc = check_yuv_layout(h, layout, H, W)) return rc;
-  return submit(h, lane, frames, n_frames, H, W, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d);
+  return submit(h, lane, frames, n_frames, H, W, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d,
+                scores);
 }
 
 int vnect_track_set_box(vnect_t* h, int32_t stream_id, int32_t x, int32_t y, int32_t w, int32_t hh) {
@@ -1959,9 +2059,42 @@ int vnect_get_orientation(vnect_t* h, int32_t stream_id, int32_t* code) {
   return VNECT_OK;
 }
 
+int vnect_request_scores(vnect_t* h, double* scores) {
+  if (!h) return fail(h, VNECT_E_INVALID, "null handle");
+  h->score_req = scores;
+  return VNECT_OK;
+}
+
+int vnect_set_track_recovery(vnect_t* h, int32_t n, const int32_t* stream_ids, const double* min_mean_score) {
+  if (!h || h->recover.empty()) return fail(h, VNECT_E_INVALID, "handle not created");
+  if (n < 0) return fail(h, VNECT_E_INVALID, "n %d below 0", n);
+  if (n == 0) return VNECT_OK;
+  if (!stream_ids || !min_mean_score) return fail(h, VNECT_E_INVALID, "null buffer");
+  h->seen_stamp.resize(h->cfg.max_streams, 0);
+  const unsigned int stamp = ++h->seen_epoch;
+  for (int i = 0; i < n; ++i) {  // everything is checked before the first change
+    const int sid = stream_ids[i];
+    if (sid < 0 || sid >= h->cfg.max_streams) return fail(h, VNECT_E_INVALID, "stream id %d not in [0, %d)", sid, h->cfg.max_streams);
+    if (h->seen_stamp[sid] == stamp) return fail(h, VNECT_E_INVALID, "stream id %d appears twice", sid);
+    h->seen_stamp[sid] = stamp;
+    if (!(min_mean_score[i] >= 0.0 && min_mean_score[i] < INFINITY))
+      return fail(h, VNECT_E_INVALID, "recovery threshold %g of stream %d is not a finite value >= 0", min_mean_score[i], sid);
+  }
+  for (int i = 0; i < n; ++i) h->recover[stream_ids[i]] = min_mean_score[i];
+  return VNECT_OK;
+}
+
+int vnect_get_track_recovery(vnect_t* h, int32_t stream_id, double* min_mean_score) {
+  if (!h || h->recover.empty() || !min_mean_score) return fail(h, VNECT_E_INVALID, "handle not created / null buffer");
+  if (stream_id < 0 || stream_id >= h->cfg.max_streams) return fail(h, VNECT_E_INVALID, "stream id out of range");
+  *min_mean_score = h->recover[stream_id];
+  return VNECT_OK;
+}
+
 int vnect_track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW, int64_t pitch,
                 int64_t frame_stride, const int32_t* stream_ids, const double* t2d, const double* t3d, double* joints2d,
                 float* joints3d, int32_t* boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!frames || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
@@ -1969,19 +2102,21 @@ int vnect_track(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH,
   if (int rc = check_host_frame_size(h, FH, FW)) return rc;
   if (pitch < (int64_t)FW * 3) return fail(h, VNECT_E_INVALID, "pitch smaller than a row");
   return track(h, frames, n_frames, FH, FW, bgr_source(pitch, frame_stride), stream_ids, t2d, t3d, joints2d, joints3d,
-               boxes_used);
+               boxes_used, scores);
 }
 
 int vnect_track_yuv(vnect_t* h, const uint8_t* frames, int32_t n_frames, int32_t FH, int32_t FW,
                     const vnect_yuv_layout* layout, const int32_t* stream_ids, const double* t2d, const double* t3d,
                     double* joints2d, float* joints3d, int32_t* boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->finalized) return fail(h, VNECT_E_INVALID, "handle not finalized");
   ON_DEVICE(h);
   if (!frames || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
   if (n_frames < 1 || n_frames > h->cfg.max_frames) return fail(h, VNECT_E_INVALID, "n_frames %d not in [1, %d]", n_frames, h->cfg.max_frames);
   if (int rc = check_host_frame_size(h, FH, FW)) return rc;
   if (int rc = check_yuv_layout(h, layout, FH, FW)) return rc;
-  return track(h, frames, n_frames, FH, FW, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d, boxes_used);
+  return track(h, frames, n_frames, FH, FW, yuv_source(*layout), stream_ids, t2d, t3d, joints2d, joints3d, boxes_used,
+               scores);
 }
 
 int vnect_wait(vnect_t* h, int32_t lane) {
@@ -2047,6 +2182,7 @@ static int stage_maps(vnect_t* h, const float* hm, const float* xm, const float*
 int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm, int32_t n_frames,
                       const int32_t* stream_ids, const double* t2d, const double* t3d, double scaler, int32_t offset_x,
                       int32_t offset_y, double* joints2d, float* joints3d, int32_t* raw_argmax) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
   ON_DEVICE(h);
   if (!hm || !xm || !ym || !zm || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
@@ -2054,11 +2190,14 @@ int vnect_postprocess(vnect_t* h, const float* hm, const float* xm, const float*
   if (rc) return rc;
   if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream))) return rc;
   if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
-  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false))) return rc;
+  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, h->cur->d_out2d, h->cur->d_out3d, nullptr, false,
+                            nullptr, scores != nullptr)))
+    return rc;
   CU(h, cudaMemcpyAsync(joints2d, h->cur->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, h->cur->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (raw_argmax)
     CU(h, cudaMemcpyAsync(raw_argmax, h->d_raw_argmax, (size_t)n_frames * kJoints * 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   CU(h, cudaStreamSynchronize(h->stream));
   return VNECT_OK;
 }
@@ -2068,6 +2207,7 @@ int vnect_postprocess_sequence(vnect_t* h, const float* hm, const float* xm, con
                                int32_t n_frames, const int32_t* stream_ids, const double* t2d, const double* t3d,
                                double scaler, int32_t offset_x, int32_t offset_y, double* joints2d, float* joints3d,
                                int32_t* raw_argmax) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
   ON_DEVICE(h);
   if (!hm || !xm || !ym || !zm || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
@@ -2076,12 +2216,14 @@ int vnect_postprocess_sequence(vnect_t* h, const float* hm, const float* xm, con
   vnect_handle::Lane* L = h->cur;
   if ((rc = stage_sequence_meta(h, n_frames, stream_ids, t2d, t3d, h->stream))) return rc;
   if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
-  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, L->d_out2d, L->d_out3d, nullptr, false, L->d_seg)))
+  if ((rc = run_postprocess(h, n_frames, scaler, offset_x, offset_y, L->d_out2d, L->d_out3d, nullptr, false, L->d_seg,
+                            scores != nullptr)))
     return rc;
   CU(h, cudaMemcpyAsync(joints2d, L->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, L->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (raw_argmax)
     CU(h, cudaMemcpyAsync(raw_argmax, h->d_raw_argmax, (size_t)n_frames * kJoints * 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   CU(h, cudaStreamSynchronize(h->stream));
   return VNECT_OK;
 }
@@ -2092,6 +2234,7 @@ int vnect_postprocess_sequence(vnect_t* h, const float* hm, const float* xm, con
 int vnect_track_postprocess(vnect_t* h, const float* hm, const float* xm, const float* ym, const float* zm,
                             int32_t n_frames, const int32_t* frame_hw, const int32_t* stream_ids, const double* t2d,
                             const double* t3d, double* joints2d, float* joints3d, int32_t* boxes_used) {
+  double* const scores = take_scores(h);  // consumed, accepted or refused
   if (!h || !h->x1) return fail(h, VNECT_E_INVALID, "handle not created");
   ON_DEVICE(h);
   if (!hm || !xm || !ym || !zm || !frame_hw || !joints2d || !joints3d) return fail(h, VNECT_E_INVALID, "null buffer");
@@ -2108,20 +2251,28 @@ int vnect_track_postprocess(vnect_t* h, const float* hm, const float* xm, const 
     t.height = frame_hw[2 * i];
     t.width = frame_hw[2 * i + 1];
   }
-  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream, n_frames))) return rc;
+  const bool recover = any_recovering(h, n_frames, stream_ids);
+  if ((rc = stage_frame_meta(h, n_frames, stream_ids, t2d, t3d, h->stream, n_frames, false, recover))) return rc;
   if ((rc = stage_maps(h, hm, xm, ym, zm, n_frames))) return rc;
   frame_geometry_kernel<<<(n_frames + 63) / 64, 64, 0, h->stream>>>(L->d_table, h->d_boxes, L->d_stream_ids, n_frames,
                                                                     h->S, L->d_geoms, h->d_boxes_used);
   CU(h, cudaGetLastError());
   ++h->launches;
-  if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, L->d_out2d, L->d_out3d, L->d_geoms, false))) return rc;
-  track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(L->d_out2d, L->d_stream_ids, L->d_table, h->d_boxes);
+  if ((rc = run_postprocess(h, n_frames, 1.0, 0, 0, L->d_out2d, L->d_out3d, L->d_geoms, false, nullptr,
+                            scores != nullptr || recover)))
+    return rc;
+  if (recover)
+    track_update_frames_recover_kernel<<<n_frames, 32, 0, h->stream>>>(L->d_out2d, L->d_stream_ids, L->d_table, nullptr,
+                                                                       h->d_scores, L->d_recover, h->d_boxes);
+  else
+    track_update_frames_kernel<<<n_frames, 32, 0, h->stream>>>(L->d_out2d, L->d_stream_ids, L->d_table, h->d_boxes);
   CU(h, cudaGetLastError());
   ++h->launches;
   CU(h, cudaMemcpyAsync(joints2d, L->d_out2d, (size_t)n_frames * kJoints * 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(h, cudaMemcpyAsync(joints3d, L->d_out3d, (size_t)n_frames * kJoints * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   if (boxes_used)
     CU(h, cudaMemcpyAsync(boxes_used, h->d_boxes_used, (size_t)n_frames * 4 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_scores(h, scores, n_frames, cudaMemcpyDeviceToHost))) return rc;
   CU(h, cudaStreamSynchronize(h->stream));
   return VNECT_OK;
 }

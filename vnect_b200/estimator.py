@@ -325,54 +325,86 @@ class VNectEngine:
             raise ValueError("stream_ids must have one entry per frame")
         return ids, t2d, t3d
 
-    def estimate(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    @staticmethod
+    def _scores_out(scores, n):
+        """The ``scores`` argument of a host-result method -> None (False) or the float64 [n, 21] array the call writes
+        every joint's score to (True: a new one; an array: that array, which must be C-contiguous and writable)."""
+        if scores is False or scores is None:
+            return None
+        if scores is True:
+            return np.empty((n, JOINTS), np.float64)
+        if not (isinstance(scores, np.ndarray) and scores.dtype == np.float64 and scores.shape == (n, JOINTS)
+                and scores.flags.c_contiguous and scores.flags.writeable):
+            raise ValueError(f"scores must be True, False or a writable C-contiguous float64 [{n}, {JOINTS}] array")
+        return scores
+
+    def _request_scores(self, ptr):
+        """vnect_request_scores: the C call made right after this one also writes its scores to ``ptr`` (a host
+        array's or a device address); nothing that can raise may run in between."""
+        if ptr is not None:
+            self._check(self._lib.vnect_request_scores(self._h, ptr))
+
+    def estimate(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr", scores=False):
         """VNectEstimator.__call__ for n independent frames (host arrays in, host arrays out).  ``pixel_format``
         "nv12" / "i420" takes YUV 4:2:0 frames (uint8 [n,3H/2,W]) and gives exactly the results of the BGR frames
-        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420); the conversion runs inside the pre-processing."""
+        cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / _I420); the conversion runs inside the pre-processing.
+        ``scores``: True, or a float64 [n, 21] array, adds every joint's confidence (vnect_request_scores: the
+        reference's float64 upsampled heat-map value at its argmax) as a last result.  The same holds for every
+        host-result method below."""
         if pixel_format != "bgr":
-            j2, j3 = self.submit(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+            res = self.submit(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format, scores=scores)
             self.wait(0)
-            return j2, j3
+            return res
         frames, st = self._frames(frames)
         n, h, w = frames.shape[:3]
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_estimate(self._h, _ptr(frames), n, h, w, st[1], st[0] if n > 1 else st[1] * h,
                                              _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
-        return j2, j3
+        return (j2, j3) if sc is None else (j2, j3, sc)
 
-    def submit(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def _enqueued(self, lane, keep, results, sc):
+        """Records a submitted call's buffers until wait(lane) and returns its results (+ scores when asked)."""
+        results = tuple(results) + ((sc,) if sc is not None else ())
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[int(lane)] = (keep, *results)  # keep the buffers alive
+        return results
+
+    def submit(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr", scores=False):
         """Pipelined estimate(): enqueue a batch on lane 0/1 and return (joints_2d, joints_3d) arrays that are filled
         once wait(lane) returns.  `frames` and the result arrays must stay alive until then (pinned memory makes the
-        copies truly asynchronous).  ``pixel_format`` as in estimate()."""
+        copies truly asynchronous).  ``pixel_format`` and ``scores`` as in estimate()."""
         frames, n, h, w, layout = self._source(frames, pixel_format)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        sc = self._scores_out(scores, n)
         fn = self._lib.vnect_submit if pixel_format == "bgr" else self._lib.vnect_submit_yuv
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(fn(self._h, int(lane), _ptr(frames), n, h, w, *layout, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2),
                        _ptr(j3)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[int(lane)] = (frames, j2, j3)  # keep the buffers alive
-        return j2, j3
+        return self._enqueued(lane, frames, (j2, j3), sc)
 
-    def estimate_frames(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def estimate_frames(self, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr", scores=False):
         """estimate() for frames of different sizes in one batch: ``frames`` is a sequence of host arrays as
         frame_table() takes them.  Frame i gives exactly what estimate() gives for that frame alone."""
-        j2, j3 = self.submit_frames(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+        res = self.submit_frames(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format, scores=scores)
         self.wait(0)
-        return j2, j3
+        return res
 
-    def submit_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def submit_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr",
+                      scores=False):
         """submit() for frames of different sizes (see estimate_frames); completes with wait(lane)."""
         table, keep = frame_table(frames, pixel_format)
         n = len(table)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_submit_frames(self._h, int(lane), table, n, _format_code(pixel_format), _ptr(ids),
                                                   _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[int(lane)] = (keep, j2, j3)  # keep the buffers alive
-        return j2, j3
+        return self._enqueued(lane, keep, (j2, j3), sc)
 
     def _sequence_meta(self, n, stream_ids, t2d, t3d):
         """_meta for a sequence call: ids are required and, with filters on, one 2D and one 3D reading per frame (a
@@ -383,40 +415,42 @@ class VNectEngine:
             raise ValueError("a sequence call with filters on needs t2d and t3d for every frame")
         return self._meta(n, stream_ids, 0.0 if t2d is None else t2d, 0.0 if t3d is None else t3d)
 
-    def estimate_sequence(self, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def estimate_sequence(self, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr", scores=False):
         """estimate_frames() where a stream id may appear several times: the frames of one stream are consecutive in
         time in call order (they may be interleaved with other streams' frames).  Frame i gets bit for bit what
         estimate_frames() gives when the frames go in one per call in call order; the CNN runs over the whole call at
         batch size.  A call refused for its ids or timestamps processes none of its frames."""
-        j2, j3 = self.submit_sequence(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format)
+        res = self.submit_sequence(0, frames, stream_ids, t2d, t3d, out, pixel_format=pixel_format, scores=scores)
         self.wait(0)
-        return j2, j3
+        return res
 
-    def submit_sequence(self, lane, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def submit_sequence(self, lane, frames, stream_ids, t2d=None, t3d=None, out=None, pixel_format="bgr",
+                        scores=False):
         """submit_frames() for a sequence call (see estimate_sequence); completes with wait(lane)."""
         table, keep = frame_table(frames, pixel_format)
         n = len(table)
         ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
         j2, j3 = out if out is not None else (np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32))
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_submit_sequence(self._h, int(lane), table, n, _format_code(pixel_format),
                                                     _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[int(lane)] = (keep, j2, j3)  # keep the buffers alive
-        return j2, j3
+        return self._enqueued(lane, keep, (j2, j3), sc)
 
     def estimate_device_sequence(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids, t2d=None, t3d=None,
-                                 pixel_format="bgr"):
+                                 pixel_format="bgr", dev_scores_ptr=None):
         """estimate_device_frames() for a sequence call (see estimate_sequence).  Asynchronous."""
         table = device_frame_table(frames, pixel_format)
         n = len(table)
         ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
+        self._request_scores(C.c_void_p(dev_scores_ptr) if dev_scores_ptr else None)
         self._check(self._lib.vnect_estimate_device_sequence(self._h, table, n, _format_code(pixel_format), _ptr(ids),
                                                              _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
                                                              C.c_void_p(dev_j3_ptr)))
 
     def wait(self, lane):
         """Completes the lane's submission: (joints_2d, joints_3d), or (joints_2d, joints_3d, boxes_used) after
-        submit_track / submit_track_frames."""
+        submit_track / submit_track_frames, followed by the scores when the submission asked for them."""
         self._check(self._lib.vnect_wait(self._h, int(lane)))
         return self.__dict__.get("_inflight", {}).pop(int(lane), (None, None, None))[1:]
 
@@ -430,7 +464,7 @@ class VNectEngine:
         self._check(self._lib.vnect_track_get_box(self._h, int(stream_id), out))
         return tuple(out)
 
-    def track(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr"):
+    def track(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr", scores=False):
         """One step of the reference's video loop (run_estimator.py:98-119) for n streams: crop each full frame by
         its stream's box, estimate, shift joints_2d to full-frame coordinates, update the box on the device.
         Returns (joints_2d [n,21,2], joints_3d [n,21,3], boxes_used [n,4]).  ``pixel_format`` as in estimate()."""
@@ -438,12 +472,14 @@ class VNectEngine:
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         boxes = np.empty((n, 4), np.int32)
+        sc = self._scores_out(scores, n)
         fn = self._lib.vnect_track if pixel_format == "bgr" else self._lib.vnect_track_yuv
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(fn(self._h, _ptr(frames), n, h, w, *layout, _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3),
                        _ptr(boxes)))
-        return j2, j3, boxes
+        return (j2, j3, boxes) if sc is None else (j2, j3, boxes, sc)
 
-    def track_frames(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr"):
+    def track_frames(self, frames, stream_ids=None, t2d=None, t3d=None, pixel_format="bgr", scores=False):
         """track() for streams whose full frames differ in size: each frame is cropped by its stream's box clipped to
         that frame.  Returns (joints_2d [n,21,2], joints_3d [n,21,3], boxes_used [n,4])."""
         table, keep = frame_table(frames, pixel_format)
@@ -451,53 +487,61 @@ class VNectEngine:
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         boxes = np.empty((n, 4), np.int32)
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_track_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids), _ptr(t2d),
                                                  _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
-        return j2, j3, boxes
+        return (j2, j3, boxes) if sc is None else (j2, j3, boxes, sc)
 
-    def submit_track(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def submit_track(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr",
+                     scores=False):
         """Pipelined track(): enqueue one tracked step on lane 0/1 and return (joints_2d, joints_3d, boxes_used)
         arrays that are filled once wait(lane) returns.  Same frames as track(); the call reads them in place
         (uniform_frame_table), so they, and ``out`` if given, must stay alive until the wait (pinned memory makes the
         copies truly asynchronous).  Steps of one stream may alternate between the lanes."""
         table, keep = uniform_frame_table(frames, pixel_format)
-        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format)
+        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format, scores)
 
-    def submit_track_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr"):
+    def submit_track_frames(self, lane, frames, stream_ids=None, t2d=None, t3d=None, out=None, pixel_format="bgr",
+                            scores=False):
         """submit_track() for streams whose full frames differ in size, as track_frames() takes them."""
         table, keep = frame_table(frames, pixel_format)
-        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format)
+        return self._submit_track(lane, table, keep, stream_ids, t2d, t3d, out, pixel_format, scores)
 
-    def _submit_track(self, lane, table, keep, stream_ids, t2d, t3d, out, pixel_format):
+    def _submit_track(self, lane, table, keep, stream_ids, t2d, t3d, out, pixel_format, scores):
         n = len(table)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3, boxes = out if out is not None else (np.empty((n, JOINTS, 2), np.float64),
                                                      np.empty((n, JOINTS, 3), np.float32), np.empty((n, 4), np.int32))
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_submit_track_frames(self._h, int(lane), table, n, _format_code(pixel_format),
                                                         _ptr(ids), _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3),
                                                         _ptr(boxes)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[int(lane)] = (keep, j2, j3, boxes)  # keep the buffers alive
-        return j2, j3, boxes
+        return self._enqueued(lane, keep, (j2, j3, boxes), sc)
 
     def track_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr=None, stream_ids=None, t2d=None,
-                            t3d=None, pixel_format="bgr"):
+                            t3d=None, pixel_format="bgr", dev_scores_ptr=None):
         """track_frames() on device full frames (``frames`` as device_frame_table() takes them) with device results:
         joints_2d float64 [n,21,2], joints_3d float32 [n,21,3] and, when ``dev_boxes_ptr`` is given, boxes_used int32
-        [n,4].  Asynchronous on the engine's stream."""
+        [n,4]; when ``dev_scores_ptr`` is given, every joint's score float64 [n,21] (as for every *_device* method).
+        Asynchronous on the engine's stream."""
         table = device_frame_table(frames, pixel_format)
         n = len(table)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        self._request_scores(C.c_void_p(dev_scores_ptr) if dev_scores_ptr else None)
         self._check(self._lib.vnect_track_device_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids),
                                                         _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
                                                         C.c_void_p(dev_j3_ptr),
                                                         C.c_void_p(dev_boxes_ptr) if dev_boxes_ptr else None))
 
     def track_device(self, dev_frames_ptr, n, h, w, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr=None, stream_ids=None,
-                     t2d=None, t3d=None, pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
+                     t2d=None, t3d=None, pitch=None, frame_stride=None, pixel_format="bgr", layout=None,
+                     dev_scores_ptr=None):
         """track_device_frames() on n equal-size device frames described as estimate_device() takes them."""
         frames = strided_device_frames(dev_frames_ptr, n, h, w, pitch, frame_stride, pixel_format, layout)
-        self.track_device_frames(frames, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr, stream_ids, t2d, t3d, pixel_format)
+        self.track_device_frames(frames, dev_j2_ptr, dev_j3_ptr, dev_boxes_ptr, stream_ids, t2d, t3d, pixel_format,
+                                 dev_scores_ptr)
 
     def set_boxes(self, stream_ids, rects):
         """set_box() for several streams, in submission order: after every call already submitted and before every
@@ -529,34 +573,57 @@ class VNectEngine:
         self._check(self._lib.vnect_get_orientation(self._h, int(stream_id), C.byref(out)))
         return out.value
 
+    def set_track_recovery(self, stream_ids, min_mean_scores):
+        """Recover lost people in tracked streams: when the mean score (sum(scores[f]) / 21, summed in joint order)
+        of a stream's tracked frame falls below its threshold, its next frame is cropped to the whole frame instead of
+        the box built from the current joints.  One threshold per stream id; 0 turns recovery off (the default).
+        Calls already submitted keep the thresholds they were submitted with; reset() keeps them and
+        export_stream_state() does not carry them."""
+        ids = np.ascontiguousarray(stream_ids, dtype=np.int32).reshape(-1)
+        tau = np.ascontiguousarray(min_mean_scores, dtype=np.float64).reshape(-1)
+        if tau.shape != ids.shape:
+            raise ValueError(f"expected one threshold per stream id: {len(ids)} ids, {len(tau)} thresholds")
+        self._check(self._lib.vnect_set_track_recovery(self._h, len(ids), _ptr(ids), _ptr(tau)))
+
+    def track_recovery(self, stream_id):
+        """The recovery threshold of a stream (0 = off)."""
+        out = C.c_double()
+        self._check(self._lib.vnect_get_track_recovery(self._h, int(stream_id), C.byref(out)))
+        return out.value
+
     def estimate_device_frames(self, frames, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
-                               pixel_format="bgr"):
+                               pixel_format="bgr", dev_scores_ptr=None):
         """estimate_device() for device frames of different sizes, each at its own address (e.g. one tensor or
         decoder surface per camera): ``frames`` as device_frame_table() takes them.  Asynchronous."""
         table = device_frame_table(frames, pixel_format)
         n = len(table)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        self._request_scores(C.c_void_p(dev_scores_ptr) if dev_scores_ptr else None)
         self._check(self._lib.vnect_estimate_device_frames(self._h, table, n, _format_code(pixel_format), _ptr(ids),
                                                            _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
                                                            C.c_void_p(dev_j3_ptr)))
 
     def estimate_device(self, dev_frames_ptr, n, h, w, dev_j2_ptr, dev_j3_ptr, stream_ids=None, t2d=None, t3d=None,
-                        pitch=None, frame_stride=None, pixel_format="bgr", layout=None):
+                        pitch=None, frame_stride=None, pixel_format="bgr", layout=None, dev_scores_ptr=None):
         """Same path with frames / results resident in device memory (raw device pointers, e.g. tensor.data_ptr()).
         For "nv12" / "i420" frames of h x w pixels, ``layout`` is a dict of yuv_layout() fields (y_pitch, uv_pitch,
         u_offset, v_offset, frame_stride) describing e.g. a padded decoder surface; by default cv2's contiguous
-        layout.  ``pitch`` and ``frame_stride`` describe BGR frames only."""
+        layout.  ``pitch`` and ``frame_stride`` describe BGR frames only.  ``dev_scores_ptr``: device float64 [n,21]
+        that also receives every joint's score, in stream order."""
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
+        sc = C.c_void_p(dev_scores_ptr) if dev_scores_ptr else None
         if pixel_format != "bgr":
             if pitch is not None or frame_stride is not None:
                 raise ValueError("YUV frames are described by `layout`, not by pitch / frame_stride")
             lay = yuv_layout(pixel_format, h, w, **(layout or {}))
+            self._request_scores(sc)
             self._check(self._lib.vnect_estimate_device_yuv(self._h, C.c_void_p(dev_frames_ptr), n, h, w, C.byref(lay),
                                                             _ptr(ids), _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
                                                             C.c_void_p(dev_j3_ptr)))
             return
         pitch = pitch or w * 3
         frame_stride = frame_stride or pitch * h
+        self._request_scores(sc)
         self._check(self._lib.vnect_estimate_device(self._h, C.c_void_p(dev_frames_ptr), n, h, w, pitch, frame_stride,
                                                     _ptr(ids), _ptr(t2d), _ptr(t3d), C.c_void_p(dev_j2_ptr),
                                                     C.c_void_p(dev_j3_ptr)))
@@ -572,31 +639,36 @@ class VNectEngine:
                                                _ptr(out), _ptr(meta)))
         return out, float(meta[0]), [int(meta[1]), int(meta[2])]
 
-    def postprocess(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None):
+    def postprocess(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None, scores=False):
         """src/estimator.py:105-142 on given (hm, xm, ym, zm) maps, each [n*n_scales, S/8, S/8, 21] float32.
-        Returns (joints_2d, joints_3d, raw_argmax)."""
+        Returns (joints_2d, joints_3d, raw_argmax) (+ scores, as in estimate())."""
         maps, n = check_maps(maps, len(self.scales), self.hm_size)
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         raw = np.empty((n, JOINTS, 2), np.int32)
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_postprocess(self._h, *[_ptr(m) for m in maps], n, _ptr(ids), _ptr(t2d), _ptr(t3d),
                                                 float(scaler), int(offsets[0]), int(offsets[1]), _ptr(j2), _ptr(j3),
                                                 _ptr(raw)))
-        return j2, j3, raw
+        return (j2, j3, raw) if sc is None else (j2, j3, raw, sc)
 
-    def postprocess_sequence(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None):
+    def postprocess_sequence(self, maps, scaler=1.0, offsets=(0, 0), stream_ids=None, t2d=None, t3d=None,
+                             scores=False):
         """postprocess() for a sequence call (see estimate_sequence) on given maps.  Returns (joints_2d, joints_3d,
-        raw_argmax)."""
+        raw_argmax) (+ scores, as in estimate())."""
         maps, n = check_maps(maps, len(self.scales), self.hm_size)
         ids, t2d, t3d = self._sequence_meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         raw = np.empty((n, JOINTS, 2), np.int32)
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_postprocess_sequence(self._h, *[_ptr(m) for m in maps], n, _ptr(ids), _ptr(t2d),
                                                          _ptr(t3d), float(scaler), int(offsets[0]), int(offsets[1]),
                                                          _ptr(j2), _ptr(j3), _ptr(raw)))
-        return j2, j3, raw
+        return (j2, j3, raw) if sc is None else (j2, j3, raw, sc)
 
-    def track_postprocess(self, maps, frame_hw, stream_ids=None, t2d=None, t3d=None):
+    def track_postprocess(self, maps, frame_hw, stream_ids=None, t2d=None, t3d=None, scores=False):
         """The tracked tail of track_frames() on given (hm, xm, ym, zm) maps, each [n*n_scales, S/8, S/8, 21] float32:
         frame f of stream stream_ids[f] is a full frame of frame_hw[f] = (height, width), cropped by the stream's box.
         Returns (joints_2d [n,21,2] in full-frame pixels, joints_3d [n,21,3], boxes_used [n,4]); the box update runs on
@@ -608,9 +680,11 @@ class VNectEngine:
         ids, t2d, t3d = self._meta(n, stream_ids, t2d, t3d)
         j2, j3 = np.empty((n, JOINTS, 2), np.float64), np.empty((n, JOINTS, 3), np.float32)
         boxes = np.empty((n, 4), np.int32)
+        sc = self._scores_out(scores, n)
+        self._request_scores(None if sc is None else _ptr(sc))
         self._check(self._lib.vnect_track_postprocess(self._h, *[_ptr(m) for m in maps], n, _ptr(hw), _ptr(ids),
                                                       _ptr(t2d), _ptr(t3d), _ptr(j2), _ptr(j3), _ptr(boxes)))
-        return j2, j3, boxes
+        return (j2, j3, boxes) if sc is None else (j2, j3, boxes, sc)
 
     def maps(self, n_frames=1):
         """The CNN output maps of the first n_frames frames of the last call (all their scales) as the 4-tuple
